@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — batched AFSK decode throughput on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Line of record (BASELINE.json configs[1], "c2"): 4096 independent 1200-baud captures per GPU, 1 KB random
@@ -493,6 +493,35 @@ def roofline_record(wl, B, total, steps, elapsed_ms, demod_ms, demod_launches, k
             "step_frac_of_peak": 2.0 * total / (elapsed_ms / steps / 1000) / 1e9 / peak}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(batch, out_dir: str) -> None:
+    """--dump-outputs: what a caller of the timed decode receives (an RxBatch) as out_dir/<name>.npy, so that
+    two builds run with the same arguments can be compared output for output.  Per capture: its index in the
+    corpus and the five stage integers (float64, exact); payload_bytes.npy (float32) holds the payloads one
+    after another, payload_offsets.npy where each starts.  When that could pass 64 MB, the captures written
+    are a prefix of a fixed permutation (seed 0) of the corpus that fits.  A capture is budgeted at its payload
+    capacity, which the plan derives from the inputs alone, so every build writes the same captures."""
+    res = batch.results
+    fields = res.dtype.names
+    nbytes = np.maximum(res["nbytes"].astype(np.int64), 0)
+    cost = 8 * (len(fields) + 2) + 4 * np.diff(batch.out_off)    # index, stage integers, offset, payload capacity
+    order = np.random.default_rng(0).permutation(len(res))
+    keep = np.sort(order[np.cumsum(cost[order]) <= DUMP_BYTES - (1 << 16)])   # room for the headers
+    off = np.zeros(len(keep) + 1, dtype=np.int64)
+    np.cumsum(nbytes[keep], out=off[1:])
+    pay = np.zeros(int(off[-1]), dtype=np.float32)
+    for i, c in enumerate(keep):
+        o = int(batch.out_off[c])
+        pay[off[i]:off[i + 1]] = batch.blob[o:o + int(nbytes[c])]
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"capture_index": keep, "payload_offsets": off, **{f: res[f][keep] for f in fields}}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
+    np.save(os.path.join(out_dir, "payload_bytes.npy"), pay)
+
+
 def results_sha256(batch) -> str:
     """SHA-256 over the stage integers of every capture and its payload bytes, in corpus order."""
     h = hashlib.sha256()
@@ -547,6 +576,11 @@ def run_workload(args, wl, captures, steps, main=False):
     elapsed, demod_ms, demod_launches = time_resident(sess, stream, steps, args.warmup,
                                                       float(os.environ.get("AFSK_BENCH_PRELOAD_S", "1.0" if main else "0.3")), sampler)
     clocks = sampler.stop() if sampler else None
+    if main and args.dump_outputs and args.scaling == "weak":
+        from afskmodem_b200 import shard
+        final = shard.gather_rx(sess.download(stream), dst=0)      # the last timed decode, all ranks in corpus order
+        if Ctx.rank == 0:
+            dump_outputs(final, args.dump_outputs)
     rank_ms = allgather_floats(elapsed / steps)
     ms_per_step = max(rank_ms)
     all_samples, all_bytes = allreduce([total, decoded_bytes])
@@ -823,6 +857,10 @@ def run_sharded(args, total_captures, steps):
     bad += int(int((batch.status < 0).sum()) != int(raising.sum()))
     checked_all, bad_all = allreduce([checked, bad])
     elapsed, demod_ms, demod_launches = time_resident(sess, stream, steps, args.warmup, 0.3)
+    if args.dump_outputs and args.scaling == "strong":
+        final = shard.gather_rx(sess.download(stream), dst=0)
+        if Ctx.rank == 0:
+            dump_outputs(final, args.dump_outputs)
     rank_ms = allgather_floats(elapsed / steps)
     ms = max(rank_ms)
     barrier()
@@ -880,7 +918,11 @@ def main():
     ap.add_argument("--no-sharded", action="store_true")
     ap.add_argument("--no-sharded-api", action="store_true")
     ap.add_argument("--file-captures", type=int, default=1024)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the line's last timed decode returned as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -935,7 +977,8 @@ def main():
         if Ctx.rank == 0 and Ctx.world == 1 and not args.no_files:
             latency = run_latency(args)
     if (extras and not args.no_sharded) or args.scaling == "strong":
-        sharded = run_sharded(args, args.corpus_captures, max(5, min(args.steps, 10)))
+        # as the line's own value the sharded corpus takes --steps; as a sub-record, 5 to 10
+        sharded = run_sharded(args, args.corpus_captures, args.steps if args.scaling == "strong" else max(5, min(args.steps, 10)))
 
     if Ctx.rank != 0:
         if Ctx.world > 1:

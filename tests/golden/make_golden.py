@@ -1,4 +1,5 @@
-"""Generates tests/golden/{rx_cases.npz,rx_cases.json,tx_cases.npz,tx_cases.json,gate_cases.json,gate_multi_cases.json}
+"""Generates tests/golden/{rx_cases.npz,rx_cases.json,tx_cases.npz,tx_cases.json,gate_cases.json,gate_multi_cases.json,
+random_trials.json}
 by running the UNMODIFIED reference (/root/reference/afskmodem.py) in this container through
 oracle/ref_harness.py.  The reference ships no golden vectors of its own (SURVEY.md §4), so these
 files ARE the pin: the oracle (oracle/afsk_oracle.c) is checked against them on CPU, and the CUDA
@@ -201,7 +202,15 @@ def main():
                                  "ret_hex": c["ret"].hex() if isinstance(c["ret"], (bytes, bytearray)) else None,
                                  "clock": c["clock"], "train_end": c["train_end"], "nbits": c["nbits"]} for c in calls]})
     json.dump(multi, open(os.path.join(HERE, "gate_multi_cases.json"), "w"), indent=1)
-    for f in ("rx_cases.npz", "rx_cases.json", "tx_cases.npz", "tx_cases.json", "gate_cases.json", "gate_multi_cases.json"):
+
+    # the 48 seeded random trials of tests/test_oracle_vs_reference.py: recipes are stored, not samples
+    sys.path.insert(0, os.path.dirname(HERE))
+    import test_oracle_vs_reference as T
+    trials = T.record(R.ref_save, lambda t: T.reference_result(R.ref_load(t["x"], t["baud"], t["amp_start"], t["amp_end"])))
+    json.dump({"source": "the unmodified reference, by tests/golden/make_golden.py", "trials": trials},
+              open(os.path.join(HERE, "random_trials.json"), "w"), indent=1)
+    for f in ("rx_cases.npz", "rx_cases.json", "tx_cases.npz", "tx_cases.json", "gate_cases.json", "gate_multi_cases.json",
+              "random_trials.json"):
         print(f, os.path.getsize(os.path.join(HERE, f)))
 
 

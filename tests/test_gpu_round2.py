@@ -276,7 +276,7 @@ def test_load_batch_ring_equals_pinned_corpus_mode(tmp_path):
     rx.close()
 
 
-def test_python_side_bounds_are_errors_not_device_faults():
+def test_python_side_bounds_are_errors_not_device_faults(tmp_path):
     caps, baud, thr, _ = _mixed_corpus(36, 3, bauds=(1200,))
     samples, offsets = A.modem._concat(caps)
     s = A.RxSession(offsets, baud, thr)
@@ -297,7 +297,7 @@ def test_python_side_bounds_are_errors_not_device_faults():
         p.decode(samples[:100])
     p.close()
     with pytest.raises(ValueError):
-        A.write_wav_batch(["/tmp/never_written.wav"], samples, [len(samples) - 5], [10])
+        A.write_wav_batch([str(tmp_path / "never_written.wav")], samples, [len(samples) - 5], [10])
 
 
 def test_empty_tx_batch(tmp_path):

@@ -3,6 +3,8 @@ import ast
 import ctypes as C
 import os
 import re
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -10,7 +12,7 @@ import pytest
 import afskmodem_b200 as A
 from afskmodem_b200 import _cabi
 from afskmodem_b200.shard import shard_captures
-from conftest import ROOT, has_cuda
+from conftest import ROOT
 
 
 def test_library_exports_every_declared_symbol():
@@ -92,12 +94,17 @@ def test_shard_captures_balanced_contiguous():
 
 
 def test_no_device_means_loud_failure():
-    if has_cuda():
-        pytest.skip("GPU present")
-    with pytest.raises(A.AfskError):
-        A.Receiver(1200).decode_batch([np.zeros(5000, np.int16)])
-    with pytest.raises(A.AfskError):
-        A.Transmitter(1200).encode_batch([b"x"])
+    """With no visible CUDA device every compute call raises AfskError.  A fresh process with
+    CUDA_VISIBLE_DEVICES empty sees no device on a GPU machine too."""
+    code = ("import sys; sys.path.insert(0, sys.argv[1])\n"
+            "import numpy as np, pytest, afskmodem_b200 as A\n"
+            "with pytest.raises(A.AfskError):\n"
+            "    A.Receiver(1200).decode_batch([np.zeros(5000, np.int16)])\n"
+            "with pytest.raises(A.AfskError):\n"
+            "    A.Transmitter(1200).encode_batch([b'x'])\n")
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    proc = subprocess.run([sys.executable, "-c", code, ROOT], env=env, capture_output=True, text=True, timeout=300)
+    assert proc.returncode == 0, proc.stderr
 
 
 def test_product_never_imports_the_oracle():

@@ -1,5 +1,5 @@
 """CPU: host logic added in round 2 — cost-balanced sharding, the host gather of per-rank batches on a
-world-size-2 gloo group, the file halves of SoundInput / SoundOutput, the bench corpus recipe."""
+world-size-2 gloo group, the file halves of SoundInput / SoundOutput, the bench corpus recipe and its output dump."""
 import os
 import socket
 import sys
@@ -145,6 +145,49 @@ def test_bench_corpus_is_seeded_by_capture_index():
         assert lens[i] == c.lead[i] + len(fr)
     w = bench.Corpus("c2", 8 * 64)
     assert w.payloads(64, 128) == bench.Corpus("c2", 8 * 64).payloads(0, 512)[64:128]
+
+
+def _fake_batch(B, seed):
+    rng = np.random.default_rng(seed)
+    res = np.zeros(B, _cabi.RX_RESULT_DTYPE)
+    res["status"] = rng.choice([0, 1, 2, -3], B)
+    res["clock"] = rng.integers(-1, 40, B)
+    res["train_end"] = rng.integers(2**40, 2**52, B)
+    res["nbits"] = rng.integers(0, 9000, B)
+    res["nbytes"] = np.where(res["status"] < 0, 0, rng.integers(0, 1100, B))
+    out_off = np.zeros(B + 1, np.int64)
+    np.cumsum(res["nbytes"] + rng.integers(0, 50, B), out=out_off[1:])
+    return A.RxBatch(res, rng.integers(0, 256, int(out_off[-1]), dtype=np.uint8), out_off)
+
+
+def test_bench_dump_outputs(tmp_path, monkeypatch):
+    """--dump-outputs writes every capture's stage integers and payload exactly in float32 / float64; over the
+    size budget, the same seeded sample of captures on every run, within the budget."""
+    import bench
+    b = _fake_batch(300, 5)
+    bench.dump_outputs(b, str(tmp_path / "all"))
+    got = {f[:-4]: np.load(tmp_path / "all" / f) for f in os.listdir(tmp_path / "all")}
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+    assert np.array_equal(got["capture_index"], np.arange(300))
+    for f in b.results.dtype.names:
+        assert np.array_equal(got[f], b.results[f].astype(np.float64)), f
+    off, pay = got["payload_offsets"].astype(np.int64), got["payload_bytes"]
+    assert [pay[off[c]:off[c + 1]].astype(np.uint8).tobytes() for c in range(300)] == b.payloads()
+    monkeypatch.setattr(bench, "DUMP_BYTES", (1 << 16) + 200_000)
+    for run in ("a", "b"):
+        bench.dump_outputs(b, str(tmp_path / run))
+    total = sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a"))
+    assert total <= bench.DUMP_BYTES
+    idx = np.load(tmp_path / "a" / "capture_index.npy").astype(np.int64)
+    assert 0 < len(idx) < 300 and np.all(np.diff(idx) > 0)
+    assert np.array_equal(np.load(tmp_path / "a" / "nbits.npy"), b.nbits[idx].astype(np.float64))
+    for f in os.listdir(tmp_path / "a"):
+        assert np.array_equal(np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)), f
+    # the sample follows the inputs (the capacity layout), not what was decoded
+    other = _fake_batch(300, 6).results
+    other["nbytes"] = np.minimum(other["nbytes"], np.diff(b.out_off))
+    bench.dump_outputs(A.RxBatch(other, b.blob, b.out_off), str(tmp_path / "c"))
+    assert np.array_equal(np.load(tmp_path / "c" / "capture_index.npy"), idx.astype(np.float64))
 
 
 def test_h2d_gate_serialises_a_group_only(tmp_path, monkeypatch):
