@@ -28,7 +28,9 @@ SYMBOLS = [
     "afsk_rx_plan_launches", "afsk_rx_plan_set_timing", "afsk_rx_plan_demod_time", "afsk_rx_decode", "afsk_rx_plan_planes", "afsk_rx_decode_host", "afsk_rx_host_release",
     "afsk_rx_out_capacity", "afsk_rx_gate", "afsk_rx_gate_multi", "afsk_tx_num_samples", "afsk_tx_plan_create",
     "afsk_tx_plan_destroy", "afsk_tx_plan_out_offsets", "afsk_tx_synth", "afsk_tx_synth_host",
-    "afsk_wav_probe", "afsk_wav_load", "afsk_wav_save",
+    "afsk_wav_probe", "afsk_wav_load", "afsk_wav_save", "afsk_rx_streams_create", "afsk_rx_streams_push",
+    "afsk_rx_streams_finish", "afsk_rx_streams_events", "afsk_rx_streams_state", "afsk_rx_streams_arena_bytes",
+    "afsk_rx_streams_counters", "afsk_rx_streams_destroy",
 ]
 
 
@@ -46,6 +48,10 @@ class RxResult(C.Structure):
 RX_RESULT_DTYPE = np.dtype([("status", "<i4"), ("clock", "<i4"), ("train_end", "<i8"),
                             ("nbits", "<i8"), ("nbytes", "<i8")])
 assert RX_RESULT_DTYPE.itemsize == C.sizeof(RxResult) == 32
+
+# AfskRxStreamEvent
+STREAM_EVENT_DTYPE = np.dtype([("stream", "<i4"), ("recorded", "<i4"), ("call", "<i8"), ("start", "<i8"), ("end", "<i8")])
+assert STREAM_EVENT_DTYPE.itemsize == 32
 
 _lib = None
 
@@ -94,6 +100,14 @@ def lib():
     L.afsk_rx_out_capacity.restype = C.c_int64
     L.afsk_rx_gate.argtypes = [C.c_int, vp, i64p, C.c_int, C.c_int, C.c_int, C.c_int64, vp, vp]
     L.afsk_rx_gate_multi.argtypes = [C.c_int, vp, i64p, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_int, vp, vp, vp]
+    L.afsk_rx_streams_create.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int64, C.POINTER(vp)]
+    L.afsk_rx_streams_push.argtypes = [vp, vp, C.c_int, i64p, vp, i64p]
+    L.afsk_rx_streams_finish.argtypes = [vp, vp, i64p]
+    L.afsk_rx_streams_events.argtypes = [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(vp)]
+    L.afsk_rx_streams_state.argtypes = [vp, C.c_int, i64p, i64p, i64p]
+    L.afsk_rx_streams_arena_bytes.argtypes = [vp, i64p]
+    L.afsk_rx_streams_counters.argtypes = [vp, i64p, i64p, i64p]
+    L.afsk_rx_streams_destroy.argtypes = [vp]
     L.afsk_tx_num_samples.argtypes = [C.c_int, C.c_int64, C.c_int64, u8p]
     L.afsk_tx_num_samples.restype = C.c_int64
     L.afsk_tx_plan_create.argtypes = [C.c_int, C.c_int, i64p, i32p, i64p, u8p, C.POINTER(vp)]

@@ -2082,13 +2082,26 @@ __global__ void __launch_bounds__(kFrameThreads) k_gate_scan(const int32_t *__re
     }
 }
 
-// Successive Receiver.receive() calls over one recorded stream (the reference keeps its input stream
-// open between calls, afskmodem.py:283): every call discards one chunk (:303), examines up to
+// Successive Receiver.receive() calls over one stream (the reference keeps its input stream open
+// between calls, afskmodem.py:283): every call discards one chunk (:303), examines up to
 // ceil(timeout / 2048) chunks for an opening (:304-310) and, once open, records through the first
 // chunk quieter than amp_end (:313-318); the next call starts at the chunk after.  One warp per
-// stream walks the chunk amplitudes 32 at a time.  Finite-stream conventions: a call that reaches
-// the end of the recording before opening or timing out does not return (the walk stops); a
-// recording still open at the end keeps everything up to the last full chunk.
+// stream walks the chunk amplitudes 32 at a time.
+//
+// The walk is resumable: it starts from a saved GateState (afsk_rx_gate_multi: a fresh one) over the
+// chunks that arrived since, emits only the calls that became final (timed out with all their chunks
+// present, or closed by a quiet chunk) and saves where it stopped.  After every walk `pos` equals the
+// number of chunks seen, so the next walk needs the amplitudes of the new chunks only.  finish applies
+// the finite-stream conventions: a recording still open keeps everything up to the last full chunk;
+// a call that has neither opened nor timed out does not return.
+struct GateState {
+    long long pos;      // next chunk to read
+    long long mark;     // phase 1: first chunk the call listens at; phase 2: chunk that opened the recording
+    long long call;     // calls finished so far
+    int phase;          // 0: the call discards chunk `pos` first; 1: listening; 2: recording
+    int pad;
+};
+static_assert(sizeof(GateState) == 32, "GateState layout");
 __device__ __forceinline__ long long warp_find_first(const int32_t *A, long long lo, long long hi, int thr, bool greater)
 {
     const int lane = threadIdx.x & 31;
@@ -2105,34 +2118,110 @@ __device__ __forceinline__ long long warp_find_first(const int32_t *A, long long
     return -1;
 }
 
+// amp[chunk_first[s] ..] are the amplitudes of stream s's chunks from state[s].pos on (state == NULL: a
+// fresh state).  Call k of this walk goes to ranges[3 * (out_first ? out_first[s] : s * max_calls) + 3k].
+// Every call emitted before finish reads at least one new chunk, so new chunks + 1 slots always suffice.
 __global__ void __launch_bounds__(32) k_gate_multi(const int32_t *__restrict__ amp, const int64_t *__restrict__ chunk_first,
                                                    int amp_start, int amp_end, long long timeout_frames, int max_calls,
-                                                   int64_t *__restrict__ ranges, int32_t *__restrict__ counts)
+                                                   GateState *__restrict__ state, int finish,
+                                                   const int64_t *__restrict__ out_first, int64_t *__restrict__ ranges,
+                                                   int32_t *__restrict__ counts)
 {
     const int s = blockIdx.x, lane = threadIdx.x;
-    const int32_t *A = amp + chunk_first[s];
-    const long long nch = chunk_first[s + 1] - chunk_first[s];
+    GateState g = {0, 0, 0, 0, 0};
+    if (state) g = state[s];
+    const int32_t *A = amp + chunk_first[s] - g.pos;             // A[j]: chunk j of the stream
+    const long long nch = g.pos + chunk_first[s + 1] - chunk_first[s];
     const long long lim = timeout_frames <= 0 ? 0 : (timeout_frames + AFSK_GATE_CHUNK - 1) / AFSK_GATE_CHUNK;
-    int64_t *out = ranges + (size_t)s * max_calls * 3;
-    long long pos = 0;
+    int64_t *out = ranges + (out_first ? (long long)out_first[s] : (long long)s * max_calls) * 3;
     int calls = 0;
-    while (calls < max_calls && pos < nch) {
-        const long long first = pos + 1;                          // chunk `pos` is discarded :303
-        const long long open = warp_find_first(A, first, min(first + lim, nch), amp_start, true);   // :306
+    while (calls < max_calls) {
+        if (g.phase == 0) {
+            if (g.pos >= nch) break;
+            g.pos++;                                              // chunk discarded :303
+            g.phase = 1; g.mark = g.pos;
+        }
         long long rec = 0, a = 0, b = 0;
-        if (open < 0) {
-            if (first + lim > nch) break;                         // recording ends before the timeout does
-            pos = first + lim;                                    // "Timed out." :311-312, :405-407
-        } else {
-            const long long close = warp_find_first(A, open + 1, nch, amp_end, false);               // :316
-            const long long end = close < 0 ? nch : close + 1;
-            rec = 1; a = open * AFSK_GATE_CHUNK; b = end * AFSK_GATE_CHUNK;
-            pos = end;
+        if (g.phase == 1) {
+            const long long stop = g.mark + lim;
+            const long long open = warp_find_first(A, g.pos, min(stop, nch), amp_start, true);     // :306
+            if (open < 0) {
+                if (stop > nch) { g.pos = nch; break; }           // not timed out yet
+                g.pos = stop;                                     // "Timed out." :311-312, :405-407
+            } else {
+                g.phase = 2; g.mark = open; g.pos = open + 1;
+            }
+        }
+        if (g.phase == 2) {
+            const long long close = warp_find_first(A, g.pos, nch, amp_end, false);                 // :316
+            if (close < 0) { g.pos = nch; break; }                // still recording
+            rec = 1; a = g.mark * AFSK_GATE_CHUNK; b = (close + 1) * AFSK_GATE_CHUNK;
+            g.pos = close + 1;
         }
         if (lane == 0) { out[3 * calls] = rec; out[3 * calls + 1] = a; out[3 * calls + 2] = b; }
         calls++;
+        g.phase = 0;
     }
-    if (lane == 0) counts[s] = calls;
+    if (finish && g.phase == 2 && calls < max_calls) {
+        if (lane == 0) { out[3 * calls] = 1; out[3 * calls + 1] = g.mark * AFSK_GATE_CHUNK; out[3 * calls + 2] = nch * AFSK_GATE_CHUNK; }
+        calls++;
+        g.phase = 0;
+    }
+    g.call += calls;
+    if (lane == 0) {
+        counts[s] = calls;
+        if (state) state[s] = g;
+    }
+}
+
+// Copies segments of samples between buffers at any frame alignment, one launch for all of them: every
+// thread writes one aligned 16-byte vector of the destination from the (at most two) aligned source
+// vectors that hold its frames, realigned with funnel shifts.  Only the partial head and tail vectors
+// of a segment are written frame by frame (the frames around them belong to other data).
+struct CopySeg { long long src, dst, len; };                     // samples
+constexpr int kCopyThreads = 256, kCopyTileVecs = 4 * kCopyThreads;
+
+__global__ void __launch_bounds__(kCopyThreads) k_stream_copy(const int16_t *__restrict__ src, int16_t *__restrict__ dst,
+                                                              const CopySeg *__restrict__ seg,
+                                                              const int64_t *__restrict__ tile_first, int n)
+{
+    const long long tile = blockIdx.x;
+    int a = 0, b = n;                                             // segment of this tile
+    while (b - a > 1) {
+        const int mid = (a + b) >> 1;
+        if (tile_first[mid] <= tile) a = mid; else b = mid;
+    }
+    const CopySeg g = seg[a];
+    const long long v0 = (g.dst >> 3) + (tile - tile_first[a]) * kCopyTileVecs, vend = (g.dst + g.len + 7) >> 3;
+    const long long s_lo = g.src >> 3, s_hi = (g.src + g.len - 1) >> 3;
+#pragma unroll
+    for (int i = 0; i < kCopyTileVecs / kCopyThreads; i++) {
+        const long long dv = v0 + i * kCopyThreads + threadIdx.x;
+        if (dv >= vend) break;
+        const long long q = dv * 8 - g.dst + g.src;               // source frame of the vector's first frame
+        const long long sv = q >> 3;                              // (floor: q < 0 only at a head vector)
+        const int k = (int)(q - sv * 8);
+        uint4 lo = make_uint4(0, 0, 0, 0), hi = make_uint4(0, 0, 0, 0);
+        if (sv >= s_lo && sv <= s_hi) lo = ld_nc_v4(src + sv * 8);
+        if (k && sv + 1 >= s_lo && sv + 1 <= s_hi) hi = ld_nc_v4(src + (sv + 1) * 8);
+        const uint32_t w[8] = {lo.x, lo.y, lo.z, lo.w, hi.x, hi.y, hi.z, hi.w};
+        const int j = k >> 1;
+        uint32_t o[4];
+#pragma unroll
+        for (int t = 0; t < 4; t++) {                             // bytes 2k .. 2k + 15 of the 32 loaded
+            const uint32_t x0 = j == 0 ? w[t] : j == 1 ? w[t + 1] : j == 2 ? w[t + 2] : w[t + 3];
+            const uint32_t x1 = j == 0 ? w[t + 1] : j == 1 ? w[t + 2] : j == 2 ? w[t + 3] : w[t + 4];
+            o[t] = (k & 1) ? __funnelshift_r(x0, x1, 16) : x0;
+        }
+        const long long d0 = dv * 8;
+        if (d0 >= g.dst && d0 + 8 <= g.dst + g.len) {
+            *reinterpret_cast<uint4 *>(dst + d0) = make_uint4(o[0], o[1], o[2], o[3]);
+        } else {
+#pragma unroll
+            for (int e = 0; e < 8; e++)
+                if (d0 + e >= g.dst && d0 + e < g.dst + g.len) dst[d0 + e] = (int16_t)(o[e >> 1] >> (16 * (e & 1)));
+        }
+    }
 }
 
 struct Group {
@@ -2422,7 +2511,8 @@ static int gate_run(int device, const int16_t *d_samples, const int64_t *h_offse
         k_gate_amp<<<(unsigned)((total + wpb - 1) / wpb), wpb * 32, 0, st>>>(d_samples, g.d_first, g.d_off, S, total, g.d_amp);
     }
     if (max_calls < 0) k_gate_scan<<<S, kFrameThreads, 0, st>>>(g.d_amp, g.d_first, amp_start, amp_end, timeout_frames, d_ranges);
-    else k_gate_multi<<<S, 32, 0, st>>>(g.d_amp, g.d_first, amp_start, amp_end, timeout_frames, max_calls, d_ranges, d_counts);
+    else k_gate_multi<<<S, 32, 0, st>>>(g.d_amp, g.d_first, amp_start, amp_end, timeout_frames, max_calls, nullptr, 1, nullptr,
+                                         d_ranges, d_counts);
     AFSK_CUDA(cudaGetLastError());
     AFSK_CUDA(cudaStreamSynchronize(st));     // the host staging vector and the scratch go out of scope
     return AFSK_OK;
@@ -3064,6 +3154,388 @@ int afsk_rx_gate_multi(int device, const int16_t *d_samples, const int64_t *h_of
         return AFSK_E_ARG;
     }
     return gate_run(device, d_samples, h_offsets, S, amp_start, amp_end, timeout_frames, max_calls, d_ranges, d_counts, stream);
+}
+
+// ---------------------------------------------------------------- streaming receiver ----
+// S channels, each one Receiver calling receive(timeout) again and again on its own open input stream,
+// fed piece by piece.  Every channel keeps its samples from its pending recording's first chunk (or,
+// with none, from its partial chunk) on in a slot of a device arena.  A push appends the pieces
+// (k_stream_copy), measures the chunks they completed (k_gate_amp), resumes every channel's walk
+// (k_gate_multi) and decodes the recordings that became final in place, through one plan re-targeted
+// with afsk_rx_plan_reset.
+//
+// Retention moves only the channel whose piece does not fit behind its slot.  Its retained samples go back
+// to the start of its slot when they fill at most half of it, else into a new slot of twice its need (plus
+// two chunks) at the top of the arena.  Only when the top has no room for those does every channel move,
+// into the other arena: slots of twice their need, and half as much again free above them.  A move costs
+// at most the frames its channel pushed since the slot was assigned, and a compaction moves at most what
+// the channels pushed while the free space filled, so every pushed frame causes O(1) moved frames
+// (afsk_rx_streams_counters reports them), and one long recording widens only its own slot.
+namespace {
+cudaError_t grow_pinned(void **p, size_t *cap, size_t need)
+{
+    if (need <= *cap) return cudaSuccess;
+    if (*p) cudaFreeHost(*p);
+    *p = nullptr; *cap = 0;
+    const size_t want = need + need / 4 + 4096;
+    const cudaError_t e = cudaMallocHost(p, want);
+    if (e == cudaSuccess) *cap = want;
+    return e;
+}
+constexpr int64_t kSlotPad = 64;           // samples after the last slot (vector over-reads of the kernels)
+int64_t arena_frames(size_t bytes) { return bytes ? (int64_t)(bytes / 2) - kSlotPad : 0; }
+}  // namespace
+
+struct AfskRxStreams {
+    int device = 0, S = 0, baud = 0, amp_start = 0, amp_end = 0;
+    int64_t timeout = 0;
+    // per channel (host): frames pushed, first retained frame (a chunk start), start of the pending recording
+    // (-1: none), calls finished, and the slot: first arena sample, capacity, stream frame at the slot's start
+    std::vector<int64_t> pushed, keep, pending, calls, slot_off, slot_cap, slot_base;
+    std::vector<int64_t> np, new_off, new_cap, chunk_first;       // scratch of one push
+    int16_t *arena[2] = {nullptr, nullptr};
+    size_t arena_cap[2] = {0, 0};
+    int cur = 0;
+    int64_t top = 0;                                              // arena samples below the free space
+    bool failed = false;                                          // an error after this push's state was committed
+    int64_t n_launches = 0, n_moved = 0, n_compactions = 0;       // since creation
+    int16_t *d_stage = nullptr; size_t stage_cap = 0;             // host input
+    // descriptors of one push, built in pinned memory and sent with one copy
+    uint8_t *d_desc = nullptr, *h_desc = nullptr;
+    size_t desc_bytes = 0, o_seg_app = 0, o_tf_app = 0, o_seg_mov = 0, o_tf_mov = 0, o_first = 0, o_amp_off = 0, o_out_first = 0;
+    GateState *d_state = nullptr, *h_state = nullptr;
+    int32_t *d_counts = nullptr, *h_counts = nullptr;
+    int32_t *d_amp = nullptr; size_t amp_cap = 0;
+    int64_t *d_ranges = nullptr, *h_ranges = nullptr; size_t ranges_cap = 0, h_ranges_cap = 0;
+    AfskRxPlan *plan = nullptr;
+    uint8_t *d_out = nullptr; size_t out_cap = 0;
+    AfskRxResult *d_res = nullptr; size_t res_cap = 0;
+    uint8_t *h_dec = nullptr; size_t h_dec_cap = 0;               // pinned: results, then payloads
+    std::vector<int64_t> rec_start, rec_len;
+    std::vector<int32_t> rec_baud, rec_amp_end;
+    // what the last push / finish returned
+    std::vector<AfskRxStreamEvent> ev;
+    std::vector<AfskRxResult> res;
+    std::vector<uint8_t> payload;
+    std::vector<int64_t> payload_off;
+};
+
+static int streams_fail(cudaError_t e)
+{
+    afsk_set_error("afsk_rx_streams: %s", cudaGetErrorString(e));
+    return AFSK_E_CUDA;
+}
+
+// one push (finish = 0) or the end of the streams (finish = 1, no samples)
+static int streams_run(AfskRxStreams *H, const int16_t *samples, int on_device, const int64_t *off, cudaStream_t st,
+                       int finish, int64_t *n_events)
+{
+    const int S = H->S;
+    const int64_t C = AFSK_GATE_CHUNK;
+    auto piece = [&](int s) -> int64_t { return finish ? 0 : off[s + 1] - off[s]; };
+    int64_t nch = 0;                               // chunks completed by this push
+    for (int s = 0; s < S; s++) {
+        H->np[s] = H->pushed[s] + piece(s);
+        nch += H->np[s] / C - H->pushed[s] / C;
+    }
+    // buffers first: a failed allocation leaves the channels as they were
+    const int64_t in_samples = finish ? 0 : off[S] - off[0];
+    cudaError_t e = cudaSuccess;
+    if (!on_device && in_samples > 0) e = grow_device((void **)&H->d_stage, &H->stage_cap, (size_t)in_samples * 2 + 32);
+    if (e == cudaSuccess) e = grow_device((void **)&H->d_amp, &H->amp_cap, sizeof(int32_t) * (size_t)nch);
+    if (e == cudaSuccess) e = grow_device((void **)&H->d_ranges, &H->ranges_cap, sizeof(int64_t) * 3 * (size_t)(nch + S));
+    if (e == cudaSuccess) e = grow_pinned((void **)&H->h_ranges, &H->h_ranges_cap, sizeof(int64_t) * 3 * (size_t)(nch + S));
+    if (e != cudaSuccess) return streams_fail(e);
+    uint8_t *hd = H->h_desc;
+    CopySeg *seg_app = reinterpret_cast<CopySeg *>(hd + H->o_seg_app), *seg_mov = reinterpret_cast<CopySeg *>(hd + H->o_seg_mov);
+    int64_t *tf_app = reinterpret_cast<int64_t *>(hd + H->o_tf_app), *tf_mov = reinterpret_cast<int64_t *>(hd + H->o_tf_mov);
+    int64_t *first = reinterpret_cast<int64_t *>(hd + H->o_first), *amp_off = reinterpret_cast<int64_t *>(hd + H->o_amp_off);
+    int64_t *out_first = reinterpret_cast<int64_t *>(hd + H->o_out_first);
+    auto add_seg = [](CopySeg *seg, int64_t *tf, int &n, int64_t src, int64_t dst, int64_t len) {
+        if (len <= 0) return;
+        const int64_t vecs = ((dst + len + 7) >> 3) - (dst >> 3);
+        seg[n] = CopySeg{src, dst, len};
+        tf[n + 1] = tf[n] + (vecs + kCopyTileVecs - 1) / kCopyTileVecs;
+        n++;
+    };
+    // retention (see above): which channels overflow, and do their new slots fit above the top?
+    auto overflows = [&](int s) { return H->np[s] - H->slot_base[s] > H->slot_cap[s]; };
+    auto rewinds = [&](int s) { return 2 * (H->np[s] - H->keep[s]) <= H->slot_cap[s]; };
+    auto fresh_cap = [&](int s) { return (2 * (H->np[s] - H->keep[s]) + 2 * C + 7) & ~(int64_t)7; };
+    int64_t want = 0;
+    bool any = false;
+    for (int s = 0; s < S; s++)
+        if (overflows(s)) {
+            any = true;
+            if (!rewinds(s)) want += fresh_cap(s);
+        }
+    const bool compact = any && H->top + want > arena_frames(H->arena_cap[H->cur]);
+    int nmov = 0, napp = 0;
+    tf_mov[0] = tf_app[0] = 0;
+    if (compact) {
+        int64_t total = 0;
+        for (int s = 0; s < S; s++) {
+            H->new_off[s] = total;
+            H->new_cap[s] = fresh_cap(s);
+            total += H->new_cap[s];
+        }
+        const int nxt = H->cur ^ 1;
+        e = grow_device((void **)&H->arena[nxt], &H->arena_cap[nxt], (size_t)(total + total / 2 + kSlotPad) * 2);
+        if (e != cudaSuccess) return streams_fail(e);
+        for (int s = 0; s < S; s++) {
+            add_seg(seg_mov, tf_mov, nmov, H->slot_off[s] + H->keep[s] - H->slot_base[s], H->new_off[s], H->pushed[s] - H->keep[s]);
+            H->slot_off[s] = H->new_off[s]; H->slot_cap[s] = H->new_cap[s]; H->slot_base[s] = H->keep[s];
+        }
+        H->top = total;
+        H->n_compactions++;
+    } else if (any) {
+        // within the arena: sources are the retained spans, destinations the slot starts (below the span: a
+        // rewind happens only when the span fills at most half the slot) or fresh space above the top
+        for (int s = 0; s < S; s++) {
+            if (!overflows(s)) continue;
+            const int64_t src = H->slot_off[s] + H->keep[s] - H->slot_base[s];
+            if (!rewinds(s)) {
+                H->slot_off[s] = H->top;
+                H->slot_cap[s] = fresh_cap(s);
+                H->top += H->slot_cap[s];
+            }
+            add_seg(seg_mov, tf_mov, nmov, src, H->slot_off[s], H->pushed[s] - H->keep[s]);
+            H->slot_base[s] = H->keep[s];
+        }
+    }
+    for (int i = 0; i < nmov; i++) H->n_moved += seg_mov[i].len;
+    first[0] = 0;
+    for (int s = 0; s < S; s++) {
+        add_seg(seg_app, tf_app, napp, finish ? 0 : off[s] - (on_device ? 0 : off[0]), H->slot_off[s] + H->pushed[s] - H->slot_base[s],
+                piece(s));
+        const int64_t c_old = H->pushed[s] / C;
+        first[s + 1] = first[s] + H->np[s] / C - c_old;
+        amp_off[s] = H->slot_off[s] + c_old * C - H->slot_base[s];
+        out_first[s] = first[s] + s;
+    }
+    AFSK_CUDA(cudaMemcpyAsync(H->d_desc, H->h_desc, H->desc_bytes, cudaMemcpyHostToDevice, st));
+    const uint8_t *dd = H->d_desc;
+    if (nmov > 0) {
+        k_stream_copy<<<(unsigned)tf_mov[nmov], kCopyThreads, 0, st>>>(H->arena[H->cur], H->arena[compact ? H->cur ^ 1 : H->cur],
+                                                                      reinterpret_cast<const CopySeg *>(dd + H->o_seg_mov),
+                                                                      reinterpret_cast<const int64_t *>(dd + H->o_tf_mov), nmov);
+        H->n_launches++;
+    }
+    if (compact) H->cur ^= 1;
+    int16_t *x = H->arena[H->cur];
+    if (napp > 0) {
+        const int16_t *src = samples;
+        if (!on_device) {
+            AFSK_CUDA(cudaMemcpyAsync(H->d_stage, samples + off[0], (size_t)in_samples * 2, cudaMemcpyHostToDevice, st));
+            src = H->d_stage;
+        }
+        k_stream_copy<<<(unsigned)tf_app[napp], kCopyThreads, 0, st>>>(src, x, reinterpret_cast<const CopySeg *>(dd + H->o_seg_app),
+                                                                      reinterpret_cast<const int64_t *>(dd + H->o_tf_app), napp);
+        H->n_launches++;
+    }
+    const int64_t *d_first = reinterpret_cast<const int64_t *>(dd + H->o_first);
+    if (nch > 0) {
+        const int wpb = 8;
+        k_gate_amp<<<(unsigned)((nch + wpb - 1) / wpb), wpb * 32, 0, st>>>(x, d_first, reinterpret_cast<const int64_t *>(dd + H->o_amp_off),
+                                                                           S, nch, H->d_amp);
+        H->n_launches++;
+    }
+    H->n_launches++;
+    k_gate_multi<<<S, 32, 0, st>>>(H->d_amp, d_first, H->amp_start, H->amp_end, H->timeout, 0x7FFFFFFF, H->d_state, finish,
+                                   reinterpret_cast<const int64_t *>(dd + H->o_out_first), H->d_ranges, H->d_counts);
+    AFSK_CUDA(cudaGetLastError());
+    AFSK_CUDA(cudaMemcpyAsync(H->h_counts, H->d_counts, sizeof(int32_t) * S, cudaMemcpyDeviceToHost, st));
+    AFSK_CUDA(cudaMemcpyAsync(H->h_state, H->d_state, sizeof(GateState) * S, cudaMemcpyDeviceToHost, st));
+    AFSK_CUDA(cudaMemcpyAsync(H->h_ranges, H->d_ranges, sizeof(int64_t) * 3 * (size_t)(nch + S), cudaMemcpyDeviceToHost, st));
+    AFSK_CUDA(cudaStreamSynchronize(st));
+
+    // final calls, ordered by (channel, call); recordings as ranges of the arena
+    H->ev.clear();
+    H->rec_start.clear();
+    H->rec_len.clear();
+    for (int s = 0; s < S; s++) {
+        const int64_t *r = H->h_ranges + 3 * out_first[s];
+        for (int k = 0; k < H->h_counts[s]; k++) {
+            AfskRxStreamEvent v;
+            v.stream = s; v.recorded = (int32_t)r[3 * k]; v.call = H->calls[s] + k; v.start = r[3 * k + 1]; v.end = r[3 * k + 2];
+            H->ev.push_back(v);
+            if (v.recorded) {
+                H->rec_start.push_back(H->slot_off[s] + v.start - H->slot_base[s]);
+                H->rec_len.push_back(v.end - v.start);
+            }
+        }
+        const GateState &g = H->h_state[s];
+        H->calls[s] = g.call;
+        H->pushed[s] = H->np[s];
+        H->pending[s] = g.phase == 2 ? g.mark * C : -1;
+        H->keep[s] = g.phase == 2 ? g.mark * C : g.pos * C;
+    }
+    const int nev = (int)H->ev.size(), nrec = (int)H->rec_start.size();
+    H->res.assign((size_t)nev, AfskRxResult{0, -1, -1, 0, 0});
+    H->payload_off.assign((size_t)nev + 1, 0);
+    H->payload.clear();
+    if (nrec > 0) {
+        H->rec_baud.assign((size_t)nrec, H->baud);
+        H->rec_amp_end.assign((size_t)nrec, H->amp_end);
+        int rc = H->plan ? afsk_rx_plan_reset(H->plan, nrec, H->rec_start.data(), H->rec_len.data(), H->rec_baud.data(), H->rec_amp_end.data())
+                         : afsk_rx_plan_create_ranges(H->device, nrec, H->rec_start.data(), H->rec_len.data(), H->rec_baud.data(),
+                                                      H->rec_amp_end.data(), &H->plan);
+        if (rc != AFSK_OK) return rc;
+        const int64_t *oo = H->plan->out_off.data();
+        const size_t res_bytes = sizeof(AfskRxResult) * (size_t)nrec, out_bytes = (size_t)oo[nrec];
+        e = grow_device((void **)&H->d_out, &H->out_cap, out_bytes);
+        if (e == cudaSuccess) e = grow_device((void **)&H->d_res, &H->res_cap, res_bytes);
+        if (e == cudaSuccess) e = grow_pinned((void **)&H->h_dec, &H->h_dec_cap, res_bytes + out_bytes);
+        if (e != cudaSuccess) return streams_fail(e);
+        rc = afsk_rx_decode(H->plan, x, H->d_out, H->d_res, st);
+        if (rc != AFSK_OK) return rc;
+        int nl = 0;
+        afsk_rx_plan_launches(H->plan, &nl);
+        H->n_launches += nl;
+        AFSK_CUDA(cudaMemcpyAsync(H->h_dec, H->d_res, res_bytes, cudaMemcpyDeviceToHost, st));
+        AFSK_CUDA(cudaMemcpyAsync(H->h_dec + res_bytes, H->d_out, out_bytes, cudaMemcpyDeviceToHost, st));
+        AFSK_CUDA(cudaStreamSynchronize(st));
+        const AfskRxResult *rr = reinterpret_cast<const AfskRxResult *>(H->h_dec);
+        H->payload.assign(H->h_dec + res_bytes, H->h_dec + res_bytes + out_bytes);
+        int k = 0;
+        for (int i = 0; i < nev; i++) {
+            H->payload_off[i] = oo[k];
+            if (H->ev[i].recorded) H->res[i] = rr[k++];
+        }
+        H->payload_off[nev] = oo[nrec];
+    }
+    if (finish) {                                  // the next push is frame 0 of new streams
+        for (int s = 0; s < S; s++) {
+            H->pushed[s] = H->keep[s] = H->calls[s] = H->slot_base[s] = 0;
+            H->pending[s] = -1;
+        }
+        AFSK_CUDA(cudaMemsetAsync(H->d_state, 0, sizeof(GateState) * S, st));
+        AFSK_CUDA(cudaStreamSynchronize(st));
+    }
+    *n_events = nev;
+    return AFSK_OK;
+}
+
+// a push or finish with valid arguments: any failure may leave the channels between two states, so the
+// handle refuses every later push / finish
+static int streams_call(AfskRxStreams *H, const int16_t *samples, int on_device, const int64_t *off, void *stream, int finish,
+                        int64_t *n_events)
+{
+    if (H->failed) { afsk_set_error("afsk_rx_streams: an earlier push failed; destroy the handle"); return AFSK_E_CUDA; }
+    AfskDeviceGuard guard(H->device);
+    if (!guard.ok) { afsk_set_error("cannot select device %d", H->device); return AFSK_E_CUDA; }
+    const int rc = streams_run(H, samples, on_device, off, (cudaStream_t)stream, finish, n_events);
+    if (rc != AFSK_OK) {
+        H->failed = true;
+        H->ev.clear(); H->res.clear(); H->payload.clear(); H->payload_off.clear();
+    }
+    return rc;
+}
+
+int afsk_rx_streams_create(int device, int S, int baud, int amp_start, int amp_end, int64_t timeout_frames, AfskRxStreams **h)
+{
+    if (!h || S < 1) { afsk_set_error("afsk_rx_streams_create: bad argument (S >= 1)"); return AFSK_E_ARG; }
+    int bf, ml, sl;
+    if (!afsk_tone_geometry(baud, &bf, &ml, &sl)) { afsk_set_error("Invalid baud rate."); return AFSK_E_BAUD; }
+    AfskDeviceGuard guard(device);
+    if (!guard.ok) { afsk_set_error("cannot select device %d", device); return AFSK_E_CUDA; }
+    AfskRxStreams *H = new (std::nothrow) AfskRxStreams();
+    if (!H) return AFSK_E_ARG;
+    H->device = device; H->S = S; H->baud = baud; H->amp_start = amp_start; H->amp_end = amp_end; H->timeout = timeout_frames;
+    for (auto *v : {&H->pushed, &H->keep, &H->calls, &H->slot_off, &H->slot_cap, &H->slot_base, &H->np, &H->new_off, &H->new_cap})
+        v->assign((size_t)S, 0);
+    H->pending.assign((size_t)S, -1);
+    size_t o = 0;
+    auto carve = [&](size_t bytes) { const size_t at = o; o += (bytes + 15) & ~(size_t)15; return at; };
+    H->o_seg_app = carve(sizeof(CopySeg) * S); H->o_tf_app = carve(8 * ((size_t)S + 1));
+    H->o_seg_mov = carve(sizeof(CopySeg) * S); H->o_tf_mov = carve(8 * ((size_t)S + 1));
+    H->o_first = carve(8 * ((size_t)S + 1)); H->o_amp_off = carve(8 * (size_t)S); H->o_out_first = carve(8 * (size_t)S);
+    H->desc_bytes = o;
+    cudaError_t e = cudaMalloc((void **)&H->d_desc, H->desc_bytes);
+    if (e == cudaSuccess) e = cudaMallocHost((void **)&H->h_desc, H->desc_bytes);
+    if (e == cudaSuccess) e = cudaMalloc((void **)&H->d_state, sizeof(GateState) * S);
+    if (e == cudaSuccess) e = cudaMallocHost((void **)&H->h_state, sizeof(GateState) * S);
+    if (e == cudaSuccess) e = cudaMalloc((void **)&H->d_counts, sizeof(int32_t) * S);
+    if (e == cudaSuccess) e = cudaMallocHost((void **)&H->h_counts, sizeof(int32_t) * S);
+    if (e == cudaSuccess) e = cudaMemset(H->d_state, 0, sizeof(GateState) * S);
+    if (e != cudaSuccess) {
+        afsk_rx_streams_destroy(H);
+        return streams_fail(e);
+    }
+    *h = H;
+    return AFSK_OK;
+}
+
+int afsk_rx_streams_push(AfskRxStreams *H, const int16_t *samples, int on_device, const int64_t *h_offsets, void *stream,
+                         int64_t *n_events)
+{
+    if (!H || !h_offsets || !n_events) { afsk_set_error("afsk_rx_streams_push: null argument"); return AFSK_E_ARG; }
+    if (h_offsets[0] < 0) { afsk_set_error("afsk_rx_streams_push: negative offset"); return AFSK_E_ARG; }
+    for (int s = 0; s < H->S; s++)
+        if (h_offsets[s + 1] < h_offsets[s]) { afsk_set_error("afsk_rx_streams_push: offsets decrease at channel %d", s); return AFSK_E_ARG; }
+    if (h_offsets[H->S] > h_offsets[0] && !samples) { afsk_set_error("afsk_rx_streams_push: null samples"); return AFSK_E_ARG; }
+    if (on_device && (reinterpret_cast<uintptr_t>(samples) & 15) != 0) {
+        afsk_set_error("afsk_rx_streams_push: device samples must be 16-byte aligned");
+        return AFSK_E_ARG;
+    }
+    return streams_call(H, samples, on_device, h_offsets, stream, 0, n_events);
+}
+
+int afsk_rx_streams_finish(AfskRxStreams *H, void *stream, int64_t *n_events)
+{
+    if (!H || !n_events) { afsk_set_error("afsk_rx_streams_finish: null argument"); return AFSK_E_ARG; }
+    return streams_call(H, nullptr, 0, nullptr, stream, 1, n_events);
+}
+
+int afsk_rx_streams_events(const AfskRxStreams *H, const AfskRxStreamEvent **ev, const AfskRxResult **res, const uint8_t **payload,
+                           const int64_t **payload_off)
+{
+    if (!H) return AFSK_E_ARG;
+    if (ev) *ev = H->ev.data();
+    if (res) *res = H->res.data();
+    if (payload) *payload = H->payload.data();
+    if (payload_off) *payload_off = H->payload_off.empty() ? nullptr : H->payload_off.data();
+    return AFSK_OK;
+}
+
+int afsk_rx_streams_state(const AfskRxStreams *H, int s, int64_t *pushed, int64_t *pending_start, int64_t *retained)
+{
+    if (!H || s < 0 || s >= H->S) { afsk_set_error("afsk_rx_streams_state: bad argument"); return AFSK_E_ARG; }
+    if (pushed) *pushed = H->pushed[s];
+    if (pending_start) *pending_start = H->pending[s];
+    if (retained) *retained = H->pushed[s] - H->keep[s];
+    return AFSK_OK;
+}
+
+int afsk_rx_streams_arena_bytes(const AfskRxStreams *H, int64_t *bytes)
+{
+    if (!H || !bytes) return AFSK_E_ARG;
+    *bytes = (int64_t)(H->arena_cap[0] + H->arena_cap[1] + H->stage_cap + H->desc_bytes + H->amp_cap + H->ranges_cap + H->out_cap +
+                       H->res_cap + (sizeof(GateState) + sizeof(int32_t)) * (size_t)H->S);
+    return AFSK_OK;
+}
+
+int afsk_rx_streams_counters(const AfskRxStreams *H, int64_t *launches, int64_t *moved_frames, int64_t *compactions)
+{
+    if (!H) return AFSK_E_ARG;
+    if (launches) *launches = H->n_launches;
+    if (moved_frames) *moved_frames = H->n_moved;
+    if (compactions) *compactions = H->n_compactions;
+    return AFSK_OK;
+}
+
+int afsk_rx_streams_destroy(AfskRxStreams *H)
+{
+    if (!H) return AFSK_OK;
+    AfskDeviceGuard guard(H->device);
+    if (H->plan) afsk_rx_plan_destroy(H->plan);
+    for (void *p : {(void *)H->arena[0], (void *)H->arena[1], (void *)H->d_stage, (void *)H->d_desc, (void *)H->d_state,
+                    (void *)H->d_counts, (void *)H->d_amp, (void *)H->d_ranges, (void *)H->d_out, (void *)H->d_res})
+        cudaFree(p);
+    for (void *p : {(void *)H->h_desc, (void *)H->h_state, (void *)H->h_counts, (void *)H->h_ranges, (void *)H->h_dec})
+        if (p) cudaFreeHost(p);
+    delete H;
+    return AFSK_OK;
 }
 
 }  // extern "C"

@@ -899,8 +899,13 @@ class Receiver:
                     sess.close()
         finally:
             d_s.close()
+        return self._receive_values([rec for rec, _, _ in calls], batch, string, keep_timeouts, errors)
+
+    def _receive_values(self, recorded, batch, string: bool, keep_timeouts: bool, errors: str) -> list:
+        """What successive ``receive`` calls return, with the reference's log lines (:402-417): one entry
+        per call flagged in ``recorded``; the recorded calls are ``batch``'s captures, in order."""
         out, k = [], 0
-        for rec, _, _ in calls:
+        for rec in recorded:
             self._log.info("Listening...")
             if not rec:
                 self._log.warn("Timed out.")
@@ -918,10 +923,162 @@ class Receiver:
             k += 1
         return out
 
+    def open_streams(self, n_streams: int, timeout: float, device: int | None = None) -> StreamReceiver:
+        """``receive(timeout)`` called again and again on ``n_streams`` open input streams at once, fed
+        piece by piece as the audio arrives (see ``StreamReceiver``)."""
+        return StreamReceiver(self, n_streams, timeout, self._device if device is None else device)
+
     def receive(self, timeout: float, string: bool = True) -> bytes | str:
         """Live microphone path (:402-417).  Needs an audio device; out of scope for the GPU core —
         record with any tool and use ``receive_recording`` / ``load``."""
         raise RuntimeError("afskmodem_b200 has no live audio input; use receive_recording() or load()")
+
+
+class StreamEvents:
+    """The ``receive`` calls that became final with one push (or ``finish``), ordered by (stream, call):
+    numpy arrays ``stream``, ``call``, ``recorded``, ``start``, ``end`` (stream frames of the recording)
+    and ``batch``, an RxBatch of the recorded calls' decodes in the same order."""
+
+    def __init__(self, receiver: Receiver, ev: np.ndarray, batch: RxBatch):
+        self._receiver = receiver
+        self.stream = ev["stream"].astype(np.int64)
+        self.call = ev["call"].copy()
+        self.recorded = ev["recorded"].astype(bool)
+        self.start = ev["start"].copy()
+        self.end = ev["end"].copy()
+        self.batch = batch
+
+    def __len__(self) -> int:
+        return len(self.stream)
+
+    def values(self, string: bool = True, errors: str = "raise") -> list:
+        """What each of these ``receive`` calls returned (``b""`` / ``""`` for "Timed out.") with the
+        reference's log lines; errors="return" puts the exception a call raises in the list instead."""
+        return self._receiver._receive_values(self.recorded, self.batch, string, True, errors)
+
+
+class StreamReceiver:
+    """Continuous reception on S channels at once (``Receiver.open_streams``).  Each channel behaves like
+    one reference Receiver calling ``receive(timeout)`` again and again on its own open input stream
+    (afskmodem.py:283, 299-319, 402-417).  ``push`` appends the next piece of every channel (any length,
+    including 0) and returns the calls that became final with it, already decoded: a call that timed
+    out, or a recording whose closing quiet chunk has arrived.  A recording still open stays on the
+    device.  ``finish`` ends the streams (a pending recording ends at its last full chunk, a call that
+    has neither opened nor timed out is dropped); the next push then starts new streams.  Over any way
+    of cutting a stream into pushes, the events of all pushes plus ``finish`` are ``listen_gate_multi``
+    over the whole stream, and their values ``receive_all(stream, keep_timeouts=True)``."""
+
+    def __init__(self, receiver: Receiver, n_streams: int, timeout: float, device: int = 0):
+        _cabi.require_device(device)
+        self.receiver, self.S, self.device = receiver, int(n_streams), device
+        self._destroy = _cabi.lib().afsk_rx_streams_destroy
+        h = C.c_void_p()
+        _cabi.check(_cabi.lib().afsk_rx_streams_create(device, self.S, receiver._baud, int(np.floor(receiver._amp_start)),
+                                                        _as_int_threshold(receiver._amp_end), int(timeout * 48000), C.byref(h)))
+        self._h = h
+        self._pinned = None
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self._destroy(self._h)
+            self._h = None
+        if getattr(self, "_pinned", None) is not None:
+            self._pinned.close()
+            self._pinned = None
+
+    __del__ = close
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def _host_input(self, pieces) -> tuple[np.ndarray, np.ndarray]:
+        """S host pieces -> one grow-only pinned int16 buffer (asynchronous copy to the device) and offsets."""
+        offsets = np.zeros(len(pieces) + 1, dtype=np.int64)
+        np.cumsum([len(p) for p in pieces], out=offsets[1:])
+        n = int(offsets[-1])
+        if self._pinned is None or self._pinned.array.size < n:
+            if self._pinned is not None:
+                self._pinned.close()
+            self._pinned = _cabi.PinnedArray((max(n + n // 4, 16),), np.int16)
+        buf = self._pinned.array
+        for p, a, b in zip(pieces, offsets[:-1], offsets[1:]):
+            buf[a:b] = p
+        return buf, offsets
+
+    def push(self, samples, offsets=None, stream=None) -> StreamEvents:
+        """``samples``: a list of S int16 arrays; or one int16 array (numpy, or a CUDA torch tensor on this
+        receiver's device) holding the S pieces concatenated, with ``offsets`` (S+1, CSR)."""
+        if offsets is None:
+            if len(samples) != self.S:
+                raise ValueError(f"push needs one piece per stream ({self.S}), got {len(samples)}")
+            arr, offsets = self._host_input(samples)
+            return self._run(arr.ctypes.data, 0, offsets, stream)
+        offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+        if len(offsets) != self.S + 1:
+            raise ValueError(f"offsets must have S + 1 = {self.S + 1} entries, got {len(offsets)}")
+        if hasattr(samples, "data_ptr"):                       # a torch tensor: passed by device pointer
+            if not samples.is_cuda or samples.device.index != self.device:
+                raise ValueError(f"device samples must live on cuda:{self.device}")
+            if str(samples.dtype) != "torch.int16" or not samples.is_contiguous():
+                raise ValueError("device samples must be a contiguous int16 tensor")
+            if int(offsets[-1]) > samples.numel():
+                raise ValueError(f"tensor holds {samples.numel()} frames, the offsets need {int(offsets[-1])}")
+            return self._run(samples.data_ptr(), 1, offsets, stream)
+        arr = np.ascontiguousarray(samples, dtype=np.int16)
+        if int(offsets[-1]) > len(arr):
+            raise ValueError(f"samples holds {len(arr)} frames, the offsets need {int(offsets[-1])}")
+        return self._run(arr.ctypes.data, 0, offsets, stream)
+
+    def finish(self, stream=None) -> StreamEvents:
+        n = C.c_int64(0)
+        _cabi.check(_cabi.lib().afsk_rx_streams_finish(self._h, C.c_void_p(stream or 0), C.byref(n)))
+        return self._events(n.value)
+
+    def _run(self, ptr: int, on_device: int, offsets: np.ndarray, stream) -> StreamEvents:
+        n = C.c_int64(0)
+        _cabi.check(_cabi.lib().afsk_rx_streams_push(self._h, C.c_void_p(ptr), on_device, _cabi.ptr(offsets, C.c_int64),
+                                                      C.c_void_p(stream or 0), C.byref(n)))
+        return self._events(n.value)
+
+    def _events(self, n: int) -> StreamEvents:
+        ev = np.zeros(n, dtype=_cabi.STREAM_EVENT_DTYPE)
+        res = np.zeros(n, dtype=_cabi.RX_RESULT_DTYPE)
+        off = np.zeros(n + 1, dtype=np.int64)
+        blob = np.zeros(0, dtype=np.uint8)
+        if n:
+            pe, pr, pp, po = C.c_void_p(), C.c_void_p(), C.c_void_p(), C.c_void_p()
+            _cabi.check(_cabi.lib().afsk_rx_streams_events(self._h, C.byref(pe), C.byref(pr), C.byref(pp), C.byref(po)))
+            C.memmove(ev.ctypes.data, pe, ev.nbytes)
+            C.memmove(res.ctypes.data, pr, res.nbytes)
+            C.memmove(off.ctypes.data, po, off.nbytes)
+            blob = np.zeros(int(off[-1]), dtype=np.uint8)
+            if len(blob):
+                C.memmove(blob.ctypes.data, pp, blob.nbytes)
+        rec = ev["recorded"] != 0
+        out_off = np.append(off[:-1][rec], off[-1]).astype(np.int64)
+        return StreamEvents(self.receiver, ev, RxBatch(res[rec], blob, out_off))
+
+    def state(self, s: int) -> tuple[int, int, int]:
+        """(frames pushed, start of the pending recording or -1, frames retained on the device) of stream s."""
+        a, b, c = C.c_int64(0), C.c_int64(0), C.c_int64(0)
+        _cabi.check(_cabi.lib().afsk_rx_streams_state(self._h, int(s), C.byref(a), C.byref(b), C.byref(c)))
+        return a.value, b.value, c.value
+
+    def counters(self) -> dict:
+        """Since this receiver was opened: kernel launches (decodes included), frames moved to keep retained
+        samples (appends aside) and whole-arena compactions."""
+        a, b, c = C.c_int64(0), C.c_int64(0), C.c_int64(0)
+        _cabi.check(_cabi.lib().afsk_rx_streams_counters(self._h, C.byref(a), C.byref(b), C.byref(c)))
+        return {"launches": a.value, "moved_frames": b.value, "compactions": c.value}
+
+    def arena_bytes(self) -> int:
+        """Device bytes this receiver holds (sample arenas, staging, scratch)."""
+        n = C.c_int64(0)
+        _cabi.check(_cabi.lib().afsk_rx_streams_arena_bytes(self._h, C.byref(n)))
+        return n.value
 
 
 class _NullLog:

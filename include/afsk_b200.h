@@ -189,6 +189,51 @@ int afsk_rx_gate_multi(int device, const int16_t *d_samples, const int64_t *h_of
                        int amp_end, int64_t timeout_frames, int max_calls, int64_t *d_ranges,
                        int32_t *d_counts, void *stream);
 
+/*
+ * Streaming receiver: S channels, each one Receiver calling receive(timeout) again and again on its own
+ * open input stream (afskmodem.py:283, 299-319, 402-417), fed piece by piece as the audio arrives.
+ * Chunks lie on the grid of stream frames 2048*k from the first frame pushed to the channel; a partial
+ * chunk at the end of a push waits for the next one.  A push returns the receive() calls that became
+ * final with it, decoded: calls that timed out (all their ceil(timeout / 2048) chunks present, none
+ * loud) and recordings whose closing quiet chunk is present.  A recording without one yet is pending:
+ * its samples stay on the device.  For every way of cutting a stream into pushes, the events of all
+ * pushes and of afsk_rx_streams_finish are the calls afsk_rx_gate_multi reports over the whole stream.
+ * Positions are int64 stream frames.
+ */
+typedef struct AfskRxStreams AfskRxStreams;
+typedef struct AfskRxStreamEvent {      /* 32 bytes, one per final receive() call */
+    int32_t stream, recorded;           /* recorded 0 = "Timed out." */
+    int64_t call;                       /* index of the call on its channel */
+    int64_t start, end;                 /* stream frames of the recording */
+} AfskRxStreamEvent;
+/* baud / amp_end as for afsk_rx_plan_create, amp_start / timeout_frames as for afsk_rx_gate_multi */
+int afsk_rx_streams_create(int device, int S, int baud, int amp_start, int amp_end, int64_t timeout_frames,
+                           AfskRxStreams **h);     /* AFSK_E_BAUD where the reference constructor raises */
+/* samples: the S pieces concatenated, h_offsets[S+1] (CSR, any length including 0); on_device != 0: a
+ * device pointer (16-byte aligned, allocation extending to the next 16-byte boundary past h_offsets[S]),
+ * else host memory (pinned recommended).  Synchronizes `stream`.  A bad argument returns AFSK_E_ARG and
+ * changes nothing; after any other error the handle refuses every later push / finish (AFSK_E_CUDA) and
+ * can only be destroyed. */
+int afsk_rx_streams_push(AfskRxStreams *h, const int16_t *samples, int on_device, const int64_t *h_offsets,
+                         void *stream, int64_t *n_events);
+/* ends every stream (finite-stream conventions of afsk_rx_gate_multi: a pending recording ends at the
+ * last full chunk, a call that has neither opened nor timed out is dropped, a partial chunk is ignored);
+ * the next push is frame 0 of new streams */
+int afsk_rx_streams_finish(AfskRxStreams *h, void *stream, int64_t *n_events);
+/* host arrays owned by the handle, valid until the next push / finish: n_events events ordered by
+ * (stream, call); per event an AfskRxResult (zero with clock = train_end = -1 for a timed-out call) and
+ * payload[payload_off[i] .. + res[i].nbytes) (capacity offsets, n_events + 1 entries) */
+int afsk_rx_streams_events(const AfskRxStreams *h, const AfskRxStreamEvent **ev, const AfskRxResult **res,
+                           const uint8_t **payload, const int64_t **payload_off);
+/* channel s: frames pushed, start of the pending recording (-1: none), frames retained on the device */
+int afsk_rx_streams_state(const AfskRxStreams *h, int s, int64_t *pushed, int64_t *pending_start, int64_t *retained);
+/* device bytes the handle holds (sample arenas, staging and scratch; the decode plan's own arena aside) */
+int afsk_rx_streams_arena_bytes(const AfskRxStreams *h, int64_t *bytes);
+/* since creation: kernel launches (decodes included), frames moved to keep retained samples (excluding
+ * appends), whole-arena compactions */
+int afsk_rx_streams_counters(const AfskRxStreams *h, int64_t *launches, int64_t *moved_frames, int64_t *compactions);
+int afsk_rx_streams_destroy(AfskRxStreams *h);
+
 /* ---------------------------------------------------------------- transmitter ---------- */
 /* frames Transmitter.save writes for a payload of n bytes (afskmodem.py:452-469 then :239-244).
  * Needs the payload only when mark/space tone lengths differ (e.g. 4800 baud); pass NULL else. */

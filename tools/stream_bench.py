@@ -1,0 +1,193 @@
+"""Streaming receiver throughput: S channels of 1200-baud transmissions separated by silence, pushed
+piece by piece through Receiver.open_streams, host-pinned or device-resident input.
+
+    python tools/stream_bench.py [--S 1,64,4096] [--piece 2048,48000] [--seconds 8] [--out FILE]
+
+Channel s hears one long traffic recording from frame s * 12345 on, so recordings land at different
+places on every channel.  Each configuration runs its push sequence twice on one receiver (finish in
+between) and times the second: host wall time of every push, which ends in a synchronize.  Beside it,
+receive_all and listen_gate_multi over whole streams of the same traffic (one stream per call, the
+only way they run) on the same card.  Card name and power limit are read in the same run."""
+from __future__ import annotations
+
+import argparse
+import json
+import os
+import subprocess
+import sys
+import time
+
+import numpy as np
+
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), ".."))
+import afskmodem_b200 as A  # noqa: E402
+from afskmodem_b200 import _cabi  # noqa: E402
+
+SHIFT = 12345
+
+
+def card():
+    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                       capture_output=True, text=True)
+    return q.stdout.strip().splitlines()[0] if q.returncode == 0 and q.stdout.strip() else "unknown"
+
+
+def traffic(n: int, rng) -> np.ndarray:
+    """1200-baud transmissions (10-60 byte payloads, 0.1 s training) separated by 0.2-1.5 s of silence, light noise"""
+    tx = A.Transmitter(1200, 0.1)
+    msgs = [rng.integers(0, 256, size=int(rng.integers(10, 61)), dtype=np.uint8).tobytes() for _ in range(64)]
+    batch = tx.encode_batch(msgs)
+    parts, total = [], 0
+    while total < n:
+        gap = np.zeros(int(rng.integers(9600, 72000)), np.int16)
+        fr = batch.frames(int(rng.integers(0, len(msgs))))
+        parts += [gap, fr]
+        total += len(gap) + len(fr)
+    x = np.concatenate(parts)[:n].astype(np.float64) * 0.8 + rng.normal(0, 1500, n)
+    return np.clip(np.round(x), -32768, 32767).astype(np.int16)
+
+
+def run_config(base: np.ndarray, d_base, S: int, piece: int, T: int, device: bool, timeout: float):
+    import torch
+    n_push = T // piece
+    offsets = np.arange(S + 1, dtype=np.int64) * piece
+    rx = A.Receiver(1200)
+    pinned = _cabi.PinnedArray((S * piece + 8,), np.int16)
+    out = {"S": S, "piece": piece, "input": "device" if device else "host-pinned", "pushes": n_push}
+    with rx.open_streams(S, timeout) as st:
+        for rep in range(2):
+            c0 = st.counters()
+            times, n_ev, n_rec, rec_frames, n_dec = [], 0, 0, 0, 0
+            for i in range(n_push):
+                if device:
+                    t = torch.as_strided(d_base, (S, piece), (SHIFT, 1), i * piece).contiguous().view(-1)
+                    torch.cuda.synchronize()
+                    t0 = time.perf_counter()
+                    ev = st.push(t, offsets)
+                else:
+                    np.copyto(pinned.array[:S * piece].reshape(S, piece),
+                              np.lib.stride_tricks.as_strided(base[i * piece:], shape=(S, piece), strides=(SHIFT * 2, 2)))
+                    t0 = time.perf_counter()
+                    ev = st.push(pinned.array, offsets)
+                times.append(time.perf_counter() - t0)
+                n_ev += len(ev)
+                n_rec += int(ev.recorded.sum())
+                rec_frames += int((ev.end - ev.start)[ev.recorded].sum())
+                n_dec += int(ev.recorded.any())
+            c1 = st.counters()
+            arena = st.arena_bytes()
+            st.finish()
+        frames = S * piece * n_push
+        t = np.array(times)
+        out.update({
+            "frames": frames, "seconds": float(t.sum()), "frames_per_s": frames / float(t.sum()),
+            "push_ms_median": float(np.median(t) * 1e3), "push_ms_p90": float(np.percentile(t, 90) * 1e3),
+            "push_ms_max": float(t.max() * 1e3), "events": n_ev, "recorded": n_rec,
+            "recorded_share": rec_frames / frames,
+            # counted by the receiver over the timed pushes (afsk_rx_streams_counters)
+            "launches_per_push": (c1["launches"] - c0["launches"]) / n_push, "pushes_with_decode": n_dec,
+            "moved_frames": c1["moved_frames"] - c0["moved_frames"], "compactions": c1["compactions"] - c0["compactions"],
+            # bytes the kernels move per pushed frame: append reads 2 + writes 2, the amplitudes read 2, the decode reads
+            # the recorded share (2 per recorded frame), retention moves read 2 + write 2 per moved frame; the host-input
+            # staging copy is not in this figure
+            "device_bytes_per_frame": 4 + 2 + (2 * rec_frames + 4 * (c1["moved_frames"] - c0["moved_frames"])) / frames,
+            "arena_bytes": arena,
+        })
+    pinned.close()
+    return out
+
+
+def profile_config(d_base, S: int, piece: int, T: int, timeout: float, out_dir: str | None):
+    """Device time of every kernel and copy over one device-input push sequence (torch.profiler, CUDA activity),
+    beside the host wall time of the same pushes: what share of a push the GPU is busy."""
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+    n_push = T // piece
+    offsets = np.arange(S + 1, dtype=np.int64) * piece
+    pieces = [torch.as_strided(d_base, (S, piece), (SHIFT, 1), i * piece).contiguous().view(-1) for i in range(n_push)]
+    rx = A.Receiver(1200)
+    with rx.open_streams(S, timeout) as st:
+        for t in pieces:                                  # warm-up: same shapes
+            st.push(t, offsets)
+        st.finish()
+        torch.cuda.synchronize()
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            t0 = time.perf_counter()
+            for t in pieces:
+                st.push(t, offsets)
+            wall = time.perf_counter() - t0
+        st.finish()
+    rows = {}
+    for e in prof.key_averages():
+        us = getattr(e, "device_time_total", None)
+        if us is None:
+            us = getattr(e, "cuda_time_total", 0.0)
+        if us > 0:
+            rows[e.key] = {"count": int(e.count), "ms": us / 1e3}
+    busy = sum(r["ms"] for r in rows.values())
+    if out_dir:
+        prof.export_chrome_trace(os.path.join(out_dir, "r3_stream_profile.pt.trace.json"))
+    return {"S": S, "piece": piece, "pushes": n_push, "input": "device", "host_wall_ms": wall * 1e3,
+            "device_busy_ms": busy, "device_busy_share": busy / (wall * 1e3),
+            "by_kernel_or_copy": dict(sorted(rows.items(), key=lambda kv: -kv[1]["ms"]))}
+
+
+def whole_stream_reference(base: np.ndarray, T: int, n_streams: int, timeout: float):
+    rx = A.Receiver(1200)
+    streams = [base[s * SHIFT:s * SHIFT + T] for s in range(n_streams)]
+    rx.receive_all(streams[0], timeout, False, keep_timeouts=True)               # warm-up
+    t0 = time.perf_counter()
+    for x in streams:
+        rx.receive_all(x, timeout, False, keep_timeouts=True)
+    t_all = time.perf_counter() - t0
+    t0 = time.perf_counter()
+    for x in streams:
+        rx.listen_gate_multi(x, timeout)
+    t_gate = time.perf_counter() - t0
+    frames = n_streams * T
+    return {"streams": n_streams, "frames": frames, "receive_all_frames_per_s": frames / t_all,
+            "receive_all_ms_per_stream": t_all / n_streams * 1e3, "listen_gate_multi_frames_per_s": frames / t_gate,
+            "listen_gate_multi_ms_per_stream": t_gate / n_streams * 1e3}
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--S", default="1,64,4096")
+    ap.add_argument("--piece", default="2048,48000")
+    ap.add_argument("--seconds", type=float, default=8.0)
+    ap.add_argument("--timeout", type=float, default=1.0)
+    ap.add_argument("--input", default="host,device")
+    ap.add_argument("--out", default=None)
+    ap.add_argument("--no-profile", action="store_true", help="skip the profiled run of the largest device configuration")
+    a = ap.parse_args()
+    import torch
+    _cabi.require_device(0)
+    A.LOG_LEVEL = 5
+    Ss = [int(v) for v in a.S.split(",")]
+    pieces = [int(v) for v in a.piece.split(",")]
+    T = int(a.seconds * 48000)
+    rng = np.random.default_rng(0)
+    base = traffic(max(Ss) * SHIFT + T + max(pieces), rng)
+    d_base = torch.from_numpy(base).cuda()
+    res = {"card": card(), "torch_device": torch.cuda.get_device_name(0), "seconds_per_channel": a.seconds,
+           "timeout_s": a.timeout, "configs": []}
+    for S in Ss:
+        for piece in pieces:
+            for inp in a.input.split(","):
+                r = run_config(base, d_base, S, piece, T, inp == "device", a.timeout)
+                print(json.dumps(r), flush=True)
+                res["configs"].append(r)
+    if not a.no_profile:
+        res["profile"] = profile_config(d_base, max(Ss), max(pieces), T, a.timeout,
+                                        os.path.dirname(os.path.abspath(a.out)) if a.out else None)
+        print(json.dumps({k: v for k, v in res["profile"].items() if k != "by_kernel_or_copy"}), flush=True)
+    res["whole_stream"] = whole_stream_reference(base, T, 16, a.timeout)
+    print(json.dumps(res["whole_stream"]), flush=True)
+    res["card_after"] = card()
+    if a.out:
+        os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
+        json.dump(res, open(a.out, "w"), indent=1)
+
+
+if __name__ == "__main__":
+    main()
