@@ -30,7 +30,9 @@ SYMBOLS = [
     "afsk_tx_plan_destroy", "afsk_tx_plan_out_offsets", "afsk_tx_synth", "afsk_tx_synth_host",
     "afsk_wav_probe", "afsk_wav_load", "afsk_wav_save", "afsk_rx_streams_create", "afsk_rx_streams_push",
     "afsk_rx_streams_finish", "afsk_rx_streams_events", "afsk_rx_streams_state", "afsk_rx_streams_arena_bytes",
-    "afsk_rx_streams_counters", "afsk_rx_streams_destroy",
+    "afsk_rx_streams_counters", "afsk_rx_streams_destroy", "afsk_tx_streams_create", "afsk_tx_streams_send",
+    "afsk_tx_streams_pull", "afsk_tx_streams_state", "afsk_tx_streams_arena_bytes", "afsk_tx_streams_counters",
+    "afsk_tx_streams_destroy",
 ]
 
 
@@ -115,6 +117,13 @@ def lib():
     L.afsk_tx_plan_out_offsets.argtypes = [vp, C.POINTER(i64p), C.POINTER(i64p)]
     L.afsk_tx_synth.argtypes = [vp, vp, vp, vp]
     L.afsk_tx_synth_host.argtypes = [C.c_int, u8p, i64p, C.c_int, i32p, i64p, i16p, i64p]
+    L.afsk_tx_streams_create.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int64, C.POINTER(vp)]
+    L.afsk_tx_streams_send.argtypes = [vp, C.c_int, i32p, i64p, u8p, i64p, i64p]
+    L.afsk_tx_streams_pull.argtypes = [vp, C.c_int64, vp, C.c_int, vp]
+    L.afsk_tx_streams_state.argtypes = [vp, C.c_int, i64p, i64p, i64p]
+    L.afsk_tx_streams_arena_bytes.argtypes = [vp, i64p]
+    L.afsk_tx_streams_counters.argtypes = [vp, i64p, i64p, i64p]
+    L.afsk_tx_streams_destroy.argtypes = [vp]
     cpp = C.POINTER(C.c_char_p)
     L.afsk_wav_probe.argtypes = [cpp, C.c_int, C.c_int, i64p, i64p, i32p]
     L.afsk_wav_load.argtypes = [cpp, C.c_int, C.c_int, i64p, i64p, i64p, vp, C.c_int, vp, C.c_int64, vp, i32p]

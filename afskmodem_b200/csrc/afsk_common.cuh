@@ -36,6 +36,28 @@ struct AfskDeviceGuard {
     }
 };
 
+// grow-only buffers: reallocated (contents dropped) with a quarter more than asked when `need` exceeds `*cap`
+static inline cudaError_t grow_device(void **p, size_t *cap, size_t need)
+{
+    if (need <= *cap) return cudaSuccess;
+    if (*p) cudaFree(*p);
+    *p = nullptr; *cap = 0;
+    const size_t want = need + need / 4 + 4096;
+    const cudaError_t e = cudaMalloc(p, want);
+    if (e == cudaSuccess) *cap = want;
+    return e;
+}
+static inline cudaError_t grow_pinned(void **p, size_t *cap, size_t need)
+{
+    if (need <= *cap) return cudaSuccess;
+    if (*p) cudaFreeHost(*p);
+    *p = nullptr; *cap = 0;
+    const size_t want = need + need / 4 + 4096;
+    const cudaError_t e = cudaMallocHost(p, want);
+    if (e == cudaSuccess) *cap = want;
+    return e;
+}
+
 // Tone geometry of a baud rate (Waveforms.getSpaceTone/getMarkTone, afskmodem.py:68-85;
 // Receiver.__bit_frames :277).  Returns false where the constructor raises "Invalid baud rate.".
 static inline bool afsk_tone_geometry(int baud, int *bf, int *mark_len, int *space_len)

@@ -3046,16 +3046,6 @@ struct HostCtx {
 };
 HostCtx g_host_ctx[64];
 
-cudaError_t grow_device(void **p, size_t *cap, size_t need)
-{
-    if (need <= *cap) return cudaSuccess;
-    if (*p) cudaFree(*p);
-    *p = nullptr; *cap = 0;
-    const size_t want = need + need / 4 + 4096;
-    const cudaError_t e = cudaMalloc(p, want);
-    if (e == cudaSuccess) *cap = want;
-    return e;
-}
 }  // namespace
 
 int afsk_rx_decode_host(int device, const int16_t *h_samples, const int64_t *h_offsets, int B, const int32_t *h_baud,
@@ -3172,16 +3162,6 @@ int afsk_rx_gate_multi(int device, const int16_t *d_samples, const int64_t *h_of
 // the channels pushed while the free space filled, so every pushed frame causes O(1) moved frames
 // (afsk_rx_streams_counters reports them), and one long recording widens only its own slot.
 namespace {
-cudaError_t grow_pinned(void **p, size_t *cap, size_t need)
-{
-    if (need <= *cap) return cudaSuccess;
-    if (*p) cudaFreeHost(*p);
-    *p = nullptr; *cap = 0;
-    const size_t want = need + need / 4 + 4096;
-    const cudaError_t e = cudaMallocHost(p, want);
-    if (e == cudaSuccess) *cap = want;
-    return e;
-}
 constexpr int64_t kSlotPad = 64;           // samples after the last slot (vector over-reads of the kernels)
 int64_t arena_frames(size_t bytes) { return bytes ? (int64_t)(bytes / 2) - kSlotPad : 0; }
 }  // namespace

@@ -10,6 +10,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <deque>
 #include <new>
 #include <vector>
 
@@ -377,6 +378,135 @@ static size_t synth_smem_bytes(int bf)
     return (size_t)(G == 1 ? 3 : 9) * VG * 16 + kMaxSymbols;
 }
 
+// ------------------------------------------------------------------ streaming transmitter ----
+// S channels on one shared timeline; channel s's frames [start, start + out_len) of a queued message are
+// that message's save() frames, every other frame is 0.  k_tx_window synthesizes the window [P, P + n) of
+// every channel straight from payload bytes, as the flat row-major S x n output (row s = channel s).  Its
+// descriptors are the TxDescs of the messages that overlap the window, with out_off = the message's first
+// frame on the timeline, listed per row (CSR row_off[S + 1]).
+//
+// Every frame of a message is the even frame of its pair (SoundOutput.__convertFrames :239-244, counted from
+// the message's own first frame).  All tone lengths are even (0 included: the 24000-baud mark), so a pair never
+// straddles two bits and a frame's value is the tone at its bit phase rounded down to even.
+constexpr int kWinThreads = 256;
+
+// bit b and phase u (frames into the bit's tone) of even message frame p: one divide (32-bit below 2^31
+// frames) for equal tones, var_locate for unequal ones
+__device__ __forceinline__ void win_locate(long long p, const TxDesc &d, const uint8_t *__restrict__ pay,
+                                           const int64_t *__restrict__ nib, long long &b, int &u)
+{
+    if (d.ml != d.bf) { var_locate(p, d, pay, nib + d.nib_off, b, u); return; }
+    if (p < 0x7FFFFFFFLL) {
+        const uint32_t q = (uint32_t)p / (uint32_t)d.bf;
+        b = q; u = (int)((uint32_t)p - q * (uint32_t)d.bf);
+    } else {
+        b = p / d.bf; u = (int)(p - b * d.bf);
+    }
+}
+
+__device__ __forceinline__ void win_bit(long long b, const TxDesc &d, const uint8_t *__restrict__ pay, uint32_t &sym, int &L)
+{
+    sym = b < d.total_bits ? tx_bit(b, d, pay) : 2u;           // 4800 zero frames :468
+    L = sym == 2u ? 0x7FFFFFFF : (sym ? d.ml : d.bf);
+}
+
+// the window message of row `row` that holds or follows timeline frame t (first with end > t); hi if none
+__device__ __forceinline__ int win_find(const TxDesc *__restrict__ descs, int lo, int hi, long long t)
+{
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (descs[mid].out_off + descs[mid].out_len <= t) lo = mid + 1; else hi = mid;
+    }
+    return lo;
+}
+
+// one frame of row `row` at timeline frame t (boundary vectors only)
+__device__ int16_t win_frame(const TxDesc *__restrict__ descs, const int32_t *__restrict__ row_off, long long row,
+                             long long t, const uint8_t *__restrict__ pay, const int64_t *__restrict__ nib)
+{
+    const int hi = row_off[row + 1];
+    const int k = win_find(descs, row_off[row], hi, t);
+    if (k >= hi || descs[k].out_off > t) return 0;
+    const TxDesc d = descs[k];
+    long long b;
+    int u;
+    win_locate((t - d.out_off) & ~1LL, d, pay, nib, b, u);
+    uint32_t sym;
+    int L;
+    win_bit(b, d, pay, sym, L);
+    return (int16_t)(tone_pair(sym, u, d.bf) & 0xFFFFu);
+}
+
+// One thread per 16-byte output vector.  A vector inside one row and one message locates its first pair once
+// and walks five pairs (the short-tone walk of k_synth_var: at 24000 baud a mark has no frames); its words
+// are the pair values, shifted by one frame when the message starts on an odd frame of the vector.  A vector
+// across a row or message boundary, or the end of the output, writes its frames one by one.
+__global__ void __launch_bounds__(kWinThreads) k_tx_window(const uint8_t *__restrict__ pay, const int64_t *__restrict__ nib,
+                                                           const TxDesc *__restrict__ descs, const int32_t *__restrict__ row_off,
+                                                           long long P, long long n, long long total, int16_t *__restrict__ out)
+{
+    const long long v = (long long)blockIdx.x * kWinThreads + threadIdx.x;
+    const long long f0 = 8 * v;
+    if (f0 >= total) return;
+    long long row, col;
+    if (f0 < 0xFFFFFFFFLL && n < 0xFFFFFFFFLL) {
+        const uint32_t r32 = (uint32_t)f0 / (uint32_t)n;
+        row = r32; col = f0 - (long long)r32 * n;
+    } else {
+        row = f0 / n; col = f0 - row * n;
+    }
+    const long long t0 = P + col;
+    if (col + 8 <= n) {
+        const int hi = row_off[row + 1];
+        const int k = win_find(descs, row_off[row], hi, t0);
+        if (k >= hi || descs[k].out_off >= t0 + 8) {           // silence
+            *reinterpret_cast<uint4 *>(out + f0) = make_uint4(0u, 0u, 0u, 0u);
+            return;
+        }
+        const TxDesc d = descs[k];
+        if (d.out_off <= t0 && d.out_off + d.out_len >= t0 + 8) {
+            const long long m0 = t0 - d.out_off;
+            long long b;
+            int u;
+            win_locate(m0 & ~1LL, d, pay, nib, b, u);
+            uint32_t sym;
+            int L;
+            win_bit(b, d, pay, sym, L);
+            uint32_t pv[5];
+#pragma unroll
+            for (int j = 0; j < 5; j++) {
+                pv[j] = tone_pair(sym, u, d.bf);
+                u += 2;
+                while (u >= L) {                               // next bit (__getFrames :463-467 appends tone after tone)
+                    u -= L;
+                    b++;
+                    win_bit(b, d, pay, sym, L);
+                }
+            }
+            uint32_t w[4];
+#pragma unroll
+            for (int j = 0; j < 4; j++) w[j] = (m0 & 1) ? ((pv[j] & 0xFFFFu) | (pv[j + 1] & 0xFFFF0000u)) : pv[j];
+            *reinterpret_cast<uint4 *>(out + f0) = make_uint4(w[0], w[1], w[2], w[3]);
+            return;
+        }
+    }
+#pragma unroll 1
+    for (int e = 0; e < 8 && f0 + e < total; e++) {
+        out[f0 + e] = win_frame(descs, row_off, row, P + col, pay, nib);
+        if (++col == n) { col = 0; row++; }
+    }
+}
+
+// Moves live arena blocks (16-byte aligned, whole 16-byte units) into the other arena: one CTA per block.
+struct TxMove { long long src, dst, len; };
+
+__global__ void __launch_bounds__(kWinThreads) k_tx_compact(const uint4 *__restrict__ src, uint4 *__restrict__ dst,
+                                                            const TxMove *__restrict__ mv)
+{
+    const TxMove m = mv[blockIdx.x];
+    for (long long i = threadIdx.x; i < m.len / 16; i += kWinThreads) dst[m.dst / 16 + i] = src[m.src / 16 + i];
+}
+
 }  // namespace
 
 struct AfskTxPlan {
@@ -561,6 +691,289 @@ int afsk_tx_synth_host(int device, const uint8_t *h_payload, const int64_t *h_pa
     afsk_tx_plan_destroy(P);
     if (e != cudaSuccess) { afsk_set_error("afsk_tx_synth_host: %s", cudaGetErrorString(e)); return AFSK_E_CUDA; }
     return rc;
+}
+
+}  // extern "C"
+
+// ---------------------------------------------------------------- streaming transmitter (host) ----
+// Device state is O(payload bytes): one arena of 16-byte aligned blocks, one per queued message: its payload
+// and, for unequal tones, its codeword start table (k_tx_nibscan at send time).  New blocks go on top.  When
+// they do not fit, the live blocks move (k_tx_compact) to the bottom of the other arena, whose capacity doubles
+// until the live blocks and the new ones fill at most half of it.  A compaction therefore follows at least half
+// an arena of sent bytes and moves at most one arena: moved bytes per sent byte stay below 2.  A message is
+// retired once the timeline has passed its end; when none is left, the top returns to the bottom.
+namespace {
+constexpr int64_t kTxArenaMin = 65536;
+int64_t round16(int64_t x) { return (x + 15) & ~(int64_t)15; }
+
+struct TxMsg {
+    int64_t block_off, block_bytes;
+    TxDesc d;                       // pay_off / nib_off into the arena, out_off = first frame on the timeline
+};
+}  // namespace
+
+struct AfskTxStreams {
+    int device = 0, S = 0, bf = 0, ml = 0, baud = 0;
+    int64_t ts_cycles = 0;
+    int64_t P = 0;                                        // frames pulled
+    std::vector<std::deque<TxMsg>> q;                     // per channel: messages not yet fully pulled
+    std::vector<int64_t> last_end;                        // per channel: end of the last message sent
+    uint8_t *arena[2] = {nullptr, nullptr};
+    size_t arena_alloc[2] = {0, 0};
+    int cur = 0;
+    int64_t cap = 0, top = 0, live = 0;                   // bytes: capacity of the current arena, used, in live blocks
+    bool failed = false;
+    int64_t n_launches = 0, n_moved = 0, n_compactions = 0;
+    uint8_t *h_stage = nullptr; size_t h_stage_cap = 0;   // pinned: new blocks / descriptors of one call
+    uint8_t *d_scratch = nullptr; size_t d_scratch_cap = 0;
+    int16_t *d_out = nullptr; size_t out_cap = 0;         // pull into host memory
+};
+
+// a send or pull with valid arguments: any failure may leave the queues and the arena between two states, so the
+// handle refuses every later send / pull
+template <typename F> static int tx_streams_call(AfskTxStreams *H, F run)
+{
+    if (H->failed) { afsk_set_error("afsk_tx_streams: an earlier call failed; destroy the handle"); return AFSK_E_CUDA; }
+    AfskDeviceGuard guard(H->device);
+    if (!guard.ok) { afsk_set_error("cannot select device %d", H->device); return AFSK_E_CUDA; }
+    const int rc = run();
+    if (rc != AFSK_OK) H->failed = true;
+    return rc;
+}
+
+// a send with valid arguments: synchronous on the legacy default stream
+static int tx_send_run(AfskTxStreams *H, int n, const int32_t *h_stream, const int64_t *h_pay_off, const uint8_t *h_payload,
+                       int64_t *h_start, int64_t *h_end)
+{
+    if (n == 0) return AFSK_OK;
+    const bool var = H->ml != H->bf;
+    cudaStream_t st = nullptr;
+
+    // the new blocks, in order, above the top (after a compaction if they do not fit)
+    std::vector<TxMsg> msgs((size_t)n);
+    int64_t W = 0;
+    for (int i = 0; i < n; i++) {
+        TxMsg &m = msgs[i];
+        TxDesc &d = m.d;
+        memset(&d, 0, sizeof(d));
+        d.pay_len = h_pay_off[i + 1] - h_pay_off[i];
+        d.bf = H->bf; d.ml = H->ml;
+        d.ts_bits = 2 * H->ts_cycles;
+        d.total_bits = d.ts_bits + 4 + 14 * d.pay_len;
+        d.out_len = afsk_tx_num_samples(H->baud, H->ts_cycles, d.pay_len, d.pay_len ? h_payload + h_pay_off[i] : nullptr);
+        m.block_off = W;
+        m.block_bytes = round16(d.pay_len) + (var ? round16(8 * (2 * d.pay_len + 1)) : 0);
+        W += m.block_bytes;
+    }
+    if (H->top + W > H->cap) {
+        int64_t newcap = H->cap;
+        while (2 * (H->live + W) > newcap) newcap *= 2;
+        const int nxt = H->cur ^ 1;
+        std::vector<TxMove> mv;
+        int64_t o = 0;
+        for (auto &qs : H->q)
+            for (TxMsg &m : qs) {
+                if (m.block_bytes) mv.push_back(TxMove{m.block_off, o, m.block_bytes});
+                m.block_off = o;
+                m.d.pay_off = o;
+                m.d.nib_off = (o + round16(m.d.pay_len)) / 8;
+                o += m.block_bytes;
+            }
+        AFSK_CUDA(grow_device((void **)&H->arena[nxt], &H->arena_alloc[nxt], (size_t)newcap));
+        if (!mv.empty()) {
+            AFSK_CUDA(grow_pinned((void **)&H->h_stage, &H->h_stage_cap, sizeof(TxMove) * mv.size()));
+            AFSK_CUDA(grow_device((void **)&H->d_scratch, &H->d_scratch_cap, sizeof(TxMove) * mv.size()));
+            memcpy(H->h_stage, mv.data(), sizeof(TxMove) * mv.size());
+            AFSK_CUDA(cudaMemcpyAsync(H->d_scratch, H->h_stage, sizeof(TxMove) * mv.size(), cudaMemcpyHostToDevice, st));
+            k_tx_compact<<<(unsigned)mv.size(), kWinThreads, 0, st>>>(reinterpret_cast<const uint4 *>(H->arena[H->cur]),
+                                                                     reinterpret_cast<uint4 *>(H->arena[nxt]),
+                                                                     reinterpret_cast<const TxMove *>(H->d_scratch));
+            AFSK_CUDA(cudaGetLastError());
+            AFSK_CUDA(cudaStreamSynchronize(st));    // the scratch and staging are reused below
+            H->n_launches++;
+        }
+        H->n_moved += H->live;
+        H->n_compactions++;
+        H->cur = nxt;
+        H->cap = newcap;
+        H->top = H->live;
+    }
+    // payload image of the new blocks (one copy), then the codeword start tables of unequal-tone messages
+    const size_t desc_bytes = var ? sizeof(TxDesc) * (size_t)n : 0, caps_bytes = var ? sizeof(int32_t) * (size_t)n : 0;
+    AFSK_CUDA(grow_pinned((void **)&H->h_stage, &H->h_stage_cap, (size_t)W + desc_bytes + caps_bytes));
+    AFSK_CUDA(grow_device((void **)&H->d_scratch, &H->d_scratch_cap, desc_bytes + caps_bytes + 16));
+    for (int i = 0; i < n; i++) {
+        TxMsg &m = msgs[i];
+        if (m.d.pay_len) memcpy(H->h_stage + m.block_off, h_payload + h_pay_off[i], (size_t)m.d.pay_len);
+        m.block_off += H->top;
+        m.d.pay_off = m.block_off;
+        m.d.nib_off = (m.block_off + round16(m.d.pay_len)) / 8;
+    }
+    if (W > 0) AFSK_CUDA(cudaMemcpyAsync(H->arena[H->cur] + H->top, H->h_stage, (size_t)W, cudaMemcpyHostToDevice, st));
+    if (var) {
+        TxDesc *hd = reinterpret_cast<TxDesc *>(H->h_stage + W);        // W is a multiple of 16
+        int32_t *hc = reinterpret_cast<int32_t *>(H->h_stage + W + desc_bytes);
+        for (int i = 0; i < n; i++) { hd[i] = msgs[i].d; hc[i] = i; }
+        AFSK_CUDA(cudaMemcpyAsync(H->d_scratch, hd, desc_bytes + caps_bytes, cudaMemcpyHostToDevice, st));
+        k_tx_nibscan<<<(unsigned)n, kScanThreads, 0, st>>>(H->arena[H->cur], reinterpret_cast<const TxDesc *>(H->d_scratch),
+                                                           reinterpret_cast<const int32_t *>(H->d_scratch + desc_bytes),
+                                                           reinterpret_cast<int64_t *>(H->arena[H->cur]));
+        AFSK_CUDA(cudaGetLastError());
+        H->n_launches++;
+    }
+    AFSK_CUDA(cudaStreamSynchronize(st));
+    H->top += W;
+    H->live += W;
+    for (int i = 0; i < n; i++) {
+        TxMsg &m = msgs[i];
+        const int s = h_stream[i];
+        m.d.out_off = std::max(H->P, H->last_end[s]);
+        H->last_end[s] = m.d.out_off + m.d.out_len;
+        h_start[i] = m.d.out_off;
+        h_end[i] = H->last_end[s];
+        H->q[s].push_back(m);
+    }
+    return AFSK_OK;
+}
+
+static int tx_pull_run(AfskTxStreams *H, int64_t n_frames, int16_t *dst, int on_device, cudaStream_t st)
+{
+    if (n_frames == 0) return AFSK_OK;
+    const int S = H->S;
+    const int64_t n = n_frames, total = (int64_t)S * n, wend = H->P + n;
+    const int64_t nvec = (total + 7) >> 3;
+    // per row, the messages that overlap [P, P + n): a prefix of the channel's queue (retired ones are gone)
+    int64_t nwin = 0;
+    for (int s = 0; s < S; s++)
+        for (const TxMsg &m : H->q[s]) {
+            if (m.d.out_off >= wend) break;
+            nwin++;
+        }
+    const size_t desc_bytes = sizeof(TxDesc) * (size_t)nwin, bytes = desc_bytes + sizeof(int32_t) * ((size_t)S + 1);
+    AFSK_CUDA(grow_pinned((void **)&H->h_stage, &H->h_stage_cap, bytes));
+    AFSK_CUDA(grow_device((void **)&H->d_scratch, &H->d_scratch_cap, bytes));
+    if (!on_device) AFSK_CUDA(grow_device((void **)&H->d_out, &H->out_cap, (size_t)nvec * 16));
+    TxDesc *hd = reinterpret_cast<TxDesc *>(H->h_stage);
+    int32_t *row_off = reinterpret_cast<int32_t *>(H->h_stage + desc_bytes);
+    int32_t k = 0;
+    for (int s = 0; s < S; s++) {
+        row_off[s] = k;
+        for (const TxMsg &m : H->q[s]) {
+            if (m.d.out_off >= wend) break;
+            hd[k++] = m.d;
+        }
+    }
+    row_off[S] = k;
+    AFSK_CUDA(cudaMemcpyAsync(H->d_scratch, H->h_stage, bytes, cudaMemcpyHostToDevice, st));
+    int16_t *out = on_device ? dst : H->d_out;
+    const uint8_t *a = H->arena[H->cur];
+    k_tx_window<<<(unsigned)((nvec + kWinThreads - 1) / kWinThreads), kWinThreads, 0, st>>>(
+        a, reinterpret_cast<const int64_t *>(a), reinterpret_cast<const TxDesc *>(H->d_scratch),
+        reinterpret_cast<const int32_t *>(H->d_scratch + desc_bytes), H->P, n, total, out);
+    AFSK_CUDA(cudaGetLastError());
+    H->n_launches++;
+    if (!on_device) AFSK_CUDA(cudaMemcpyAsync(dst, H->d_out, (size_t)total * 2, cudaMemcpyDeviceToHost, st));
+    AFSK_CUDA(cudaStreamSynchronize(st));
+    H->P = wend;
+    for (auto &qs : H->q)
+        while (!qs.empty() && qs.front().d.out_off + qs.front().d.out_len <= H->P) {
+            H->live -= qs.front().block_bytes;
+            qs.pop_front();
+        }
+    if (H->live == 0) H->top = 0;
+    return AFSK_OK;
+}
+
+extern "C" {
+
+int afsk_tx_streams_create(int device, int S, int baud, int64_t ts_cycles, AfskTxStreams **h)
+{
+    if (!h || S < 1) { afsk_set_error("afsk_tx_streams_create: bad argument (S >= 1)"); return AFSK_E_ARG; }
+    int bf, ml, sl;
+    if (!afsk_tone_geometry(baud, &bf, &ml, &sl)) { afsk_set_error("Invalid baud rate."); return AFSK_E_BAUD; }
+    AfskDeviceGuard guard(device);
+    if (!guard.ok) { afsk_set_error("cannot select device %d", device); return AFSK_E_CUDA; }
+    AfskTxStreams *H = new (std::nothrow) AfskTxStreams();
+    if (!H) return AFSK_E_ARG;
+    H->device = device; H->S = S; H->baud = baud; H->bf = bf; H->ml = ml;
+    H->ts_cycles = ts_cycles < 0 ? 0 : ts_cycles;
+    H->q.resize((size_t)S);
+    H->last_end.assign((size_t)S, 0);
+    H->cap = kTxArenaMin;
+    const cudaError_t e = grow_device((void **)&H->arena[0], &H->arena_alloc[0], (size_t)H->cap);
+    if (e != cudaSuccess) {
+        afsk_set_error("afsk_tx_streams_create: %s", cudaGetErrorString(e));
+        afsk_tx_streams_destroy(H);
+        return AFSK_E_CUDA;
+    }
+    *h = H;
+    return AFSK_OK;
+}
+
+int afsk_tx_streams_send(AfskTxStreams *H, int n, const int32_t *h_stream, const int64_t *h_pay_off, const uint8_t *h_payload,
+                         int64_t *h_start, int64_t *h_end)
+{
+    if (!H || n < 0 || (n > 0 && (!h_stream || !h_pay_off || !h_start || !h_end))) {
+        afsk_set_error("afsk_tx_streams_send: bad argument");
+        return AFSK_E_ARG;
+    }
+    if (n > 0 && h_pay_off[0] < 0) { afsk_set_error("afsk_tx_streams_send: negative payload offset"); return AFSK_E_ARG; }
+    for (int i = 0; i < n; i++) {
+        if (h_stream[i] < 0 || h_stream[i] >= H->S) { afsk_set_error("afsk_tx_streams_send: stream %d out of range", h_stream[i]); return AFSK_E_ARG; }
+        if (h_pay_off[i + 1] < h_pay_off[i]) { afsk_set_error("afsk_tx_streams_send: payload offsets decrease at message %d", i); return AFSK_E_ARG; }
+    }
+    if (n > 0 && h_pay_off[n] > h_pay_off[0] && !h_payload) { afsk_set_error("afsk_tx_streams_send: null payload"); return AFSK_E_ARG; }
+    return tx_streams_call(H, [&] { return tx_send_run(H, n, h_stream, h_pay_off, h_payload, h_start, h_end); });
+}
+
+int afsk_tx_streams_pull(AfskTxStreams *H, int64_t n_frames, int16_t *dst, int on_device, void *stream)
+{
+    if (!H || n_frames < 0 || (n_frames > 0 && !dst)) { afsk_set_error("afsk_tx_streams_pull: bad argument"); return AFSK_E_ARG; }
+    if (n_frames > (INT64_MAX / 16) / H->S) { afsk_set_error("afsk_tx_streams_pull: S * n_frames overflows"); return AFSK_E_ARG; }
+    if (on_device && (reinterpret_cast<uintptr_t>(dst) & 15) != 0) {
+        afsk_set_error("afsk_tx_streams_pull: device output must be 16-byte aligned");
+        return AFSK_E_ARG;
+    }
+    if ((((int64_t)H->S * n_frames + 7) / 8 + kWinThreads - 1) / kWinThreads > 0x7FFFFFFFLL) {
+        afsk_set_error("afsk_tx_streams_pull: window too large");
+        return AFSK_E_ARG;
+    }
+    return tx_streams_call(H, [&] { return tx_pull_run(H, n_frames, dst, on_device, (cudaStream_t)stream); });
+}
+
+int afsk_tx_streams_state(const AfskTxStreams *H, int s, int64_t *pulled, int64_t *busy_until, int64_t *pending)
+{
+    if (!H || s < 0 || s >= H->S) { afsk_set_error("afsk_tx_streams_state: bad argument"); return AFSK_E_ARG; }
+    if (pulled) *pulled = H->P;
+    if (busy_until) *busy_until = H->last_end[s];
+    if (pending) *pending = (int64_t)H->q[s].size();
+    return AFSK_OK;
+}
+
+int afsk_tx_streams_arena_bytes(const AfskTxStreams *H, int64_t *bytes)
+{
+    if (!H || !bytes) return AFSK_E_ARG;
+    *bytes = (int64_t)(H->arena_alloc[0] + H->arena_alloc[1] + H->d_scratch_cap + H->out_cap);
+    return AFSK_OK;
+}
+
+int afsk_tx_streams_counters(const AfskTxStreams *H, int64_t *launches, int64_t *moved_bytes, int64_t *compactions)
+{
+    if (!H) return AFSK_E_ARG;
+    if (launches) *launches = H->n_launches;
+    if (moved_bytes) *moved_bytes = H->n_moved;
+    if (compactions) *compactions = H->n_compactions;
+    return AFSK_OK;
+}
+
+int afsk_tx_streams_destroy(AfskTxStreams *H)
+{
+    if (!H) return AFSK_OK;
+    AfskDeviceGuard guard(H->device);
+    for (void *p : {(void *)H->arena[0], (void *)H->arena[1], (void *)H->d_scratch, (void *)H->d_out}) cudaFree(p);
+    if (H->h_stage) cudaFreeHost(H->h_stage);
+    delete H;
+    return AFSK_OK;
 }
 
 }  // extern "C"

@@ -1256,6 +1256,106 @@ class Transmitter:
 
     write = save         # README.md:119 name
 
+    def open_streams(self, n_streams: int, device: int | None = None) -> StreamTransmitter:
+        """``transmit`` called again and again on ``n_streams`` open output streams at once, pulled piece by
+        piece as the sound card asks for frames (see ``StreamTransmitter``)."""
+        return StreamTransmitter(self, n_streams, self._device if device is None else device)
+
     def transmit(self, data: str | bytes):
         """Live speaker path (:472-478).  Needs an audio device; out of scope — use ``save``."""
         raise RuntimeError("afskmodem_b200 has no live audio output; use save()")
+
+
+class StreamTransmitter:
+    """Continuous transmission on S channels at once (``Transmitter.open_streams``).  Each channel behaves like
+    one reference Transmitter whose output stream stays open, calling ``transmit(data)`` again and again
+    (afskmodem.py:472-478: ``SoundOutput.play`` writes what ``save`` writes, :247-252).  The channels share one
+    timeline, pulled ``n`` frames at a time like the periods of a multi-channel sound card.  ``send`` queues
+    messages; one starts at ``max(frames pulled, end of its channel's last message)`` and its frames are exactly
+    what ``save`` writes for it; every other frame is silence (0).  Only payload bytes are kept on the device:
+    each ``pull`` synthesizes its window from them."""
+
+    def __init__(self, transmitter: Transmitter, n_streams: int, device: int = 0):
+        _cabi.require_device(device)
+        self.transmitter, self.S, self.device = transmitter, int(n_streams), device
+        self._destroy = _cabi.lib().afsk_tx_streams_destroy
+        h = C.c_void_p()
+        _cabi.check(_cabi.lib().afsk_tx_streams_create(device, self.S, transmitter._baud, transmitter._ts_cycles, C.byref(h)))
+        self._h = h
+        self._pinned = None
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self._destroy(self._h)
+            self._h = None
+        if getattr(self, "_pinned", None) is not None:
+            self._pinned.close()
+            self._pinned = None
+
+    __del__ = close
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def send(self, streams, payloads) -> tuple[np.ndarray, np.ndarray]:
+        """Queues ``payloads[i]`` (str is UTF-8 encoded, as in ``save``) on channel ``streams[i]``, in list order.
+        Returns the int64 arrays (start, end): the timeline frames of each message."""
+        data = [Transmitter._as_bytes(p) for p in payloads]
+        ids = np.ascontiguousarray(streams, dtype=np.int32).reshape(-1)
+        if len(ids) != len(data):
+            raise ValueError(f"send needs one stream per payload, got {len(ids)} streams and {len(data)} payloads")
+        off = np.zeros(len(data) + 1, dtype=np.int64)
+        np.cumsum([len(p) for p in data], out=off[1:])
+        blob = np.frombuffer(b"".join(data), dtype=np.uint8) if off[-1] else np.zeros(1, dtype=np.uint8)
+        start, end = np.zeros(len(data), np.int64), np.zeros(len(data), np.int64)
+        _cabi.check(_cabi.lib().afsk_tx_streams_send(self._h, len(data), _cabi.ptr(ids, C.c_int32), _cabi.ptr(off, C.c_int64),
+                                                     _cabi.ptr(blob, C.c_uint8), _cabi.ptr(start, C.c_int64),
+                                                     _cabi.ptr(end, C.c_int64)))
+        return start, end
+
+    def pull(self, n: int, out=None, stream=None):
+        """The next ``n`` frames of every channel.  Default: a host (S, n) int16 array in a grow-only pinned
+        buffer, valid until the next pull unless copied.  ``out``: a contiguous CUDA int16 tensor of at least
+        S * n elements on this transmitter's device, written row-major (row s = channel s, no padding) and
+        returned; nothing past S * n is written."""
+        n = int(n)
+        if n < 0:
+            raise ValueError("pull needs n >= 0")
+        total = self.S * n
+        if out is not None:
+            if not out.is_cuda or out.device.index != self.device:
+                raise ValueError(f"out must live on cuda:{self.device}")
+            if str(out.dtype) != "torch.int16" or not out.is_contiguous():
+                raise ValueError("out must be a contiguous int16 tensor")
+            if out.numel() < total:
+                raise ValueError(f"out holds {out.numel()} frames, the pull needs {total}")
+            _cabi.check(_cabi.lib().afsk_tx_streams_pull(self._h, n, C.c_void_p(out.data_ptr()), 1, C.c_void_p(stream or 0)))
+            return out
+        if self._pinned is None or self._pinned.array.size < total:
+            if self._pinned is not None:
+                self._pinned.close()
+            self._pinned = _cabi.PinnedArray((max(total + total // 4, 16),), np.int16)
+        buf = self._pinned.array[:total]
+        _cabi.check(_cabi.lib().afsk_tx_streams_pull(self._h, n, C.c_void_p(buf.ctypes.data), 0, C.c_void_p(stream or 0)))
+        return buf.reshape(self.S, n)
+
+    def state(self, s: int) -> tuple[int, int, int]:
+        """(frames pulled, end of channel s's last message (<= frames pulled: idle), its messages not yet fully pulled)."""
+        a, b, c = C.c_int64(0), C.c_int64(0), C.c_int64(0)
+        _cabi.check(_cabi.lib().afsk_tx_streams_state(self._h, int(s), C.byref(a), C.byref(b), C.byref(c)))
+        return a.value, b.value, c.value
+
+    def counters(self) -> dict:
+        """Since this transmitter was opened: kernel launches, payload-arena bytes moved by compactions, compactions."""
+        a, b, c = C.c_int64(0), C.c_int64(0), C.c_int64(0)
+        _cabi.check(_cabi.lib().afsk_tx_streams_counters(self._h, C.byref(a), C.byref(b), C.byref(c)))
+        return {"launches": a.value, "moved_bytes": b.value, "compactions": c.value}
+
+    def arena_bytes(self) -> int:
+        """Device bytes this transmitter holds (payload arenas, descriptors, host-output staging)."""
+        n = C.c_int64(0)
+        _cabi.check(_cabi.lib().afsk_tx_streams_arena_bytes(self._h, C.byref(n)))
+        return n.value

@@ -253,6 +253,35 @@ int afsk_tx_synth_host(int device, const uint8_t *h_payload, const int64_t *h_pa
                        const int32_t *h_baud, const int64_t *h_ts_cycles, int16_t *h_out,
                        const int64_t *h_out_off);
 
+/*
+ * Streaming transmitter: S channels, each one Transmitter whose output stream stays open, calling
+ * transmit(data) again and again (afskmodem.py:472-478 hands __getFrames to SoundOutput.play, :247-252,
+ * which writes what save() writes).  The channels share one timeline of frames, pulled in windows like
+ * the periods of a multi-channel sound card; P = frames pulled so far.  A message sent to channel s starts
+ * at max(P, end of s's last message) and lasts afsk_tx_num_samples frames (always even); its frames are
+ * exactly save()'s, every frame outside a message is 0.  The device keeps payload bytes only (plus, for
+ * unequal tone lengths, each message's codeword start table); every pull synthesizes its window from them.
+ */
+typedef struct AfskTxStreams AfskTxStreams;
+/* baud / ts_cycles as for afsk_tx_plan_create; AFSK_E_BAUD where the reference constructor raises */
+int afsk_tx_streams_create(int device, int S, int baud, int64_t ts_cycles, AfskTxStreams **h);
+/* queues n messages (message i = h_payload[h_pay_off[i] .. h_pay_off[i+1]) on channel h_stream[i], in order)
+ * and returns their timeline frames [h_start[i], h_end[i]).  Synchronous. */
+int afsk_tx_streams_send(AfskTxStreams *h, int n, const int32_t *h_stream, const int64_t *h_pay_off,
+                         const uint8_t *h_payload, int64_t *h_start, int64_t *h_end);
+/* the next n_frames frames of every channel as an S x n_frames row-major int16 array: on_device != 0, a
+ * 16-byte aligned device pointer, else host memory (pinned recommended); nothing past S * n_frames is
+ * written.  Synchronizes `stream`.  A bad argument returns AFSK_E_ARG and changes nothing; after any other
+ * error the handle refuses every later send / pull (AFSK_E_CUDA) and can only be destroyed. */
+int afsk_tx_streams_pull(AfskTxStreams *h, int64_t n_frames, int16_t *dst, int on_device, void *stream);
+/* channel s: frames pulled (P), end of its last message sent (<= P: idle), messages not yet fully pulled */
+int afsk_tx_streams_state(const AfskTxStreams *h, int s, int64_t *pulled, int64_t *busy_until, int64_t *pending);
+/* device bytes the handle holds (payload arenas, descriptors, host-output staging) */
+int afsk_tx_streams_arena_bytes(const AfskTxStreams *h, int64_t *bytes);
+/* since creation: kernel launches, arena bytes moved by compactions, compactions */
+int afsk_tx_streams_counters(const AfskTxStreams *h, int64_t *launches, int64_t *moved_bytes, int64_t *compactions);
+int afsk_tx_streams_destroy(AfskTxStreams *h);
+
 /* ---------------------------------------------------------------- wav files ------------ */
 /*
  * Host ingest / egress for batches of files (one pool of host threads; threads <= 0: all cores).

@@ -1,0 +1,173 @@
+"""Streaming transmitter throughput: S channels of 1200-baud messages separated by silence, pulled window by window
+through Transmitter.open_streams into a CUDA tensor or a host (pinned) array.
+
+    python tools/stream_tx_bench.py [--S 1,64,4096] [--pull 2048,48000] [--seconds 8] [--out FILE]
+
+Every channel sends a 10-60 byte message (0.1 s training) whenever its previous one has ended and a random gap of
+up to twice a message's mean length has passed, so a channel is busy about half the time; the sends due inside a
+window go in one send() call before its pull.  Each configuration runs its sequence twice on one transmitter and
+times the second: host wall time of every pull (it ends in a synchronize) and of every send.  A separate
+torch.profiler run of the largest device-output configuration gives k_tx_window's kernel time (bytes written per
+second of kernel time, against the 7.7 TB/s of HBM3e on a B200's data sheet) and the share of a pull the GPU is busy.
+Card name and power limit are read in the same run."""
+from __future__ import annotations
+
+import argparse
+import json
+import os
+import subprocess
+import sys
+import time
+
+import numpy as np
+
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), ".."))
+import afskmodem_b200 as A  # noqa: E402
+from afskmodem_b200 import _cabi  # noqa: E402
+
+HBM_TBS = 7.7
+
+
+def card():
+    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                       capture_output=True, text=True)
+    return q.stdout.strip().splitlines()[0] if q.returncode == 0 and q.stdout.strip() else "unknown"
+
+
+class Traffic:
+    """per channel: the next frame at which it sends, and a pool of payloads"""
+
+    def __init__(self, S: int, baud: int, seed: int):
+        self.rng = np.random.default_rng(seed)
+        self.S = S
+        self.msgs = [self.rng.integers(0, 256, size=int(self.rng.integers(10, 61)), dtype=np.uint8).tobytes() for _ in range(256)]
+        bf = 48000 // baud
+        self.mean_len = int(0.1 * baud) * bf + 5 * bf + 4800 + 35 * 14 * bf
+        self.next_at = self.rng.integers(0, 2 * self.mean_len, S).astype(np.int64)
+
+    def due(self, P: int, n: int):
+        s = np.nonzero(self.next_at < P + n)[0]
+        return s.astype(np.int32), [self.msgs[i] for i in self.rng.integers(0, len(self.msgs), len(s))]
+
+    def sent(self, streams, end):
+        self.next_at[streams] = end + self.rng.integers(0, 2 * self.mean_len, len(streams))
+
+
+def run_sequence(st, S, n, n_pull, baud, seed, out_t=None):
+    tr = Traffic(S, baud, seed)
+    t_pull, t_send, busy = [], [], 0
+    P = st.state(0)[0]                      # the timeline goes on from the previous sequence
+    tr.next_at += P
+    for _ in range(n_pull):
+        streams, pays = tr.due(P, n)
+        t0 = time.perf_counter()
+        if len(streams):
+            a, b = st.send(streams, pays)
+            tr.sent(streams, b)
+            busy += int((b - a).sum())
+        t1 = time.perf_counter()
+        st.pull(n, out=out_t)
+        t2 = time.perf_counter()
+        t_send.append(t1 - t0)
+        t_pull.append(t2 - t1)
+        P += n
+    return np.array(t_pull), np.array(t_send), busy
+
+
+def run_config(S: int, n: int, T: int, device: bool, baud: int):
+    import torch
+    n_pull = max(T // n, 1)
+    out_t = torch.empty(S * n, dtype=torch.int16, device="cuda") if device else None
+    tx = A.Transmitter(baud, 0.1)
+    res = {"S": S, "pull": n, "baud": baud, "output": "device" if device else "host-pinned", "pulls": n_pull}
+    with tx.open_streams(S) as st:
+        run_sequence(st, S, n, n_pull, baud, 1, out_t)                # warm-up: same shapes
+        c0 = st.counters()
+        tp, ts, busy = run_sequence(st, S, n, n_pull, baud, 2, out_t)
+        c1 = st.counters()
+        arena = st.arena_bytes()
+    frames = S * n * n_pull
+    res.update({
+        "frames": frames, "pull_seconds": float(tp.sum()), "send_seconds": float(ts.sum()),
+        "frames_per_s": frames / float(tp.sum()), "frames_per_s_with_send": frames / float(tp.sum() + ts.sum()),
+        "pull_ms_median": float(np.median(tp) * 1e3), "pull_ms_p90": float(np.percentile(tp, 90) * 1e3),
+        "send_ms_median": float(np.median(ts) * 1e3), "busy_fraction": busy / frames,
+        "launches_per_pull": (c1["launches"] - c0["launches"]) / n_pull,
+        "moved_bytes": c1["moved_bytes"] - c0["moved_bytes"], "compactions": c1["compactions"] - c0["compactions"],
+        "arena_bytes": arena,
+    })
+    return res
+
+
+def profile_config(S: int, n: int, T: int, baud: int, out_dir: str | None):
+    """Device time of every kernel and copy over one device-output pull sequence (torch.profiler, CUDA activity),
+    beside the host wall time of the same pulls."""
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+    n_pull = max(T // n, 1)
+    out_t = torch.empty(S * n, dtype=torch.int16, device="cuda")
+    tx = A.Transmitter(baud, 0.1)
+    with tx.open_streams(S) as st:
+        run_sequence(st, S, n, n_pull, baud, 1, out_t)
+        torch.cuda.synchronize()
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            t0 = time.perf_counter()
+            tp, ts, _ = run_sequence(st, S, n, n_pull, baud, 2, out_t)
+            wall = time.perf_counter() - t0
+    rows = {}
+    for e in prof.key_averages():
+        us = getattr(e, "device_time_total", None)
+        if us is None:
+            us = getattr(e, "cuda_time_total", 0.0)
+        if us > 0:
+            rows[e.key] = {"count": int(e.count), "ms": us / 1e3}
+    busy = sum(r["ms"] for r in rows.values())
+    win = [v for k, v in rows.items() if "k_tx_window" in k]
+    win_ms = sum(r["ms"] for r in win)
+    win_bytes = 2 * S * n * n_pull
+    if out_dir:
+        prof.export_chrome_trace(os.path.join(out_dir, "r4_stream_tx_profile.pt.trace.json"))
+    return {"S": S, "pull": n, "baud": baud, "pulls": n_pull, "output": "device", "host_wall_ms": wall * 1e3,
+            "host_ms_per_pull": wall * 1e3 / n_pull, "pull_ms_per_pull": float(tp.sum()) * 1e3 / n_pull,
+            "send_ms_per_pull": float(ts.sum()) * 1e3 / n_pull,
+            "device_busy_ms": busy, "device_busy_ms_per_pull": busy / n_pull, "device_busy_share": busy / (wall * 1e3),
+            "k_tx_window_ms": win_ms, "k_tx_window_us_per_pull": win_ms * 1e3 / n_pull,
+            "k_tx_window_bytes_written": win_bytes,
+            "k_tx_window_TBps": win_bytes / (win_ms * 1e-3) / 1e12 if win_ms else None,
+            "k_tx_window_share_of_hbm_peak": (win_bytes / (win_ms * 1e-3) / 1e12) / HBM_TBS if win_ms else None,
+            "by_kernel_or_copy": dict(sorted(rows.items(), key=lambda kv: -kv[1]["ms"]))}
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--S", default="1,64,4096")
+    ap.add_argument("--pull", default="2048,48000")
+    ap.add_argument("--seconds", type=float, default=8.0)
+    ap.add_argument("--output", default="device,host")
+    ap.add_argument("--out", default=None)
+    ap.add_argument("--no-profile", action="store_true", help="skip the profiled run of the largest device configuration")
+    a = ap.parse_args()
+    import torch
+    _cabi.require_device(0)
+    A.LOG_LEVEL = 5
+    Ss = [int(v) for v in a.S.split(",")]
+    pulls = [int(v) for v in a.pull.split(",")]
+    T = int(a.seconds * 48000)
+    res = {"card": card(), "torch_device": torch.cuda.get_device_name(0), "seconds_per_channel": a.seconds, "configs": []}
+    lines = [(S, n, o == "device", 1200) for S in Ss for n in pulls for o in a.output.split(",")]
+    lines.append((max(Ss), max(pulls), True, 4800))
+    for S, n, dev, baud in lines:
+        r = run_config(S, n, T, dev, baud)
+        print(json.dumps(r), flush=True)
+        res["configs"].append(r)
+    if not a.no_profile:
+        res["profile"] = profile_config(max(Ss), max(pulls), T, 1200, os.path.dirname(os.path.abspath(a.out)) if a.out else None)
+        print(json.dumps({k: v for k, v in res["profile"].items() if k != "by_kernel_or_copy"}), flush=True)
+    res["card_after"] = card()
+    if a.out:
+        os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
+        json.dump(res, open(a.out, "w"), indent=1)
+
+
+if __name__ == "__main__":
+    main()
