@@ -12,10 +12,11 @@ LOG_LEVEL = 0
 
 from ._cabi import AfskError, LIB_PATH  # noqa: E402
 from .modem import (ECC, Log, PipelinedRxSession, Receiver, RxBatch, RxSession, ShardedRxSession, SoundInput,  # noqa: E402
-                    SoundOutput, StreamEvents, StreamReceiver, StreamTransmitter, Transmitter, TxBatch, TxSession, Waveforms, WavBatch, read_wav_frames, write_wav_batch,
-                    write_wav_frames)
+                    SoundOutput, StreamEvents, StreamReceiver, StreamTransmitter, Transmitter, TxBatch, TxSession, Waveforms, WavBatch,
+                    open_receive_streams, open_transmit_streams, read_wav_frames, write_wav_batch, write_wav_frames)
 from .shard import capture_cost, gather_rx, shard_captures  # noqa: E402
 
-__all__ = ["LOG_LEVEL", "Log", "Waveforms", "ECC", "Receiver", "Transmitter", "RxBatch", "RxSession", "PipelinedRxSession", "ShardedRxSession", "StreamReceiver", "StreamEvents", "StreamTransmitter", "SoundInput", "SoundOutput",
+__all__ = ["LOG_LEVEL", "Log", "Waveforms", "ECC", "Receiver", "Transmitter", "RxBatch", "RxSession", "PipelinedRxSession", "ShardedRxSession", "StreamReceiver", "StreamEvents", "StreamTransmitter",
+           "open_receive_streams", "open_transmit_streams", "SoundInput", "SoundOutput",
            "TxBatch", "TxSession", "AfskError", "LIB_PATH", "read_wav_frames", "write_wav_frames", "WavBatch", "write_wav_batch",
            "shard_captures", "capture_cost", "gather_rx"]

@@ -2118,21 +2118,33 @@ __device__ __forceinline__ long long warp_find_first(const int32_t *A, long long
     return -1;
 }
 
+// One receiver's gate settings (Receiver amp_start / amp_end thresholds, receive() timeout in frames).
+struct GateParams {
+    int amp_start, amp_end;
+    long long timeout_frames;
+};
+static_assert(sizeof(GateParams) == 16, "GateParams layout");
+
 // amp[chunk_first[s] ..] are the amplitudes of stream s's chunks from state[s].pos on (state == NULL: a
-// fresh state).  Call k of this walk goes to ranges[3 * (out_first ? out_first[s] : s * max_calls) + 3k].
-// Every call emitted before finish reads at least one new chunk, so new chunks + 1 slots always suffice.
+// fresh state).  Stream s gates with params[s] (params == NULL: `uni` for every stream) and finishes when
+// fin[s] != 0 (fin == NULL: when `finish`); a finished stream's state is reset to a fresh one.  Call k of
+// this walk goes to ranges[3 * (out_first ? out_first[s] : s * max_calls) + 3k].  Every call emitted before
+// finish reads at least one new chunk, so new chunks + 1 slots always suffice.
 __global__ void __launch_bounds__(32) k_gate_multi(const int32_t *__restrict__ amp, const int64_t *__restrict__ chunk_first,
-                                                   int amp_start, int amp_end, long long timeout_frames, int max_calls,
-                                                   GateState *__restrict__ state, int finish,
+                                                   GateParams uni, const GateParams *__restrict__ params, int max_calls,
+                                                   GateState *__restrict__ state, int finish, const uint8_t *__restrict__ fin,
                                                    const int64_t *__restrict__ out_first, int64_t *__restrict__ ranges,
                                                    int32_t *__restrict__ counts)
 {
     const int s = blockIdx.x, lane = threadIdx.x;
+    const GateParams p = params ? params[s] : uni;
+    const int amp_start = p.amp_start, amp_end = p.amp_end;
+    if (fin) finish = fin[s];
     GateState g = {0, 0, 0, 0, 0};
     if (state) g = state[s];
     const int32_t *A = amp + chunk_first[s] - g.pos;             // A[j]: chunk j of the stream
     const long long nch = g.pos + chunk_first[s + 1] - chunk_first[s];
-    const long long lim = timeout_frames <= 0 ? 0 : (timeout_frames + AFSK_GATE_CHUNK - 1) / AFSK_GATE_CHUNK;
+    const long long lim = p.timeout_frames <= 0 ? 0 : (p.timeout_frames + AFSK_GATE_CHUNK - 1) / AFSK_GATE_CHUNK;
     int64_t *out = ranges + (out_first ? (long long)out_first[s] : (long long)s * max_calls) * 3;
     int calls = 0;
     while (calls < max_calls) {
@@ -2170,7 +2182,7 @@ __global__ void __launch_bounds__(32) k_gate_multi(const int32_t *__restrict__ a
     g.call += calls;
     if (lane == 0) {
         counts[s] = calls;
-        if (state) state[s] = g;
+        if (state) state[s] = finish ? GateState{0, 0, 0, 0, 0} : g;
     }
 }
 
@@ -2511,8 +2523,8 @@ static int gate_run(int device, const int16_t *d_samples, const int64_t *h_offse
         k_gate_amp<<<(unsigned)((total + wpb - 1) / wpb), wpb * 32, 0, st>>>(d_samples, g.d_first, g.d_off, S, total, g.d_amp);
     }
     if (max_calls < 0) k_gate_scan<<<S, kFrameThreads, 0, st>>>(g.d_amp, g.d_first, amp_start, amp_end, timeout_frames, d_ranges);
-    else k_gate_multi<<<S, 32, 0, st>>>(g.d_amp, g.d_first, amp_start, amp_end, timeout_frames, max_calls, nullptr, 1, nullptr,
-                                         d_ranges, d_counts);
+    else k_gate_multi<<<S, 32, 0, st>>>(g.d_amp, g.d_first, GateParams{amp_start, amp_end, timeout_frames}, nullptr, max_calls,
+                                         nullptr, 1, nullptr, nullptr, d_ranges, d_counts);
     AFSK_CUDA(cudaGetLastError());
     AFSK_CUDA(cudaStreamSynchronize(st));     // the host staging vector and the scratch go out of scope
     return AFSK_OK;
@@ -3167,8 +3179,11 @@ int64_t arena_frames(size_t bytes) { return bytes ? (int64_t)(bytes / 2) - kSlot
 }  // namespace
 
 struct AfskRxStreams {
-    int device = 0, S = 0, baud = 0, amp_start = 0, amp_end = 0;
-    int64_t timeout = 0;
+    int device = 0, S = 0;
+    // per channel: the receiver's baud, and its gate settings (host copy of d_params)
+    std::vector<int32_t> baud;
+    std::vector<GateParams> params;
+    GateParams *d_params = nullptr;
     // per channel (host): frames pushed, first retained frame (a chunk start), start of the pending recording
     // (-1: none), calls finished, and the slot: first arena sample, capacity, stream frame at the slot's start
     std::vector<int64_t> pushed, keep, pending, calls, slot_off, slot_cap, slot_base;
@@ -3182,7 +3197,9 @@ struct AfskRxStreams {
     int16_t *d_stage = nullptr; size_t stage_cap = 0;             // host input
     // descriptors of one push, built in pinned memory and sent with one copy
     uint8_t *d_desc = nullptr, *h_desc = nullptr;
-    size_t desc_bytes = 0, o_seg_app = 0, o_tf_app = 0, o_seg_mov = 0, o_tf_mov = 0, o_first = 0, o_amp_off = 0, o_out_first = 0;
+    // (the finish flags come last: a push copies the block up to o_fin only)
+    size_t desc_bytes = 0, o_seg_app = 0, o_tf_app = 0, o_seg_mov = 0, o_tf_mov = 0, o_first = 0, o_amp_off = 0, o_out_first = 0,
+           o_fin = 0;
     GateState *d_state = nullptr, *h_state = nullptr;
     int32_t *d_counts = nullptr, *h_counts = nullptr;
     int32_t *d_amp = nullptr; size_t amp_cap = 0;
@@ -3206,11 +3223,13 @@ static int streams_fail(cudaError_t e)
     return AFSK_E_CUDA;
 }
 
-// one push (finish = 0) or the end of the streams (finish = 1, no samples)
+// one push (fin == NULL) or the end of the streams s with fin[s] != 0 (no samples); then, when new_baud is
+// given, every channel's settings become new_baud[s] / new_params[s] for its next stream
 static int streams_run(AfskRxStreams *H, const int16_t *samples, int on_device, const int64_t *off, cudaStream_t st,
-                       int finish, int64_t *n_events)
+                       const uint8_t *fin, const int32_t *new_baud, const GateParams *new_params, int64_t *n_events)
 {
     const int S = H->S;
+    const bool finish = fin != nullptr;
     const int64_t C = AFSK_GATE_CHUNK;
     auto piece = [&](int s) -> int64_t { return finish ? 0 : off[s + 1] - off[s]; };
     int64_t nch = 0;                               // chunks completed by this push
@@ -3293,7 +3312,8 @@ static int streams_run(AfskRxStreams *H, const int16_t *samples, int on_device, 
         amp_off[s] = H->slot_off[s] + c_old * C - H->slot_base[s];
         out_first[s] = first[s] + s;
     }
-    AFSK_CUDA(cudaMemcpyAsync(H->d_desc, H->h_desc, H->desc_bytes, cudaMemcpyHostToDevice, st));
+    if (finish) memcpy(hd + H->o_fin, fin, (size_t)S);
+    AFSK_CUDA(cudaMemcpyAsync(H->d_desc, H->h_desc, finish ? H->desc_bytes : H->o_fin, cudaMemcpyHostToDevice, st));
     const uint8_t *dd = H->d_desc;
     if (nmov > 0) {
         k_stream_copy<<<(unsigned)tf_mov[nmov], kCopyThreads, 0, st>>>(H->arena[H->cur], H->arena[compact ? H->cur ^ 1 : H->cur],
@@ -3321,8 +3341,9 @@ static int streams_run(AfskRxStreams *H, const int16_t *samples, int on_device, 
         H->n_launches++;
     }
     H->n_launches++;
-    k_gate_multi<<<S, 32, 0, st>>>(H->d_amp, d_first, H->amp_start, H->amp_end, H->timeout, 0x7FFFFFFF, H->d_state, finish,
-                                   reinterpret_cast<const int64_t *>(dd + H->o_out_first), H->d_ranges, H->d_counts);
+    k_gate_multi<<<S, 32, 0, st>>>(H->d_amp, d_first, GateParams{}, H->d_params, 0x7FFFFFFF, H->d_state, 0,
+                                   finish ? dd + H->o_fin : nullptr, reinterpret_cast<const int64_t *>(dd + H->o_out_first),
+                                   H->d_ranges, H->d_counts);
     AFSK_CUDA(cudaGetLastError());
     AFSK_CUDA(cudaMemcpyAsync(H->h_counts, H->d_counts, sizeof(int32_t) * S, cudaMemcpyDeviceToHost, st));
     AFSK_CUDA(cudaMemcpyAsync(H->h_state, H->d_state, sizeof(GateState) * S, cudaMemcpyDeviceToHost, st));
@@ -3333,6 +3354,8 @@ static int streams_run(AfskRxStreams *H, const int16_t *samples, int on_device, 
     H->ev.clear();
     H->rec_start.clear();
     H->rec_len.clear();
+    H->rec_baud.clear();
+    H->rec_amp_end.clear();
     for (int s = 0; s < S; s++) {
         const int64_t *r = H->h_ranges + 3 * out_first[s];
         for (int k = 0; k < H->h_counts[s]; k++) {
@@ -3342,6 +3365,8 @@ static int streams_run(AfskRxStreams *H, const int16_t *samples, int on_device, 
             if (v.recorded) {
                 H->rec_start.push_back(H->slot_off[s] + v.start - H->slot_base[s]);
                 H->rec_len.push_back(v.end - v.start);
+                H->rec_baud.push_back(H->baud[s]);
+                H->rec_amp_end.push_back(H->params[s].amp_end);
             }
         }
         const GateState &g = H->h_state[s];
@@ -3355,8 +3380,6 @@ static int streams_run(AfskRxStreams *H, const int16_t *samples, int on_device, 
     H->payload_off.assign((size_t)nev + 1, 0);
     H->payload.clear();
     if (nrec > 0) {
-        H->rec_baud.assign((size_t)nrec, H->baud);
-        H->rec_amp_end.assign((size_t)nrec, H->amp_end);
         int rc = H->plan ? afsk_rx_plan_reset(H->plan, nrec, H->rec_start.data(), H->rec_len.data(), H->rec_baud.data(), H->rec_amp_end.data())
                          : afsk_rx_plan_create_ranges(H->device, nrec, H->rec_start.data(), H->rec_len.data(), H->rec_baud.data(),
                                                       H->rec_amp_end.data(), &H->plan);
@@ -3384,13 +3407,17 @@ static int streams_run(AfskRxStreams *H, const int16_t *samples, int on_device, 
         }
         H->payload_off[nev] = oo[nrec];
     }
-    if (finish) {                                  // the next push is frame 0 of new streams
-        for (int s = 0; s < S; s++) {
-            H->pushed[s] = H->keep[s] = H->calls[s] = H->slot_base[s] = 0;
-            H->pending[s] = -1;
-        }
-        AFSK_CUDA(cudaMemsetAsync(H->d_state, 0, sizeof(GateState) * S, st));
+    if (finish)                                    // the next push is frame 0 of a new stream (k_gate_multi reset its state)
+        for (int s = 0; s < S; s++)
+            if (fin[s]) {
+                H->pushed[s] = H->keep[s] = H->calls[s] = H->slot_base[s] = 0;
+                H->pending[s] = -1;
+            }
+    if (new_baud) {
+        AFSK_CUDA(cudaMemcpyAsync(H->d_params, new_params, sizeof(GateParams) * S, cudaMemcpyHostToDevice, st));
         AFSK_CUDA(cudaStreamSynchronize(st));
+        H->baud.assign(new_baud, new_baud + S);
+        H->params.assign(new_params, new_params + S);
     }
     *n_events = nev;
     return AFSK_OK;
@@ -3398,13 +3425,13 @@ static int streams_run(AfskRxStreams *H, const int16_t *samples, int on_device, 
 
 // a push or finish with valid arguments: any failure may leave the channels between two states, so the
 // handle refuses every later push / finish
-static int streams_call(AfskRxStreams *H, const int16_t *samples, int on_device, const int64_t *off, void *stream, int finish,
-                        int64_t *n_events)
+static int streams_call(AfskRxStreams *H, const int16_t *samples, int on_device, const int64_t *off, void *stream,
+                        const uint8_t *fin, const int32_t *new_baud, const GateParams *new_params, int64_t *n_events)
 {
     if (H->failed) { afsk_set_error("afsk_rx_streams: an earlier push failed; destroy the handle"); return AFSK_E_CUDA; }
     AfskDeviceGuard guard(H->device);
     if (!guard.ok) { afsk_set_error("cannot select device %d", H->device); return AFSK_E_CUDA; }
-    const int rc = streams_run(H, samples, on_device, off, (cudaStream_t)stream, finish, n_events);
+    const int rc = streams_run(H, samples, on_device, off, (cudaStream_t)stream, fin, new_baud, new_params, n_events);
     if (rc != AFSK_OK) {
         H->failed = true;
         H->ev.clear(); H->res.clear(); H->payload.clear(); H->payload_off.clear();
@@ -3412,16 +3439,35 @@ static int streams_call(AfskRxStreams *H, const int16_t *samples, int on_device,
     return rc;
 }
 
-int afsk_rx_streams_create(int device, int S, int baud, int amp_start, int amp_end, int64_t timeout_frames, AfskRxStreams **h)
+// checks one channel's settings: AFSK_E_ARG for a negative timeout, AFSK_E_BAUD where the reference
+// constructor raises
+static int rx_settings_check(const char *fn, int s, int baud, int64_t timeout_frames)
 {
-    if (!h || S < 1) { afsk_set_error("afsk_rx_streams_create: bad argument (S >= 1)"); return AFSK_E_ARG; }
+    if (timeout_frames < 0) { afsk_set_error("%s: negative timeout on channel %d", fn, s); return AFSK_E_ARG; }
     int bf, ml, sl;
-    if (!afsk_tone_geometry(baud, &bf, &ml, &sl)) { afsk_set_error("Invalid baud rate."); return AFSK_E_BAUD; }
+    if (!afsk_tone_geometry(baud, &bf, &ml, &sl)) { afsk_set_error("Invalid baud rate. (%s: channel %d, baud %d)", fn, s, baud); return AFSK_E_BAUD; }
+    return AFSK_OK;
+}
+
+int afsk_rx_streams_create_each(int device, int S, const int32_t *h_baud, const int32_t *h_amp_start, const int32_t *h_amp_end,
+                                const int64_t *h_timeout_frames, AfskRxStreams **h)
+{
+    if (!h || S < 1 || !h_baud || !h_amp_start || !h_amp_end || !h_timeout_frames) {
+        afsk_set_error("afsk_rx_streams_create_each: bad argument (S >= 1, non-null arrays)");
+        return AFSK_E_ARG;
+    }
+    for (int s = 0; s < S; s++) {
+        const int rc = rx_settings_check("afsk_rx_streams_create_each", s, h_baud[s], h_timeout_frames[s]);
+        if (rc != AFSK_OK) return rc;
+    }
     AfskDeviceGuard guard(device);
     if (!guard.ok) { afsk_set_error("cannot select device %d", device); return AFSK_E_CUDA; }
     AfskRxStreams *H = new (std::nothrow) AfskRxStreams();
     if (!H) return AFSK_E_ARG;
-    H->device = device; H->S = S; H->baud = baud; H->amp_start = amp_start; H->amp_end = amp_end; H->timeout = timeout_frames;
+    H->device = device; H->S = S;
+    H->baud.assign(h_baud, h_baud + S);
+    H->params.resize((size_t)S);
+    for (int s = 0; s < S; s++) H->params[s] = GateParams{h_amp_start[s], h_amp_end[s], h_timeout_frames[s]};
     for (auto *v : {&H->pushed, &H->keep, &H->calls, &H->slot_off, &H->slot_cap, &H->slot_base, &H->np, &H->new_off, &H->new_cap})
         v->assign((size_t)S, 0);
     H->pending.assign((size_t)S, -1);
@@ -3430,6 +3476,7 @@ int afsk_rx_streams_create(int device, int S, int baud, int amp_start, int amp_e
     H->o_seg_app = carve(sizeof(CopySeg) * S); H->o_tf_app = carve(8 * ((size_t)S + 1));
     H->o_seg_mov = carve(sizeof(CopySeg) * S); H->o_tf_mov = carve(8 * ((size_t)S + 1));
     H->o_first = carve(8 * ((size_t)S + 1)); H->o_amp_off = carve(8 * (size_t)S); H->o_out_first = carve(8 * (size_t)S);
+    H->o_fin = carve((size_t)S);
     H->desc_bytes = o;
     cudaError_t e = cudaMalloc((void **)&H->d_desc, H->desc_bytes);
     if (e == cudaSuccess) e = cudaMallocHost((void **)&H->h_desc, H->desc_bytes);
@@ -3437,6 +3484,8 @@ int afsk_rx_streams_create(int device, int S, int baud, int amp_start, int amp_e
     if (e == cudaSuccess) e = cudaMallocHost((void **)&H->h_state, sizeof(GateState) * S);
     if (e == cudaSuccess) e = cudaMalloc((void **)&H->d_counts, sizeof(int32_t) * S);
     if (e == cudaSuccess) e = cudaMallocHost((void **)&H->h_counts, sizeof(int32_t) * S);
+    if (e == cudaSuccess) e = cudaMalloc((void **)&H->d_params, sizeof(GateParams) * S);
+    if (e == cudaSuccess) e = cudaMemcpy(H->d_params, H->params.data(), sizeof(GateParams) * S, cudaMemcpyHostToDevice);
     if (e == cudaSuccess) e = cudaMemset(H->d_state, 0, sizeof(GateState) * S);
     if (e != cudaSuccess) {
         afsk_rx_streams_destroy(H);
@@ -3444,6 +3493,14 @@ int afsk_rx_streams_create(int device, int S, int baud, int amp_start, int amp_e
     }
     *h = H;
     return AFSK_OK;
+}
+
+int afsk_rx_streams_create(int device, int S, int baud, int amp_start, int amp_end, int64_t timeout_frames, AfskRxStreams **h)
+{
+    const size_t n = S > 0 ? (size_t)S : 1;
+    const std::vector<int32_t> b(n, baud), a0(n, amp_start), a1(n, amp_end);
+    const std::vector<int64_t> t(n, timeout_frames < 0 ? 0 : timeout_frames);     // any timeout <= 0 gates alike
+    return afsk_rx_streams_create_each(device, S, b.data(), a0.data(), a1.data(), t.data(), h);
 }
 
 int afsk_rx_streams_push(AfskRxStreams *H, const int16_t *samples, int on_device, const int64_t *h_offsets, void *stream,
@@ -3458,13 +3515,43 @@ int afsk_rx_streams_push(AfskRxStreams *H, const int16_t *samples, int on_device
         afsk_set_error("afsk_rx_streams_push: device samples must be 16-byte aligned");
         return AFSK_E_ARG;
     }
-    return streams_call(H, samples, on_device, h_offsets, stream, 0, n_events);
+    return streams_call(H, samples, on_device, h_offsets, stream, nullptr, nullptr, nullptr, n_events);
+}
+
+int afsk_rx_streams_finish_some(AfskRxStreams *H, int n, const int32_t *h_streams, const int32_t *h_baud, const int32_t *h_amp_start,
+                                const int32_t *h_amp_end, const int64_t *h_timeout_frames, void *stream, int64_t *n_events)
+{
+    const char *fn = "afsk_rx_streams_finish_some";
+    if (!H || !n_events || n < 0 || n > H->S || (n > 0 && !h_streams)) { afsk_set_error("%s: bad argument", fn); return AFSK_E_ARG; }
+    const int given = (h_baud != nullptr) + (h_amp_start != nullptr) + (h_amp_end != nullptr) + (h_timeout_frames != nullptr);
+    if (given != 0 && given != 4) { afsk_set_error("%s: the settings arrays are all given or all NULL", fn); return AFSK_E_ARG; }
+    std::vector<uint8_t> fin((size_t)H->S, 0);
+    for (int i = 0; i < n; i++) {
+        const int s = h_streams[i];
+        if (s < 0 || s >= H->S) { afsk_set_error("%s: stream %d out of range", fn, s); return AFSK_E_ARG; }
+        if (fin[s]) { afsk_set_error("%s: stream %d listed twice", fn, s); return AFSK_E_ARG; }
+        fin[s] = 1;
+    }
+    if (!given) return streams_call(H, nullptr, 0, nullptr, stream, fin.data(), nullptr, nullptr, n_events);
+    for (int i = 0; i < n; i++) {
+        const int rc = rx_settings_check(fn, h_streams[i], h_baud[i], h_timeout_frames[i]);
+        if (rc != AFSK_OK) return rc;
+    }
+    std::vector<int32_t> baud = H->baud;
+    std::vector<GateParams> params = H->params;
+    for (int i = 0; i < n; i++) {
+        baud[h_streams[i]] = h_baud[i];
+        params[h_streams[i]] = GateParams{h_amp_start[i], h_amp_end[i], h_timeout_frames[i]};
+    }
+    return streams_call(H, nullptr, 0, nullptr, stream, fin.data(), baud.data(), params.data(), n_events);
 }
 
 int afsk_rx_streams_finish(AfskRxStreams *H, void *stream, int64_t *n_events)
 {
     if (!H || !n_events) { afsk_set_error("afsk_rx_streams_finish: null argument"); return AFSK_E_ARG; }
-    return streams_call(H, nullptr, 0, nullptr, stream, 1, n_events);
+    std::vector<int32_t> all((size_t)H->S);
+    for (int s = 0; s < H->S; s++) all[s] = s;
+    return afsk_rx_streams_finish_some(H, H->S, all.data(), nullptr, nullptr, nullptr, nullptr, stream, n_events);
 }
 
 int afsk_rx_streams_events(const AfskRxStreams *H, const AfskRxStreamEvent **ev, const AfskRxResult **res, const uint8_t **payload,
@@ -3491,7 +3578,7 @@ int afsk_rx_streams_arena_bytes(const AfskRxStreams *H, int64_t *bytes)
 {
     if (!H || !bytes) return AFSK_E_ARG;
     *bytes = (int64_t)(H->arena_cap[0] + H->arena_cap[1] + H->stage_cap + H->desc_bytes + H->amp_cap + H->ranges_cap + H->out_cap +
-                       H->res_cap + (sizeof(GateState) + sizeof(int32_t)) * (size_t)H->S);
+                       H->res_cap + (sizeof(GateState) + sizeof(int32_t) + sizeof(GateParams)) * (size_t)H->S);
     return AFSK_OK;
 }
 
@@ -3510,7 +3597,7 @@ int afsk_rx_streams_destroy(AfskRxStreams *H)
     AfskDeviceGuard guard(H->device);
     if (H->plan) afsk_rx_plan_destroy(H->plan);
     for (void *p : {(void *)H->arena[0], (void *)H->arena[1], (void *)H->d_stage, (void *)H->d_desc, (void *)H->d_state,
-                    (void *)H->d_counts, (void *)H->d_amp, (void *)H->d_ranges, (void *)H->d_out, (void *)H->d_res})
+                    (void *)H->d_counts, (void *)H->d_params, (void *)H->d_amp, (void *)H->d_ranges, (void *)H->d_out, (void *)H->d_res})
         cudaFree(p);
     for (void *p : {(void *)H->h_desc, (void *)H->h_state, (void *)H->h_counts, (void *)H->h_ranges, (void *)H->h_dec})
         if (p) cudaFreeHost(p);

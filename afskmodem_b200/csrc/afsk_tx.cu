@@ -713,8 +713,10 @@ struct TxMsg {
 }  // namespace
 
 struct AfskTxStreams {
-    int device = 0, S = 0, bf = 0, ml = 0, baud = 0;
-    int64_t ts_cycles = 0;
+    int device = 0, S = 0;
+    // per channel: the settings of the messages it is sent next (bf, ml: tone lengths of baud)
+    std::vector<int32_t> baud, bf, ml;
+    std::vector<int64_t> ts_cycles;
     int64_t P = 0;                                        // frames pulled
     std::vector<std::deque<TxMsg>> q;                     // per channel: messages not yet fully pulled
     std::vector<int64_t> last_end;                        // per channel: end of the last message sent
@@ -746,23 +748,26 @@ static int tx_send_run(AfskTxStreams *H, int n, const int32_t *h_stream, const i
                        int64_t *h_start, int64_t *h_end)
 {
     if (n == 0) return AFSK_OK;
-    const bool var = H->ml != H->bf;
     cudaStream_t st = nullptr;
 
-    // the new blocks, in order, above the top (after a compaction if they do not fit)
+    // the new blocks, in order, above the top (after a compaction if they do not fit), each with its channel's
+    // settings; var: the messages with unequal tone lengths, whose blocks also hold a codeword start table
     std::vector<TxMsg> msgs((size_t)n);
+    std::vector<int32_t> var;
     int64_t W = 0;
     for (int i = 0; i < n; i++) {
+        const int s = h_stream[i];
         TxMsg &m = msgs[i];
         TxDesc &d = m.d;
         memset(&d, 0, sizeof(d));
         d.pay_len = h_pay_off[i + 1] - h_pay_off[i];
-        d.bf = H->bf; d.ml = H->ml;
-        d.ts_bits = 2 * H->ts_cycles;
+        d.bf = H->bf[s]; d.ml = H->ml[s];
+        d.ts_bits = 2 * H->ts_cycles[s];
         d.total_bits = d.ts_bits + 4 + 14 * d.pay_len;
-        d.out_len = afsk_tx_num_samples(H->baud, H->ts_cycles, d.pay_len, d.pay_len ? h_payload + h_pay_off[i] : nullptr);
+        d.out_len = afsk_tx_num_samples(H->baud[s], H->ts_cycles[s], d.pay_len, d.pay_len ? h_payload + h_pay_off[i] : nullptr);
+        if (d.ml != d.bf) var.push_back(i);
         m.block_off = W;
-        m.block_bytes = round16(d.pay_len) + (var ? round16(8 * (2 * d.pay_len + 1)) : 0);
+        m.block_bytes = round16(d.pay_len) + (d.ml != d.bf ? round16(8 * (2 * d.pay_len + 1)) : 0);
         W += m.block_bytes;
     }
     if (H->top + W > H->cap) {
@@ -799,7 +804,7 @@ static int tx_send_run(AfskTxStreams *H, int n, const int32_t *h_stream, const i
         H->top = H->live;
     }
     // payload image of the new blocks (one copy), then the codeword start tables of unequal-tone messages
-    const size_t desc_bytes = var ? sizeof(TxDesc) * (size_t)n : 0, caps_bytes = var ? sizeof(int32_t) * (size_t)n : 0;
+    const size_t desc_bytes = var.empty() ? 0 : sizeof(TxDesc) * (size_t)n, caps_bytes = sizeof(int32_t) * var.size();
     AFSK_CUDA(grow_pinned((void **)&H->h_stage, &H->h_stage_cap, (size_t)W + desc_bytes + caps_bytes));
     AFSK_CUDA(grow_device((void **)&H->d_scratch, &H->d_scratch_cap, desc_bytes + caps_bytes + 16));
     for (int i = 0; i < n; i++) {
@@ -810,12 +815,13 @@ static int tx_send_run(AfskTxStreams *H, int n, const int32_t *h_stream, const i
         m.d.nib_off = (m.block_off + round16(m.d.pay_len)) / 8;
     }
     if (W > 0) AFSK_CUDA(cudaMemcpyAsync(H->arena[H->cur] + H->top, H->h_stage, (size_t)W, cudaMemcpyHostToDevice, st));
-    if (var) {
+    if (!var.empty()) {
         TxDesc *hd = reinterpret_cast<TxDesc *>(H->h_stage + W);        // W is a multiple of 16
         int32_t *hc = reinterpret_cast<int32_t *>(H->h_stage + W + desc_bytes);
-        for (int i = 0; i < n; i++) { hd[i] = msgs[i].d; hc[i] = i; }
+        for (int i = 0; i < n; i++) hd[i] = msgs[i].d;
+        memcpy(hc, var.data(), caps_bytes);
         AFSK_CUDA(cudaMemcpyAsync(H->d_scratch, hd, desc_bytes + caps_bytes, cudaMemcpyHostToDevice, st));
-        k_tx_nibscan<<<(unsigned)n, kScanThreads, 0, st>>>(H->arena[H->cur], reinterpret_cast<const TxDesc *>(H->d_scratch),
+        k_tx_nibscan<<<(unsigned)var.size(), kScanThreads, 0, st>>>(H->arena[H->cur], reinterpret_cast<const TxDesc *>(H->d_scratch),
                                                            reinterpret_cast<const int32_t *>(H->d_scratch + desc_bytes),
                                                            reinterpret_cast<int64_t *>(H->arena[H->cur]));
         AFSK_CUDA(cudaGetLastError());
@@ -886,17 +892,29 @@ static int tx_pull_run(AfskTxStreams *H, int64_t n_frames, int16_t *dst, int on_
 
 extern "C" {
 
-int afsk_tx_streams_create(int device, int S, int baud, int64_t ts_cycles, AfskTxStreams **h)
+int afsk_tx_streams_create_each(int device, int S, const int32_t *h_baud, const int64_t *h_ts_cycles, AfskTxStreams **h)
 {
-    if (!h || S < 1) { afsk_set_error("afsk_tx_streams_create: bad argument (S >= 1)"); return AFSK_E_ARG; }
+    if (!h || S < 1 || !h_baud || !h_ts_cycles) {
+        afsk_set_error("afsk_tx_streams_create_each: bad argument (S >= 1, non-null arrays)");
+        return AFSK_E_ARG;
+    }
     int bf, ml, sl;
-    if (!afsk_tone_geometry(baud, &bf, &ml, &sl)) { afsk_set_error("Invalid baud rate."); return AFSK_E_BAUD; }
+    for (int s = 0; s < S; s++)
+        if (!afsk_tone_geometry(h_baud[s], &bf, &ml, &sl)) {
+            afsk_set_error("Invalid baud rate. (afsk_tx_streams_create_each: channel %d, baud %d)", s, h_baud[s]);
+            return AFSK_E_BAUD;
+        }
     AfskDeviceGuard guard(device);
     if (!guard.ok) { afsk_set_error("cannot select device %d", device); return AFSK_E_CUDA; }
     AfskTxStreams *H = new (std::nothrow) AfskTxStreams();
     if (!H) return AFSK_E_ARG;
-    H->device = device; H->S = S; H->baud = baud; H->bf = bf; H->ml = ml;
-    H->ts_cycles = ts_cycles < 0 ? 0 : ts_cycles;
+    H->device = device; H->S = S;
+    H->baud.resize((size_t)S); H->bf.resize((size_t)S); H->ml.resize((size_t)S); H->ts_cycles.resize((size_t)S);
+    for (int s = 0; s < S; s++) {
+        afsk_tone_geometry(h_baud[s], &bf, &ml, &sl);
+        H->baud[s] = h_baud[s]; H->bf[s] = bf; H->ml[s] = ml;
+        H->ts_cycles[s] = h_ts_cycles[s] < 0 ? 0 : h_ts_cycles[s];
+    }
     H->q.resize((size_t)S);
     H->last_end.assign((size_t)S, 0);
     H->cap = kTxArenaMin;
@@ -908,6 +926,42 @@ int afsk_tx_streams_create(int device, int S, int baud, int64_t ts_cycles, AfskT
     }
     *h = H;
     return AFSK_OK;
+}
+
+int afsk_tx_streams_create(int device, int S, int baud, int64_t ts_cycles, AfskTxStreams **h)
+{
+    const size_t n = S > 0 ? (size_t)S : 1;
+    const std::vector<int32_t> b(n, baud);
+    const std::vector<int64_t> t(n, ts_cycles);
+    return afsk_tx_streams_create_each(device, S, b.data(), t.data(), h);
+}
+
+int afsk_tx_streams_configure(AfskTxStreams *H, int n, const int32_t *h_streams, const int32_t *h_baud, const int64_t *h_ts_cycles)
+{
+    const char *fn = "afsk_tx_streams_configure";
+    if (!H || n < 0 || n > H->S || (n > 0 && (!h_streams || !h_baud || !h_ts_cycles))) { afsk_set_error("%s: bad argument", fn); return AFSK_E_ARG; }
+    std::vector<uint8_t> seen((size_t)H->S, 0);
+    for (int i = 0; i < n; i++) {
+        const int s = h_streams[i];
+        if (s < 0 || s >= H->S) { afsk_set_error("%s: stream %d out of range", fn, s); return AFSK_E_ARG; }
+        if (seen[s]) { afsk_set_error("%s: stream %d listed twice", fn, s); return AFSK_E_ARG; }
+        seen[s] = 1;
+    }
+    int bf, ml, sl;
+    for (int i = 0; i < n; i++)
+        if (!afsk_tone_geometry(h_baud[i], &bf, &ml, &sl)) {
+            afsk_set_error("Invalid baud rate. (%s: channel %d, baud %d)", fn, h_streams[i], h_baud[i]);
+            return AFSK_E_BAUD;
+        }
+    return tx_streams_call(H, [&] {
+        for (int i = 0; i < n; i++) {
+            const int s = h_streams[i];
+            afsk_tone_geometry(h_baud[i], &bf, &ml, &sl);
+            H->baud[s] = h_baud[i]; H->bf[s] = bf; H->ml[s] = ml;
+            H->ts_cycles[s] = h_ts_cycles[i] < 0 ? 0 : h_ts_cycles[i];
+        }
+        return AFSK_OK;
+    });
 }
 
 int afsk_tx_streams_send(AfskTxStreams *H, int n, const int32_t *h_stream, const int64_t *h_pay_off, const uint8_t *h_payload,

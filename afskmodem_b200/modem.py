@@ -901,10 +901,10 @@ class Receiver:
             d_s.close()
         return self._receive_values([rec for rec, _, _ in calls], batch, string, keep_timeouts, errors)
 
-    def _receive_values(self, recorded, batch, string: bool, keep_timeouts: bool, errors: str) -> list:
+    def _receive_values(self, recorded, batch, string: bool, keep_timeouts: bool, errors: str, first: int = 0) -> list:
         """What successive ``receive`` calls return, with the reference's log lines (:402-417): one entry
-        per call flagged in ``recorded``; the recorded calls are ``batch``'s captures, in order."""
-        out, k = [], 0
+        per call flagged in ``recorded``; the recorded calls are ``batch``'s captures from ``first`` on, in order."""
+        out, k = [], first
         for rec in recorded:
             self._log.info("Listening...")
             if not rec:
@@ -926,7 +926,7 @@ class Receiver:
     def open_streams(self, n_streams: int, timeout: float, device: int | None = None) -> StreamReceiver:
         """``receive(timeout)`` called again and again on ``n_streams`` open input streams at once, fed
         piece by piece as the audio arrives (see ``StreamReceiver``)."""
-        return StreamReceiver(self, n_streams, timeout, self._device if device is None else device)
+        return open_receive_streams([self] * int(n_streams), timeout, self._device if device is None else device)
 
     def receive(self, timeout: float, string: bool = True) -> bytes | str:
         """Live microphone path (:402-417).  Needs an audio device; out of scope for the GPU core —
@@ -934,13 +934,33 @@ class Receiver:
         raise RuntimeError("afskmodem_b200 has no live audio input; use receive_recording() or load()")
 
 
+def open_receive_streams(receivers, timeout, device: int | None = None) -> StreamReceiver:
+    """``receive(timeout)`` called again and again on S open input streams at once, channel s by
+    ``receivers[s]`` with ``timeout`` (seconds: one for all channels, or S of them).  The same Receiver may
+    serve many channels, e.g. ``[rx300] * 2048 + [rx1200] * 2048``.  ``device`` defaults to the first
+    receiver's.  See ``StreamReceiver``."""
+    receivers = list(receivers)
+    if not receivers:
+        raise ValueError("open_receive_streams needs at least one receiver")
+    return StreamReceiver(receivers, timeout, receivers[0]._device if device is None else device)
+
+
+def _timeout_frames(timeout, n: int) -> np.ndarray:
+    """receive() timeouts in seconds (one, or n) -> int64 frames; the reference's gate treats a negative timeout
+    like 0 (no chunk is examined, :304)"""
+    t = [timeout] * n if np.ndim(timeout) == 0 else list(timeout)
+    if len(t) != n:
+        raise ValueError(f"need one timeout or {n}, got {len(t)}")
+    return np.array([max(0, int(float(x) * 48000)) for x in t], dtype=np.int64)
+
+
 class StreamEvents:
     """The ``receive`` calls that became final with one push (or ``finish``), ordered by (stream, call):
     numpy arrays ``stream``, ``call``, ``recorded``, ``start``, ``end`` (stream frames of the recording)
     and ``batch``, an RxBatch of the recorded calls' decodes in the same order."""
 
-    def __init__(self, receiver: Receiver, ev: np.ndarray, batch: RxBatch):
-        self._receiver = receiver
+    def __init__(self, receivers, ev: np.ndarray, batch: RxBatch):
+        self._receivers = receivers                             # per channel, as when these calls were made
         self.stream = ev["stream"].astype(np.int64)
         self.call = ev["call"].copy()
         self.recorded = ev["recorded"].astype(bool)
@@ -954,29 +974,52 @@ class StreamEvents:
     def values(self, string: bool = True, errors: str = "raise") -> list:
         """What each of these ``receive`` calls returned (``b""`` / ``""`` for "Timed out.") with the
         reference's log lines; errors="return" puts the exception a call raises in the list instead."""
-        return self._receiver._receive_values(self.recorded, self.batch, string, True, errors)
+        out, i, k, n = [], 0, 0, len(self)
+        while i < n:                                            # runs of events whose channels share a Receiver
+            rx, j = self._receivers[self.stream[i]], i + 1
+            while j < n and self._receivers[self.stream[j]] is rx:
+                j += 1
+            out += rx._receive_values(self.recorded[i:j], self.batch, string, True, errors, first=k)
+            k += int(self.recorded[i:j].sum())
+            i = j
+        return out
 
 
 class StreamReceiver:
-    """Continuous reception on S channels at once (``Receiver.open_streams``).  Each channel behaves like
-    one reference Receiver calling ``receive(timeout)`` again and again on its own open input stream
+    """Continuous reception on S channels at once (``open_receive_streams``, ``Receiver.open_streams``).  Each
+    channel behaves like its own reference Receiver calling ``receive(timeout)`` again and again on its own open input stream
     (afskmodem.py:283, 299-319, 402-417).  ``push`` appends the next piece of every channel (any length,
     including 0) and returns the calls that became final with it, already decoded: a call that timed
     out, or a recording whose closing quiet chunk has arrived.  A recording still open stays on the
-    device.  ``finish`` ends the streams (a pending recording ends at its last full chunk, a call that
-    has neither opened nor timed out is dropped); the next push then starts new streams.  Over any way
+    device.  ``finish`` ends the streams of all or some channels (a pending recording ends at its last full
+    chunk, a call that has neither opened nor timed out is dropped); their next push starts new streams, which
+    may be received with other settings.  Over any way
     of cutting a stream into pushes, the events of all pushes plus ``finish`` are ``listen_gate_multi``
     over the whole stream, and their values ``receive_all(stream, keep_timeouts=True)``."""
 
-    def __init__(self, receiver: Receiver, n_streams: int, timeout: float, device: int = 0):
+    def __init__(self, receivers, timeout, device: int = 0):
         _cabi.require_device(device)
-        self.receiver, self.S, self.device = receiver, int(n_streams), device
+        self.receivers, self.S, self.device = tuple(receivers), len(receivers), device
+        self.timeout_frames = _timeout_frames(timeout, self.S)
         self._destroy = _cabi.lib().afsk_rx_streams_destroy
         h = C.c_void_p()
-        _cabi.check(_cabi.lib().afsk_rx_streams_create(device, self.S, receiver._baud, int(np.floor(receiver._amp_start)),
-                                                        _as_int_threshold(receiver._amp_end), int(timeout * 48000), C.byref(h)))
+        b, a0, a1 = self._settings(self.receivers)
+        _cabi.check(_cabi.lib().afsk_rx_streams_create_each(device, self.S, _cabi.ptr(b, C.c_int32), _cabi.ptr(a0, C.c_int32),
+                                                             _cabi.ptr(a1, C.c_int32), _cabi.ptr(self.timeout_frames, C.c_int64),
+                                                             C.byref(h)))
         self._h = h
         self._pinned = None
+
+    @property
+    def receiver(self) -> Receiver:
+        """channel 0's Receiver (every channel's for ``Receiver.open_streams``)"""
+        return self.receivers[0]
+
+    @staticmethod
+    def _settings(receivers):
+        """int32 arrays (baud, amp_start, amp_end) of the receivers, as the gate and the decoder use them"""
+        return (np.array([r._baud for r in receivers], np.int32), np.array([int(np.floor(r._amp_start)) for r in receivers], np.int32),
+                np.array([_as_int_threshold(r._amp_end) for r in receivers], np.int32))
 
     def close(self):
         if getattr(self, "_h", None):
@@ -1032,10 +1075,39 @@ class StreamReceiver:
             raise ValueError(f"samples holds {len(arr)} frames, the offsets need {int(offsets[-1])}")
         return self._run(arr.ctypes.data, 0, offsets, stream)
 
-    def finish(self, stream=None) -> StreamEvents:
+    def finish(self, streams=None, receivers=None, timeout=None, stream=None) -> StreamEvents:
+        """Ends the streams of the channels ``streams`` (default: all) and returns their final calls.  Each of
+        them then starts a new stream at its next push, received by ``receivers`` (one Receiver, or one per
+        listed channel) with ``timeout`` (seconds: one, or one per listed channel); either one left out keeps
+        the channel's current setting.  Other channels are untouched."""
         n = C.c_int64(0)
-        _cabi.check(_cabi.lib().afsk_rx_streams_finish(self._h, C.c_void_p(stream or 0), C.byref(n)))
-        return self._events(n.value)
+        if streams is None and receivers is None and timeout is None:
+            _cabi.check(_cabi.lib().afsk_rx_streams_finish(self._h, C.c_void_p(stream or 0), C.byref(n)))
+            return self._events(n.value)
+        ids = np.arange(self.S, dtype=np.int32) if streams is None else np.ascontiguousarray(streams, dtype=np.int32).reshape(-1)
+        new = None
+        if receivers is not None or timeout is not None:
+            cur = [i if 0 <= i < self.S else 0 for i in ids]      # (the library rejects a channel out of range)
+            if receivers is None:
+                rxs = [self.receivers[i] for i in cur]
+            else:
+                rxs = [receivers] * len(ids) if isinstance(receivers, Receiver) else list(receivers)
+            if len(rxs) != len(ids):
+                raise ValueError(f"finish needs one receiver per listed channel ({len(ids)}), got {len(rxs)}")
+            t = self.timeout_frames[cur] if timeout is None else _timeout_frames(timeout, len(ids))
+            new = (rxs, t) + self._settings(rxs)
+        args = [None] * 4 if new is None else [_cabi.ptr(new[2], C.c_int32), _cabi.ptr(new[3], C.c_int32),
+                                               _cabi.ptr(new[4], C.c_int32), _cabi.ptr(new[1], C.c_int64)]
+        _cabi.check(_cabi.lib().afsk_rx_streams_finish_some(self._h, len(ids), _cabi.ptr(ids, C.c_int32), *args,
+                                                             C.c_void_p(stream or 0), C.byref(n)))
+        ev = self._events(n.value)                               # decoded with the settings of the streams that ended
+        if new is not None:
+            rx = list(self.receivers)
+            for i, r, t in zip(ids, new[0], new[1]):
+                rx[i] = r
+                self.timeout_frames[i] = t
+            self.receivers = tuple(rx)
+        return ev
 
     def _run(self, ptr: int, on_device: int, offsets: np.ndarray, stream) -> StreamEvents:
         n = C.c_int64(0)
@@ -1059,7 +1131,7 @@ class StreamReceiver:
                 C.memmove(blob.ctypes.data, pp, blob.nbytes)
         rec = ev["recorded"] != 0
         out_off = np.append(off[:-1][rec], off[-1]).astype(np.int64)
-        return StreamEvents(self.receiver, ev, RxBatch(res[rec], blob, out_off))
+        return StreamEvents(self.receivers, ev, RxBatch(res[rec], blob, out_off))
 
     def state(self, s: int) -> tuple[int, int, int]:
         """(frames pushed, start of the pending recording or -1, frames retained on the device) of stream s."""
@@ -1259,30 +1331,67 @@ class Transmitter:
     def open_streams(self, n_streams: int, device: int | None = None) -> StreamTransmitter:
         """``transmit`` called again and again on ``n_streams`` open output streams at once, pulled piece by
         piece as the sound card asks for frames (see ``StreamTransmitter``)."""
-        return StreamTransmitter(self, n_streams, self._device if device is None else device)
+        return open_transmit_streams([self] * int(n_streams), self._device if device is None else device)
 
     def transmit(self, data: str | bytes):
         """Live speaker path (:472-478).  Needs an audio device; out of scope — use ``save``."""
         raise RuntimeError("afskmodem_b200 has no live audio output; use save()")
 
 
+def open_transmit_streams(transmitters, device: int | None = None) -> StreamTransmitter:
+    """``transmit`` called again and again on S open output streams at once, channel s by ``transmitters[s]``
+    (the same Transmitter may serve many channels).  ``device`` defaults to the first transmitter's.  See
+    ``StreamTransmitter``."""
+    transmitters = list(transmitters)
+    if not transmitters:
+        raise ValueError("open_transmit_streams needs at least one transmitter")
+    return StreamTransmitter(transmitters, transmitters[0]._device if device is None else device)
+
+
 class StreamTransmitter:
-    """Continuous transmission on S channels at once (``Transmitter.open_streams``).  Each channel behaves like
-    one reference Transmitter whose output stream stays open, calling ``transmit(data)`` again and again
+    """Continuous transmission on S channels at once (``open_transmit_streams``, ``Transmitter.open_streams``).
+    Each channel behaves like its own reference Transmitter whose output stream stays open, calling ``transmit(data)`` again and again
     (afskmodem.py:472-478: ``SoundOutput.play`` writes what ``save`` writes, :247-252).  The channels share one
     timeline, pulled ``n`` frames at a time like the periods of a multi-channel sound card.  ``send`` queues
     messages; one starts at ``max(frames pulled, end of its channel's last message)`` and its frames are exactly
     what ``save`` writes for it; every other frame is silence (0).  Only payload bytes are kept on the device:
-    each ``pull`` synthesizes its window from them."""
+    each ``pull`` synthesizes its window from them.  ``configure`` gives channels other settings for the messages
+    sent to them afterwards."""
 
-    def __init__(self, transmitter: Transmitter, n_streams: int, device: int = 0):
+    def __init__(self, transmitters, device: int = 0):
         _cabi.require_device(device)
-        self.transmitter, self.S, self.device = transmitter, int(n_streams), device
+        self.transmitters, self.S, self.device = tuple(transmitters), len(transmitters), device
         self._destroy = _cabi.lib().afsk_tx_streams_destroy
         h = C.c_void_p()
-        _cabi.check(_cabi.lib().afsk_tx_streams_create(device, self.S, transmitter._baud, transmitter._ts_cycles, C.byref(h)))
+        b, t = self._settings(self.transmitters)
+        _cabi.check(_cabi.lib().afsk_tx_streams_create_each(device, self.S, _cabi.ptr(b, C.c_int32), _cabi.ptr(t, C.c_int64),
+                                                             C.byref(h)))
         self._h = h
         self._pinned = None
+
+    @property
+    def transmitter(self) -> Transmitter:
+        """channel 0's Transmitter (every channel's for ``Transmitter.open_streams``)"""
+        return self.transmitters[0]
+
+    @staticmethod
+    def _settings(transmitters):
+        return (np.array([t._baud for t in transmitters], np.int32), np.array([t._ts_cycles for t in transmitters], np.int64))
+
+    def configure(self, streams, transmitters) -> None:
+        """Messages sent from now on to channels ``streams`` use ``transmitters`` (one Transmitter, or one per listed
+        channel); messages already queued keep their settings."""
+        ids = np.ascontiguousarray(streams, dtype=np.int32).reshape(-1)
+        txs = [transmitters] * len(ids) if isinstance(transmitters, Transmitter) else list(transmitters)
+        if len(txs) != len(ids):
+            raise ValueError(f"configure needs one transmitter per listed channel ({len(ids)}), got {len(txs)}")
+        b, t = self._settings(txs)
+        _cabi.check(_cabi.lib().afsk_tx_streams_configure(self._h, len(ids), _cabi.ptr(ids, C.c_int32), _cabi.ptr(b, C.c_int32),
+                                                           _cabi.ptr(t, C.c_int64)))
+        tx = list(self.transmitters)
+        for i, x in zip(ids, txs):
+            tx[i] = x
+        self.transmitters = tuple(tx)
 
     def close(self):
         if getattr(self, "_h", None):

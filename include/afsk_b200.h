@@ -206,9 +206,14 @@ typedef struct AfskRxStreamEvent {      /* 32 bytes, one per final receive() cal
     int64_t call;                       /* index of the call on its channel */
     int64_t start, end;                 /* stream frames of the recording */
 } AfskRxStreamEvent;
-/* baud / amp_end as for afsk_rx_plan_create, amp_start / timeout_frames as for afsk_rx_gate_multi */
+/* channel s is a Receiver(h_baud[s], h_amp_start[s], h_amp_end[s]) calling receive() with a timeout of
+ * h_timeout_frames[s] frames (>= 0): baud / amp_end as for afsk_rx_plan_create, amp_start / timeout_frames as for
+ * afsk_rx_gate_multi.  AFSK_E_BAUD where the reference constructor raises (afsk_last_error names the channel). */
+int afsk_rx_streams_create_each(int device, int S, const int32_t *h_baud, const int32_t *h_amp_start,
+                                const int32_t *h_amp_end, const int64_t *h_timeout_frames, AfskRxStreams **h);
+/* the same settings on every channel (a timeout below 0 counts as 0) */
 int afsk_rx_streams_create(int device, int S, int baud, int amp_start, int amp_end, int64_t timeout_frames,
-                           AfskRxStreams **h);     /* AFSK_E_BAUD where the reference constructor raises */
+                           AfskRxStreams **h);
 /* samples: the S pieces concatenated, h_offsets[S+1] (CSR, any length including 0); on_device != 0: a
  * device pointer (16-byte aligned, allocation extending to the next 16-byte boundary past h_offsets[S]),
  * else host memory (pinned recommended).  Synchronizes `stream`.  A bad argument returns AFSK_E_ARG and
@@ -216,9 +221,16 @@ int afsk_rx_streams_create(int device, int S, int baud, int amp_start, int amp_e
  * can only be destroyed. */
 int afsk_rx_streams_push(AfskRxStreams *h, const int16_t *samples, int on_device, const int64_t *h_offsets,
                          void *stream, int64_t *n_events);
-/* ends every stream (finite-stream conventions of afsk_rx_gate_multi: a pending recording ends at the
- * last full chunk, a call that has neither opened nor timed out is dropped, a partial chunk is ignored);
- * the next push is frame 0 of new streams */
+/* ends the streams of the n distinct channels h_streams[n] (finite-stream conventions of afsk_rx_gate_multi: a
+ * pending recording ends at the last full chunk, a call that has neither opened nor timed out is dropped, a
+ * partial chunk is ignored) and returns their final calls.  Each listed channel's next push is frame 0 of a new
+ * stream, whose calls count from 0; with the four settings arrays given (one entry per listed channel, as for
+ * afsk_rx_streams_create_each) that stream is received with those settings, with all four NULL with the old
+ * ones.  Other channels are untouched.  Synchronizes `stream`; errors as for afsk_rx_streams_push. */
+int afsk_rx_streams_finish_some(AfskRxStreams *h, int n, const int32_t *h_streams, const int32_t *h_baud,
+                                const int32_t *h_amp_start, const int32_t *h_amp_end, const int64_t *h_timeout_frames,
+                                void *stream, int64_t *n_events);
+/* afsk_rx_streams_finish_some over every channel, settings kept */
 int afsk_rx_streams_finish(AfskRxStreams *h, void *stream, int64_t *n_events);
 /* host arrays owned by the handle, valid until the next push / finish: n_events events ordered by
  * (stream, call); per event an AfskRxResult (zero with clock = train_end = -1 for a timed-out call) and
@@ -263,8 +275,16 @@ int afsk_tx_synth_host(int device, const uint8_t *h_payload, const int64_t *h_pa
  * unequal tone lengths, each message's codeword start table); every pull synthesizes its window from them.
  */
 typedef struct AfskTxStreams AfskTxStreams;
-/* baud / ts_cycles as for afsk_tx_plan_create; AFSK_E_BAUD where the reference constructor raises */
+/* channel s is a Transmitter with h_baud[s] / h_ts_cycles[s] (as for afsk_tx_plan_create); AFSK_E_BAUD where the
+ * reference constructor raises (afsk_last_error names the channel) */
+int afsk_tx_streams_create_each(int device, int S, const int32_t *h_baud, const int64_t *h_ts_cycles, AfskTxStreams **h);
+/* the same settings on every channel */
 int afsk_tx_streams_create(int device, int S, int baud, int64_t ts_cycles, AfskTxStreams **h);
+/* messages sent from now on to the n distinct channels h_streams[n] use h_baud[i] / h_ts_cycles[i]; messages
+ * already queued keep theirs.  A bad argument returns AFSK_E_ARG (AFSK_E_BAUD for a baud the reference
+ * constructor rejects) and changes nothing. */
+int afsk_tx_streams_configure(AfskTxStreams *h, int n, const int32_t *h_streams, const int32_t *h_baud,
+                              const int64_t *h_ts_cycles);
 /* queues n messages (message i = h_payload[h_pay_off[i] .. h_pay_off[i+1]) on channel h_stream[i], in order)
  * and returns their timeline frames [h_start[i], h_end[i]).  Synchronous. */
 int afsk_tx_streams_send(AfskTxStreams *h, int n, const int32_t *h_stream, const int64_t *h_pay_off,

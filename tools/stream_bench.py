@@ -1,13 +1,18 @@
 """Streaming receiver throughput: S channels of 1200-baud transmissions separated by silence, pushed
 piece by piece through Receiver.open_streams, host-pinned or device-resident input.
 
-    python tools/stream_bench.py [--S 1,64,4096] [--piece 2048,48000] [--seconds 8] [--out FILE]
+    python tools/stream_bench.py [--S 1,64,4096] [--piece 2048,48000] [--seconds 8] [--mix] [--out FILE]
 
 Channel s hears one long traffic recording from frame s * 12345 on, so recordings land at different
 places on every channel.  Each configuration runs its push sequence twice on one receiver (finish in
 between) and times the second: host wall time of every push, which ends in a synchronize.  Beside it,
 receive_all and listen_gate_multi over whole streams of the same traffic (one stream per call, the
-only way they run) on the same card.  Card name and power limit are read in the same run."""
+only way they run) on the same card.  Card name and power limit are read in the same run.
+
+--mix splits the channels into six equal groups at 300, 600, 1200, 2400, 4000 and 6000 baud, each hearing
+traffic at its own baud, and within a group cycles through the three (amp_start, amp_end) threshold pairs of
+the c5 corpus; the handle is then opened with open_receive_streams.  A push then decodes one group per distinct
+baud among its final recordings."""
 from __future__ import annotations
 
 import argparse
@@ -24,6 +29,8 @@ import afskmodem_b200 as A  # noqa: E402
 from afskmodem_b200 import _cabi  # noqa: E402
 
 SHIFT = 12345
+MIX_BAUDS = [300, 600, 1200, 2400, 4000, 6000]
+MIX_THRESHOLDS = [(18000, 14000), (14000, 11000), (9000, 8000)]
 
 
 def card():
@@ -32,9 +39,9 @@ def card():
     return q.stdout.strip().splitlines()[0] if q.returncode == 0 and q.stdout.strip() else "unknown"
 
 
-def traffic(n: int, rng) -> np.ndarray:
-    """1200-baud transmissions (10-60 byte payloads, 0.1 s training) separated by 0.2-1.5 s of silence, light noise"""
-    tx = A.Transmitter(1200, 0.1)
+def traffic(n: int, rng, baud: int = 1200) -> np.ndarray:
+    """transmissions (10-60 byte payloads, 0.1 s training) separated by 0.2-1.5 s of silence, light noise"""
+    tx = A.Transmitter(baud, 0.1)
     msgs = [rng.integers(0, 256, size=int(rng.integers(10, 61)), dtype=np.uint8).tobytes() for _ in range(64)]
     batch = tx.encode_batch(msgs)
     parts, total = [], 0
@@ -47,26 +54,42 @@ def traffic(n: int, rng) -> np.ndarray:
     return np.clip(np.round(x), -32768, 32767).astype(np.int16)
 
 
-def run_config(base: np.ndarray, d_base, S: int, piece: int, T: int, device: bool, timeout: float):
+def mix_groups(S: int):
+    """--mix: (baud, first channel, channels) of the six groups"""
+    cuts = [S * g // len(MIX_BAUDS) for g in range(len(MIX_BAUDS) + 1)]
+    return [(b, cuts[g], cuts[g + 1] - cuts[g]) for g, b in enumerate(MIX_BAUDS)]
+
+
+def run_config(base, d_base, S: int, piece: int, T: int, device: bool, timeout: float, mix: bool = False):
+    """base / d_base: one traffic stream, or with mix one per baud of MIX_BAUDS"""
     import torch
     n_push = T // piece
     offsets = np.arange(S + 1, dtype=np.int64) * piece
-    rx = A.Receiver(1200)
     pinned = _cabi.PinnedArray((S * piece + 8,), np.int16)
-    out = {"S": S, "piece": piece, "input": "device" if device else "host-pinned", "pushes": n_push}
-    with rx.open_streams(S, timeout) as st:
+    out = {"S": S, "piece": piece, "input": "device" if device else "host-pinned", "pushes": n_push, "mix": mix}
+    if mix:
+        groups = mix_groups(S)
+        rxs = [A.Receiver(b, *MIX_THRESHOLDS[k % 3]) for b, _, n in groups for k in range(n)]
+        st = A.open_receive_streams(rxs, timeout)
+    else:
+        groups = [(1200, 0, S)]
+        st = A.Receiver(1200).open_streams(S, timeout)
+        base, d_base = [base], [d_base]
+    with st:
         for rep in range(2):
             c0 = st.counters()
             times, n_ev, n_rec, rec_frames, n_dec = [], 0, 0, 0, 0
             for i in range(n_push):
                 if device:
-                    t = torch.as_strided(d_base, (S, piece), (SHIFT, 1), i * piece).contiguous().view(-1)
+                    t = torch.cat([torch.as_strided(d_base[g], (n, piece), (SHIFT, 1), i * piece).reshape(-1)
+                                   for g, (_, _, n) in enumerate(groups)])
                     torch.cuda.synchronize()
                     t0 = time.perf_counter()
                     ev = st.push(t, offsets)
                 else:
-                    np.copyto(pinned.array[:S * piece].reshape(S, piece),
-                              np.lib.stride_tricks.as_strided(base[i * piece:], shape=(S, piece), strides=(SHIFT * 2, 2)))
+                    for g, (_, c, n) in enumerate(groups):
+                        np.copyto(pinned.array[c * piece:(c + n) * piece].reshape(n, piece),
+                                  np.lib.stride_tricks.as_strided(base[g][i * piece:], shape=(n, piece), strides=(SHIFT * 2, 2)))
                     t0 = time.perf_counter()
                     ev = st.push(pinned.array, offsets)
                 times.append(time.perf_counter() - t0)
@@ -157,6 +180,7 @@ def main():
     ap.add_argument("--seconds", type=float, default=8.0)
     ap.add_argument("--timeout", type=float, default=1.0)
     ap.add_argument("--input", default="host,device")
+    ap.add_argument("--mix", action="store_true", help="six bauds and three threshold pairs across the channels")
     ap.add_argument("--out", default=None)
     ap.add_argument("--no-profile", action="store_true", help="skip the profiled run of the largest device configuration")
     a = ap.parse_args()
@@ -167,22 +191,29 @@ def main():
     pieces = [int(v) for v in a.piece.split(",")]
     T = int(a.seconds * 48000)
     rng = np.random.default_rng(0)
-    base = traffic(max(Ss) * SHIFT + T + max(pieces), rng)
-    d_base = torch.from_numpy(base).cuda()
+    n = max(Ss) * SHIFT + T + max(pieces)
+    if a.mix:
+        bases = [traffic(n, rng, b) for b in MIX_BAUDS]
+        d_bases = [torch.from_numpy(x).cuda() for x in bases]
+    else:
+        base = traffic(n, rng)
+        d_base = torch.from_numpy(base).cuda()
     res = {"card": card(), "torch_device": torch.cuda.get_device_name(0), "seconds_per_channel": a.seconds,
-           "timeout_s": a.timeout, "configs": []}
+           "timeout_s": a.timeout, "mix": a.mix, "configs": []}
     for S in Ss:
         for piece in pieces:
             for inp in a.input.split(","):
-                r = run_config(base, d_base, S, piece, T, inp == "device", a.timeout)
+                r = run_config(bases, d_bases, S, piece, T, inp == "device", a.timeout, True) if a.mix else \
+                    run_config(base, d_base, S, piece, T, inp == "device", a.timeout)
                 print(json.dumps(r), flush=True)
                 res["configs"].append(r)
-    if not a.no_profile:
+    if not a.mix and not a.no_profile:                    # the profile and whole-stream lines use uniform traffic
         res["profile"] = profile_config(d_base, max(Ss), max(pieces), T, a.timeout,
                                         os.path.dirname(os.path.abspath(a.out)) if a.out else None)
         print(json.dumps({k: v for k, v in res["profile"].items() if k != "by_kernel_or_copy"}), flush=True)
-    res["whole_stream"] = whole_stream_reference(base, T, 16, a.timeout)
-    print(json.dumps(res["whole_stream"]), flush=True)
+    if not a.mix:
+        res["whole_stream"] = whole_stream_reference(base, T, 16, a.timeout)
+        print(json.dumps(res["whole_stream"]), flush=True)
     res["card_after"] = card()
     if a.out:
         os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)

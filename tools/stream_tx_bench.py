@@ -1,7 +1,7 @@
 """Streaming transmitter throughput: S channels of 1200-baud messages separated by silence, pulled window by window
 through Transmitter.open_streams into a CUDA tensor or a host (pinned) array.
 
-    python tools/stream_tx_bench.py [--S 1,64,4096] [--pull 2048,48000] [--seconds 8] [--out FILE]
+    python tools/stream_tx_bench.py [--S 1,64,4096] [--pull 2048,48000] [--seconds 8] [--mix] [--out FILE]
 
 Every channel sends a 10-60 byte message (0.1 s training) whenever its previous one has ended and a random gap of
 up to twice a message's mean length has passed, so a channel is busy about half the time; the sends due inside a
@@ -9,7 +9,10 @@ window go in one send() call before its pull.  Each configuration runs its seque
 times the second: host wall time of every pull (it ends in a synchronize) and of every send.  A separate
 torch.profiler run of the largest device-output configuration gives k_tx_window's kernel time (bytes written per
 second of kernel time, against the 7.7 TB/s of HBM3e on a B200's data sheet) and the share of a pull the GPU is busy.
-Card name and power limit are read in the same run."""
+Card name and power limit are read in the same run.
+
+--mix splits the channels into six equal groups at 300, 600, 1200, 2400, 4000 and 6000 baud (open_transmit_streams),
+each sending messages of its own length at the same duty."""
 from __future__ import annotations
 
 import argparse
@@ -26,6 +29,7 @@ import afskmodem_b200 as A  # noqa: E402
 from afskmodem_b200 import _cabi  # noqa: E402
 
 HBM_TBS = 7.7
+MIX_BAUDS = [300, 600, 1200, 2400, 4000, 6000]
 
 
 def card():
@@ -37,12 +41,13 @@ def card():
 class Traffic:
     """per channel: the next frame at which it sends, and a pool of payloads"""
 
-    def __init__(self, S: int, baud: int, seed: int):
+    def __init__(self, S: int, baud, seed: int):
+        """baud: one for every channel, or an array of S (mean message length per channel)"""
         self.rng = np.random.default_rng(seed)
         self.S = S
         self.msgs = [self.rng.integers(0, 256, size=int(self.rng.integers(10, 61)), dtype=np.uint8).tobytes() for _ in range(256)]
         bf = 48000 // baud
-        self.mean_len = int(0.1 * baud) * bf + 5 * bf + 4800 + 35 * 14 * bf
+        self.mean_len = (baud // 10) * bf + 5 * bf + 4800 + 35 * 14 * bf
         self.next_at = self.rng.integers(0, 2 * self.mean_len, S).astype(np.int64)
 
     def due(self, P: int, n: int):
@@ -50,7 +55,8 @@ class Traffic:
         return s.astype(np.int32), [self.msgs[i] for i in self.rng.integers(0, len(self.msgs), len(s))]
 
     def sent(self, streams, end):
-        self.next_at[streams] = end + self.rng.integers(0, 2 * self.mean_len, len(streams))
+        hi = 2 * (self.mean_len if np.ndim(self.mean_len) == 0 else self.mean_len[streams])
+        self.next_at[streams] = end + self.rng.integers(0, hi, len(streams))
 
 
 def run_sequence(st, S, n, n_pull, baud, seed, out_t=None):
@@ -74,13 +80,23 @@ def run_sequence(st, S, n, n_pull, baud, seed, out_t=None):
     return np.array(t_pull), np.array(t_send), busy
 
 
-def run_config(S: int, n: int, T: int, device: bool, baud: int):
+def mix_bauds(S: int) -> np.ndarray:
+    """--mix: channel s's baud (six equal groups)"""
+    return np.array([MIX_BAUDS[s * len(MIX_BAUDS) // S] for s in range(S)], np.int64)
+
+
+def run_config(S: int, n: int, T: int, device: bool, baud):
+    """baud: one for every channel, or "mix" (mix_bauds)"""
     import torch
     n_pull = max(T // n, 1)
     out_t = torch.empty(S * n, dtype=torch.int16, device="cuda") if device else None
-    tx = A.Transmitter(baud, 0.1)
     res = {"S": S, "pull": n, "baud": baud, "output": "device" if device else "host-pinned", "pulls": n_pull}
-    with tx.open_streams(S) as st:
+    if baud == "mix":
+        baud = mix_bauds(S)
+        st = A.open_transmit_streams([A.Transmitter(int(b), 0.1) for b in baud])
+    else:
+        st = A.Transmitter(baud, 0.1).open_streams(S)
+    with st:
         run_sequence(st, S, n, n_pull, baud, 1, out_t)                # warm-up: same shapes
         c0 = st.counters()
         tp, ts, busy = run_sequence(st, S, n, n_pull, baud, 2, out_t)
@@ -144,6 +160,7 @@ def main():
     ap.add_argument("--pull", default="2048,48000")
     ap.add_argument("--seconds", type=float, default=8.0)
     ap.add_argument("--output", default="device,host")
+    ap.add_argument("--mix", action="store_true", help="six bauds across the channels")
     ap.add_argument("--out", default=None)
     ap.add_argument("--no-profile", action="store_true", help="skip the profiled run of the largest device configuration")
     a = ap.parse_args()
@@ -153,14 +170,16 @@ def main():
     Ss = [int(v) for v in a.S.split(",")]
     pulls = [int(v) for v in a.pull.split(",")]
     T = int(a.seconds * 48000)
-    res = {"card": card(), "torch_device": torch.cuda.get_device_name(0), "seconds_per_channel": a.seconds, "configs": []}
-    lines = [(S, n, o == "device", 1200) for S in Ss for n in pulls for o in a.output.split(",")]
-    lines.append((max(Ss), max(pulls), True, 4800))
+    res = {"card": card(), "torch_device": torch.cuda.get_device_name(0), "seconds_per_channel": a.seconds, "mix": a.mix,
+           "configs": []}
+    lines = [(S, n, o == "device", "mix" if a.mix else 1200) for S in Ss for n in pulls for o in a.output.split(",")]
+    if not a.mix:
+        lines.append((max(Ss), max(pulls), True, 4800))
     for S, n, dev, baud in lines:
         r = run_config(S, n, T, dev, baud)
         print(json.dumps(r), flush=True)
         res["configs"].append(r)
-    if not a.no_profile:
+    if not a.mix and not a.no_profile:
         res["profile"] = profile_config(max(Ss), max(pulls), T, 1200, os.path.dirname(os.path.abspath(a.out)) if a.out else None)
         print(json.dumps({k: v for k, v in res["profile"].items() if k != "by_kernel_or_copy"}), flush=True)
     res["card_after"] = card()
