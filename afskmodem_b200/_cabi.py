@@ -33,7 +33,7 @@ SYMBOLS = [
     "afsk_rx_streams_counters", "afsk_rx_streams_destroy", "afsk_tx_streams_create", "afsk_tx_streams_send",
     "afsk_tx_streams_pull", "afsk_tx_streams_state", "afsk_tx_streams_arena_bytes", "afsk_tx_streams_counters",
     "afsk_tx_streams_destroy", "afsk_rx_streams_create_each", "afsk_rx_streams_finish_some", "afsk_tx_streams_create_each",
-    "afsk_tx_streams_configure",
+    "afsk_tx_streams_configure", "afsk_rx_streams_push_interleaved", "afsk_tx_streams_pull_interleaved",
 ]
 
 
@@ -105,6 +105,7 @@ def lib():
     L.afsk_rx_gate_multi.argtypes = [C.c_int, vp, i64p, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_int, vp, vp, vp]
     L.afsk_rx_streams_create.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int64, C.POINTER(vp)]
     L.afsk_rx_streams_push.argtypes = [vp, vp, C.c_int, i64p, vp, i64p]
+    L.afsk_rx_streams_push_interleaved.argtypes = [vp, vp, C.c_int, C.c_int64, vp, i64p]
     L.afsk_rx_streams_create_each.argtypes = [C.c_int, C.c_int, i32p, i32p, i32p, i64p, C.POINTER(vp)]
     L.afsk_rx_streams_finish.argtypes = [vp, vp, i64p]
     L.afsk_rx_streams_finish_some.argtypes = [vp, C.c_int, i32p, i32p, i32p, i32p, i64p, vp, i64p]
@@ -125,6 +126,7 @@ def lib():
     L.afsk_tx_streams_configure.argtypes = [vp, C.c_int, i32p, i32p, i64p]
     L.afsk_tx_streams_send.argtypes = [vp, C.c_int, i32p, i64p, u8p, i64p, i64p]
     L.afsk_tx_streams_pull.argtypes = [vp, C.c_int64, vp, C.c_int, vp]
+    L.afsk_tx_streams_pull_interleaved.argtypes = [vp, C.c_int64, vp, C.c_int, vp]
     L.afsk_tx_streams_state.argtypes = [vp, C.c_int, i64p, i64p, i64p]
     L.afsk_tx_streams_arena_bytes.argtypes = [vp, i64p]
     L.afsk_tx_streams_counters.argtypes = [vp, i64p, i64p, i64p]

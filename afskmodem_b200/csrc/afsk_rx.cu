@@ -2236,6 +2236,78 @@ __global__ void __launch_bounds__(kCopyThreads) k_stream_copy(const int16_t *__r
     }
 }
 
+// Appends one interleaved piece (src[f * S + s] = frame f of channel s, n frames, 16-byte aligned) to every
+// channel's slot: frame f of channel s goes to dst[seg[s].dst + f], an arbitrary alignment per channel.
+// A CTA owns kDiC consecutive channels x kDiF destination frames, in destination-vector coordinates: tile fb
+// writes channel s's vectors (seg[s].dst >> 3) + fb * kDiF / 8 + j, j < kDiF / 8, which hold frames
+// fb * kDiF - a + 8j .. + 7 with a = seg[s].dst & 7.  So the tile reads frame rows fb * kDiF - 7 .. fb * kDiF +
+// kDiF - 1 (a halo of 7 frames in front), each row's kDiC channels as 128 contiguous bytes: eight lanes per row,
+// aligned 128-bit loads realigned with funnel shifts when S % 8 != 0.  Each frame lands in shared memory at its
+// channel's destination position, so every thread then writes aligned 16-byte vectors of one channel, sixteen
+// lanes one 256-byte run; only a channel's head and tail vectors are written frame by frame.  64 x 128 keeps a
+// row load at one 128-byte line and the tile at 17 KB (several CTAs per SM); the halo costs 7 / 128 extra reads.
+// Shared rows are channels in the order (s & 7) * 8 + (s >> 3), 136 samples apart (68 words = 4 banks): the
+// eight lanes of a row load write eight consecutive rows, in disjoint bank groups.
+constexpr int kDiC = 64, kDiF = 128, kDiHalo = 7, kDiThreads = 256, kDiStride = kDiF + 8;
+
+__device__ __forceinline__ int di_row(int c) { return (c & 7) * 8 + (c >> 3); }
+
+__global__ void __launch_bounds__(kDiThreads) k_stream_deinterleave(const int16_t *__restrict__ src, int16_t *__restrict__ dst,
+                                                                     const CopySeg *__restrict__ seg, int S, long long n,
+                                                                     int cblocks)
+{
+    __shared__ __align__(16) int16_t T[kDiC * kDiStride];
+    __shared__ long long sdst[kDiC];
+    const int c0 = (int)(blockIdx.x % cblocks) * kDiC, nc = min(kDiC, S - c0);
+    const long long F0 = (long long)(blockIdx.x / cblocks) * kDiF;
+    if (threadIdx.x < nc) sdst[threadIdx.x] = seg[c0 + threadIdx.x].dst;
+    __syncthreads();
+    const long long f_lo = max(F0 - kDiHalo, 0LL), f_hi = min(F0 + kDiF, n);
+    const int nq = (nc + 7) >> 3;
+    for (int i = threadIdx.x; i < (int)(f_hi - f_lo) * 8; i += kDiThreads) {
+        const int q = i & 7;
+        if (q >= nq) continue;
+        const long long f = f_lo + (i >> 3), row_end = f * S + c0 + nc;
+        const long long qs = f * S + c0 + 8 * q;                  // first sample of channels c0 + 8q ..
+        const long long sv = qs >> 3;
+        const int k = (int)(qs & 7);
+        const uint4 lo = ld_nc_v4(src + sv * 8);                  // holds qs, inside the row
+        const uint4 hi = k && (sv + 1) * 8 < row_end ? ld_nc_v4(src + (sv + 1) * 8) : make_uint4(0, 0, 0, 0);
+        const uint32_t w[8] = {lo.x, lo.y, lo.z, lo.w, hi.x, hi.y, hi.z, hi.w};
+        const int j = k >> 1;
+        uint32_t o[4];
+#pragma unroll
+        for (int t = 0; t < 4; t++) {                             // samples k .. k + 7 of the 16 loaded
+            const uint32_t x0 = j == 0 ? w[t] : j == 1 ? w[t + 1] : j == 2 ? w[t + 2] : w[t + 3];
+            const uint32_t x1 = j == 0 ? w[t + 1] : j == 1 ? w[t + 2] : j == 2 ? w[t + 3] : w[t + 4];
+            o[t] = (k & 1) ? __funnelshift_r(x0, x1, 16) : x0;
+        }
+#pragma unroll
+        for (int e = 0; e < 8; e++) {
+            const int c = 8 * q + e;
+            if (c >= nc) break;
+            const long long p = f - F0 + (sdst[c] & 7);           // destination position in the tile
+            if (p >= 0 && p < kDiF) T[di_row(c) * kDiStride + p] = (int16_t)(o[e >> 1] >> (16 * (e & 1)));
+        }
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < nc * (kDiF / 8); i += kDiThreads) {
+        const int j = i % (kDiF / 8), c = i / (kDiF / 8);
+        const long long g = sdst[c];
+        const long long d0 = ((g >> 3) * 8) + F0 + 8 * j, f0 = d0 - g;   // the vector and its first frame
+        if (f0 >= n) continue;
+        const uint4 v = *reinterpret_cast<const uint4 *>(T + di_row(c) * kDiStride + 8 * j);
+        if (f0 >= 0 && f0 + 8 <= n) {
+            *reinterpret_cast<uint4 *>(dst + d0) = v;
+        } else {
+            const uint32_t o[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+            for (int e = 0; e < 8; e++)
+                if (f0 + e >= 0 && f0 + e < n) dst[d0 + e] = (int16_t)(o[e >> 1] >> (16 * (e & 1)));
+        }
+    }
+}
+
 struct Group {
     int bf = 0, tpw_log2 = 0, seg = 0, nv = 0, nt = 0, merge = 0, wt = 0, nsub = 1, stage_bytes = 0, stages = 0;
     int small_wpt = 0;            // > 0: k_demod_lane<bf/8, small_wpt>
@@ -3224,21 +3296,23 @@ static int streams_fail(cudaError_t e)
 }
 
 // one push (fin == NULL) or the end of the streams s with fin[s] != 0 (no samples); then, when new_baud is
-// given, every channel's settings become new_baud[s] / new_params[s] for its next stream
-static int streams_run(AfskRxStreams *H, const int16_t *samples, int on_device, const int64_t *off, cudaStream_t st,
+// given, every channel's settings become new_baud[s] / new_params[s] for its next stream.  A push is planar
+// (inter < 0: channel s's piece is samples[off[s] .. off[s + 1])) or interleaved (inter frames of every
+// channel, samples[f * S + s] = frame f of channel s; off unused)
+static int streams_run(AfskRxStreams *H, const int16_t *samples, int on_device, const int64_t *off, int64_t inter, cudaStream_t st,
                        const uint8_t *fin, const int32_t *new_baud, const GateParams *new_params, int64_t *n_events)
 {
     const int S = H->S;
-    const bool finish = fin != nullptr;
+    const bool finish = fin != nullptr, interleaved = inter >= 0;
     const int64_t C = AFSK_GATE_CHUNK;
-    auto piece = [&](int s) -> int64_t { return finish ? 0 : off[s + 1] - off[s]; };
+    auto piece = [&](int s) -> int64_t { return finish ? 0 : interleaved ? inter : off[s + 1] - off[s]; };
     int64_t nch = 0;                               // chunks completed by this push
     for (int s = 0; s < S; s++) {
         H->np[s] = H->pushed[s] + piece(s);
         nch += H->np[s] / C - H->pushed[s] / C;
     }
     // buffers first: a failed allocation leaves the channels as they were
-    const int64_t in_samples = finish ? 0 : off[S] - off[0];
+    const int64_t in_samples = finish ? 0 : interleaved ? inter * S : off[S] - off[0];
     cudaError_t e = cudaSuccess;
     if (!on_device && in_samples > 0) e = grow_device((void **)&H->d_stage, &H->stage_cap, (size_t)in_samples * 2 + 32);
     if (e == cudaSuccess) e = grow_device((void **)&H->d_amp, &H->amp_cap, sizeof(int32_t) * (size_t)nch);
@@ -3305,8 +3379,9 @@ static int streams_run(AfskRxStreams *H, const int16_t *samples, int on_device, 
     for (int i = 0; i < nmov; i++) H->n_moved += seg_mov[i].len;
     first[0] = 0;
     for (int s = 0; s < S; s++) {
-        add_seg(seg_app, tf_app, napp, finish ? 0 : off[s] - (on_device ? 0 : off[0]), H->slot_off[s] + H->pushed[s] - H->slot_base[s],
-                piece(s));
+        // (interleaved: src is the channel's column, which only a one-channel push reads as a k_stream_copy segment)
+        const int64_t src = finish ? 0 : interleaved ? s : off[s] - (on_device ? 0 : off[0]);
+        add_seg(seg_app, tf_app, napp, src, H->slot_off[s] + H->pushed[s] - H->slot_base[s], piece(s));
         const int64_t c_old = H->pushed[s] / C;
         first[s + 1] = first[s] + H->np[s] / C - c_old;
         amp_off[s] = H->slot_off[s] + c_old * C - H->slot_base[s];
@@ -3326,11 +3401,18 @@ static int streams_run(AfskRxStreams *H, const int16_t *samples, int on_device, 
     if (napp > 0) {
         const int16_t *src = samples;
         if (!on_device) {
-            AFSK_CUDA(cudaMemcpyAsync(H->d_stage, samples + off[0], (size_t)in_samples * 2, cudaMemcpyHostToDevice, st));
+            AFSK_CUDA(cudaMemcpyAsync(H->d_stage, samples + (interleaved ? 0 : off[0]), (size_t)in_samples * 2, cudaMemcpyHostToDevice, st));
             src = H->d_stage;
         }
-        k_stream_copy<<<(unsigned)tf_app[napp], kCopyThreads, 0, st>>>(src, x, reinterpret_cast<const CopySeg *>(dd + H->o_seg_app),
-                                                                      reinterpret_cast<const int64_t *>(dd + H->o_tf_app), napp);
+        if (interleaved && S > 1) {
+            const int cblocks = (S + kDiC - 1) / kDiC;
+            const int64_t ftiles = (inter + kDiF + kDiHalo - 1) / kDiF;
+            k_stream_deinterleave<<<(unsigned)(cblocks * ftiles), kDiThreads, 0, st>>>(
+                src, x, reinterpret_cast<const CopySeg *>(dd + H->o_seg_app), S, inter, cblocks);
+        } else {
+            k_stream_copy<<<(unsigned)tf_app[napp], kCopyThreads, 0, st>>>(src, x, reinterpret_cast<const CopySeg *>(dd + H->o_seg_app),
+                                                                          reinterpret_cast<const int64_t *>(dd + H->o_tf_app), napp);
+        }
         H->n_launches++;
     }
     const int64_t *d_first = reinterpret_cast<const int64_t *>(dd + H->o_first);
@@ -3425,13 +3507,13 @@ static int streams_run(AfskRxStreams *H, const int16_t *samples, int on_device, 
 
 // a push or finish with valid arguments: any failure may leave the channels between two states, so the
 // handle refuses every later push / finish
-static int streams_call(AfskRxStreams *H, const int16_t *samples, int on_device, const int64_t *off, void *stream,
+static int streams_call(AfskRxStreams *H, const int16_t *samples, int on_device, const int64_t *off, int64_t inter, void *stream,
                         const uint8_t *fin, const int32_t *new_baud, const GateParams *new_params, int64_t *n_events)
 {
     if (H->failed) { afsk_set_error("afsk_rx_streams: an earlier push failed; destroy the handle"); return AFSK_E_CUDA; }
     AfskDeviceGuard guard(H->device);
     if (!guard.ok) { afsk_set_error("cannot select device %d", H->device); return AFSK_E_CUDA; }
-    const int rc = streams_run(H, samples, on_device, off, (cudaStream_t)stream, fin, new_baud, new_params, n_events);
+    const int rc = streams_run(H, samples, on_device, off, inter, (cudaStream_t)stream, fin, new_baud, new_params, n_events);
     if (rc != AFSK_OK) {
         H->failed = true;
         H->ev.clear(); H->res.clear(); H->payload.clear(); H->payload_off.clear();
@@ -3515,7 +3597,24 @@ int afsk_rx_streams_push(AfskRxStreams *H, const int16_t *samples, int on_device
         afsk_set_error("afsk_rx_streams_push: device samples must be 16-byte aligned");
         return AFSK_E_ARG;
     }
-    return streams_call(H, samples, on_device, h_offsets, stream, nullptr, nullptr, nullptr, n_events);
+    return streams_call(H, samples, on_device, h_offsets, -1, stream, nullptr, nullptr, nullptr, n_events);
+}
+
+int afsk_rx_streams_push_interleaved(AfskRxStreams *H, const int16_t *frames, int on_device, int64_t n_frames, void *stream,
+                                     int64_t *n_events)
+{
+    const char *fn = "afsk_rx_streams_push_interleaved";
+    if (!H || !n_events || n_frames < 0 || (n_frames > 0 && !frames)) { afsk_set_error("%s: bad argument", fn); return AFSK_E_ARG; }
+    if (n_frames > (INT64_MAX / 16) / H->S) { afsk_set_error("%s: S * n_frames overflows", fn); return AFSK_E_ARG; }
+    if ((int64_t)((H->S + kDiC - 1) / kDiC) * ((n_frames + kDiF + kDiHalo - 1) / kDiF) > 0x7FFFFFFFLL) {
+        afsk_set_error("%s: piece too large", fn);
+        return AFSK_E_ARG;
+    }
+    if (on_device && (reinterpret_cast<uintptr_t>(frames) & 15) != 0) {
+        afsk_set_error("%s: device frames must be 16-byte aligned", fn);
+        return AFSK_E_ARG;
+    }
+    return streams_call(H, frames, on_device, nullptr, n_frames, stream, nullptr, nullptr, nullptr, n_events);
 }
 
 int afsk_rx_streams_finish_some(AfskRxStreams *H, int n, const int32_t *h_streams, const int32_t *h_baud, const int32_t *h_amp_start,
@@ -3532,7 +3631,7 @@ int afsk_rx_streams_finish_some(AfskRxStreams *H, int n, const int32_t *h_stream
         if (fin[s]) { afsk_set_error("%s: stream %d listed twice", fn, s); return AFSK_E_ARG; }
         fin[s] = 1;
     }
-    if (!given) return streams_call(H, nullptr, 0, nullptr, stream, fin.data(), nullptr, nullptr, n_events);
+    if (!given) return streams_call(H, nullptr, 0, nullptr, -1, stream, fin.data(), nullptr, nullptr, n_events);
     for (int i = 0; i < n; i++) {
         const int rc = rx_settings_check(fn, h_streams[i], h_baud[i], h_timeout_frames[i]);
         if (rc != AFSK_OK) return rc;
@@ -3543,7 +3642,7 @@ int afsk_rx_streams_finish_some(AfskRxStreams *H, int n, const int32_t *h_stream
         baud[h_streams[i]] = h_baud[i];
         params[h_streams[i]] = GateParams{h_amp_start[i], h_amp_end[i], h_timeout_frames[i]};
     }
-    return streams_call(H, nullptr, 0, nullptr, stream, fin.data(), baud.data(), params.data(), n_events);
+    return streams_call(H, nullptr, 0, nullptr, -1, stream, fin.data(), baud.data(), params.data(), n_events);
 }
 
 int afsk_rx_streams_finish(AfskRxStreams *H, void *stream, int64_t *n_events)

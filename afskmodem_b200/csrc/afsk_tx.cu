@@ -437,10 +437,50 @@ __device__ int16_t win_frame(const TxDesc *__restrict__ descs, const int32_t *__
     return (int16_t)(tone_pair(sym, u, d.bf) & 0xFFFFu);
 }
 
-// One thread per 16-byte output vector.  A vector inside one row and one message locates its first pair once
-// and walks five pairs (the short-tone walk of k_synth_var: at 24000 baud a mark has no frames); its words
-// are the pair values, shifted by one frame when the message starts on an odd frame of the vector.  A vector
-// across a row or message boundary, or the end of the output, writes its frames one by one.
+// Frames t0 .. t0 + 7 of row `row` (all inside the window row) as one 16-byte vector, into o; false when they
+// straddle a message boundary (the caller then computes them frame by frame with win_frame).  A vector inside one
+// message locates its first pair once and walks five pairs (the short-tone walk of k_synth_var: at 24000 baud a
+// mark has no frames); its words are the pair values, shifted by one frame when the message starts on an odd frame
+// of the vector.  Silence is zero.
+__device__ __forceinline__ bool win_vec(const TxDesc *__restrict__ descs, const int32_t *__restrict__ row_off, long long row,
+                                        long long t0, const uint8_t *__restrict__ pay, const int64_t *__restrict__ nib, uint4 &o)
+{
+    const int hi = row_off[row + 1];
+    const int k = win_find(descs, row_off[row], hi, t0);
+    if (k >= hi || descs[k].out_off >= t0 + 8) {               // silence
+        o = make_uint4(0u, 0u, 0u, 0u);
+        return true;
+    }
+    const TxDesc d = descs[k];
+    if (d.out_off > t0 || d.out_off + d.out_len < t0 + 8) return false;
+    const long long m0 = t0 - d.out_off;
+    long long b;
+    int u;
+    win_locate(m0 & ~1LL, d, pay, nib, b, u);
+    uint32_t sym;
+    int L;
+    win_bit(b, d, pay, sym, L);
+    uint32_t pv[5];
+#pragma unroll
+    for (int j = 0; j < 5; j++) {
+        pv[j] = tone_pair(sym, u, d.bf);
+        u += 2;
+        while (u >= L) {                                       // next bit (__getFrames :463-467 appends tone after tone)
+            u -= L;
+            b++;
+            win_bit(b, d, pay, sym, L);
+        }
+    }
+    uint32_t w[4];
+#pragma unroll
+    for (int j = 0; j < 4; j++) w[j] = (m0 & 1) ? ((pv[j] & 0xFFFFu) | (pv[j + 1] & 0xFFFF0000u)) : pv[j];
+    o = make_uint4(w[0], w[1], w[2], w[3]);
+    return true;
+}
+
+// The planar window, out[s * n + c] = frame P + c of channel s: one thread per 16-byte output vector.  A vector
+// inside one row is win_vec's; one across a row or message boundary, or at the end of the output, writes its frames
+// one by one.
 __global__ void __launch_bounds__(kWinThreads) k_tx_window(const uint8_t *__restrict__ pay, const int64_t *__restrict__ nib,
                                                            const TxDesc *__restrict__ descs, const int32_t *__restrict__ row_off,
                                                            long long P, long long n, long long total, int16_t *__restrict__ out)
@@ -455,45 +495,75 @@ __global__ void __launch_bounds__(kWinThreads) k_tx_window(const uint8_t *__rest
     } else {
         row = f0 / n; col = f0 - row * n;
     }
-    const long long t0 = P + col;
-    if (col + 8 <= n) {
-        const int hi = row_off[row + 1];
-        const int k = win_find(descs, row_off[row], hi, t0);
-        if (k >= hi || descs[k].out_off >= t0 + 8) {           // silence
-            *reinterpret_cast<uint4 *>(out + f0) = make_uint4(0u, 0u, 0u, 0u);
-            return;
-        }
-        const TxDesc d = descs[k];
-        if (d.out_off <= t0 && d.out_off + d.out_len >= t0 + 8) {
-            const long long m0 = t0 - d.out_off;
-            long long b;
-            int u;
-            win_locate(m0 & ~1LL, d, pay, nib, b, u);
-            uint32_t sym;
-            int L;
-            win_bit(b, d, pay, sym, L);
-            uint32_t pv[5];
-#pragma unroll
-            for (int j = 0; j < 5; j++) {
-                pv[j] = tone_pair(sym, u, d.bf);
-                u += 2;
-                while (u >= L) {                               // next bit (__getFrames :463-467 appends tone after tone)
-                    u -= L;
-                    b++;
-                    win_bit(b, d, pay, sym, L);
-                }
-            }
-            uint32_t w[4];
-#pragma unroll
-            for (int j = 0; j < 4; j++) w[j] = (m0 & 1) ? ((pv[j] & 0xFFFFu) | (pv[j + 1] & 0xFFFF0000u)) : pv[j];
-            *reinterpret_cast<uint4 *>(out + f0) = make_uint4(w[0], w[1], w[2], w[3]);
-            return;
-        }
+    uint4 o;
+    if (col + 8 <= n && win_vec(descs, row_off, row, P + col, pay, nib, o)) {
+        *reinterpret_cast<uint4 *>(out + f0) = o;
+        return;
     }
 #pragma unroll 1
     for (int e = 0; e < 8 && f0 + e < total; e++) {
         out[f0 + e] = win_frame(descs, row_off, row, P + col, pay, nib);
         if (++col == n) { col = 0; row++; }
+    }
+}
+
+// The interleaved window, out[c * S + s] = frame P + c of channel s (what a multi-channel sound card takes).  A CTA
+// computes kIlC consecutive channels x kIlV column vectors of 8 frames (aligned on the window column, so no vector
+// straddles two channels) with win_vec, or win_frame for a vector across a message boundary or the window's end: one
+// thread per vector, consecutive threads along a channel as in k_tx_window, into shared memory.  It then writes the
+// tile frame-major: each of its frame rows is the contiguous run out[f * S + c0 .. + kIlC), as aligned 16-byte
+// vectors of the output, the row's partial head and tail vectors (S % 8 != 0) sample by sample.  Shared rows are
+// channels in the order (s & 7) * 8 + (s >> 3), 136 samples apart, so that the lanes of one output row read
+// consecutive shared rows in distinct bank groups.
+constexpr int kIlC = 64, kIlV = 16, kIlStride = 8 * kIlV + 8;
+
+__global__ void __launch_bounds__(kWinThreads) k_tx_window_interleaved(const uint8_t *__restrict__ pay, const int64_t *__restrict__ nib,
+                                                                       const TxDesc *__restrict__ descs,
+                                                                       const int32_t *__restrict__ row_off, long long P, long long n,
+                                                                       int S, int cblocks, int16_t *__restrict__ out)
+{
+    __shared__ __align__(16) int16_t T[kIlC * kIlStride];
+    const int c0 = (int)(blockIdx.x % cblocks) * kIlC, nc = min(kIlC, S - c0);
+    const long long F0 = (long long)(blockIdx.x / cblocks) * (8 * kIlV);
+    const int nf = (int)min(8LL * kIlV, n - F0);
+    const int col = 8 * (threadIdx.x % kIlV);                    // this thread's column vector, on every channel
+    if (col < nf) {
+        const long long t0 = P + F0 + col;
+        const int m = min(8, nf - col);
+#pragma unroll 1
+        for (int c = threadIdx.x / kIlV; c < nc; c += kWinThreads / kIlV) {
+            uint4 o;
+            if (m < 8 || !win_vec(descs, row_off, c0 + c, t0, pay, nib, o)) {   // frame by frame, 0 past the window
+                unsigned long long w = 0, x = 0;
+#pragma unroll 1
+                for (int e = 0; e < m; e++) {
+                    const unsigned long long f = (uint16_t)win_frame(descs, row_off, c0 + c, t0 + e, pay, nib);
+                    if (e < 4) w |= f << (16 * e); else x |= f << (16 * (e - 4));
+                }
+                o = make_uint4((uint32_t)w, (uint32_t)(w >> 32), (uint32_t)x, (uint32_t)(x >> 32));
+            }
+            *reinterpret_cast<uint4 *>(T + ((c & 7) * 8 + (c >> 3)) * kIlStride + col) = o;
+        }
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < nf * 9; i += kWinThreads) {     // a row of kIlC samples spans at most 9 vectors
+        const int q = i % 9, fl = i / 9;
+        const long long a = (F0 + fl) * S + c0, b = a + nc;      // the row's samples in out
+        const long long d0 = ((a >> 3) + q) * 8;
+        if (d0 >= b) continue;
+        uint32_t w[4] = {0u, 0u, 0u, 0u};
+#pragma unroll
+        for (int e = 0; e < 8; e++) {
+            const int c = (int)(d0 + e - a);
+            if (c >= 0 && c < nc) w[e >> 1] |= (uint32_t)(uint16_t)T[((c & 7) * 8 + (c >> 3)) * kIlStride + fl] << (16 * (e & 1));
+        }
+        if (d0 >= a && d0 + 8 <= b) {
+            *reinterpret_cast<uint4 *>(out + d0) = make_uint4(w[0], w[1], w[2], w[3]);
+        } else {
+#pragma unroll
+            for (int e = 0; e < 8; e++)
+                if (d0 + e >= a && d0 + e < b) out[d0 + e] = (int16_t)(w[e >> 1] >> (16 * (e & 1)));
+        }
     }
 }
 
@@ -842,7 +912,8 @@ static int tx_send_run(AfskTxStreams *H, int n, const int32_t *h_stream, const i
     return AFSK_OK;
 }
 
-static int tx_pull_run(AfskTxStreams *H, int64_t n_frames, int16_t *dst, int on_device, cudaStream_t st)
+// the window as S x n_frames row-major (planar) or n_frames x S (interleaved)
+static int tx_pull_run(AfskTxStreams *H, int64_t n_frames, int16_t *dst, int on_device, bool interleaved, cudaStream_t st)
 {
     if (n_frames == 0) return AFSK_OK;
     const int S = H->S;
@@ -873,9 +944,17 @@ static int tx_pull_run(AfskTxStreams *H, int64_t n_frames, int16_t *dst, int on_
     AFSK_CUDA(cudaMemcpyAsync(H->d_scratch, H->h_stage, bytes, cudaMemcpyHostToDevice, st));
     int16_t *out = on_device ? dst : H->d_out;
     const uint8_t *a = H->arena[H->cur];
-    k_tx_window<<<(unsigned)((nvec + kWinThreads - 1) / kWinThreads), kWinThreads, 0, st>>>(
-        a, reinterpret_cast<const int64_t *>(a), reinterpret_cast<const TxDesc *>(H->d_scratch),
-        reinterpret_cast<const int32_t *>(H->d_scratch + desc_bytes), H->P, n, total, out);
+    const TxDesc *d_descs = reinterpret_cast<const TxDesc *>(H->d_scratch);
+    const int32_t *d_row_off = reinterpret_cast<const int32_t *>(H->d_scratch + desc_bytes);
+    if (interleaved) {
+        const int cblocks = (S + kIlC - 1) / kIlC;
+        const int64_t ftiles = (n + 8 * kIlV - 1) / (8 * kIlV);
+        k_tx_window_interleaved<<<(unsigned)(cblocks * ftiles), kWinThreads, 0, st>>>(a, reinterpret_cast<const int64_t *>(a), d_descs,
+                                                                                     d_row_off, H->P, n, S, cblocks, out);
+    } else {
+        k_tx_window<<<(unsigned)((nvec + kWinThreads - 1) / kWinThreads), kWinThreads, 0, st>>>(
+            a, reinterpret_cast<const int64_t *>(a), d_descs, d_row_off, H->P, n, total, out);
+    }
     AFSK_CUDA(cudaGetLastError());
     H->n_launches++;
     if (!on_device) AFSK_CUDA(cudaMemcpyAsync(dst, H->d_out, (size_t)total * 2, cudaMemcpyDeviceToHost, st));
@@ -992,7 +1071,23 @@ int afsk_tx_streams_pull(AfskTxStreams *H, int64_t n_frames, int16_t *dst, int o
         afsk_set_error("afsk_tx_streams_pull: window too large");
         return AFSK_E_ARG;
     }
-    return tx_streams_call(H, [&] { return tx_pull_run(H, n_frames, dst, on_device, (cudaStream_t)stream); });
+    return tx_streams_call(H, [&] { return tx_pull_run(H, n_frames, dst, on_device, false, (cudaStream_t)stream); });
+}
+
+int afsk_tx_streams_pull_interleaved(AfskTxStreams *H, int64_t n_frames, int16_t *dst, int on_device, void *stream)
+{
+    const char *fn = "afsk_tx_streams_pull_interleaved";
+    if (!H || n_frames < 0 || (n_frames > 0 && !dst)) { afsk_set_error("%s: bad argument", fn); return AFSK_E_ARG; }
+    if (n_frames > (INT64_MAX / 16) / H->S) { afsk_set_error("%s: S * n_frames overflows", fn); return AFSK_E_ARG; }
+    if (on_device && (reinterpret_cast<uintptr_t>(dst) & 15) != 0) {
+        afsk_set_error("%s: device output must be 16-byte aligned", fn);
+        return AFSK_E_ARG;
+    }
+    if ((int64_t)((H->S + kIlC - 1) / kIlC) * ((n_frames + 8 * kIlV - 1) / (8 * kIlV)) > 0x7FFFFFFFLL) {
+        afsk_set_error("%s: window too large", fn);
+        return AFSK_E_ARG;
+    }
+    return tx_streams_call(H, [&] { return tx_pull_run(H, n_frames, dst, on_device, true, (cudaStream_t)stream); });
 }
 
 int afsk_tx_streams_state(const AfskTxStreams *H, int s, int64_t *pulled, int64_t *busy_until, int64_t *pending)

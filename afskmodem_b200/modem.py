@@ -1037,16 +1037,19 @@ class StreamReceiver:
     def __exit__(self, *exc):
         self.close()
 
-    def _host_input(self, pieces) -> tuple[np.ndarray, np.ndarray]:
-        """S host pieces -> one grow-only pinned int16 buffer (asynchronous copy to the device) and offsets."""
-        offsets = np.zeros(len(pieces) + 1, dtype=np.int64)
-        np.cumsum([len(p) for p in pieces], out=offsets[1:])
-        n = int(offsets[-1])
+    def _staging(self, n: int) -> np.ndarray:
+        """the grow-only pinned int16 buffer host input is copied into (asynchronous copy to the device), >= n samples"""
         if self._pinned is None or self._pinned.array.size < n:
             if self._pinned is not None:
                 self._pinned.close()
             self._pinned = _cabi.PinnedArray((max(n + n // 4, 16),), np.int16)
-        buf = self._pinned.array
+        return self._pinned.array
+
+    def _host_input(self, pieces) -> tuple[np.ndarray, np.ndarray]:
+        """S host pieces -> the pinned staging buffer and offsets."""
+        offsets = np.zeros(len(pieces) + 1, dtype=np.int64)
+        np.cumsum([len(p) for p in pieces], out=offsets[1:])
+        buf = self._staging(int(offsets[-1]))
         for p, a, b in zip(pieces, offsets[:-1], offsets[1:]):
             buf[a:b] = p
         return buf, offsets
@@ -1074,6 +1077,43 @@ class StreamReceiver:
         if int(offsets[-1]) > len(arr):
             raise ValueError(f"samples holds {len(arr)} frames, the offsets need {int(offsets[-1])}")
         return self._run(arr.ctypes.data, 0, offsets, stream)
+
+    def push_interleaved(self, frames, stream=None) -> StreamEvents:
+        """``push`` of the next n frames of every channel, given interleaved as a multi-channel sound card
+        delivers them: frame f of channel s is ``frames[f, s]``.  ``frames``: a C-contiguous (n, S) int16 numpy
+        array; any buffer (bytes, bytearray, memoryview) of 2 * n * S bytes of little-endian int16, which is what
+        pyaudio's ``Stream.read(n)`` returns for ``channels=S``; or a contiguous CUDA int16 tensor on this
+        receiver's device, of shape (n, S) or (n * S,).  Host input is copied once, as is, into a pinned
+        buffer; the GPU de-interleaves it.  Returns what ``push([frames[:, s] for s in range(S)])`` returns."""
+        S = self.S
+        if hasattr(frames, "data_ptr"):                         # a torch tensor: passed by device pointer
+            if not frames.is_cuda or frames.device.index != self.device:
+                raise ValueError(f"device frames must live on cuda:{self.device}")
+            if str(frames.dtype) != "torch.int16" or not frames.is_contiguous():
+                raise ValueError("device frames must be a contiguous int16 tensor")
+            if not (frames.dim() == 2 and frames.shape[1] == S) and not (frames.dim() == 1 and frames.numel() % S == 0):
+                raise ValueError(f"device frames must have shape (n, {S}) or (n * {S},), got {tuple(frames.shape)}")
+            return self._run_interleaved(frames.data_ptr(), 1, frames.numel() // S, stream)
+        if isinstance(frames, np.ndarray):
+            if frames.dtype != np.int16 or not frames.flags.c_contiguous:
+                raise ValueError("host frames must be a C-contiguous int16 array")
+            if not (frames.ndim == 2 and frames.shape[1] == S) and not (frames.ndim == 1 and frames.size % S == 0):
+                raise ValueError(f"host frames must have shape (n, {S}) or (n * {S},), got {frames.shape}")
+            src = frames.reshape(-1)
+        else:
+            mv = memoryview(frames).cast("B")
+            if mv.nbytes % (2 * S):
+                raise ValueError(f"{mv.nbytes} bytes are not whole frames of {S} int16 samples")
+            src = np.frombuffer(mv, dtype="<i2")
+        buf = self._staging(src.size)
+        buf[:src.size] = src
+        return self._run_interleaved(buf.ctypes.data, 0, src.size // S, stream)
+
+    def _run_interleaved(self, ptr: int, on_device: int, n_frames: int, stream) -> StreamEvents:
+        n = C.c_int64(0)
+        _cabi.check(_cabi.lib().afsk_rx_streams_push_interleaved(self._h, C.c_void_p(ptr), on_device, n_frames,
+                                                                  C.c_void_p(stream or 0), C.byref(n)))
+        return self._events(n.value)
 
     def finish(self, streams=None, receivers=None, timeout=None, stream=None) -> StreamEvents:
         """Ends the streams of the channels ``streams`` (default: all) and returns their final calls.  Each of
@@ -1430,6 +1470,21 @@ class StreamTransmitter:
         buffer, valid until the next pull unless copied.  ``out``: a contiguous CUDA int16 tensor of at least
         S * n elements on this transmitter's device, written row-major (row s = channel s, no padding) and
         returned; nothing past S * n is written."""
+        r = self._pull(_cabi.lib().afsk_tx_streams_pull, n, out, stream)
+        return r if out is not None else r.reshape(self.S, int(n))
+
+    def pull_interleaved(self, n: int, out=None, stream=None):
+        """``pull`` with the window interleaved, as a multi-channel sound card takes it: frame f of channel s is
+        element [f, s], bitwise ``pull(n).T``.  Default: a host (n, S) int16 array in the grow-only pinned buffer,
+        valid until the next pull; its ``tobytes()`` is what pyaudio's ``Stream.write`` takes for ``channels=S``.
+        ``out``: a contiguous CUDA int16 tensor of at least n * S elements on this transmitter's device, written
+        frame-major and returned; nothing past n * S is written."""
+        r = self._pull(_cabi.lib().afsk_tx_streams_pull_interleaved, n, out, stream)
+        return r if out is not None else r.reshape(int(n), self.S)
+
+    def _pull(self, fn, n, out, stream):
+        """the next n frames of every channel through fn (planar or interleaved pull): into ``out``, or into the
+        pinned buffer, returned flat"""
         n = int(n)
         if n < 0:
             raise ValueError("pull needs n >= 0")
@@ -1441,15 +1496,15 @@ class StreamTransmitter:
                 raise ValueError("out must be a contiguous int16 tensor")
             if out.numel() < total:
                 raise ValueError(f"out holds {out.numel()} frames, the pull needs {total}")
-            _cabi.check(_cabi.lib().afsk_tx_streams_pull(self._h, n, C.c_void_p(out.data_ptr()), 1, C.c_void_p(stream or 0)))
+            _cabi.check(fn(self._h, n, C.c_void_p(out.data_ptr()), 1, C.c_void_p(stream or 0)))
             return out
         if self._pinned is None or self._pinned.array.size < total:
             if self._pinned is not None:
                 self._pinned.close()
             self._pinned = _cabi.PinnedArray((max(total + total // 4, 16),), np.int16)
         buf = self._pinned.array[:total]
-        _cabi.check(_cabi.lib().afsk_tx_streams_pull(self._h, n, C.c_void_p(buf.ctypes.data), 0, C.c_void_p(stream or 0)))
-        return buf.reshape(self.S, n)
+        _cabi.check(fn(self._h, n, C.c_void_p(buf.ctypes.data), 0, C.c_void_p(stream or 0)))
+        return buf
 
     def state(self, s: int) -> tuple[int, int, int]:
         """(frames pulled, end of channel s's last message (<= frames pulled: idle), its messages not yet fully pulled)."""

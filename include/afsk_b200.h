@@ -221,6 +221,13 @@ int afsk_rx_streams_create(int device, int S, int baud, int amp_start, int amp_e
  * can only be destroyed. */
 int afsk_rx_streams_push(AfskRxStreams *h, const int16_t *samples, int on_device, const int64_t *h_offsets,
                          void *stream, int64_t *n_events);
+/* afsk_rx_streams_push of n_frames frames of every channel, given interleaved as a sound card delivers them:
+ * frames[f * S + s] = frame f of channel s (n_frames * S samples, frame-major).  Device and host pointers, the
+ * host copy and errors as for afsk_rx_streams_push; AFSK_E_ARG also for a negative n_frames, a NULL frames with
+ * n_frames > 0 or an n_frames * S that overflows.  Events, state, counters and arena bytes are those of the
+ * planar push of the same pieces. */
+int afsk_rx_streams_push_interleaved(AfskRxStreams *h, const int16_t *frames, int on_device, int64_t n_frames,
+                                     void *stream, int64_t *n_events);
 /* ends the streams of the n distinct channels h_streams[n] (finite-stream conventions of afsk_rx_gate_multi: a
  * pending recording ends at the last full chunk, a call that has neither opened nor timed out is dropped, a
  * partial chunk is ignored) and returns their final calls.  Each listed channel's next push is frame 0 of a new
@@ -294,6 +301,10 @@ int afsk_tx_streams_send(AfskTxStreams *h, int n, const int32_t *h_stream, const
  * written.  Synchronizes `stream`.  A bad argument returns AFSK_E_ARG and changes nothing; after any other
  * error the handle refuses every later send / pull (AFSK_E_CUDA) and can only be destroyed. */
 int afsk_tx_streams_pull(AfskTxStreams *h, int64_t n_frames, int16_t *dst, int on_device, void *stream);
+/* afsk_tx_streams_pull with the window written interleaved, as a sound card takes it: dst[f * S + s] = frame f
+ * of channel s (n_frames x S, frame-major), the transpose of afsk_tx_streams_pull's array; nothing past
+ * S * n_frames is written.  Arguments and errors as for afsk_tx_streams_pull. */
+int afsk_tx_streams_pull_interleaved(AfskTxStreams *h, int64_t n_frames, int16_t *dst, int on_device, void *stream);
 /* channel s: frames pulled (P), end of its last message sent (<= P: idle), messages not yet fully pulled */
 int afsk_tx_streams_state(const AfskTxStreams *h, int s, int64_t *pulled, int64_t *busy_until, int64_t *pending);
 /* device bytes the handle holds (payload arenas, descriptors, host-output staging) */

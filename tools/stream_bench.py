@@ -12,7 +12,13 @@ only way they run) on the same card.  Card name and power limit are read in the 
 --mix splits the channels into six equal groups at 300, 600, 1200, 2400, 4000 and 6000 baud, each hearing
 traffic at its own baud, and within a group cycles through the three (amp_start, amp_end) threshold pairs of
 the c5 corpus; the handle is then opened with open_receive_streams.  A push then decodes one group per distinct
-baud among its final recordings."""
+baud among its final recordings.
+
+--layout interleaved feeds each piece as a multi-channel sound card delivers it, n x S frame-major (host input: a
+pageable array, as pyaudio's read returns it), three ways in one run: push_interleaved (the GPU de-interleaves it),
+a host numpy transpose into the pinned planar buffer followed by push, and .t().contiguous() on the device followed
+by push, which is what a user had to do without push_interleaved.  The profiled run then times
+k_stream_deinterleave and k_stream_copy's planar append over the same pieces (4 bytes moved per appended frame)."""
 from __future__ import annotations
 
 import argparse
@@ -60,13 +66,18 @@ def mix_groups(S: int):
     return [(b, cuts[g], cuts[g + 1] - cuts[g]) for g, b in enumerate(MIX_BAUDS)]
 
 
-def run_config(base, d_base, S: int, piece: int, T: int, device: bool, timeout: float, mix: bool = False):
-    """base / d_base: one traffic stream, or with mix one per baud of MIX_BAUDS"""
+def run_config(base, d_base, S: int, piece: int, T: int, device: bool, timeout: float, mix: bool = False,
+               route: str = "planar"):
+    """base / d_base: one traffic stream, or with mix one per baud of MIX_BAUDS; route: planar, interleaved,
+    host-transpose or device-transpose (see --layout)"""
     import torch
     n_push = T // piece
     offsets = np.arange(S + 1, dtype=np.int64) * piece
     pinned = _cabi.PinnedArray((S * piece + 8,), np.int16)
-    out = {"S": S, "piece": piece, "input": "device" if device else "host-pinned", "pushes": n_push, "mix": mix}
+    out = {"S": S, "piece": piece, "input": "device" if device else "host-pinned", "pushes": n_push, "mix": mix,
+           "route": route}
+    if route != "planar" and not device:
+        out["input"] = "host"
     if mix:
         groups = mix_groups(S)
         rxs = [A.Receiver(b, *MIX_THRESHOLDS[k % 3]) for b, _, n in groups for k in range(n)]
@@ -83,15 +94,30 @@ def run_config(base, d_base, S: int, piece: int, T: int, device: bool, timeout: 
                 if device:
                     t = torch.cat([torch.as_strided(d_base[g], (n, piece), (SHIFT, 1), i * piece).reshape(-1)
                                    for g, (_, _, n) in enumerate(groups)])
+                    if route != "planar":
+                        t = t.view(S, piece).t().contiguous()        # the piece as a sound card delivers it
                     torch.cuda.synchronize()
                     t0 = time.perf_counter()
-                    ev = st.push(t, offsets)
+                    if route == "interleaved":
+                        ev = st.push_interleaved(t)
+                    elif route == "device-transpose":
+                        ev = st.push(t.t().contiguous().view(-1), offsets)
+                    else:
+                        ev = st.push(t, offsets)
                 else:
                     for g, (_, c, n) in enumerate(groups):
                         np.copyto(pinned.array[c * piece:(c + n) * piece].reshape(n, piece),
                                   np.lib.stride_tricks.as_strided(base[g][i * piece:], shape=(n, piece), strides=(SHIFT * 2, 2)))
+                    if route != "planar":
+                        x = pinned.array[:S * piece].reshape(S, piece).T.copy()   # pageable, frame-major
                     t0 = time.perf_counter()
-                    ev = st.push(pinned.array, offsets)
+                    if route == "interleaved":
+                        ev = st.push_interleaved(x)
+                    elif route == "host-transpose":
+                        np.copyto(pinned.array[:S * piece].reshape(S, piece), x.T)
+                        ev = st.push(pinned.array, offsets)
+                    else:
+                        ev = st.push(pinned.array, offsets)
                 times.append(time.perf_counter() - t0)
                 n_ev += len(ev)
                 n_rec += int(ev.recorded.sum())
@@ -120,24 +146,30 @@ def run_config(base, d_base, S: int, piece: int, T: int, device: bool, timeout: 
     return out
 
 
-def profile_config(d_base, S: int, piece: int, T: int, timeout: float, out_dir: str | None):
+def profile_config(d_base, S: int, piece: int, T: int, timeout: float, out_dir: str | None, route: str = "planar"):
     """Device time of every kernel and copy over one device-input push sequence (torch.profiler, CUDA activity),
-    beside the host wall time of the same pushes: what share of a push the GPU is busy."""
+    beside the host wall time of the same pushes: what share of a push the GPU is busy.  route interleaved: the
+    same pieces frame-major, through push_interleaved."""
     import torch
     from torch.profiler import ProfilerActivity, profile
     n_push = T // piece
     offsets = np.arange(S + 1, dtype=np.int64) * piece
     pieces = [torch.as_strided(d_base, (S, piece), (SHIFT, 1), i * piece).contiguous().view(-1) for i in range(n_push)]
+    if route == "interleaved":
+        pieces = [t.view(S, piece).t().contiguous() for t in pieces]
+
+    def push(st, t):
+        return st.push_interleaved(t) if route == "interleaved" else st.push(t, offsets)
     rx = A.Receiver(1200)
     with rx.open_streams(S, timeout) as st:
         for t in pieces:                                  # warm-up: same shapes
-            st.push(t, offsets)
+            push(st, t)
         st.finish()
         torch.cuda.synchronize()
         with profile(activities=[ProfilerActivity.CUDA]) as prof:
             t0 = time.perf_counter()
             for t in pieces:
-                st.push(t, offsets)
+                push(st, t)
             wall = time.perf_counter() - t0
         st.finish()
     rows = {}
@@ -149,8 +181,16 @@ def profile_config(d_base, S: int, piece: int, T: int, timeout: float, out_dir: 
             rows[e.key] = {"count": int(e.count), "ms": us / 1e3}
     busy = sum(r["ms"] for r in rows.values())
     if out_dir:
-        prof.export_chrome_trace(os.path.join(out_dir, "r3_stream_profile.pt.trace.json"))
-    return {"S": S, "piece": piece, "pushes": n_push, "input": "device", "host_wall_ms": wall * 1e3,
+        prof.export_chrome_trace(os.path.join(out_dir, f"stream_profile_{route}.pt.trace.json"))
+    # the append: k_stream_deinterleave, or k_stream_copy's launches (its retention moves included, which the
+    # interleaved run also counts under k_stream_copy); 4 bytes per appended frame
+    kernel = "k_stream_deinterleave" if route == "interleaved" else "k_stream_copy"
+    app_ms = sum(r["ms"] for k, r in rows.items() if kernel in k)
+    app_bytes = 4 * S * piece * n_push
+    return {"S": S, "piece": piece, "pushes": n_push, "input": "device", "route": route, "host_wall_ms": wall * 1e3,
+            "host_ms_per_push": wall * 1e3 / n_push, "append_kernel": kernel, "append_ms": app_ms,
+            "append_us_per_push": app_ms * 1e3 / n_push,
+            "append_TBps": app_bytes / (app_ms * 1e-3) / 1e12 if app_ms else None,
             "device_busy_ms": busy, "device_busy_share": busy / (wall * 1e3),
             "by_kernel_or_copy": dict(sorted(rows.items(), key=lambda kv: -kv[1]["ms"]))}
 
@@ -181,6 +221,7 @@ def main():
     ap.add_argument("--timeout", type=float, default=1.0)
     ap.add_argument("--input", default="host,device")
     ap.add_argument("--mix", action="store_true", help="six bauds and three threshold pairs across the channels")
+    ap.add_argument("--layout", default="planar", choices=["planar", "interleaved"])
     ap.add_argument("--out", default=None)
     ap.add_argument("--no-profile", action="store_true", help="skip the profiled run of the largest device configuration")
     a = ap.parse_args()
@@ -199,18 +240,25 @@ def main():
         base = traffic(n, rng)
         d_base = torch.from_numpy(base).cuda()
     res = {"card": card(), "torch_device": torch.cuda.get_device_name(0), "seconds_per_channel": a.seconds,
-           "timeout_s": a.timeout, "mix": a.mix, "configs": []}
+           "timeout_s": a.timeout, "mix": a.mix, "layout": a.layout, "configs": []}
+    routes = {False: ["planar"], True: ["planar"]}
+    if a.layout == "interleaved":
+        routes = {False: ["interleaved", "host-transpose"], True: ["interleaved", "device-transpose"]}
     for S in Ss:
         for piece in pieces:
             for inp in a.input.split(","):
-                r = run_config(bases, d_bases, S, piece, T, inp == "device", a.timeout, True) if a.mix else \
-                    run_config(base, d_base, S, piece, T, inp == "device", a.timeout)
-                print(json.dumps(r), flush=True)
-                res["configs"].append(r)
+                for route in routes[inp == "device"]:
+                    r = run_config(bases, d_bases, S, piece, T, inp == "device", a.timeout, True, route) if a.mix else \
+                        run_config(base, d_base, S, piece, T, inp == "device", a.timeout, route=route)
+                    print(json.dumps(r), flush=True)
+                    res["configs"].append(r)
     if not a.mix and not a.no_profile:                    # the profile and whole-stream lines use uniform traffic
-        res["profile"] = profile_config(d_base, max(Ss), max(pieces), T, a.timeout,
-                                        os.path.dirname(os.path.abspath(a.out)) if a.out else None)
+        out_dir = os.path.dirname(os.path.abspath(a.out)) if a.out else None
+        res["profile"] = profile_config(d_base, max(Ss), max(pieces), T, a.timeout, out_dir)
         print(json.dumps({k: v for k, v in res["profile"].items() if k != "by_kernel_or_copy"}), flush=True)
+        if a.layout == "interleaved":
+            res["profile_interleaved"] = profile_config(d_base, max(Ss), max(pieces), T, a.timeout, out_dir, "interleaved")
+            print(json.dumps({k: v for k, v in res["profile_interleaved"].items() if k != "by_kernel_or_copy"}), flush=True)
     if not a.mix:
         res["whole_stream"] = whole_stream_reference(base, T, 16, a.timeout)
         print(json.dumps(res["whole_stream"]), flush=True)

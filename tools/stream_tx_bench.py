@@ -12,12 +12,19 @@ second of kernel time, against the 7.7 TB/s of HBM3e on a B200's data sheet) and
 Card name and power limit are read in the same run.
 
 --mix splits the channels into six equal groups at 300, 600, 1200, 2400, 4000 and 6000 baud (open_transmit_streams),
-each sending messages of its own length at the same duty."""
+each sending messages of its own length at the same duty.
+
+--layout interleaved measures the window as a multi-channel sound card takes it, n x S frame-major, three ways in one
+run: pull_interleaved (the GPU writes it interleaved), a planar pull followed by a host numpy transpose into a
+preallocated array (host output), and a planar pull into a CUDA tensor followed by .t().contiguous() (device output),
+which is what a user had to do without pull_interleaved.  The profiled run then times k_tx_window_interleaved and
+k_tx_window over the same sequence (2 bytes written per pulled frame)."""
 from __future__ import annotations
 
 import argparse
 import json
 import os
+import re
 import subprocess
 import sys
 import time
@@ -59,7 +66,24 @@ class Traffic:
         self.next_at[streams] = end + self.rng.integers(0, hi, len(streams))
 
 
-def run_sequence(st, S, n, n_pull, baud, seed, out_t=None):
+def pull_route(st, S, n, route, out_t):
+    """the pull of one window by route: planar, interleaved, or the planar pull transposed on the host / device"""
+    import torch
+    if route == "planar":
+        return lambda: st.pull(n, out=out_t)
+    if route == "interleaved":
+        return lambda: st.pull_interleaved(n, out=out_t)
+    if route == "host-transpose":
+        dst = np.empty((n, S), np.int16)
+        return lambda: np.copyto(dst, st.pull(n).T)
+
+    def dev():                                            # device-transpose
+        st.pull(n, out=out_t)[:S * n].view(S, n).t().contiguous()
+        torch.cuda.synchronize()
+    return dev
+
+
+def run_sequence(st, S, n, n_pull, baud, seed, out_t=None, pull=None):
     tr = Traffic(S, baud, seed)
     t_pull, t_send, busy = [], [], 0
     P = st.state(0)[0]                      # the timeline goes on from the previous sequence
@@ -72,7 +96,10 @@ def run_sequence(st, S, n, n_pull, baud, seed, out_t=None):
             tr.sent(streams, b)
             busy += int((b - a).sum())
         t1 = time.perf_counter()
-        st.pull(n, out=out_t)
+        if pull:
+            pull()
+        else:
+            st.pull(n, out=out_t)
         t2 = time.perf_counter()
         t_send.append(t1 - t0)
         t_pull.append(t2 - t1)
@@ -85,21 +112,22 @@ def mix_bauds(S: int) -> np.ndarray:
     return np.array([MIX_BAUDS[s * len(MIX_BAUDS) // S] for s in range(S)], np.int64)
 
 
-def run_config(S: int, n: int, T: int, device: bool, baud):
-    """baud: one for every channel, or "mix" (mix_bauds)"""
+def run_config(S: int, n: int, T: int, device: bool, baud, route: str = "planar"):
+    """baud: one for every channel, or "mix" (mix_bauds); route: see pull_route"""
     import torch
     n_pull = max(T // n, 1)
     out_t = torch.empty(S * n, dtype=torch.int16, device="cuda") if device else None
-    res = {"S": S, "pull": n, "baud": baud, "output": "device" if device else "host-pinned", "pulls": n_pull}
+    res = {"S": S, "pull": n, "baud": baud, "output": "device" if device else "host-pinned", "pulls": n_pull, "route": route}
     if baud == "mix":
         baud = mix_bauds(S)
         st = A.open_transmit_streams([A.Transmitter(int(b), 0.1) for b in baud])
     else:
         st = A.Transmitter(baud, 0.1).open_streams(S)
     with st:
-        run_sequence(st, S, n, n_pull, baud, 1, out_t)                # warm-up: same shapes
+        pull = pull_route(st, S, n, route, out_t)
+        run_sequence(st, S, n, n_pull, baud, 1, out_t, pull)          # warm-up: same shapes
         c0 = st.counters()
-        tp, ts, busy = run_sequence(st, S, n, n_pull, baud, 2, out_t)
+        tp, ts, busy = run_sequence(st, S, n, n_pull, baud, 2, out_t, pull)
         c1 = st.counters()
         arena = st.arena_bytes()
     frames = S * n * n_pull
@@ -115,7 +143,7 @@ def run_config(S: int, n: int, T: int, device: bool, baud):
     return res
 
 
-def profile_config(S: int, n: int, T: int, baud: int, out_dir: str | None):
+def profile_config(S: int, n: int, T: int, baud: int, out_dir: str | None, route: str = "planar"):
     """Device time of every kernel and copy over one device-output pull sequence (torch.profiler, CUDA activity),
     beside the host wall time of the same pulls."""
     import torch
@@ -124,11 +152,12 @@ def profile_config(S: int, n: int, T: int, baud: int, out_dir: str | None):
     out_t = torch.empty(S * n, dtype=torch.int16, device="cuda")
     tx = A.Transmitter(baud, 0.1)
     with tx.open_streams(S) as st:
-        run_sequence(st, S, n, n_pull, baud, 1, out_t)
+        pull = pull_route(st, S, n, route, out_t)
+        run_sequence(st, S, n, n_pull, baud, 1, out_t, pull)
         torch.cuda.synchronize()
         with profile(activities=[ProfilerActivity.CUDA]) as prof:
             t0 = time.perf_counter()
-            tp, ts, _ = run_sequence(st, S, n, n_pull, baud, 2, out_t)
+            tp, ts, _ = run_sequence(st, S, n, n_pull, baud, 2, out_t, pull)
             wall = time.perf_counter() - t0
     rows = {}
     for e in prof.key_averages():
@@ -138,12 +167,14 @@ def profile_config(S: int, n: int, T: int, baud: int, out_dir: str | None):
         if us > 0:
             rows[e.key] = {"count": int(e.count), "ms": us / 1e3}
     busy = sum(r["ms"] for r in rows.values())
-    win = [v for k, v in rows.items() if "k_tx_window" in k]
+    kernel = "k_tx_window_interleaved" if route == "interleaved" else "k_tx_window"
+    win = [v for k, v in rows.items() if re.search(kernel + r"\b(?!_)", k)]
     win_ms = sum(r["ms"] for r in win)
     win_bytes = 2 * S * n * n_pull
     if out_dir:
-        prof.export_chrome_trace(os.path.join(out_dir, "r4_stream_tx_profile.pt.trace.json"))
-    return {"S": S, "pull": n, "baud": baud, "pulls": n_pull, "output": "device", "host_wall_ms": wall * 1e3,
+        prof.export_chrome_trace(os.path.join(out_dir, f"stream_tx_profile_{route}.pt.trace.json"))
+    return {"S": S, "pull": n, "baud": baud, "pulls": n_pull, "output": "device", "route": route, "kernel": kernel,
+            "host_wall_ms": wall * 1e3,
             "host_ms_per_pull": wall * 1e3 / n_pull, "pull_ms_per_pull": float(tp.sum()) * 1e3 / n_pull,
             "send_ms_per_pull": float(ts.sum()) * 1e3 / n_pull,
             "device_busy_ms": busy, "device_busy_ms_per_pull": busy / n_pull, "device_busy_share": busy / (wall * 1e3),
@@ -161,6 +192,7 @@ def main():
     ap.add_argument("--seconds", type=float, default=8.0)
     ap.add_argument("--output", default="device,host")
     ap.add_argument("--mix", action="store_true", help="six bauds across the channels")
+    ap.add_argument("--layout", default="planar", choices=["planar", "interleaved"])
     ap.add_argument("--out", default=None)
     ap.add_argument("--no-profile", action="store_true", help="skip the profiled run of the largest device configuration")
     a = ap.parse_args()
@@ -172,16 +204,25 @@ def main():
     T = int(a.seconds * 48000)
     res = {"card": card(), "torch_device": torch.cuda.get_device_name(0), "seconds_per_channel": a.seconds, "mix": a.mix,
            "configs": []}
-    lines = [(S, n, o == "device", "mix" if a.mix else 1200) for S in Ss for n in pulls for o in a.output.split(",")]
+    res["layout"] = a.layout
+    routes = {False: ["planar"], True: ["planar"]}
+    if a.layout == "interleaved":
+        routes = {False: ["interleaved", "host-transpose"], True: ["interleaved", "device-transpose"]}
+    lines = [(S, n, o == "device", "mix" if a.mix else 1200, r) for S in Ss for n in pulls for o in a.output.split(",")
+             for r in routes[o == "device"]]
     if not a.mix:
-        lines.append((max(Ss), max(pulls), True, 4800))
-    for S, n, dev, baud in lines:
-        r = run_config(S, n, T, dev, baud)
+        lines += [(max(Ss), max(pulls), True, 4800, r) for r in routes[True]]
+    for S, n, dev, baud, route in lines:
+        r = run_config(S, n, T, dev, baud, route)
         print(json.dumps(r), flush=True)
         res["configs"].append(r)
     if not a.mix and not a.no_profile:
-        res["profile"] = profile_config(max(Ss), max(pulls), T, 1200, os.path.dirname(os.path.abspath(a.out)) if a.out else None)
+        out_dir = os.path.dirname(os.path.abspath(a.out)) if a.out else None
+        res["profile"] = profile_config(max(Ss), max(pulls), T, 1200, out_dir)
         print(json.dumps({k: v for k, v in res["profile"].items() if k != "by_kernel_or_copy"}), flush=True)
+        if a.layout == "interleaved":
+            res["profile_interleaved"] = profile_config(max(Ss), max(pulls), T, 1200, out_dir, "interleaved")
+            print(json.dumps({k: v for k, v in res["profile_interleaved"].items() if k != "by_kernel_or_copy"}), flush=True)
     res["card_after"] = card()
     if a.out:
         os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
