@@ -12,7 +12,7 @@ import pytest
 import afskmodem_b200 as A
 from afskmodem_b200 import _cabi
 from oracle import oracle as O
-from test_stream_tx_model import TxModel, random_payload, timeline
+from test_stream_tx_model import TimelineWindow, TxModel, random_payload, timeline
 
 pytestmark = pytest.mark.gpu
 A.LOG_LEVEL = 5
@@ -109,21 +109,25 @@ def test_seeded_sweep_64_channels(baud, tt):
 
 def test_retention_counters_match_the_model():
     """Many small messages on 64 channels: the arena compacts several times, exactly as the CPU model of the
-    retention policy does, and moves less than twice the bytes sent."""
+    retention policy does, and moves less than twice the bytes sent; every frame pulled, before and after each
+    compaction, is the oracle's timeline (a payload or codeword start table moved incompletely would show)."""
     rng = np.random.default_rng(7)
     S = 64
     for baud in (1200, 4800):
         model = TxModel(S, baud, 0.05, synth=False)
+        win = TimelineWindow(S)
         with A.Transmitter(baud, 0.05).open_streams(S) as st:
             for step in range(300):
                 k = int(rng.integers(0, 40))
                 streams = [int(x) for x in rng.integers(0, S, k)]
                 pays = [random_payload(rng, 400) for _ in range(k)]
-                a, _ = st.send(streams, pays)
+                a, b = st.send(streams, pays)
                 wa, _ = model.send(streams, pays)
                 assert np.array_equal(a, wa)
+                for s, p, x, y in zip(streams, pays, a, b):
+                    win.add(s, p, int(x), int(y), baud, 0.05)
                 n = int(rng.integers(1, 30000))
-                st.pull(n)
+                assert np.array_equal(st.pull(n), win.window(model.P, n)), (baud, step)
                 model.pull(n)
             c = st.counters()
         assert model.compactions >= 3

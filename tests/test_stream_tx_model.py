@@ -223,6 +223,35 @@ def timeline(sent, S, length, baud, training_time):
     return tl
 
 
+class TimelineWindow:
+    """timeline() one pull at a time, each message with its own baud and training time: add() the messages as they
+    are sent, window(P, n) is frames [P, P + n) of every channel.  Each message's frames are made when a window
+    first reaches them and dropped once a window has passed its end."""
+
+    def __init__(self, S):
+        self.S = S
+        self.q = [[] for _ in range(S)]
+
+    def add(self, s, pay, a, b, baud, training_time):
+        self.q[s].append([a, b, pay.encode() if isinstance(pay, str) else bytes(pay), baud, training_time, None])
+
+    def window(self, P, n):
+        out = np.zeros((self.S, n), np.int16)
+        for s, q in enumerate(self.q):
+            while q and q[0][1] <= P:
+                q.pop(0)
+            for m in q:
+                a, b = m[0], m[1]
+                if a >= P + n:
+                    break
+                if m[5] is None:
+                    m[5] = O.tx_frames(m[2], m[3], m[4])
+                    assert len(m[5]) == b - a
+                lo, hi = max(a, P), min(b, P + n)
+                out[s, lo - P:hi - P] = m[5][lo - a:hi - a]
+        return out
+
+
 def random_payload(rng, hi=12):
     k = int(rng.integers(0, hi + 1))
     return rng.integers(0, 256, size=k, dtype=np.uint8).tobytes()
