@@ -678,6 +678,16 @@ __device__ __forceinline__ void unpack_acc(int acc, int &U, int &Xn)
     Xn += (acc - u) >> 8;
 }
 
+// The bit of a window whose correlations tie (Um == Us) while Ns > Nm: mark_diff < space_diff (:346-351) compares
+// floor(M / bf) < floor(S / bf), with 2 M = 65535 bf - 65534 Um + 2 Nm and 2 S = 2 M + 2 (Ns - Nm)
+__device__ __forceinline__ bool tie_bit(int Um, int Nm, int Ns, int bf)
+{
+    const int two_bf = 2 * bf;
+    const int M2 = 65535 * bf - 65534 * Um + 2 * Nm;
+    const int S2 = M2 + 2 * (Ns - Nm);
+    return (S2 - M2 >= two_bf) || (M2 < (S2 / two_bf) * two_bf);
+}
+
 // accum4 with every slot inside the window
 __device__ __forceinline__ void accum4_full(uint32_t w0, uint32_t w1, uint32_t mw, uint32_t sw, uint32_t k512,
                                             int &accM, int &accS, int &accA)
@@ -995,7 +1005,6 @@ __global__ void __launch_bounds__(kFusedThreads2, 2) k_demod(const DemodParams p
     const int wsub = kConsumerThreads >> p.tpw_log2;          // windows per sub-tile
     const int bf = p.bf, nv = p.nv;
     const int rel0 = w * bf + part * p.seg;
-    const int two_bf = 2 * bf;
     // VIADDMNMX takes one immediate; derive the other constant from a runtime value so that it
     // lives in one register instead of being re-materialised before every use (stages < 65536)
     const uint32_t k512 = 0x02000200u | ((uint32_t)p.stages >> 16);
@@ -1114,11 +1123,7 @@ __global__ void __launch_bounds__(kFusedThreads2, 2) k_demod(const DemodParams p
                         Us += __shfl_xor_sync(0xFFFFFFFFu, Us, o);
                         Ns += __shfl_xor_sync(0xFFFFFFFFu, Ns, o);
                     }
-                    if (Um == Us && Ns > Nm) {
-                        const int M2 = 65535 * bf - 65534 * Um + 2 * Nm;
-                        const int S2 = M2 + 2 * (Ns - Nm);
-                        b1 = (S2 - M2 >= two_bf) || (M2 < (S2 / two_bf) * two_bf);   // floor(M/bf) < floor(S/bf)
-                    }
+                    if (Um == Us && Ns > Nm) b1 = tie_bit(Um, Nm, Ns, bf);
                 }
             } else {
                 if (kNT > 0) {
@@ -1160,11 +1165,7 @@ __global__ void __launch_bounds__(kFusedThreads2, 2) k_demod(const DemodParams p
                 // Um - Us decides unless the correlations tie, and only then is the floor compared.
                 const int du = Um - Us;
                 b1 = du > 0;
-                if (du == 0 && Ns > Nm) {
-                    const int M2 = 65535 * bf - 65534 * Um + 2 * Nm;
-                    const int S2 = M2 + 2 * (Ns - Nm);
-                    b1 = (S2 - M2 >= two_bf) || (M2 < (S2 / two_bf) * two_bf);   // floor(M/bf) < floor(S/bf)
-                }
+                if (du == 0 && Ns > Nm) b1 = tie_bit(Um, Nm, Ns, bf);
             }
             const bool valid = (part == 0) && (wbase + w < m.nwin);
             bit = valid && b1;
@@ -1278,11 +1279,7 @@ __device__ __forceinline__ void shift_decode(const uint4 *dp, uint32_t k512, int
         if (du == 0) {
             const int Nm = NmF + ((accM - ((int)((unsigned)accM << 24) >> 24)) >> 8);
             const int Ns = NsF + ((accS - ((int)((unsigned)accS << 24) >> 24)) >> 8);
-            if (Ns > Nm) {
-                const int M2 = 65535 * kBf - 65534 * Um + 2 * Nm;
-                const int S2 = M2 + 2 * (Ns - Nm);
-                b1 = (S2 - M2 >= 2 * kBf) || (M2 < (S2 / (2 * kBf)) * (2 * kBf));
-            }
+            if (Ns > Nm) b1 = tie_bit(Um, Nm, Ns, kBf);
         }
         const bool valid = w < nvalid;
         bits |= (uint32_t)(valid && b1) << w;
@@ -1484,9 +1481,7 @@ __device__ __forceinline__ void lane_decode(const uint4 *dp, uint32_t k512, int 
                 const int Um = (int)((unsigned)accM << 24) >> 24, Us = (int)((unsigned)accS << 24) >> 24;
                 const int Nm = (accM - Um) >> 8, Ns = (accS - Us) >> 8;
                 if (Um == Us && Ns > Nm) {
-                    const int M2 = 65535 * kBf - 65534 * Um + 2 * Nm;
-                    const int S2 = M2 + 2 * (Ns - Nm);
-                    b1 = (S2 - M2 >= 2 * kBf) || (M2 < (S2 / (2 * kBf)) * (2 * kBf));   // floor(M/bf) < floor(S/bf)
+                    b1 = tie_bit(Um, Nm, Ns, kBf);
                 } else {
                     b1 = Um > Us;
                 }
@@ -2193,6 +2188,19 @@ __global__ void __launch_bounds__(32) k_gate_multi(const int32_t *__restrict__ a
 struct CopySeg { long long src, dst, len; };                     // samples
 constexpr int kCopyThreads = 256, kCopyTileVecs = 4 * kCopyThreads;
 
+// samples k .. k + 7 of the sixteen in two consecutive aligned vectors
+__device__ __forceinline__ void realign8(const uint4 &lo, const uint4 &hi, int k, uint32_t (&o)[4])
+{
+    const uint32_t w[8] = {lo.x, lo.y, lo.z, lo.w, hi.x, hi.y, hi.z, hi.w};
+    const int j = k >> 1;
+#pragma unroll
+    for (int t = 0; t < 4; t++) {
+        const uint32_t x0 = j == 0 ? w[t] : j == 1 ? w[t + 1] : j == 2 ? w[t + 2] : w[t + 3];
+        const uint32_t x1 = j == 0 ? w[t + 1] : j == 1 ? w[t + 2] : j == 2 ? w[t + 3] : w[t + 4];
+        o[t] = (k & 1) ? __funnelshift_r(x0, x1, 16) : x0;
+    }
+}
+
 __global__ void __launch_bounds__(kCopyThreads) k_stream_copy(const int16_t *__restrict__ src, int16_t *__restrict__ dst,
                                                               const CopySeg *__restrict__ seg,
                                                               const int64_t *__restrict__ tile_first, int n)
@@ -2216,15 +2224,8 @@ __global__ void __launch_bounds__(kCopyThreads) k_stream_copy(const int16_t *__r
         uint4 lo = make_uint4(0, 0, 0, 0), hi = make_uint4(0, 0, 0, 0);
         if (sv >= s_lo && sv <= s_hi) lo = ld_nc_v4(src + sv * 8);
         if (k && sv + 1 >= s_lo && sv + 1 <= s_hi) hi = ld_nc_v4(src + (sv + 1) * 8);
-        const uint32_t w[8] = {lo.x, lo.y, lo.z, lo.w, hi.x, hi.y, hi.z, hi.w};
-        const int j = k >> 1;
         uint32_t o[4];
-#pragma unroll
-        for (int t = 0; t < 4; t++) {                             // bytes 2k .. 2k + 15 of the 32 loaded
-            const uint32_t x0 = j == 0 ? w[t] : j == 1 ? w[t + 1] : j == 2 ? w[t + 2] : w[t + 3];
-            const uint32_t x1 = j == 0 ? w[t + 1] : j == 1 ? w[t + 2] : j == 2 ? w[t + 3] : w[t + 4];
-            o[t] = (k & 1) ? __funnelshift_r(x0, x1, 16) : x0;
-        }
+        realign8(lo, hi, k, o);
         const long long d0 = dv * 8;
         if (d0 >= g.dst && d0 + 8 <= g.dst + g.len) {
             *reinterpret_cast<uint4 *>(dst + d0) = make_uint4(o[0], o[1], o[2], o[3]);
@@ -2273,15 +2274,8 @@ __global__ void __launch_bounds__(kDiThreads) k_stream_deinterleave(const int16_
         const int k = (int)(qs & 7);
         const uint4 lo = ld_nc_v4(src + sv * 8);                  // holds qs, inside the row
         const uint4 hi = k && (sv + 1) * 8 < row_end ? ld_nc_v4(src + (sv + 1) * 8) : make_uint4(0, 0, 0, 0);
-        const uint32_t w[8] = {lo.x, lo.y, lo.z, lo.w, hi.x, hi.y, hi.z, hi.w};
-        const int j = k >> 1;
         uint32_t o[4];
-#pragma unroll
-        for (int t = 0; t < 4; t++) {                             // samples k .. k + 7 of the 16 loaded
-            const uint32_t x0 = j == 0 ? w[t] : j == 1 ? w[t + 1] : j == 2 ? w[t + 2] : w[t + 3];
-            const uint32_t x1 = j == 0 ? w[t + 1] : j == 1 ? w[t + 2] : j == 2 ? w[t + 3] : w[t + 4];
-            o[t] = (k & 1) ? __funnelshift_r(x0, x1, 16) : x0;
-        }
+        realign8(lo, hi, k, o);
 #pragma unroll
         for (int e = 0; e < 8; e++) {
             const int c = 8 * q + e;
@@ -2305,6 +2299,78 @@ __global__ void __launch_bounds__(kDiThreads) k_stream_deinterleave(const int16_
             for (int e = 0; e < 8; e++)
                 if (f0 + e >= 0 && f0 + e < n) dst[d0 + e] = (int16_t)(o[e >> 1] >> (16 * (e & 1)));
         }
+    }
+}
+
+// Bit windows of open recordings, demodulated as their samples arrive (retention mode AFSK_RETAIN_BITS): job j decides
+// windows 0 .. nwin - 1 of one recording range, window k = samples x0 + k bf .. + bf - 1 of the sample arena, into
+// plane words w0, w0 + 1, ... of the plane arena.  One lane per window and one ballot per plane word; a CTA takes up to
+// kWinTileWords words of one job, so its bit length is uniform and the {mark, space} weights of every 8-sample step of
+// a window sit in shared memory (read as a broadcast).  A lane reads its window with aligned 128-bit loads realigned
+// to the window start (the window alignment is arbitrary), then the same per-sample arithmetic as k_demod: the
+// limiter and template sums of accum4_full in packed accumulators flushed every kFlushVecs vectors, the decision
+// with tie_bit, and quiet <=> sum |x| < amp_end * bf.
+struct __align__(16) WinJob {
+    int64_t x0;          // sample-arena index of window 0's first sample
+    int64_t w0;          // plane-arena word of windows 0 .. 31
+    int32_t nwin;        // windows to decide (> 0)
+    int32_t bf;          // bit length: a multiple of 4, at most kWinMaxBf
+    int32_t thr_bf;      // amp_end * bf
+    int32_t pad;
+};
+constexpr int kWinWarps = 4, kWinTileWords = 16, kWinMaxBf = 2000;
+constexpr int64_t kBitsMaxPiece = (int64_t)1 << 32;   // frames per channel and push in bits mode (WinJob.nwin < 2^31 at bf = 4)
+
+__global__ void __launch_bounds__(32 * kWinWarps) k_stream_windows(const int16_t *__restrict__ x, uint2 *__restrict__ planes,
+                                                                  const WinJob *__restrict__ jobs,
+                                                                  const int64_t *__restrict__ tile_first, int n)
+{
+    __shared__ uint4 wt[kWinMaxBf / 8 + 1];      // step i: {mark, space} of window samples 8i .. 8i + 3, then 8i + 4 .. 8i + 7
+    const long long tile = blockIdx.x;
+    int a = 0, b = n;                              // job of this tile
+    while (b - a > 1) {
+        const int mid = (a + b) >> 1;
+        if (tile_first[mid] <= tile) a = mid; else b = mid;
+    }
+    const WinJob J = jobs[a];
+    const int bf = J.bf, nvec = (bf + 7) >> 3;
+    for (int i = threadIdx.x; i < nvec; i += blockDim.x)
+        wt[i] = make_uint4(tone_weights4(bf, 8 * i, false), tone_weights4(bf, 8 * i, true), tone_weights4(bf, 8 * i + 4, false),
+                           tone_weights4(bf, 8 * i + 4, true));
+    __syncthreads();
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const long long word0 = (tile - tile_first[a]) * kWinTileWords;
+    const long long word1 = min(word0 + kWinTileWords, (long long)((J.nwin + 31) >> 5));
+    const uint32_t k512 = 0x02000200u | ((uint32_t)bf >> 16);     // (one register, as in k_demod)
+    for (long long wd = word0 + warp; wd < word1; wd += kWinWarps) {
+        const long long k = wd * 32 + lane;
+        bool bit = false, quiet = false;
+        if (k < J.nwin) {
+            const long long s0 = J.x0 + k * bf;
+            const uint4 *src = reinterpret_cast<const uint4 *>(x) + (s0 >> 3);
+            const int sh = (int)(s0 & 7);
+            int Um = 0, Nm = 0, Us = 0, Ns = 0, accA = 0;
+            uint4 lo = __ldg(src);
+            for (int i0 = 0; i0 < nvec; i0 += kFlushVecs) {
+                const int i1 = min(nvec, i0 + kFlushVecs);
+                int accM = 0, accS = 0;
+                for (int i = i0; i < i1; i++) {
+                    const uint4 hi = __ldg(src + i + 1);   // (at most one vector past the window: the arena's pad)
+                    uint32_t o[4];
+                    realign8(lo, hi, sh, o);
+                    lo = hi;
+                    const uint4 w = wt[i];
+                    accum4_full(o[0], o[1], w.x, w.y, k512, accM, accS, accA);
+                    if (8 * i + 4 < bf) accum4_full(o[2], o[3], w.z, w.w, k512, accM, accS, accA);
+                }
+                unpack_acc(accM, Um, Nm);
+                unpack_acc(accS, Us, Ns);
+            }
+            bit = Um > Us || (Um == Us && Ns > Nm && tie_bit(Um, Nm, Ns, bf));
+            quiet = accA < J.thr_bf;
+        }
+        const uint32_t bw = __ballot_sync(0xFFFFFFFFu, bit), qw = __ballot_sync(0xFFFFFFFFu, quiet);
+        if (lane == 0) planes[J.w0 + wd] = make_uint2(bw, qw);
     }
 }
 
@@ -2974,6 +3040,30 @@ int afsk_rx_plan_planes(const AfskRxPlan *P, int capture, const uint32_t **d_pla
     return AFSK_OK;
 }
 
+// The framing launch of B captures (planes at caps[c].plane_base, clocks in clock[]): automatic by capture length
+// (fk = 0), or forced (AFSK_OPT_FRAME_KERNEL) where the forced variant can represent the batch (k_frame_warp:
+// <= 2^18 windows per capture; int indices: < 2^30)
+static void launch_frame(int fk, int B, const CapDesc *caps, const int32_t *clock, const uint2 *planes, uint8_t *d_out,
+                         AfskRxResult *d_res, int64_t max_windows, int64_t sum_windows, int64_t gpu_caps, cudaStream_t st)
+{
+    if (fk == 1 && max_windows > kFrameWarpMaxWindows) fk = 0;
+    if ((fk == 2 || fk == 3) && max_windows >= ((int64_t)1 << 30)) fk = 0;
+    if (fk == 0) {
+        if (max_windows <= kFrameWarpMaxWindows) fk = 1;
+        else if (max_windows >= ((int64_t)1 << 30)) fk = 4;
+        else if (sum_windows > 65536 * std::max<int64_t>(gpu_caps, 1)) fk = 3;   // long captures on average
+        else fk = 2;
+    }
+    if (fk == 1)
+        k_frame_warp<<<(B + kFrameWarpCaps - 1) / kFrameWarpCaps, 32 * kFrameWarpCaps, 0, st>>>(caps, clock, planes, d_out, d_res, B);
+    else if (fk == 4)
+        k_frame<512, 8, long long><<<B, 512, 0, st>>>(caps, clock, planes, d_out, d_res);
+    else if (fk == 3)
+        k_frame<512, 8, int><<<B, 512, 0, st>>>(caps, clock, planes, d_out, d_res);
+    else
+        k_frame<128, 4, int><<<B, 128, 0, st>>>(caps, clock, planes, d_out, d_res);
+}
+
 int afsk_rx_decode(AfskRxPlan *P, const int16_t *d_samples, uint8_t *d_out, AfskRxResult *d_res, void *stream)
 {
     if (!P || (P->B > 0 && (!d_samples || !d_out || !d_res))) { afsk_set_error("afsk_rx_decode: null argument"); return AFSK_E_ARG; }
@@ -3092,26 +3182,7 @@ int afsk_rx_decode(AfskRxPlan *P, const int16_t *d_samples, uint8_t *d_out, Afsk
         AFSK_CUDA(cudaGetLastError());
         return AFSK_OK;
     }
-    // framing kernel: automatic by capture length, or forced (AFSK_OPT_FRAME_KERNEL) where the forced variant can
-    // represent the batch (k_frame_warp: <= 2^18 windows per capture; int indices: < 2^30)
-    int fk = P->frame_kernel;
-    if (fk == 1 && P->max_windows > kFrameWarpMaxWindows) fk = 0;
-    if ((fk == 2 || fk == 3) && P->max_windows >= ((int64_t)1 << 30)) fk = 0;
-    if (fk == 0) {
-        if (P->max_windows <= kFrameWarpMaxWindows) fk = 1;
-        else if (P->max_windows >= ((int64_t)1 << 30)) fk = 4;
-        else if (P->sum_windows > 65536 * std::max<int64_t>(P->gpu_caps, 1)) fk = 3;   // long captures on average
-        else fk = 2;
-    }
-    if (fk == 1)
-        k_frame_warp<<<(P->B + kFrameWarpCaps - 1) / kFrameWarpCaps, 32 * kFrameWarpCaps, 0, st>>>(P->d_caps, P->d_clock, P->d_planes,
-                                                                                                 d_out, d_res, P->B);
-    else if (fk == 4)
-        k_frame<512, 8, long long><<<P->B, 512, 0, st>>>(P->d_caps, P->d_clock, P->d_planes, d_out, d_res);
-    else if (fk == 3)
-        k_frame<512, 8, int><<<P->B, 512, 0, st>>>(P->d_caps, P->d_clock, P->d_planes, d_out, d_res);
-    else
-        k_frame<128, 4, int><<<P->B, 128, 0, st>>>(P->d_caps, P->d_clock, P->d_planes, d_out, d_res);
+    launch_frame(P->frame_kernel, P->B, P->d_caps, P->d_clock, P->d_planes, d_out, d_res, P->max_windows, P->sum_windows, P->gpu_caps, st);
     AFSK_CUDA(cudaGetLastError());
     return AFSK_OK;
 }
@@ -3245,9 +3316,125 @@ int afsk_rx_gate_multi(int device, const int16_t *d_samples, const int64_t *h_of
 // at most the frames its channel pushed since the slot was assigned, and a compaction moves at most what
 // the channels pushed while the free space filled, so every pushed frame causes O(1) moved frames
 // (afsk_rx_streams_counters reports them), and one long recording widens only its own slot.
+//
+// Retention mode AFSK_RETAIN_BITS demodulates open recordings as they arrive instead.  Once 4096 frames of a
+// pending recording are in, its clock is recovered (k_clock_q / k_clock, as a plan chooses them) and stored;
+// from then on every push decides the recording's complete 32-window plane words (k_stream_windows) into the
+// channel's slot of a plane arena, which follows the same policy as the sample arena (a plane word counts as
+// four samples).  The channel keeps its samples only from its first undecided window, or from its partial
+// chunk if that is earlier.  When the recording becomes final, its remaining windows are decided from that tail
+// and it is framed from its planes (k_frame_warp / k_frame).  A recording that ends before its clock is stored
+// still has all its samples and is decoded through the plan.  Each window's bit and quiet flag depend on its
+// own samples only, and the final length only decides how many windows count, so the results are the same.
 namespace {
 constexpr int64_t kSlotPad = 64;           // samples after the last slot (vector over-reads of the kernels)
 int64_t arena_frames(size_t bytes) { return bytes ? (int64_t)(bytes / 2) - kSlotPad : 0; }
+
+// an arena pair with one slot per channel, in samples (a plane word is four)
+struct Slots {
+    // per channel: first arena sample, capacity, stream position at the slot's start
+    std::vector<int64_t> off, cap, base;
+    int16_t *arena[2] = {nullptr, nullptr};
+    size_t arena_cap[2] = {0, 0};
+    int cur = 0;
+    int64_t top = 0;                                              // arena samples below the free space
+    int64_t n_moved = 0, n_compactions = 0;                       // since creation
+};
+
+void add_seg(CopySeg *seg, int64_t *tf, int &n, int64_t src, int64_t dst, int64_t len)
+{
+    if (len <= 0) return;
+    const int64_t vecs = ((dst + len + 7) >> 3) - (dst >> 3);
+    seg[n] = CopySeg{src, dst, len};
+    tf[n + 1] = tf[n] + (vecs + kCopyTileVecs - 1) / kCopyTileVecs;
+    n++;
+}
+
+// The retention step of one push (see above) for channels that have pushed[s], will have np[s] and keep from
+// keep[s] on: assigns the slots and lists the moves of the retained spans [keep[s], pushed[s]).  A compaction
+// allocates the other arena first; a failed allocation leaves A as it was.
+cudaError_t slots_retain(Slots &A, int S, const int64_t *pushed, const int64_t *np, const int64_t *keep, int64_t *new_off,
+                         int64_t *new_cap, CopySeg *seg, int64_t *tf, int &nmov, bool &compact)
+{
+    const int64_t C = AFSK_GATE_CHUNK;
+    auto overflows = [&](int s) { return np[s] - A.base[s] > A.cap[s]; };
+    auto rewinds = [&](int s) { return 2 * (np[s] - keep[s]) <= A.cap[s]; };
+    auto fresh_cap = [&](int s) { return (2 * (np[s] - keep[s]) + 2 * C + 7) & ~(int64_t)7; };
+    int64_t want = 0;
+    bool any = false;
+    for (int s = 0; s < S; s++)
+        if (overflows(s)) {
+            any = true;
+            if (!rewinds(s)) want += fresh_cap(s);
+        }
+    compact = any && A.top + want > arena_frames(A.arena_cap[A.cur]);
+    nmov = 0;
+    tf[0] = 0;
+    if (compact) {
+        int64_t total = 0;
+        for (int s = 0; s < S; s++) {
+            new_off[s] = total;
+            new_cap[s] = fresh_cap(s);
+            total += new_cap[s];
+        }
+        const int nxt = A.cur ^ 1;
+        const cudaError_t e = grow_device((void **)&A.arena[nxt], &A.arena_cap[nxt], (size_t)(total + total / 2 + kSlotPad) * 2);
+        if (e != cudaSuccess) return e;
+        for (int s = 0; s < S; s++) {
+            add_seg(seg, tf, nmov, A.off[s] + keep[s] - A.base[s], new_off[s], pushed[s] - keep[s]);
+            A.off[s] = new_off[s]; A.cap[s] = new_cap[s]; A.base[s] = keep[s];
+        }
+        A.top = total;
+        A.n_compactions++;
+    } else if (any) {
+        // within the arena: sources are the retained spans, destinations the slot starts (below the span: a
+        // rewind happens only when the span fills at most half the slot) or fresh space above the top
+        for (int s = 0; s < S; s++) {
+            if (!overflows(s)) continue;
+            const int64_t src = A.off[s] + keep[s] - A.base[s];
+            if (!rewinds(s)) {
+                A.off[s] = A.top;
+                A.cap[s] = fresh_cap(s);
+                A.top += A.cap[s];
+            }
+            add_seg(seg, tf, nmov, src, A.off[s], pushed[s] - keep[s]);
+            A.base[s] = keep[s];
+        }
+    }
+    for (int i = 0; i < nmov; i++) A.n_moved += seg[i].len;
+    return cudaSuccess;
+}
+
+// the moves slots_retain listed (descriptors already on the device), then the compacted arena becomes current
+void slots_move(Slots &A, bool compact, int nmov, const uint8_t *d_seg, const uint8_t *d_tf, int64_t tiles, cudaStream_t st,
+                int64_t &launches)
+{
+    if (nmov > 0) {
+        k_stream_copy<<<(unsigned)tiles, kCopyThreads, 0, st>>>(A.arena[A.cur], A.arena[compact ? A.cur ^ 1 : A.cur],
+                                                                reinterpret_cast<const CopySeg *>(d_seg),
+                                                                reinterpret_cast<const int64_t *>(d_tf), nmov);
+        launches++;
+    }
+    if (compact) A.cur ^= 1;
+}
+
+// K = #{k >= 0 : clk + k bf < n - bf}, as num_windows
+int64_t windows_of(int64_t n, int bf, int64_t clk)
+{
+    const int64_t span = n - bf - clk;
+    return span <= 0 ? 0 : (span + bf - 1) / bf;
+}
+
+// what bits mode does with a channel's recordings at this baud: > 0, the bit length: demodulated as they arrive;
+// 0: decided from length and baud alone (k_preset's statuses: no sample is needed); -1: kept whole
+int bits_bf(int baud)
+{
+    int bf, ml, sl;
+    if (!afsk_tone_geometry(baud, &bf, &ml, &sl) || AFSK_SYNC_FRAMES - 2 * bf <= 0 || ml != bf || sl != bf) return 0;
+    return (bf % 4 == 0 && bf <= kWinMaxBf) ? bf : -1;
+}
+
+int32_t clamp_thr(int32_t amp_end) { return std::min<int32_t>(std::max<int32_t>(amp_end, 0), 65537); }
 }  // namespace
 
 struct AfskRxStreams {
@@ -3256,16 +3443,15 @@ struct AfskRxStreams {
     std::vector<int32_t> baud;
     std::vector<GateParams> params;
     GateParams *d_params = nullptr;
-    // per channel (host): frames pushed, first retained frame (a chunk start), start of the pending recording
-    // (-1: none), calls finished, and the slot: first arena sample, capacity, stream frame at the slot's start
-    std::vector<int64_t> pushed, keep, pending, calls, slot_off, slot_cap, slot_base;
+    // per channel (host): frames pushed, first retained frame, start of the pending recording (-1: none), calls
+    // finished; the sample slots
+    std::vector<int64_t> pushed, keep, pending, calls;
+    Slots smp;
     std::vector<int64_t> np, new_off, new_cap, chunk_first;       // scratch of one push
-    int16_t *arena[2] = {nullptr, nullptr};
-    size_t arena_cap[2] = {0, 0};
-    int cur = 0;
-    int64_t top = 0;                                              // arena samples below the free space
     bool failed = false;                                          // an error after this push's state was committed
-    int64_t n_launches = 0, n_moved = 0, n_compactions = 0;       // since creation
+    bool used = false;                                            // a push or finish has run (the retention mode is fixed)
+    int retain = AFSK_RETAIN_SAMPLES;
+    int64_t n_launches = 0;                                       // since creation
     int16_t *d_stage = nullptr; size_t stage_cap = 0;             // host input
     // descriptors of one push, built in pinned memory and sent with one copy
     uint8_t *d_desc = nullptr, *h_desc = nullptr;
@@ -3282,6 +3468,18 @@ struct AfskRxStreams {
     uint8_t *h_dec = nullptr; size_t h_dec_cap = 0;               // pinned: results, then payloads
     std::vector<int64_t> rec_start, rec_len;
     std::vector<int32_t> rec_baud, rec_amp_end;
+    // bits mode, per channel: the pending recording's clock (-1: not stored), its windows decided, and the channel's
+    // plane stream (in samples, four per word): where the recording's window 0 lies, the end used, the first kept
+    std::vector<int64_t> pclock, pdecided, pw_rec, pw_pushed, pw_keep;
+    Slots pln;
+    // bits mode: descriptors (clock captures, their k_clock_q lists, plane moves, window jobs, frame captures and
+    // clocks), clocks read back, framing output
+    uint8_t *d_bdesc = nullptr, *h_bdesc = nullptr;
+    size_t bdesc_bytes = 0, o_ccap = 0, o_cq = 0, o_clk = 0, o_seg_pmov = 0, o_tf_pmov = 0, o_win = 0, o_tf_win = 0, o_fcap = 0,
+           o_fclk = 0;
+    uint8_t *d_fout = nullptr; size_t fout_cap = 0;
+    AfskRxResult *d_fres = nullptr; size_t fres_cap = 0;
+    uint8_t *h_fdec = nullptr; size_t h_fdec_cap = 0;
     // what the last push / finish returned
     std::vector<AfskRxStreamEvent> ev;
     std::vector<AfskRxResult> res;
@@ -3294,6 +3492,37 @@ static int streams_fail(cudaError_t e)
     afsk_set_error("afsk_rx_streams: %s", cudaGetErrorString(e));
     return AFSK_E_CUDA;
 }
+
+// decodes H->rec_* (recordings as ranges of the sample arena) through the plan; *rr / *oo: results and payload offsets
+// in H->h_dec, whose payloads start at *res_bytes.  Synchronizes st.
+static int streams_decode_plan(AfskRxStreams *H, const int16_t *x, cudaStream_t st, const AfskRxResult **rr, const int64_t **oo,
+                               size_t *res_bytes)
+{
+    const int nrec = (int)H->rec_start.size();
+    int rc = H->plan ? afsk_rx_plan_reset(H->plan, nrec, H->rec_start.data(), H->rec_len.data(), H->rec_baud.data(), H->rec_amp_end.data())
+                     : afsk_rx_plan_create_ranges(H->device, nrec, H->rec_start.data(), H->rec_len.data(), H->rec_baud.data(),
+                                                  H->rec_amp_end.data(), &H->plan);
+    if (rc != AFSK_OK) return rc;
+    *oo = H->plan->out_off.data();
+    const size_t rb = sizeof(AfskRxResult) * (size_t)nrec, out_bytes = (size_t)(*oo)[nrec];
+    cudaError_t e = grow_device((void **)&H->d_out, &H->out_cap, out_bytes);
+    if (e == cudaSuccess) e = grow_device((void **)&H->d_res, &H->res_cap, rb);
+    if (e == cudaSuccess) e = grow_pinned((void **)&H->h_dec, &H->h_dec_cap, rb + out_bytes);
+    if (e != cudaSuccess) return streams_fail(e);
+    rc = afsk_rx_decode(H->plan, x, H->d_out, H->d_res, st);
+    if (rc != AFSK_OK) return rc;
+    int nl = 0;
+    afsk_rx_plan_launches(H->plan, &nl);
+    H->n_launches += nl;
+    AFSK_CUDA(cudaMemcpyAsync(H->h_dec, H->d_res, rb, cudaMemcpyDeviceToHost, st));
+    AFSK_CUDA(cudaMemcpyAsync(H->h_dec + rb, H->d_out, out_bytes, cudaMemcpyDeviceToHost, st));
+    AFSK_CUDA(cudaStreamSynchronize(st));
+    *rr = reinterpret_cast<const AfskRxResult *>(H->h_dec);
+    *res_bytes = rb;
+    return AFSK_OK;
+}
+
+static int streams_bits(AfskRxStreams *H, cudaStream_t st, const int64_t *out_first);
 
 // one push (fin == NULL) or the end of the streams s with fin[s] != 0 (no samples); then, when new_baud is
 // given, every channel's settings become new_baud[s] / new_params[s] for its next stream.  A push is planar
@@ -3324,80 +3553,28 @@ static int streams_run(AfskRxStreams *H, const int16_t *samples, int on_device, 
     int64_t *tf_app = reinterpret_cast<int64_t *>(hd + H->o_tf_app), *tf_mov = reinterpret_cast<int64_t *>(hd + H->o_tf_mov);
     int64_t *first = reinterpret_cast<int64_t *>(hd + H->o_first), *amp_off = reinterpret_cast<int64_t *>(hd + H->o_amp_off);
     int64_t *out_first = reinterpret_cast<int64_t *>(hd + H->o_out_first);
-    auto add_seg = [](CopySeg *seg, int64_t *tf, int &n, int64_t src, int64_t dst, int64_t len) {
-        if (len <= 0) return;
-        const int64_t vecs = ((dst + len + 7) >> 3) - (dst >> 3);
-        seg[n] = CopySeg{src, dst, len};
-        tf[n + 1] = tf[n] + (vecs + kCopyTileVecs - 1) / kCopyTileVecs;
-        n++;
-    };
-    // retention (see above): which channels overflow, and do their new slots fit above the top?
-    auto overflows = [&](int s) { return H->np[s] - H->slot_base[s] > H->slot_cap[s]; };
-    auto rewinds = [&](int s) { return 2 * (H->np[s] - H->keep[s]) <= H->slot_cap[s]; };
-    auto fresh_cap = [&](int s) { return (2 * (H->np[s] - H->keep[s]) + 2 * C + 7) & ~(int64_t)7; };
-    int64_t want = 0;
-    bool any = false;
-    for (int s = 0; s < S; s++)
-        if (overflows(s)) {
-            any = true;
-            if (!rewinds(s)) want += fresh_cap(s);
-        }
-    const bool compact = any && H->top + want > arena_frames(H->arena_cap[H->cur]);
     int nmov = 0, napp = 0;
-    tf_mov[0] = tf_app[0] = 0;
-    if (compact) {
-        int64_t total = 0;
-        for (int s = 0; s < S; s++) {
-            H->new_off[s] = total;
-            H->new_cap[s] = fresh_cap(s);
-            total += H->new_cap[s];
-        }
-        const int nxt = H->cur ^ 1;
-        e = grow_device((void **)&H->arena[nxt], &H->arena_cap[nxt], (size_t)(total + total / 2 + kSlotPad) * 2);
-        if (e != cudaSuccess) return streams_fail(e);
-        for (int s = 0; s < S; s++) {
-            add_seg(seg_mov, tf_mov, nmov, H->slot_off[s] + H->keep[s] - H->slot_base[s], H->new_off[s], H->pushed[s] - H->keep[s]);
-            H->slot_off[s] = H->new_off[s]; H->slot_cap[s] = H->new_cap[s]; H->slot_base[s] = H->keep[s];
-        }
-        H->top = total;
-        H->n_compactions++;
-    } else if (any) {
-        // within the arena: sources are the retained spans, destinations the slot starts (below the span: a
-        // rewind happens only when the span fills at most half the slot) or fresh space above the top
-        for (int s = 0; s < S; s++) {
-            if (!overflows(s)) continue;
-            const int64_t src = H->slot_off[s] + H->keep[s] - H->slot_base[s];
-            if (!rewinds(s)) {
-                H->slot_off[s] = H->top;
-                H->slot_cap[s] = fresh_cap(s);
-                H->top += H->slot_cap[s];
-            }
-            add_seg(seg_mov, tf_mov, nmov, src, H->slot_off[s], H->pushed[s] - H->keep[s]);
-            H->slot_base[s] = H->keep[s];
-        }
-    }
-    for (int i = 0; i < nmov; i++) H->n_moved += seg_mov[i].len;
+    bool compact = false;
+    e = slots_retain(H->smp, S, H->pushed.data(), H->np.data(), H->keep.data(), H->new_off.data(), H->new_cap.data(), seg_mov, tf_mov,
+                     nmov, compact);
+    if (e != cudaSuccess) return streams_fail(e);
+    Slots &A = H->smp;
+    tf_app[0] = 0;
     first[0] = 0;
     for (int s = 0; s < S; s++) {
         // (interleaved: src is the channel's column, which only a one-channel push reads as a k_stream_copy segment)
         const int64_t src = finish ? 0 : interleaved ? s : off[s] - (on_device ? 0 : off[0]);
-        add_seg(seg_app, tf_app, napp, src, H->slot_off[s] + H->pushed[s] - H->slot_base[s], piece(s));
+        add_seg(seg_app, tf_app, napp, src, A.off[s] + H->pushed[s] - A.base[s], piece(s));
         const int64_t c_old = H->pushed[s] / C;
         first[s + 1] = first[s] + H->np[s] / C - c_old;
-        amp_off[s] = H->slot_off[s] + c_old * C - H->slot_base[s];
+        amp_off[s] = A.off[s] + c_old * C - A.base[s];
         out_first[s] = first[s] + s;
     }
     if (finish) memcpy(hd + H->o_fin, fin, (size_t)S);
     AFSK_CUDA(cudaMemcpyAsync(H->d_desc, H->h_desc, finish ? H->desc_bytes : H->o_fin, cudaMemcpyHostToDevice, st));
     const uint8_t *dd = H->d_desc;
-    if (nmov > 0) {
-        k_stream_copy<<<(unsigned)tf_mov[nmov], kCopyThreads, 0, st>>>(H->arena[H->cur], H->arena[compact ? H->cur ^ 1 : H->cur],
-                                                                      reinterpret_cast<const CopySeg *>(dd + H->o_seg_mov),
-                                                                      reinterpret_cast<const int64_t *>(dd + H->o_tf_mov), nmov);
-        H->n_launches++;
-    }
-    if (compact) H->cur ^= 1;
-    int16_t *x = H->arena[H->cur];
+    slots_move(A, compact, nmov, dd + H->o_seg_mov, dd + H->o_tf_mov, tf_mov[nmov], st, H->n_launches);
+    int16_t *x = A.arena[A.cur];
     if (napp > 0) {
         const int16_t *src = samples;
         if (!on_device) {
@@ -3432,68 +3609,63 @@ static int streams_run(AfskRxStreams *H, const int16_t *samples, int on_device, 
     AFSK_CUDA(cudaMemcpyAsync(H->h_ranges, H->d_ranges, sizeof(int64_t) * 3 * (size_t)(nch + S), cudaMemcpyDeviceToHost, st));
     AFSK_CUDA(cudaStreamSynchronize(st));
 
-    // final calls, ordered by (channel, call); recordings as ranges of the arena
-    H->ev.clear();
-    H->rec_start.clear();
-    H->rec_len.clear();
-    H->rec_baud.clear();
-    H->rec_amp_end.clear();
-    for (int s = 0; s < S; s++) {
-        const int64_t *r = H->h_ranges + 3 * out_first[s];
-        for (int k = 0; k < H->h_counts[s]; k++) {
-            AfskRxStreamEvent v;
-            v.stream = s; v.recorded = (int32_t)r[3 * k]; v.call = H->calls[s] + k; v.start = r[3 * k + 1]; v.end = r[3 * k + 2];
-            H->ev.push_back(v);
-            if (v.recorded) {
-                H->rec_start.push_back(H->slot_off[s] + v.start - H->slot_base[s]);
-                H->rec_len.push_back(v.end - v.start);
-                H->rec_baud.push_back(H->baud[s]);
-                H->rec_amp_end.push_back(H->params[s].amp_end);
+    if (H->retain == AFSK_RETAIN_BITS) {
+        const int rc = streams_bits(H, st, out_first);
+        if (rc != AFSK_OK) return rc;
+    } else {
+        // final calls, ordered by (channel, call); recordings as ranges of the arena
+        H->ev.clear();
+        H->rec_start.clear();
+        H->rec_len.clear();
+        H->rec_baud.clear();
+        H->rec_amp_end.clear();
+        for (int s = 0; s < S; s++) {
+            const int64_t *r = H->h_ranges + 3 * out_first[s];
+            for (int k = 0; k < H->h_counts[s]; k++) {
+                AfskRxStreamEvent v;
+                v.stream = s; v.recorded = (int32_t)r[3 * k]; v.call = H->calls[s] + k; v.start = r[3 * k + 1]; v.end = r[3 * k + 2];
+                H->ev.push_back(v);
+                if (v.recorded) {
+                    H->rec_start.push_back(A.off[s] + v.start - A.base[s]);
+                    H->rec_len.push_back(v.end - v.start);
+                    H->rec_baud.push_back(H->baud[s]);
+                    H->rec_amp_end.push_back(H->params[s].amp_end);
+                }
             }
+            const GateState &g = H->h_state[s];
+            H->calls[s] = g.call;
+            H->pushed[s] = H->np[s];
+            H->pending[s] = g.phase == 2 ? g.mark * C : -1;
+            H->keep[s] = g.phase == 2 ? g.mark * C : g.pos * C;
         }
-        const GateState &g = H->h_state[s];
-        H->calls[s] = g.call;
-        H->pushed[s] = H->np[s];
-        H->pending[s] = g.phase == 2 ? g.mark * C : -1;
-        H->keep[s] = g.phase == 2 ? g.mark * C : g.pos * C;
-    }
-    const int nev = (int)H->ev.size(), nrec = (int)H->rec_start.size();
-    H->res.assign((size_t)nev, AfskRxResult{0, -1, -1, 0, 0});
-    H->payload_off.assign((size_t)nev + 1, 0);
-    H->payload.clear();
-    if (nrec > 0) {
-        int rc = H->plan ? afsk_rx_plan_reset(H->plan, nrec, H->rec_start.data(), H->rec_len.data(), H->rec_baud.data(), H->rec_amp_end.data())
-                         : afsk_rx_plan_create_ranges(H->device, nrec, H->rec_start.data(), H->rec_len.data(), H->rec_baud.data(),
-                                                      H->rec_amp_end.data(), &H->plan);
-        if (rc != AFSK_OK) return rc;
-        const int64_t *oo = H->plan->out_off.data();
-        const size_t res_bytes = sizeof(AfskRxResult) * (size_t)nrec, out_bytes = (size_t)oo[nrec];
-        e = grow_device((void **)&H->d_out, &H->out_cap, out_bytes);
-        if (e == cudaSuccess) e = grow_device((void **)&H->d_res, &H->res_cap, res_bytes);
-        if (e == cudaSuccess) e = grow_pinned((void **)&H->h_dec, &H->h_dec_cap, res_bytes + out_bytes);
-        if (e != cudaSuccess) return streams_fail(e);
-        rc = afsk_rx_decode(H->plan, x, H->d_out, H->d_res, st);
-        if (rc != AFSK_OK) return rc;
-        int nl = 0;
-        afsk_rx_plan_launches(H->plan, &nl);
-        H->n_launches += nl;
-        AFSK_CUDA(cudaMemcpyAsync(H->h_dec, H->d_res, res_bytes, cudaMemcpyDeviceToHost, st));
-        AFSK_CUDA(cudaMemcpyAsync(H->h_dec + res_bytes, H->d_out, out_bytes, cudaMemcpyDeviceToHost, st));
-        AFSK_CUDA(cudaStreamSynchronize(st));
-        const AfskRxResult *rr = reinterpret_cast<const AfskRxResult *>(H->h_dec);
-        H->payload.assign(H->h_dec + res_bytes, H->h_dec + res_bytes + out_bytes);
-        int k = 0;
-        for (int i = 0; i < nev; i++) {
-            H->payload_off[i] = oo[k];
-            if (H->ev[i].recorded) H->res[i] = rr[k++];
+        const int nev = (int)H->ev.size(), nrec = (int)H->rec_start.size();
+        H->res.assign((size_t)nev, AfskRxResult{0, -1, -1, 0, 0});
+        H->payload_off.assign((size_t)nev + 1, 0);
+        H->payload.clear();
+        if (nrec > 0) {
+            const AfskRxResult *rr = nullptr;
+            const int64_t *oo = nullptr;
+            size_t res_bytes = 0;
+            const int rc = streams_decode_plan(H, x, st, &rr, &oo, &res_bytes);
+            if (rc != AFSK_OK) return rc;
+            H->payload.assign(H->h_dec + res_bytes, H->h_dec + res_bytes + oo[nrec]);
+            int k = 0;
+            for (int i = 0; i < nev; i++) {
+                H->payload_off[i] = oo[k];
+                if (H->ev[i].recorded) H->res[i] = rr[k++];
+            }
+            H->payload_off[nev] = oo[nrec];
         }
-        H->payload_off[nev] = oo[nrec];
     }
     if (finish)                                    // the next push is frame 0 of a new stream (k_gate_multi reset its state)
         for (int s = 0; s < S; s++)
             if (fin[s]) {
-                H->pushed[s] = H->keep[s] = H->calls[s] = H->slot_base[s] = 0;
+                H->pushed[s] = H->keep[s] = H->calls[s] = A.base[s] = 0;
                 H->pending[s] = -1;
+                if (H->retain == AFSK_RETAIN_BITS) {
+                    H->pclock[s] = -1;
+                    H->pdecided[s] = H->pw_rec[s] = H->pw_pushed[s] = H->pw_keep[s] = H->pln.base[s] = 0;
+                }
             }
     if (new_baud) {
         AFSK_CUDA(cudaMemcpyAsync(H->d_params, new_params, sizeof(GateParams) * S, cudaMemcpyHostToDevice, st));
@@ -3501,7 +3673,236 @@ static int streams_run(AfskRxStreams *H, const int16_t *samples, int on_device, 
         H->baud.assign(new_baud, new_baud + S);
         H->params.assign(new_params, new_params + S);
     }
-    *n_events = nev;
+    *n_events = (int64_t)H->ev.size();
+    return AFSK_OK;
+}
+
+// The rest of a bits-mode push, after the gate: the final calls (a recording that was pending with its clock stored
+// is framed from its planes, any other through the plan), clocks of the pending recordings that now have 4096
+// frames, the plane slots, the windows decided, and the channels' new state.
+static int streams_bits(AfskRxStreams *H, cudaStream_t st, const int64_t *out_first)
+{
+    const int S = H->S;
+    const int64_t C = AFSK_GATE_CHUNK;
+    Slots &A = H->smp, &Pl = H->pln;
+    const int16_t *x = A.arena[A.cur];
+    uint8_t *hb = H->h_bdesc;
+    const uint8_t *db = H->d_bdesc;
+    CapDesc *ccap = reinterpret_cast<CapDesc *>(hb + H->o_ccap), *fcap = reinterpret_cast<CapDesc *>(hb + H->o_fcap);
+    int32_t *cq = reinterpret_cast<int32_t *>(hb + H->o_cq), *fclk = reinterpret_cast<int32_t *>(hb + H->o_fclk);
+    int32_t *h_clk = reinterpret_cast<int32_t *>(hb + H->o_clk);
+    CopySeg *seg_pmov = reinterpret_cast<CopySeg *>(hb + H->o_seg_pmov);
+    int64_t *tf_pmov = reinterpret_cast<int64_t *>(hb + H->o_tf_pmov), *tf_win = reinterpret_cast<int64_t *>(hb + H->o_tf_win);
+    WinJob *win = reinterpret_cast<WinJob *>(hb + H->o_win);
+
+    // final calls, ordered by (channel, call): src[i] >= 0 plan capture, <= -2 frame capture -2 - src[i], -1 none
+    H->ev.clear();
+    H->rec_start.clear();
+    H->rec_len.clear();
+    H->rec_baud.clear();
+    H->rec_amp_end.clear();
+    std::vector<int> src, fch(S, -1), fev;         // fch[s]: the channel's frame capture, fev[j]: its event
+    int nf = 0;
+    for (int s = 0; s < S; s++) {
+        const int64_t *r = H->h_ranges + 3 * out_first[s];
+        for (int k = 0; k < H->h_counts[s]; k++) {
+            AfskRxStreamEvent v;
+            v.stream = s; v.recorded = (int32_t)r[3 * k]; v.call = H->calls[s] + k; v.start = r[3 * k + 1]; v.end = r[3 * k + 2];
+            H->ev.push_back(v);
+            if (!v.recorded) {
+                src.push_back(-1);
+            } else if (k == 0 && H->pending[s] == v.start && H->pclock[s] >= 0) {
+                fch[s] = nf;
+                fev.push_back((int)H->ev.size() - 1);
+                src.push_back(-2 - nf++);
+            } else {
+                src.push_back((int)H->rec_start.size());
+                // (a recording whose samples were not kept is one decided from its length and baud alone)
+                H->rec_start.push_back(v.start < H->keep[s] ? 0 : A.off[s] + v.start - A.base[s]);
+                H->rec_len.push_back(v.end - v.start);
+                H->rec_baud.push_back(H->baud[s]);
+                H->rec_amp_end.push_back(H->params[s].amp_end);
+            }
+        }
+    }
+    // the recordings pending after this push; clocks of those that reached 4096 frames
+    std::vector<int64_t> R(S), clk(S), dec(S, 0), pw0(S, 0), pw_np(S);
+    std::vector<uint8_t> stored(S, 0);             // the recording was pending with its clock stored, and still is
+    std::vector<int> cch;
+    uint32_t qmask = 0;
+    int nq[7] = {0};
+    for (int s = 0; s < S; s++) {
+        const GateState &g = H->h_state[s];
+        R[s] = g.phase == 2 ? g.mark * C : -1;
+        const bool same = R[s] >= 0 && R[s] == H->pending[s];
+        stored[s] = same && H->pclock[s] >= 0;
+        clk[s] = same ? H->pclock[s] : -1;
+        const int bf = bits_bf(H->baud[s]);
+        if (R[s] >= 0 && clk[s] < 0 && bf > 0 && H->np[s] - R[s] >= AFSK_SYNC_FRAMES) {
+            const int c = (int)cch.size();
+            ccap[c] = CapDesc{A.off[s] + R[s] - A.base[s], H->np[s] - R[s], 0, 0, bf, 0, 0, 0};
+            cch.push_back(s);
+            if (bf >= 8 && bf <= 24) nq[bf / 4]++;
+        }
+    }
+    const int nc = (int)cch.size();
+    if (nc > 0) {
+        int qo[7] = {0};
+        for (int q = 2, o = 0; q <= 6; q++) { qo[q] = o; o += nq[q]; }
+        int qn[7] = {0};
+        for (int c = 0; c < nc; c++)
+            if (ccap[c].bf >= 8 && ccap[c].bf <= 24) { const int q = ccap[c].bf / 4; cq[qo[q] + qn[q]++] = c; }
+        AFSK_CUDA(cudaMemcpyAsync(H->d_bdesc, hb, H->o_clk, cudaMemcpyHostToDevice, st));
+        const CapDesc *d_ccap = reinterpret_cast<const CapDesc *>(db + H->o_ccap);
+        const int32_t *d_cq = reinterpret_cast<const int32_t *>(db + H->o_cq);
+        int32_t *d_clk = reinterpret_cast<int32_t *>(H->d_bdesc + H->o_clk);
+        int nqc = 0;
+        for (int q = 2; q <= 6; q++) {
+            if (!nq[q]) continue;
+            switch (q) {
+            case 2: k_clock_q<2><<<nq[q], kClockThreads, 0, st>>>(x, d_ccap, d_cq + qo[q], d_clk); break;
+            case 3: k_clock_q<3><<<nq[q], kClockThreads, 0, st>>>(x, d_ccap, d_cq + qo[q], d_clk); break;
+            case 4: k_clock_q<4><<<nq[q], kClockThreads, 0, st>>>(x, d_ccap, d_cq + qo[q], d_clk); break;
+            case 5: k_clock_q<5><<<nq[q], kClockThreads, 0, st>>>(x, d_ccap, d_cq + qo[q], d_clk); break;
+            default: k_clock_q<6><<<nq[q], kClockThreads, 0, st>>>(x, d_ccap, d_cq + qo[q], d_clk); break;
+            }
+            qmask |= 1u << q;
+            nqc += nq[q];
+            H->n_launches++;
+        }
+        // (no capture here has a status of its own: k_clock writes no result)
+        if (nqc < nc) {
+            k_clock<<<nc, kClockThreads, 0, st>>>(x, d_ccap, d_clk, H->d_fres, qmask);
+            H->n_launches++;
+        }
+        AFSK_CUDA(cudaGetLastError());
+        AFSK_CUDA(cudaMemcpyAsync(h_clk, d_clk, sizeof(int32_t) * nc, cudaMemcpyDeviceToHost, st));
+        AFSK_CUDA(cudaStreamSynchronize(st));
+        for (int c = 0; c < nc; c++) clk[cch[c]] = h_clk[c];
+    }
+    // windows decided after this push, and the end of every channel's plane stream (a final recording's words first)
+    std::vector<int64_t> K(S, 0);
+    for (int s = 0; s < S; s++) {
+        int64_t e = H->pw_pushed[s];
+        if (fch[s] >= 0) {
+            const AfskRxStreamEvent &v = H->ev[fev[fch[s]]];
+            K[s] = windows_of(v.end - v.start, bits_bf(H->baud[s]), H->pclock[s]);
+            e = std::max(e, H->pw_rec[s] + 4 * ((K[s] + 31) / 32));
+        }
+        if (R[s] >= 0 && clk[s] >= 0) {
+            const int bf = bits_bf(H->baud[s]);
+            const int64_t span = H->np[s] - R[s] - clk[s];
+            dec[s] = span > 0 ? (span / bf) & ~(int64_t)31 : 0;
+            pw0[s] = stored[s] ? H->pw_rec[s] : e;
+            e = std::max(e, pw0[s] + 4 * (dec[s] / 32));
+        }
+        pw_np[s] = e;
+    }
+    int npm = 0;
+    bool pcompact = false;
+    cudaError_t err = slots_retain(Pl, S, H->pw_pushed.data(), pw_np.data(), H->pw_keep.data(), H->new_off.data(), H->new_cap.data(),
+                                   seg_pmov, tf_pmov, npm, pcompact);
+    if (err != cudaSuccess) return streams_fail(err);
+    // window jobs (word positions after the moves) and frame captures
+    auto word_at = [&](int s, int64_t pw) { return (Pl.off[s] + pw - Pl.base[s]) / 4; };
+    int nw = 0;
+    tf_win[0] = 0;
+    auto add_job = [&](int s, int64_t x0, int64_t w0, int64_t nwin) {
+        const int bf = bits_bf(H->baud[s]);
+        win[nw] = WinJob{x0, w0, (int32_t)nwin, bf, clamp_thr(H->params[s].amp_end) * bf, 0};
+        tf_win[nw + 1] = tf_win[nw] + ((nwin + 31) / 32 + kWinTileWords - 1) / kWinTileWords;
+        nw++;
+    };
+    int64_t fo = 0, fmax = 0, fsum = 0;
+    for (int s = 0; s < S; s++) {
+        const int bf = bits_bf(H->baud[s]);
+        if (fch[s] >= 0) {
+            const int j = fch[s];
+            const AfskRxStreamEvent &v = H->ev[fev[j]];
+            const int64_t k0 = H->pdecided[s], n = v.end - v.start;
+            if (K[s] > k0)
+                add_job(s, A.off[s] + v.start + H->pclock[s] + k0 * bf - A.base[s], word_at(s, H->pw_rec[s]) + k0 / 32, K[s] - k0);
+            fcap[j] = CapDesc{0, n, word_at(s, H->pw_rec[s]), fo, bf, clamp_thr(H->params[s].amp_end), 0, 0};
+            fclk[j] = (int32_t)H->pclock[s];
+            const int64_t kmax = (n - bf + bf - 1) / bf;
+            fo += (kmax / 14 + 16 + 15) & ~(int64_t)15;
+            fmax = std::max(fmax, kmax);
+            fsum += kmax;
+        }
+        const int64_t d0 = stored[s] ? H->pdecided[s] : 0;
+        if (R[s] >= 0 && clk[s] >= 0 && dec[s] > d0)
+            add_job(s, A.off[s] + R[s] + clk[s] + d0 * bf - A.base[s], word_at(s, pw0[s]) + d0 / 32, dec[s] - d0);
+    }
+    const size_t fres_bytes = sizeof(AfskRxResult) * (size_t)nf;
+    if (nf > 0) {
+        err = grow_device((void **)&H->d_fout, &H->fout_cap, (size_t)fo);
+        if (err == cudaSuccess) err = grow_device((void **)&H->d_fres, &H->fres_cap, fres_bytes);
+        if (err == cudaSuccess) err = grow_pinned((void **)&H->h_fdec, &H->h_fdec_cap, fres_bytes + (size_t)fo);
+        if (err != cudaSuccess) return streams_fail(err);
+    }
+    if (npm > 0 || nw > 0 || nf > 0)
+        AFSK_CUDA(cudaMemcpyAsync(H->d_bdesc + H->o_seg_pmov, hb + H->o_seg_pmov, H->bdesc_bytes - H->o_seg_pmov, cudaMemcpyHostToDevice, st));
+    slots_move(Pl, pcompact, npm, db + H->o_seg_pmov, db + H->o_tf_pmov, tf_pmov[npm], st, H->n_launches);
+    uint2 *planes = reinterpret_cast<uint2 *>(Pl.arena[Pl.cur]);
+    if (nw > 0) {
+        k_stream_windows<<<(unsigned)tf_win[nw], 32 * kWinWarps, 0, st>>>(x, planes, reinterpret_cast<const WinJob *>(db + H->o_win),
+                                                                         reinterpret_cast<const int64_t *>(db + H->o_tf_win), nw);
+        H->n_launches++;
+    }
+    if (nf > 0) {
+        launch_frame(0, nf, reinterpret_cast<const CapDesc *>(db + H->o_fcap), reinterpret_cast<const int32_t *>(db + H->o_fclk), planes,
+                     H->d_fout, H->d_fres, fmax, fsum, nf, st);
+        H->n_launches++;
+        AFSK_CUDA(cudaGetLastError());
+        AFSK_CUDA(cudaMemcpyAsync(H->h_fdec, H->d_fres, fres_bytes, cudaMemcpyDeviceToHost, st));
+        AFSK_CUDA(cudaMemcpyAsync(H->h_fdec + fres_bytes, H->d_fout, (size_t)fo, cudaMemcpyDeviceToHost, st));
+    }
+    AFSK_CUDA(cudaGetLastError());
+    const AfskRxResult *rr = nullptr;
+    const int64_t *oo = nullptr;
+    size_t res_bytes = 0;
+    if (!H->rec_start.empty()) {
+        const int rc = streams_decode_plan(H, x, st, &rr, &oo, &res_bytes);
+        if (rc != AFSK_OK) return rc;
+    } else {
+        AFSK_CUDA(cudaStreamSynchronize(st));
+    }
+    // results and payloads in event order
+    const int nev = (int)H->ev.size();
+    const AfskRxResult *fr = reinterpret_cast<const AfskRxResult *>(H->h_fdec);
+    H->res.assign((size_t)nev, AfskRxResult{0, -1, -1, 0, 0});
+    H->payload_off.assign((size_t)nev + 1, 0);
+    H->payload.clear();
+    for (int i = 0; i < nev; i++) {
+        H->payload_off[i] = (int64_t)H->payload.size();
+        if (src[i] == -1) continue;
+        const uint8_t *p;
+        if (src[i] >= 0) {
+            H->res[i] = rr[src[i]];
+            p = H->h_dec + res_bytes + oo[src[i]];
+        } else {
+            const int j = -2 - src[i];
+            H->res[i] = fr[j];
+            p = H->h_fdec + fres_bytes + fcap[j].out_off;
+        }
+        if (H->res[i].nbytes > 0) H->payload.insert(H->payload.end(), p, p + H->res[i].nbytes);
+    }
+    H->payload_off[nev] = (int64_t)H->payload.size();
+    // the channels' new state
+    for (int s = 0; s < S; s++) {
+        const GateState &g = H->h_state[s];
+        const int bf = bits_bf(H->baud[s]);
+        H->calls[s] = g.call;
+        H->pushed[s] = H->np[s];
+        H->pending[s] = R[s];
+        const bool planes_on = R[s] >= 0 && clk[s] >= 0;
+        H->keep[s] = R[s] < 0 || bf == 0 ? g.pos * C : planes_on ? std::min<int64_t>(g.pos * C, R[s] + clk[s] + dec[s] * bf) : R[s];
+        H->pclock[s] = planes_on ? clk[s] : -1;
+        H->pdecided[s] = planes_on ? dec[s] : 0;
+        H->pw_rec[s] = planes_on ? pw0[s] : 0;
+        H->pw_pushed[s] = pw_np[s];
+        H->pw_keep[s] = planes_on ? pw0[s] : pw_np[s];
+    }
     return AFSK_OK;
 }
 
@@ -3513,6 +3914,15 @@ static int streams_call(AfskRxStreams *H, const int16_t *samples, int on_device,
     if (H->failed) { afsk_set_error("afsk_rx_streams: an earlier push failed; destroy the handle"); return AFSK_E_CUDA; }
     AfskDeviceGuard guard(H->device);
     if (!guard.ok) { afsk_set_error("cannot select device %d", H->device); return AFSK_E_CUDA; }
+    if (H->retain == AFSK_RETAIN_BITS && !fin) {
+        // a window range of one push (WinJob.nwin) spans the piece plus a tail of under 33 bit lengths: below 2^31 windows
+        for (int s = 0; s < H->S; s++)
+            if ((inter >= 0 ? inter : off[s + 1] - off[s]) > kBitsMaxPiece) {
+                afsk_set_error("afsk_rx_streams: bits retention takes at most 2^32 frames per channel and push (channel %d)", s);
+                return AFSK_E_ARG;
+            }
+    }
+    H->used = true;
     const int rc = streams_run(H, samples, on_device, off, inter, (cudaStream_t)stream, fin, new_baud, new_params, n_events);
     if (rc != AFSK_OK) {
         H->failed = true;
@@ -3529,6 +3939,20 @@ static int rx_settings_check(const char *fn, int s, int baud, int64_t timeout_fr
     int bf, ml, sl;
     if (!afsk_tone_geometry(baud, &bf, &ml, &sl)) { afsk_set_error("Invalid baud rate. (%s: channel %d, baud %d)", fn, s, baud); return AFSK_E_BAUD; }
     return AFSK_OK;
+}
+
+// the bits-mode buffers of a handle (set_retention): freed when the handle goes back to samples
+static void streams_free_bits(AfskRxStreams *H)
+{
+    for (void *p : {(void *)H->pln.arena[0], (void *)H->pln.arena[1], (void *)H->d_bdesc, (void *)H->d_fout, (void *)H->d_fres})
+        cudaFree(p);
+    for (void *p : {(void *)H->h_bdesc, (void *)H->h_fdec})
+        if (p) cudaFreeHost(p);
+    H->pln.arena[0] = H->pln.arena[1] = nullptr;
+    H->pln.arena_cap[0] = H->pln.arena_cap[1] = 0;
+    H->d_bdesc = H->h_bdesc = H->d_fout = H->h_fdec = nullptr;
+    H->d_fres = nullptr;
+    H->bdesc_bytes = H->fout_cap = H->fres_cap = H->h_fdec_cap = 0;
 }
 
 int afsk_rx_streams_create_each(int device, int S, const int32_t *h_baud, const int32_t *h_amp_start, const int32_t *h_amp_end,
@@ -3550,9 +3974,11 @@ int afsk_rx_streams_create_each(int device, int S, const int32_t *h_baud, const 
     H->baud.assign(h_baud, h_baud + S);
     H->params.resize((size_t)S);
     for (int s = 0; s < S; s++) H->params[s] = GateParams{h_amp_start[s], h_amp_end[s], h_timeout_frames[s]};
-    for (auto *v : {&H->pushed, &H->keep, &H->calls, &H->slot_off, &H->slot_cap, &H->slot_base, &H->np, &H->new_off, &H->new_cap})
+    for (auto *v : {&H->pushed, &H->keep, &H->calls, &H->smp.off, &H->smp.cap, &H->smp.base, &H->np, &H->new_off, &H->new_cap,
+                    &H->pdecided, &H->pw_rec, &H->pw_pushed, &H->pw_keep, &H->pln.off, &H->pln.cap, &H->pln.base})
         v->assign((size_t)S, 0);
     H->pending.assign((size_t)S, -1);
+    H->pclock.assign((size_t)S, -1);
     size_t o = 0;
     auto carve = [&](size_t bytes) { const size_t at = o; o += (bytes + 15) & ~(size_t)15; return at; };
     H->o_seg_app = carve(sizeof(CopySeg) * S); H->o_tf_app = carve(8 * ((size_t)S + 1));
@@ -3583,6 +4009,36 @@ int afsk_rx_streams_create(int device, int S, int baud, int amp_start, int amp_e
     const std::vector<int32_t> b(n, baud), a0(n, amp_start), a1(n, amp_end);
     const std::vector<int64_t> t(n, timeout_frames < 0 ? 0 : timeout_frames);     // any timeout <= 0 gates alike
     return afsk_rx_streams_create_each(device, S, b.data(), a0.data(), a1.data(), t.data(), h);
+}
+
+int afsk_rx_streams_set_retention(AfskRxStreams *H, int mode)
+{
+    const char *fn = "afsk_rx_streams_set_retention";
+    if (!H || (mode != AFSK_RETAIN_SAMPLES && mode != AFSK_RETAIN_BITS)) { afsk_set_error("%s: bad argument", fn); return AFSK_E_ARG; }
+    if (H->used) { afsk_set_error("%s: the retention mode is chosen before the first push or finish", fn); return AFSK_E_ARG; }
+    AfskDeviceGuard guard(H->device);
+    if (!guard.ok) { afsk_set_error("cannot select device %d", H->device); return AFSK_E_CUDA; }
+    if (mode == AFSK_RETAIN_SAMPLES) {
+        streams_free_bits(H);
+    } else if (!H->d_bdesc) {
+        const size_t S = (size_t)H->S;
+        size_t o = 0;
+        auto carve = [&](size_t bytes) { const size_t at = o; o += (bytes + 15) & ~(size_t)15; return at; };
+        // (the clock part comes first: the clock launches copy the block up to o_clk only)
+        H->o_ccap = carve(sizeof(CapDesc) * S); H->o_cq = carve(sizeof(int32_t) * S); H->o_clk = carve(sizeof(int32_t) * S);
+        H->o_seg_pmov = carve(sizeof(CopySeg) * S); H->o_tf_pmov = carve(8 * (S + 1));
+        H->o_win = carve(sizeof(WinJob) * 2 * S); H->o_tf_win = carve(8 * (2 * S + 1));   // a final tail and a new recording per channel
+        H->o_fcap = carve(sizeof(CapDesc) * S); H->o_fclk = carve(sizeof(int32_t) * S);
+        H->bdesc_bytes = o;
+        cudaError_t e = cudaMalloc((void **)&H->d_bdesc, o);
+        if (e == cudaSuccess) e = cudaMallocHost((void **)&H->h_bdesc, o);
+        if (e != cudaSuccess) {
+            streams_free_bits(H);
+            return streams_fail(e);
+        }
+    }
+    H->retain = mode;
+    return AFSK_OK;
 }
 
 int afsk_rx_streams_push(AfskRxStreams *H, const int16_t *samples, int on_device, const int64_t *h_offsets, void *stream,
@@ -3673,11 +4129,20 @@ int afsk_rx_streams_state(const AfskRxStreams *H, int s, int64_t *pushed, int64_
     return AFSK_OK;
 }
 
+int afsk_rx_streams_pending_bits(const AfskRxStreams *H, int s, int32_t *clock, int64_t *windows)
+{
+    if (!H || s < 0 || s >= H->S) { afsk_set_error("afsk_rx_streams_pending_bits: bad argument"); return AFSK_E_ARG; }
+    if (clock) *clock = H->pending[s] >= 0 ? (int32_t)H->pclock[s] : -1;
+    if (windows) *windows = H->pending[s] >= 0 ? H->pdecided[s] : 0;
+    return AFSK_OK;
+}
+
 int afsk_rx_streams_arena_bytes(const AfskRxStreams *H, int64_t *bytes)
 {
     if (!H || !bytes) return AFSK_E_ARG;
-    *bytes = (int64_t)(H->arena_cap[0] + H->arena_cap[1] + H->stage_cap + H->desc_bytes + H->amp_cap + H->ranges_cap + H->out_cap +
-                       H->res_cap + (sizeof(GateState) + sizeof(int32_t) + sizeof(GateParams)) * (size_t)H->S);
+    *bytes = (int64_t)(H->smp.arena_cap[0] + H->smp.arena_cap[1] + H->stage_cap + H->desc_bytes + H->amp_cap + H->ranges_cap + H->out_cap +
+                       H->res_cap + (sizeof(GateState) + sizeof(int32_t) + sizeof(GateParams)) * (size_t)H->S +
+                       H->pln.arena_cap[0] + H->pln.arena_cap[1] + H->bdesc_bytes + H->fout_cap + H->fres_cap);
     return AFSK_OK;
 }
 
@@ -3685,8 +4150,16 @@ int afsk_rx_streams_counters(const AfskRxStreams *H, int64_t *launches, int64_t 
 {
     if (!H) return AFSK_E_ARG;
     if (launches) *launches = H->n_launches;
-    if (moved_frames) *moved_frames = H->n_moved;
-    if (compactions) *compactions = H->n_compactions;
+    if (moved_frames) *moved_frames = H->smp.n_moved;
+    if (compactions) *compactions = H->smp.n_compactions;
+    return AFSK_OK;
+}
+
+int afsk_rx_streams_plane_counters(const AfskRxStreams *H, int64_t *moved_words, int64_t *compactions)
+{
+    if (!H) { afsk_set_error("afsk_rx_streams_plane_counters: bad argument"); return AFSK_E_ARG; }
+    if (moved_words) *moved_words = H->pln.n_moved / 4;
+    if (compactions) *compactions = H->pln.n_compactions;
     return AFSK_OK;
 }
 
@@ -3695,7 +4168,8 @@ int afsk_rx_streams_destroy(AfskRxStreams *H)
     if (!H) return AFSK_OK;
     AfskDeviceGuard guard(H->device);
     if (H->plan) afsk_rx_plan_destroy(H->plan);
-    for (void *p : {(void *)H->arena[0], (void *)H->arena[1], (void *)H->d_stage, (void *)H->d_desc, (void *)H->d_state,
+    streams_free_bits(H);
+    for (void *p : {(void *)H->smp.arena[0], (void *)H->smp.arena[1], (void *)H->d_stage, (void *)H->d_desc, (void *)H->d_state,
                     (void *)H->d_counts, (void *)H->d_params, (void *)H->d_amp, (void *)H->d_ranges, (void *)H->d_out, (void *)H->d_res})
         cudaFree(p);
     for (void *p : {(void *)H->h_desc, (void *)H->h_state, (void *)H->h_counts, (void *)H->h_ranges, (void *)H->h_dec})

@@ -923,10 +923,10 @@ class Receiver:
             k += 1
         return out
 
-    def open_streams(self, n_streams: int, timeout: float, device: int | None = None) -> StreamReceiver:
+    def open_streams(self, n_streams: int, timeout: float, device: int | None = None, retain: str = "samples") -> StreamReceiver:
         """``receive(timeout)`` called again and again on ``n_streams`` open input streams at once, fed
-        piece by piece as the audio arrives (see ``StreamReceiver``)."""
-        return open_receive_streams([self] * int(n_streams), timeout, self._device if device is None else device)
+        piece by piece as the audio arrives (see ``StreamReceiver``; ``retain`` as for ``open_receive_streams``)."""
+        return open_receive_streams([self] * int(n_streams), timeout, self._device if device is None else device, retain)
 
     def receive(self, timeout: float, string: bool = True) -> bytes | str:
         """Live microphone path (:402-417).  Needs an audio device; out of scope for the GPU core —
@@ -934,15 +934,22 @@ class Receiver:
         raise RuntimeError("afskmodem_b200 has no live audio input; use receive_recording() or load()")
 
 
-def open_receive_streams(receivers, timeout, device: int | None = None) -> StreamReceiver:
+def open_receive_streams(receivers, timeout, device: int | None = None, retain: str = "samples") -> StreamReceiver:
     """``receive(timeout)`` called again and again on S open input streams at once, channel s by
     ``receivers[s]`` with ``timeout`` (seconds: one for all channels, or S of them).  The same Receiver may
     serve many channels, e.g. ``[rx300] * 2048 + [rx1200] * 2048``.  ``device`` defaults to the first
-    receiver's.  See ``StreamReceiver``."""
+    receiver's.
+
+    ``retain`` chooses what the device keeps of a recording that is still open.  ``"samples"`` (the default)
+    keeps all its samples until it ends: 96 KB per second of audio.  ``"bits"`` demodulates it as it arrives:
+    once 4096 frames are in, its clock is recovered, and every push decides its bit windows 32 at a time into
+    2 bits per window (1/320 of the samples at 1200 baud); the channel keeps its samples only from its first
+    undecided window (less than max(4096, 33 bit lengths) frames).  Both modes return the same events, results
+    and values.  See ``StreamReceiver``."""
     receivers = list(receivers)
     if not receivers:
         raise ValueError("open_receive_streams needs at least one receiver")
-    return StreamReceiver(receivers, timeout, receivers[0]._device if device is None else device)
+    return StreamReceiver(receivers, timeout, receivers[0]._device if device is None else device, retain)
 
 
 def _timeout_frames(timeout, n: int) -> np.ndarray:
@@ -997,7 +1004,11 @@ class StreamReceiver:
     of cutting a stream into pushes, the events of all pushes plus ``finish`` are ``listen_gate_multi``
     over the whole stream, and their values ``receive_all(stream, keep_timeouts=True)``."""
 
-    def __init__(self, receivers, timeout, device: int = 0):
+    RETAIN = {"samples": 0, "bits": 1}                           # AFSK_RETAIN_SAMPLES / AFSK_RETAIN_BITS
+
+    def __init__(self, receivers, timeout, device: int = 0, retain: str = "samples"):
+        if retain not in self.RETAIN:
+            raise ValueError(f"retain must be 'samples' or 'bits', got {retain!r}")
         _cabi.require_device(device)
         self.receivers, self.S, self.device = tuple(receivers), len(receivers), device
         self.timeout_frames = _timeout_frames(timeout, self.S)
@@ -1009,6 +1020,9 @@ class StreamReceiver:
                                                              C.byref(h)))
         self._h = h
         self._pinned = None
+        self.retain = retain
+        if retain != "samples":
+            _cabi.check(_cabi.lib().afsk_rx_streams_set_retention(h, self.RETAIN[retain]))
 
     @property
     def receiver(self) -> Receiver:
@@ -1181,13 +1195,23 @@ class StreamReceiver:
 
     def counters(self) -> dict:
         """Since this receiver was opened: kernel launches (decodes included), frames moved to keep retained
-        samples (appends aside) and whole-arena compactions."""
-        a, b, c = C.c_int64(0), C.c_int64(0), C.c_int64(0)
+        samples (appends aside) and whole-arena compactions; in bits mode also the plane words moved to keep
+        open recordings' planes and the plane arena's compactions (both 0 in samples mode)."""
+        a, b, c, d, e = (C.c_int64(0) for _ in range(5))
         _cabi.check(_cabi.lib().afsk_rx_streams_counters(self._h, C.byref(a), C.byref(b), C.byref(c)))
-        return {"launches": a.value, "moved_frames": b.value, "compactions": c.value}
+        _cabi.check(_cabi.lib().afsk_rx_streams_plane_counters(self._h, C.byref(d), C.byref(e)))
+        return {"launches": a.value, "moved_frames": b.value, "compactions": c.value, "moved_plane_words": d.value,
+                "plane_compactions": e.value}
+
+    def pending_bits(self, s: int) -> tuple[int, int]:
+        """(stored clock, windows decided so far) of stream s's pending recording in bits mode: (-1, 0) while its
+        clock is not recovered or no recording is pending; the windows are 0 in samples mode."""
+        a, b = C.c_int32(0), C.c_int64(0)
+        _cabi.check(_cabi.lib().afsk_rx_streams_pending_bits(self._h, int(s), C.byref(a), C.byref(b)))
+        return a.value, b.value
 
     def arena_bytes(self) -> int:
-        """Device bytes this receiver holds (sample arenas, staging, scratch)."""
+        """Device bytes this receiver holds (sample arenas, plane arenas in bits mode, staging, scratch)."""
         n = C.c_int64(0)
         _cabi.check(_cabi.lib().afsk_rx_streams_arena_bytes(self._h, C.byref(n)))
         return n.value

@@ -252,6 +252,24 @@ int afsk_rx_streams_arena_bytes(const AfskRxStreams *h, int64_t *bytes);
  * appends), whole-arena compactions */
 int afsk_rx_streams_counters(const AfskRxStreams *h, int64_t *launches, int64_t *moved_frames, int64_t *compactions);
 int afsk_rx_streams_destroy(AfskRxStreams *h);
+/* Retention modes of a receive handle.  AFSK_RETAIN_SAMPLES (the default) keeps every sample of a pending
+ * recording on the device until it ends.  AFSK_RETAIN_BITS demodulates a pending recording as it arrives: once
+ * 4096 of its frames are in, its clock is recovered and stored, every push decides its complete 32-window plane
+ * words (2 bits per window, in a plane arena with the sample arena's policy), and the channel keeps its samples
+ * only from its first undecided window (or its partial chunk, if earlier).  Recordings whose status follows from
+ * baud and length keep no samples.  Events, results and payloads are those of AFSK_RETAIN_SAMPLES; only state's
+ * retained frames, the counters and arena_bytes differ. */
+#define AFSK_RETAIN_SAMPLES 0
+#define AFSK_RETAIN_BITS 1
+/* before the first push or finish only; AFSK_E_ARG (nothing changed) after it or for an unknown mode.  A bits-mode
+ * push of more than 2^32 frames on one channel returns AFSK_E_ARG and changes nothing. */
+int afsk_rx_streams_set_retention(AfskRxStreams *h, int mode);
+/* channel s's pending recording in bits mode: its stored clock (-1: not yet, or no recording pending) and the
+ * windows decided so far (0 in samples mode) */
+int afsk_rx_streams_pending_bits(const AfskRxStreams *h, int s, int32_t *clock, int64_t *windows);
+/* since creation: plane words moved to keep pending recordings' planes, and whole plane-arena compactions (both
+ * 0 in samples mode) */
+int afsk_rx_streams_plane_counters(const AfskRxStreams *h, int64_t *moved_words, int64_t *compactions);
 
 /* ---------------------------------------------------------------- transmitter ---------- */
 /* frames Transmitter.save writes for a payload of n bytes (afskmodem.py:452-469 then :239-244).

@@ -18,7 +18,14 @@ baud among its final recordings.
 pageable array, as pyaudio's read returns it), three ways in one run: push_interleaved (the GPU de-interleaves it),
 a host numpy transpose into the pinned planar buffer followed by push, and .t().contiguous() on the device followed
 by push, which is what a user had to do without push_interleaved.  The profiled run then times
-k_stream_deinterleave and k_stream_copy's planar append over the same pieces (4 bytes moved per appended frame)."""
+k_stream_deinterleave and k_stream_copy's planar append over the same pieces (4 bytes moved per appended frame).
+
+--retain samples,bits runs every configuration once per retention mode, one after the other, on the same traffic
+(open_receive_streams(..., retain=...)), and adds a profiled bits-mode run that times k_stream_windows over the
+frames it demodulates (2 bytes read per frame of every window it decides, counted from pending_bits and the final
+calls).  --windows-bauds profiles it alone at the given bauds on channels whose recordings never close, --stuck
+records arena_bytes() against pushed seconds on such channels for each mode (samples mode stops after 60 s), and
+--loopback S times BASELINE config 4 (64 KB at 300 baud) looped back from a transmitter on S channels in bits mode."""
 from __future__ import annotations
 
 import argparse
@@ -67,7 +74,7 @@ def mix_groups(S: int):
 
 
 def run_config(base, d_base, S: int, piece: int, T: int, device: bool, timeout: float, mix: bool = False,
-               route: str = "planar"):
+               route: str = "planar", retain: str = "samples"):
     """base / d_base: one traffic stream, or with mix one per baud of MIX_BAUDS; route: planar, interleaved,
     host-transpose or device-transpose (see --layout)"""
     import torch
@@ -75,16 +82,16 @@ def run_config(base, d_base, S: int, piece: int, T: int, device: bool, timeout: 
     offsets = np.arange(S + 1, dtype=np.int64) * piece
     pinned = _cabi.PinnedArray((S * piece + 8,), np.int16)
     out = {"S": S, "piece": piece, "input": "device" if device else "host-pinned", "pushes": n_push, "mix": mix,
-           "route": route}
+           "route": route, "retain": retain}
     if route != "planar" and not device:
         out["input"] = "host"
     if mix:
         groups = mix_groups(S)
         rxs = [A.Receiver(b, *MIX_THRESHOLDS[k % 3]) for b, _, n in groups for k in range(n)]
-        st = A.open_receive_streams(rxs, timeout)
+        st = A.open_receive_streams(rxs, timeout, retain=retain)
     else:
         groups = [(1200, 0, S)]
-        st = A.Receiver(1200).open_streams(S, timeout)
+        st = A.Receiver(1200).open_streams(S, timeout, retain=retain)
         base, d_base = [base], [d_base]
     with st:
         for rep in range(2):
@@ -141,9 +148,150 @@ def run_config(base, d_base, S: int, piece: int, T: int, device: bool, timeout: 
             # staging copy is not in this figure
             "device_bytes_per_frame": 4 + 2 + (2 * rec_frames + 4 * (c1["moved_frames"] - c0["moved_frames"])) / frames,
             "arena_bytes": arena,
+            "moved_plane_words": c1["moved_plane_words"] - c0["moved_plane_words"],
+            "plane_compactions": c1["plane_compactions"] - c0["plane_compactions"],
         })
     pinned.close()
     return out
+
+
+def windows_decided(st, ev, before, bf):
+    """windows k_stream_windows decided in one bits-mode push: before[s] = (pending start, clock, windows) of channel s
+    before it; a final recording that was pending with its clock stored ends with windows [windows, K)"""
+    n = 0
+    for i in np.flatnonzero(ev.recorded):
+        s = int(ev.stream[i])
+        R, clk, w = before[s]
+        if int(ev.start[i]) == R and clk >= 0:
+            span = int(ev.end[i] - ev.start[i]) - bf - clk
+            n += max(0, (span + bf - 1) // bf - w) if span > 0 else 0
+            before[s] = (-1, -1, 0)
+    for s in range(st.S):
+        R, clk, w = before[s]
+        pend = st.state(s)[1]
+        c, w1 = st.pending_bits(s)
+        n += w1 - (w if pend == R and c == clk else 0)
+    return n
+
+
+def profile_bits(d_base, S: int, piece: int, T: int, timeout: float):
+    """k_stream_windows in a bits-mode run of its own (torch.profiler): kernel time and GB/s over the frames it
+    demodulates"""
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+    n_push = T // piece
+    offsets = np.arange(S + 1, dtype=np.int64) * piece
+    pieces = [torch.as_strided(d_base, (S, piece), (SHIFT, 1), i * piece).contiguous().view(-1) for i in range(n_push)]
+    rx, bf = A.Receiver(1200), 40
+    with rx.open_streams(S, timeout, retain="bits") as st:
+        for t in pieces:
+            st.push(t, offsets)
+        st.finish()
+        torch.cuda.synchronize()
+        wins = 0
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            for t in pieces:
+                before = [(st.state(s)[1],) + st.pending_bits(s) for s in range(S)]
+                ev = st.push(t, offsets)
+                wins += windows_decided(st, ev, before, bf)
+        st.finish()
+    ms = 0.0
+    for e in prof.key_averages():
+        if "k_stream_windows" in e.key:
+            us = getattr(e, "device_time_total", None)
+            ms += (us if us is not None else getattr(e, "cuda_time_total", 0.0)) / 1e3
+    nbytes = 2 * bf * wins
+    return {"S": S, "piece": piece, "pushes": n_push, "kernel": "k_stream_windows", "windows": wins, "frames": bf * wins,
+            "kernel_ms": ms, "kernel_us_per_push": ms * 1e3 / n_push, "GBps": nbytes / (ms * 1e-3) / 1e9 if ms else None}
+
+
+def stuck_carrier(S: int, seconds: int, mode: str, samples_cap_s: int = 60):
+    """arena_bytes() against pushed seconds on recordings that never close: a short message, then a full-scale 1200 Hz
+    carrier with no quiet chunk, 1 s device pushes at 1200 baud (samples mode stops after samples_cap_s seconds)"""
+    import torch
+    t = torch.arange(48000, device="cuda", dtype=torch.float64)
+    block = torch.round(30000 * torch.sin(2 * np.pi * 1200 * t / 48000)).to(torch.int16)
+    fr = torch.from_numpy(A.Transmitter(1200, 0.1).encode_batch([b"stuck"]).frames(0)[:-4800].copy()).cuda()
+    head = block.clone()
+    head[100:100 + len(fr)] = fr
+    offsets = np.arange(S + 1, dtype=np.int64) * 48000
+    out = []
+    with A.Receiver(1200).open_streams(S, 5.0, retain=mode) as st:
+        for i in range(seconds if mode == "bits" else min(seconds, samples_cap_s)):
+            st.push((head if i == 0 else block).repeat(S), offsets)
+            out.append([i + 1, st.arena_bytes()])
+        st.finish()
+    return {"S": S, "retain": mode, "seconds_vs_arena_bytes": out}
+
+
+def profile_windows(baud: int, S: int, pushes: int):
+    """k_stream_windows alone at one bit length (torch.profiler): S channels whose recordings never close (a message,
+    then a full-scale carrier), 1 s device pushes after the clocks are stored; GB/s over the frames of the windows it
+    decides (2 bytes each), counted from pending_bits"""
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+    bf = 48000 // baud
+    t = torch.arange(48000, device="cuda", dtype=torch.float64)
+    block = torch.round(30000 * torch.sin(2 * np.pi * 1200 * t / 48000)).to(torch.int16).repeat(S)
+    offsets = np.arange(S + 1, dtype=np.int64) * 48000
+    with A.Receiver(baud).open_streams(S, 5.0, retain="bits") as st:
+        for _ in range(3):
+            st.push(block, offsets)
+        w0 = sum(st.pending_bits(s)[1] for s in range(S))
+        torch.cuda.synchronize()
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            for _ in range(pushes):
+                st.push(block, offsets)
+        w1 = sum(st.pending_bits(s)[1] for s in range(S))
+        st.finish()
+    ms = 0.0
+    for e in prof.key_averages():
+        if "k_stream_windows" in e.key:
+            us = getattr(e, "device_time_total", None)
+            ms += (us if us is not None else getattr(e, "cuda_time_total", 0.0)) / 1e3
+    frames = (w1 - w0) * bf
+    return {"baud": baud, "bf": bf, "S": S, "pushes": pushes, "windows": w1 - w0, "frames": frames, "kernel_ms": ms,
+            "kernel_us_per_push": ms * 1e3 / pushes, "GBps": 2 * frames / (ms * 1e-3) / 1e9 if ms else None}
+
+
+def loopback_config4(S: int):
+    """BASELINE config 4 on S channels: 64 KB random payloads at 300 baud (146.8 M frames each) from a streaming
+    transmitter, pulled into a device tensor and pushed in 1 s pieces into a bits-mode receiver; start frames spread
+    over chunk phases.  Wall time, decoded messages, peak arena_bytes()"""
+    import torch
+    rng = np.random.default_rng(8400)
+    pays = [rng.integers(0, 256, 65536, dtype=np.uint8).tobytes() for _ in range(S)]
+    ok, peak = 0, 0
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    with A.open_transmit_streams([A.Transmitter(300, 0.1)] * S) as tx, A.Receiver(300).open_streams(S, 10.0, retain="bits") as st:
+        buf = torch.empty(S * 48000, dtype=torch.int16, device="cuda")
+        ends, pushed = 0, 0
+        for g in range(8):
+            ids = list(range(g, S, 8))
+            _, e = tx.send(ids, [pays[s] for s in ids])
+            ends = max(ends, int(e.max()))
+            st.push(tx.pull(257, out=buf), np.arange(S + 1, dtype=np.int64) * 257)
+            pushed += 257
+        total = ends + 4096
+        evs = []
+        while pushed < total:
+            n = min(48000, total - pushed)
+            ev = st.push(tx.pull(n, out=buf), np.arange(S + 1, dtype=np.int64) * n)
+            if len(ev):
+                evs.append(ev)
+            pushed += n
+            peak = max(peak, st.arena_bytes())
+        evs.append(st.finish())
+        for ev in evs:
+            b = ev.batch
+            k = 0
+            for i in np.flatnonzero(ev.recorded):
+                ok += int(b.status[k] == 0 and b.nbits[k] == 917504 and b.payload(k) == pays[int(ev.stream[i])])
+                k += 1
+        torch.cuda.synchronize()
+    return {"S": S, "frames_per_channel": total, "wall_s": time.perf_counter() - t0, "decoded_ok": ok,
+            "peak_arena_bytes": peak}
 
 
 def profile_config(d_base, S: int, piece: int, T: int, timeout: float, out_dir: str | None, route: str = "planar"):
@@ -222,6 +370,11 @@ def main():
     ap.add_argument("--input", default="host,device")
     ap.add_argument("--mix", action="store_true", help="six bauds and three threshold pairs across the channels")
     ap.add_argument("--layout", default="planar", choices=["planar", "interleaved"])
+    ap.add_argument("--stuck", type=int, default=0, help="seconds of stuck-carrier traffic per retention mode")
+    ap.add_argument("--stuck-S", type=int, default=256, help="channels of the stuck-carrier run")
+    ap.add_argument("--windows-bauds", default="", help="bauds at which to profile k_stream_windows alone (bits mode)")
+    ap.add_argument("--loopback", type=int, default=0, help="channels of a config-4 loopback in bits mode (0: none)")
+    ap.add_argument("--retain", default="samples", help="retention modes, run in turn per configuration: samples,bits")
     ap.add_argument("--out", default=None)
     ap.add_argument("--no-profile", action="store_true", help="skip the profiled run of the largest device configuration")
     a = ap.parse_args()
@@ -240,7 +393,8 @@ def main():
         base = traffic(n, rng)
         d_base = torch.from_numpy(base).cuda()
     res = {"card": card(), "torch_device": torch.cuda.get_device_name(0), "seconds_per_channel": a.seconds,
-           "timeout_s": a.timeout, "mix": a.mix, "layout": a.layout, "configs": []}
+           "timeout_s": a.timeout, "mix": a.mix, "layout": a.layout, "retain": a.retain, "configs": []}
+    modes = a.retain.split(",")
     routes = {False: ["planar"], True: ["planar"]}
     if a.layout == "interleaved":
         routes = {False: ["interleaved", "host-transpose"], True: ["interleaved", "device-transpose"]}
@@ -248,10 +402,11 @@ def main():
         for piece in pieces:
             for inp in a.input.split(","):
                 for route in routes[inp == "device"]:
-                    r = run_config(bases, d_bases, S, piece, T, inp == "device", a.timeout, True, route) if a.mix else \
-                        run_config(base, d_base, S, piece, T, inp == "device", a.timeout, route=route)
-                    print(json.dumps(r), flush=True)
-                    res["configs"].append(r)
+                    for mode in modes:
+                        r = run_config(bases, d_bases, S, piece, T, inp == "device", a.timeout, True, route, mode) if a.mix else \
+                            run_config(base, d_base, S, piece, T, inp == "device", a.timeout, route=route, retain=mode)
+                        print(json.dumps(r), flush=True)
+                        res["configs"].append(r)
     if not a.mix and not a.no_profile:                    # the profile and whole-stream lines use uniform traffic
         out_dir = os.path.dirname(os.path.abspath(a.out)) if a.out else None
         res["profile"] = profile_config(d_base, max(Ss), max(pieces), T, a.timeout, out_dir)
@@ -259,6 +414,20 @@ def main():
         if a.layout == "interleaved":
             res["profile_interleaved"] = profile_config(d_base, max(Ss), max(pieces), T, a.timeout, out_dir, "interleaved")
             print(json.dumps({k: v for k, v in res["profile_interleaved"].items() if k != "by_kernel_or_copy"}), flush=True)
+    if a.stuck:
+        res["stuck_carrier"] = [stuck_carrier(a.stuck_S, a.stuck, m) for m in modes]
+        for r in res["stuck_carrier"]:
+            print(json.dumps({"retain": r["retain"], "last": r["seconds_vs_arena_bytes"][-1]}), flush=True)
+    if a.windows_bauds:
+        res["windows_by_baud"] = [profile_windows(int(b), max(Ss), 4) for b in a.windows_bauds.split(",")]
+        for r in res["windows_by_baud"]:
+            print(json.dumps(r), flush=True)
+    if a.loopback:
+        res["loopback_config4"] = loopback_config4(a.loopback)
+        print(json.dumps(res["loopback_config4"]), flush=True)
+    if not a.mix and "bits" in modes:
+        res["profile_bits"] = profile_bits(d_base, max(Ss), max(pieces), T, a.timeout)
+        print(json.dumps(res["profile_bits"]), flush=True)
     if not a.mix:
         res["whole_stream"] = whole_stream_reference(base, T, 16, a.timeout)
         print(json.dumps(res["whole_stream"]), flush=True)
