@@ -35,6 +35,7 @@ SYMBOLS = [
     "afsk_tx_streams_destroy", "afsk_rx_streams_create_each", "afsk_rx_streams_finish_some", "afsk_tx_streams_create_each",
     "afsk_tx_streams_configure", "afsk_rx_streams_push_interleaved", "afsk_tx_streams_pull_interleaved",
     "afsk_rx_streams_set_retention", "afsk_rx_streams_pending_bits", "afsk_rx_streams_plane_counters",
+    "afsk_rx_streams_pending_payload", "afsk_rx_streams_payload_counters",
 ]
 
 
@@ -118,6 +119,8 @@ def lib():
     L.afsk_rx_streams_set_retention.argtypes = [vp, C.c_int]
     L.afsk_rx_streams_pending_bits.argtypes = [vp, C.c_int, i32p, i64p]
     L.afsk_rx_streams_plane_counters.argtypes = [vp, i64p, i64p]
+    L.afsk_rx_streams_pending_payload.argtypes = [vp, C.c_int, i64p, i64p, i32p, vp, C.c_int64, i64p]
+    L.afsk_rx_streams_payload_counters.argtypes = [vp, i64p, i64p]
     L.afsk_tx_num_samples.argtypes = [C.c_int, C.c_int64, C.c_int64, u8p]
     L.afsk_tx_num_samples.restype = C.c_int64
     L.afsk_tx_plan_create.argtypes = [C.c_int, C.c_int, i64p, i32p, i64p, u8p, C.POINTER(vp)]

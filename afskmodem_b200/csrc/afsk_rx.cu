@@ -1608,6 +1608,13 @@ __device__ __forceinline__ uint32_t decode_byte(uint32_t v14, const uint8_t *lut
     return ((uint32_t)lut[v14 & 0x7Fu] << 4) | (uint32_t)lut[(v14 >> 7) & 0x7Fu];
 }
 
+// __scanTraining's terminator (:362-366) over plane word `cur` (decision bits of windows 32j .. 32j + 31) and the word
+// before it: bit t is set when b[k-3] & ~b[k-2] & ~b[k-1] & ~b[k] for k = 32j + t
+__device__ __forceinline__ uint32_t term_mask(uint32_t prev, uint32_t cur)
+{
+    return __funnelshift_l(prev, cur, 3) & ~__funnelshift_l(prev, cur, 2) & ~__funnelshift_l(prev, cur, 1) & ~cur;
+}
+
 // kThreads x kWords plane words are searched per block step: <128,4> for ordinary captures,
 // <512,8> when the captures average more than 65536 windows (e.g. 64 KB payloads at 300 baud).
 // idx_t = int unless a capture has 2^30 or more windows.
@@ -1639,9 +1646,7 @@ __global__ void __launch_bounds__(kThreads) k_frame(const CapDesc *__restrict__ 
             const idx_t j = base + tid + r * kThreads;
             if (j < nwords) {
                 const uint32_t cur = PL[j].x, prev = j ? PL[j - 1].x : 0u;
-                // bit t of M: b[k-3] & ~b[k-2] & ~b[k-1] & ~b[k] for k = 32j + t
-                uint32_t M = __funnelshift_l(prev, cur, 3) & ~__funnelshift_l(prev, cur, 2) &
-                             ~__funnelshift_l(prev, cur, 1) & ~cur;
+                uint32_t M = term_mask(prev, cur);
                 const idx_t rem = K - 32 * j;
                 if (rem < 32) M &= (1u << rem) - 1u;
                 if (M) cand = 32 * j + (__ffs(M) - 1);
@@ -1752,9 +1757,7 @@ __device__ __forceinline__ void frame_capture_warp(int c, const CapDesc &d, int 
         for (int r = kWords - 1; r >= 0; r--) {
             const int j = base + lane + 32 * r;
             if (j < nwords) {
-                // bit t of M: b[k-3] & ~b[k-2] & ~b[k-1] & ~b[k] for k = 32j + t
-                uint32_t M = __funnelshift_l(prv[r], cur[r], 3) & ~__funnelshift_l(prv[r], cur[r], 2) &
-                             ~__funnelshift_l(prv[r], cur[r], 1) & ~cur[r];
+                uint32_t M = term_mask(prv[r], cur[r]);
                 const int rem = K - 32 * j;
                 if (rem < 32) M &= (1u << rem) - 1u;
                 if (M) cand = (unsigned)(32 * j + (__ffs(M) - 1));
@@ -2371,6 +2374,138 @@ __global__ void __launch_bounds__(32 * kWinWarps) k_stream_windows(const int16_t
         }
         const uint32_t bw = __ballot_sync(0xFFFFFFFFu, bit), qw = __ballot_sync(0xFFFFFFFFu, quiet);
         if (lane == 0) planes[J.w0 + wd] = make_uint2(bw, qw);
+    }
+}
+
+// Framing of open recordings as their windows are decided (retention mode AFSK_RETAIN_PAYLOAD).  A channel's pending
+// recording with a stored clock has a FrameState: training (searching for 1,0,0,0 from window `consumed` on), payload
+// (k0 known: searching for the first quiet window from `consumed` on, whole 14-window groups decoded into the channel's
+// payload slot) and ended (k1 found: the result is fixed).  Job j frames windows [consumed, k_end) of one recording from
+// the state the job carries (the host's copy of the state the last push left); a final job (the recording became final
+// with K = k_end windows) then writes its AfskRxResult as k_frame does and copies its payload to out.  A channel can have
+// two jobs in one launch (its recording became final and a new one was framed), so no job reads `state`: each only
+// writes the state it ends with to state[ch] for the host to read back, and a final job that shares its channel with
+// a pending job leaves state[ch] to that job (kFrKeepState), so every slot has at most one writer and no reader.  The
+// planes hold only the words from the one of window consumed - 3 (training) or of the next incomplete byte (payload)
+// on, so nothing below those is read.
+struct __align__(16) FrameState {
+    long long consumed;  // windows framed
+    long long k0;        // payload / ended: first payload window
+    long long k1;        // ended: first quiet window at or after k0
+    long long nbytes;    // bytes decoded into the payload slot
+    int phase;           // 0 training, 1 payload, 2 ended
+    int pad[3];
+};
+static_assert(sizeof(FrameState) == 48, "FrameState layout");
+struct __align__(16) FrameJob {
+    FrameState start;    // the recording's state before this job (zero for a recording whose clock was just stored)
+    int64_t w0;          // plane-arena word of the recording's windows 0 .. 31 (may lie below the words kept)
+    int64_t k_end;       // frame up to this window
+    int64_t y0;          // payload-arena byte of the recording's byte 0
+    int64_t out_off;     // final: offset of the payload in out
+    int32_t ch;          // FrameState of the channel
+    int32_t flags;       // kFrFinal, kFrKeepState
+    int32_t clk, bf;
+    int32_t res;         // final: result index
+    int32_t pad[3];
+};
+constexpr int kFrFinal = 1;       // the recording became final with k_end windows
+constexpr int kFrKeepState = 4;   // final: another job of this launch owns the channel's state (else it is reset)
+constexpr int kStreamFrameWarps = 4;
+
+// minimum over the warp of a non-negative 64-bit value: the high words first, then the low words of the lanes that hold it
+__device__ __forceinline__ long long warp_min64(long long v)
+{
+    const uint32_t hi = __reduce_min_sync(0xFFFFFFFFu, (uint32_t)((unsigned long long)v >> 32));
+    const uint32_t lo = __reduce_min_sync(0xFFFFFFFFu, (uint32_t)((unsigned long long)v >> 32) == hi ? (uint32_t)v : 0xFFFFFFFFu);
+    return (long long)(((unsigned long long)hi << 32) | lo);
+}
+
+__global__ void __launch_bounds__(32 * kStreamFrameWarps) k_stream_frame(const uint2 *__restrict__ planes, uint8_t *__restrict__ pay,
+                                                                        FrameState *__restrict__ state, const FrameJob *__restrict__ jobs,
+                                                                        uint8_t *__restrict__ out, AfskRxResult *__restrict__ res, int n)
+{
+    __shared__ uint8_t lut[128];
+    static_assert(32 * kStreamFrameWarps == 128, "one LUT entry per thread");
+    const int tid = threadIdx.x, lane = tid & 31;
+    lut[tid] = (uint8_t)hamming74_nibble((uint32_t)tid);
+    __syncthreads();
+    const int j = blockIdx.x * kStreamFrameWarps + (tid >> 5);
+    if (j >= n) return;
+    const FrameJob J = jobs[j];
+    FrameState F = J.start;
+    const uint32_t *PW = reinterpret_cast<const uint32_t *>(planes);        // word w: bits PW[2w], quiet PW[2w + 1]
+    const long long K = J.k_end;
+    constexpr long long NONE = 0x7FFFFFFFFFFFFFFFLL;
+    long long c = F.consumed;
+    if (F.phase == 0 && c < K) {
+        // (:362-366) from window c on; a word's predecessor is read only where its bits enter windows >= c
+        long long kt = NONE;
+        for (long long base = c >> 5; base <= (K - 1) >> 5; base += 32) {
+            const long long w = base + lane;
+            long long cand = NONE;
+            if (w <= (K - 1) >> 5) {
+                const uint32_t cur = PW[2 * (J.w0 + w)];
+                const uint32_t prev = (w > 0 && c < 32 * w + 3) ? PW[2 * (J.w0 + w - 1)] : 0u;
+                uint32_t M = term_mask(prev, cur);
+                if (w == (c >> 5)) M &= ~((1u << (c & 31)) - 1u);
+                const long long rem = K - 32 * w;
+                if (rem < 32) M &= (1u << rem) - 1u;
+                if (M) cand = 32 * w + (__ffs(M) - 1);
+            }
+            kt = warp_min64(cand);
+            if (kt != NONE) break;
+        }
+        if (kt != NONE) { F.phase = 1; F.k0 = kt + 1; c = F.k0; } else { c = K; }
+    }
+    if (F.phase == 1) {
+        long long kq = NONE;
+        if (c < K) {
+            // (:372-378) first quiet window at or after c (>= k0)
+            for (long long base = c >> 5; base <= (K - 1) >> 5; base += 32) {
+                const long long w = base + lane;
+                long long cand = NONE;
+                if (w <= (K - 1) >> 5) {
+                    uint32_t M = PW[2 * (J.w0 + w) + 1];
+                    if (w == (c >> 5)) M &= ~((1u << (c & 31)) - 1u);
+                    const long long rem = K - 32 * w;
+                    if (rem < 32) M &= (1u << rem) - 1u;
+                    if (M) cand = 32 * w + (__ffs(M) - 1);
+                }
+                kq = warp_min64(cand);
+                if (kq != NONE) break;
+            }
+        }
+        if (kq != NONE) { F.phase = 2; F.k1 = kq; }
+        c = max(c, K);
+        const long long lim = kq != NONE ? kq : c;                // decoded bytes end before window lim
+        // whole 14-window groups (:393-399), one byte per lane
+        const long long nb = (lim - F.k0) / 14;
+        for (long long i = F.nbytes + lane; i < nb; i += 32) {
+            const long long pos = F.k0 + 14 * i;
+            const uint32_t lo = PW[2 * (J.w0 + (pos >> 5))], hi = PW[2 * (J.w0 + (pos >> 5) + 1)];
+            pay[J.y0 + i] = (uint8_t)decode_byte(__funnelshift_r(lo, hi, (uint32_t)(pos & 31)) & 0x3FFFu, lut);
+        }
+        F.nbytes = max(F.nbytes, nb);
+    }
+    F.consumed = max(F.consumed, c);
+    if (J.flags & kFrFinal) {
+        const long long k0 = F.phase >= 1 ? F.k0 : K, k1 = F.phase == 2 ? F.k1 : K;
+        const long long nbits = k1 - k0;
+        __syncwarp();                                            // the bytes decoded above, read back by other lanes
+        for (long long i = lane; i < F.nbytes; i += 32) out[J.out_off + i] = pay[J.y0 + i];
+        if (lane == 0) {
+            AfskRxResult r;
+            r.status = nbits > 0 ? AFSK_ST_OK : AFSK_ST_NO_DATA;
+            r.clock = J.clk;
+            r.train_end = (long long)J.clk + k0 * J.bf;          // "Training sequence terminated on frame" :368
+            r.nbits = nbits;
+            r.nbytes = nbits > 0 ? F.nbytes : 0;
+            res[J.res] = r;
+            if (!(J.flags & kFrKeepState)) state[J.ch] = FrameState{0, 0, 0, 0, 0, {0, 0, 0}};
+        }
+    } else if (lane == 0) {
+        state[J.ch] = F;
     }
 }
 
@@ -3326,6 +3461,15 @@ int afsk_rx_gate_multi(int device, const int16_t *d_samples, const int64_t *h_of
 // and it is framed from its planes (k_frame_warp / k_frame).  A recording that ends before its clock is stored
 // still has all its samples and is decoded through the plan.  Each window's bit and quiet flag depend on its
 // own samples only, and the final length only decides how many windows count, so the results are the same.
+//
+// Retention mode AFSK_RETAIN_PAYLOAD also frames such a recording push by push (k_stream_frame) over its windows below
+// K_safe = windows_of((g.pos - mark) * 2048, bf, clock), which every later end of the recording includes (it ends at a
+// closing quiet chunk at or after g.pos, or a finish cuts it at its last full chunk), as far as they are decided.  The
+// channel then keeps plane words only from the one its search or its next incomplete byte needs, and its decoded bytes
+// in a payload slot (a third arena with the same policy, two bytes counting as one sample); once the first quiet window
+// after the terminator is found the result is fixed, and it decides no more windows, keeps no planes and keeps samples
+// only from its partial chunk.  When the recording becomes final, the same kernel frames the rest up to its K and
+// writes the result as k_frame does.
 namespace {
 constexpr int64_t kSlotPad = 64;           // samples after the last slot (vector over-reads of the kernels)
 int64_t arena_frames(size_t bytes) { return bytes ? (int64_t)(bytes / 2) - kSlotPad : 0; }
@@ -3480,6 +3624,13 @@ struct AfskRxStreams {
     uint8_t *d_fout = nullptr; size_t fout_cap = 0;
     AfskRxResult *d_fres = nullptr; size_t fres_cap = 0;
     uint8_t *h_fdec = nullptr; size_t h_fdec_cap = 0;
+    // payload mode, per channel: the framing state of the pending recording (h_fst: as the last push left it), and the
+    // channel's payload stream (in samples, two bytes each): where the recording's byte 0 lies, the end used, the first
+    // kept; descriptors (payload moves, frame jobs) in the bits-mode block
+    FrameState *d_fst = nullptr, *h_fst = nullptr;
+    std::vector<int64_t> py_rec, py_pushed, py_keep;
+    Slots pay;
+    size_t o_seg_ymov = 0, o_tf_ymov = 0, o_fjob = 0;
     // what the last push / finish returned
     std::vector<AfskRxStreamEvent> ev;
     std::vector<AfskRxResult> res;
@@ -3609,7 +3760,7 @@ static int streams_run(AfskRxStreams *H, const int16_t *samples, int on_device, 
     AFSK_CUDA(cudaMemcpyAsync(H->h_ranges, H->d_ranges, sizeof(int64_t) * 3 * (size_t)(nch + S), cudaMemcpyDeviceToHost, st));
     AFSK_CUDA(cudaStreamSynchronize(st));
 
-    if (H->retain == AFSK_RETAIN_BITS) {
+    if (H->retain != AFSK_RETAIN_SAMPLES) {
         const int rc = streams_bits(H, st, out_first);
         if (rc != AFSK_OK) return rc;
     } else {
@@ -3662,9 +3813,10 @@ static int streams_run(AfskRxStreams *H, const int16_t *samples, int on_device, 
             if (fin[s]) {
                 H->pushed[s] = H->keep[s] = H->calls[s] = A.base[s] = 0;
                 H->pending[s] = -1;
-                if (H->retain == AFSK_RETAIN_BITS) {
+                if (H->retain != AFSK_RETAIN_SAMPLES) {
                     H->pclock[s] = -1;
                     H->pdecided[s] = H->pw_rec[s] = H->pw_pushed[s] = H->pw_keep[s] = H->pln.base[s] = 0;
+                    H->py_rec[s] = H->py_pushed[s] = H->py_keep[s] = H->pay.base[s] = 0;
                 }
             }
     if (new_baud) {
@@ -3677,14 +3829,17 @@ static int streams_run(AfskRxStreams *H, const int16_t *samples, int on_device, 
     return AFSK_OK;
 }
 
-// The rest of a bits-mode push, after the gate: the final calls (a recording that was pending with its clock stored
-// is framed from its planes, any other through the plan), clocks of the pending recordings that now have 4096
-// frames, the plane slots, the windows decided, and the channels' new state.
+// The rest of a bits- or payload-mode push, after the gate: the final calls (a recording that was pending with its
+// clock stored is framed from its planes, any other through the plan), clocks of the pending recordings that now have
+// 4096 frames, the plane slots, the windows decided, and the channels' new state.  In payload mode the recordings
+// pending with a stored clock are also framed as far as the chunks the gate has walked (k_stream_frame, which frames
+// the final ones too), and a recording whose first quiet window was found decides no more windows.
 static int streams_bits(AfskRxStreams *H, cudaStream_t st, const int64_t *out_first)
 {
     const int S = H->S;
     const int64_t C = AFSK_GATE_CHUNK;
-    Slots &A = H->smp, &Pl = H->pln;
+    const bool pmode = H->retain == AFSK_RETAIN_PAYLOAD;
+    Slots &A = H->smp, &Pl = H->pln, &Y = H->pay;
     const int16_t *x = A.arena[A.cur];
     uint8_t *hb = H->h_bdesc;
     const uint8_t *db = H->d_bdesc;
@@ -3694,6 +3849,9 @@ static int streams_bits(AfskRxStreams *H, cudaStream_t st, const int64_t *out_fi
     CopySeg *seg_pmov = reinterpret_cast<CopySeg *>(hb + H->o_seg_pmov);
     int64_t *tf_pmov = reinterpret_cast<int64_t *>(hb + H->o_tf_pmov), *tf_win = reinterpret_cast<int64_t *>(hb + H->o_tf_win);
     WinJob *win = reinterpret_cast<WinJob *>(hb + H->o_win);
+    CopySeg *seg_ymov = reinterpret_cast<CopySeg *>(hb + H->o_seg_ymov);
+    int64_t *tf_ymov = reinterpret_cast<int64_t *>(hb + H->o_tf_ymov);
+    FrameJob *fjob = reinterpret_cast<FrameJob *>(hb + H->o_fjob);
 
     // final calls, ordered by (channel, call): src[i] >= 0 plan capture, <= -2 frame capture -2 - src[i], -1 none
     H->ev.clear();
@@ -3780,19 +3938,23 @@ static int streams_bits(AfskRxStreams *H, cudaStream_t st, const int64_t *out_fi
         AFSK_CUDA(cudaStreamSynchronize(st));
         for (int c = 0; c < nc; c++) clk[cch[c]] = h_clk[c];
     }
-    // windows decided after this push, and the end of every channel's plane stream (a final recording's words first)
+    // windows decided after this push, and the end of every channel's plane stream (a final recording's words first).
+    // Payload mode: fin_ended / ended, the final / pending recording's result was fixed by the last push (h_fst).
     std::vector<int64_t> K(S, 0);
+    std::vector<uint8_t> fin_ended(S, 0), ended(S, 0);
     for (int s = 0; s < S; s++) {
         int64_t e = H->pw_pushed[s];
+        fin_ended[s] = pmode && fch[s] >= 0 && H->h_fst[s].phase == 2;
+        ended[s] = pmode && stored[s] && H->h_fst[s].phase == 2;
         if (fch[s] >= 0) {
             const AfskRxStreamEvent &v = H->ev[fev[fch[s]]];
             K[s] = windows_of(v.end - v.start, bits_bf(H->baud[s]), H->pclock[s]);
-            e = std::max(e, H->pw_rec[s] + 4 * ((K[s] + 31) / 32));
+            if (!fin_ended[s]) e = std::max(e, H->pw_rec[s] + 4 * ((K[s] + 31) / 32));
         }
         if (R[s] >= 0 && clk[s] >= 0) {
             const int bf = bits_bf(H->baud[s]);
             const int64_t span = H->np[s] - R[s] - clk[s];
-            dec[s] = span > 0 ? (span / bf) & ~(int64_t)31 : 0;
+            dec[s] = ended[s] ? H->pdecided[s] : span > 0 ? (span / bf) & ~(int64_t)31 : 0;
             pw0[s] = stored[s] ? H->pw_rec[s] : e;
             e = std::max(e, pw0[s] + 4 * (dec[s] / 32));
         }
@@ -3803,8 +3965,37 @@ static int streams_bits(AfskRxStreams *H, cudaStream_t st, const int64_t *out_fi
     cudaError_t err = slots_retain(Pl, S, H->pw_pushed.data(), pw_np.data(), H->pw_keep.data(), H->new_off.data(), H->new_cap.data(),
                                    seg_pmov, tf_pmov, npm, pcompact);
     if (err != cudaSuccess) return streams_fail(err);
-    // window jobs (word positions after the moves) and frame captures
+    // payload mode: the windows each pending recording is framed up to (those of the chunks the gate has walked, which
+    // every later end of the recording includes, as far as they are decided), and the end of every channel's payload
+    // stream with room for every byte its frame jobs can write (a final recording's bytes first)
+    std::vector<int64_t> kend(S, 0), py0(S, 0), py_np(S, 0);
+    int nym = 0;
+    bool ycompact = false;
+    if (pmode) {
+        const FrameState fresh = {0, 0, 0, 0, 0, {0, 0, 0}};
+        auto room = [](const FrameState &f, int64_t k) {          // samples, after framing up to window k
+            const int64_t b = f.phase == 2 ? f.nbytes
+                                           : ((f.phase == 1 ? f.consumed - f.k0 : 0) + std::max<int64_t>(k - f.consumed, 0)) / 14 + 1;
+            return (b + 1) / 2;
+        };
+        for (int s = 0; s < S; s++) {
+            const GateState &g = H->h_state[s];
+            int64_t e = H->py_pushed[s];
+            if (fch[s] >= 0) e = std::max(e, H->py_rec[s] + room(H->h_fst[s], K[s]));
+            if (R[s] >= 0 && clk[s] >= 0) {
+                if (!ended[s]) kend[s] = std::min(windows_of((g.pos - g.mark) * C, bits_bf(H->baud[s]), clk[s]), dec[s]);
+                py0[s] = stored[s] ? H->py_rec[s] : e;
+                e = std::max(e, py0[s] + room(stored[s] ? H->h_fst[s] : fresh, kend[s]));
+            }
+            py_np[s] = e;
+        }
+        err = slots_retain(Y, S, H->py_pushed.data(), py_np.data(), H->py_keep.data(), H->new_off.data(), H->new_cap.data(), seg_ymov,
+                           tf_ymov, nym, ycompact);
+        if (err != cudaSuccess) return streams_fail(err);
+    }
+    // window jobs (word positions after the moves), frame captures and frame jobs
     auto word_at = [&](int s, int64_t pw) { return (Pl.off[s] + pw - Pl.base[s]) / 4; };
+    auto byte_at = [&](int s, int64_t py) { return 2 * (Y.off[s] + py - Y.base[s]); };
     int nw = 0;
     tf_win[0] = 0;
     auto add_job = [&](int s, int64_t x0, int64_t w0, int64_t nwin) {
@@ -3814,16 +4005,21 @@ static int streams_bits(AfskRxStreams *H, cudaStream_t st, const int64_t *out_fi
         nw++;
     };
     int64_t fo = 0, fmax = 0, fsum = 0;
+    int nj = 0;
     for (int s = 0; s < S; s++) {
         const int bf = bits_bf(H->baud[s]);
+        const bool frame_new = pmode && kend[s] > (stored[s] ? H->h_fst[s].consumed : 0);
         if (fch[s] >= 0) {
             const int j = fch[s];
             const AfskRxStreamEvent &v = H->ev[fev[j]];
             const int64_t k0 = H->pdecided[s], n = v.end - v.start;
-            if (K[s] > k0)
+            if (K[s] > k0 && !fin_ended[s])
                 add_job(s, A.off[s] + v.start + H->pclock[s] + k0 * bf - A.base[s], word_at(s, H->pw_rec[s]) + k0 / 32, K[s] - k0);
             fcap[j] = CapDesc{0, n, word_at(s, H->pw_rec[s]), fo, bf, clamp_thr(H->params[s].amp_end), 0, 0};
             fclk[j] = (int32_t)H->pclock[s];
+            if (pmode)
+                fjob[nj++] = FrameJob{H->h_fst[s], word_at(s, H->pw_rec[s]), K[s], byte_at(s, H->py_rec[s]), fo, s,
+                                      kFrFinal | (frame_new ? kFrKeepState : 0), (int32_t)H->pclock[s], bf, j, {0, 0, 0}};
             const int64_t kmax = (n - bf + bf - 1) / bf;
             fo += (kmax / 14 + 16 + 15) & ~(int64_t)15;
             fmax = std::max(fmax, kmax);
@@ -3832,6 +4028,9 @@ static int streams_bits(AfskRxStreams *H, cudaStream_t st, const int64_t *out_fi
         const int64_t d0 = stored[s] ? H->pdecided[s] : 0;
         if (R[s] >= 0 && clk[s] >= 0 && dec[s] > d0)
             add_job(s, A.off[s] + R[s] + clk[s] + d0 * bf - A.base[s], word_at(s, pw0[s]) + d0 / 32, dec[s] - d0);
+        if (frame_new)
+            fjob[nj++] = FrameJob{stored[s] ? H->h_fst[s] : FrameState{}, word_at(s, pw0[s]), kend[s], byte_at(s, py0[s]), 0, s, 0,
+                                  (int32_t)clk[s], bf, 0, {0, 0, 0}};
     }
     const size_t fres_bytes = sizeof(AfskRxResult) * (size_t)nf;
     if (nf > 0) {
@@ -3840,19 +4039,29 @@ static int streams_bits(AfskRxStreams *H, cudaStream_t st, const int64_t *out_fi
         if (err == cudaSuccess) err = grow_pinned((void **)&H->h_fdec, &H->h_fdec_cap, fres_bytes + (size_t)fo);
         if (err != cudaSuccess) return streams_fail(err);
     }
-    if (npm > 0 || nw > 0 || nf > 0)
+    if (npm > 0 || nw > 0 || nf > 0 || nym > 0 || nj > 0)
         AFSK_CUDA(cudaMemcpyAsync(H->d_bdesc + H->o_seg_pmov, hb + H->o_seg_pmov, H->bdesc_bytes - H->o_seg_pmov, cudaMemcpyHostToDevice, st));
     slots_move(Pl, pcompact, npm, db + H->o_seg_pmov, db + H->o_tf_pmov, tf_pmov[npm], st, H->n_launches);
+    if (pmode) slots_move(Y, ycompact, nym, db + H->o_seg_ymov, db + H->o_tf_ymov, tf_ymov[nym], st, H->n_launches);
     uint2 *planes = reinterpret_cast<uint2 *>(Pl.arena[Pl.cur]);
     if (nw > 0) {
         k_stream_windows<<<(unsigned)tf_win[nw], 32 * kWinWarps, 0, st>>>(x, planes, reinterpret_cast<const WinJob *>(db + H->o_win),
                                                                          reinterpret_cast<const int64_t *>(db + H->o_tf_win), nw);
         H->n_launches++;
     }
-    if (nf > 0) {
+    if (nj > 0) {
+        k_stream_frame<<<(unsigned)((nj + kStreamFrameWarps - 1) / kStreamFrameWarps), 32 * kStreamFrameWarps, 0, st>>>(
+            planes, reinterpret_cast<uint8_t *>(Y.arena[Y.cur]), H->d_fst, reinterpret_cast<const FrameJob *>(db + H->o_fjob), H->d_fout,
+            H->d_fres, nj);
+        H->n_launches++;
+        AFSK_CUDA(cudaGetLastError());
+        AFSK_CUDA(cudaMemcpyAsync(H->h_fst, H->d_fst, sizeof(FrameState) * S, cudaMemcpyDeviceToHost, st));
+    } else if (nf > 0) {
         launch_frame(0, nf, reinterpret_cast<const CapDesc *>(db + H->o_fcap), reinterpret_cast<const int32_t *>(db + H->o_fclk), planes,
                      H->d_fout, H->d_fres, fmax, fsum, nf, st);
         H->n_launches++;
+    }
+    if (nf > 0) {
         AFSK_CUDA(cudaGetLastError());
         AFSK_CUDA(cudaMemcpyAsync(H->h_fdec, H->d_fres, fres_bytes, cudaMemcpyDeviceToHost, st));
         AFSK_CUDA(cudaMemcpyAsync(H->h_fdec + fres_bytes, H->d_fout, (size_t)fo, cudaMemcpyDeviceToHost, st));
@@ -3896,12 +4105,23 @@ static int streams_bits(AfskRxStreams *H, cudaStream_t st, const int64_t *out_fi
         H->pushed[s] = H->np[s];
         H->pending[s] = R[s];
         const bool planes_on = R[s] >= 0 && clk[s] >= 0;
-        H->keep[s] = R[s] < 0 || bf == 0 ? g.pos * C : planes_on ? std::min<int64_t>(g.pos * C, R[s] + clk[s] + dec[s] * bf) : R[s];
+        // payload mode: what the pending recording's framing still needs (h_fst as this push left it)
+        const FrameState f = pmode ? H->h_fst[s] : FrameState{};
+        const bool fixed = pmode && planes_on && f.phase == 2;
+        const int64_t need = !pmode ? 0 : f.phase == 1 ? f.k0 + 14 * f.nbytes : std::max<int64_t>(f.consumed - 3, 0);
+        H->keep[s] = R[s] < 0 || bf == 0 || fixed ? g.pos * C
+                     : planes_on                  ? std::min<int64_t>(g.pos * C, R[s] + clk[s] + dec[s] * bf)
+                                                  : R[s];
         H->pclock[s] = planes_on ? clk[s] : -1;
         H->pdecided[s] = planes_on ? dec[s] : 0;
         H->pw_rec[s] = planes_on ? pw0[s] : 0;
         H->pw_pushed[s] = pw_np[s];
-        H->pw_keep[s] = planes_on ? pw0[s] : pw_np[s];
+        H->pw_keep[s] = planes_on && !fixed ? pw0[s] + 4 * (need / 32) : pw_np[s];
+        if (pmode) {
+            H->py_rec[s] = planes_on ? py0[s] : 0;
+            H->py_pushed[s] = py_np[s];
+            H->py_keep[s] = planes_on ? py0[s] : py_np[s];
+        }
     }
     return AFSK_OK;
 }
@@ -3914,11 +4134,11 @@ static int streams_call(AfskRxStreams *H, const int16_t *samples, int on_device,
     if (H->failed) { afsk_set_error("afsk_rx_streams: an earlier push failed; destroy the handle"); return AFSK_E_CUDA; }
     AfskDeviceGuard guard(H->device);
     if (!guard.ok) { afsk_set_error("cannot select device %d", H->device); return AFSK_E_CUDA; }
-    if (H->retain == AFSK_RETAIN_BITS && !fin) {
+    if (H->retain != AFSK_RETAIN_SAMPLES && !fin) {
         // a window range of one push (WinJob.nwin) spans the piece plus a tail of under 33 bit lengths: below 2^31 windows
         for (int s = 0; s < H->S; s++)
             if ((inter >= 0 ? inter : off[s + 1] - off[s]) > kBitsMaxPiece) {
-                afsk_set_error("afsk_rx_streams: bits retention takes at most 2^32 frames per channel and push (channel %d)", s);
+                afsk_set_error("afsk_rx_streams: bits and payload retention take at most 2^32 frames per channel and push (channel %d)", s);
                 return AFSK_E_ARG;
             }
     }
@@ -3941,17 +4161,19 @@ static int rx_settings_check(const char *fn, int s, int baud, int64_t timeout_fr
     return AFSK_OK;
 }
 
-// the bits-mode buffers of a handle (set_retention): freed when the handle goes back to samples
+// the bits- and payload-mode buffers of a handle (set_retention): freed when the handle changes its mode
 static void streams_free_bits(AfskRxStreams *H)
 {
-    for (void *p : {(void *)H->pln.arena[0], (void *)H->pln.arena[1], (void *)H->d_bdesc, (void *)H->d_fout, (void *)H->d_fres})
+    for (void *p : {(void *)H->pln.arena[0], (void *)H->pln.arena[1], (void *)H->d_bdesc, (void *)H->d_fout, (void *)H->d_fres,
+                    (void *)H->pay.arena[0], (void *)H->pay.arena[1], (void *)H->d_fst})
         cudaFree(p);
-    for (void *p : {(void *)H->h_bdesc, (void *)H->h_fdec})
+    for (void *p : {(void *)H->h_bdesc, (void *)H->h_fdec, (void *)H->h_fst})
         if (p) cudaFreeHost(p);
-    H->pln.arena[0] = H->pln.arena[1] = nullptr;
-    H->pln.arena_cap[0] = H->pln.arena_cap[1] = 0;
+    H->pln.arena[0] = H->pln.arena[1] = H->pay.arena[0] = H->pay.arena[1] = nullptr;
+    H->pln.arena_cap[0] = H->pln.arena_cap[1] = H->pay.arena_cap[0] = H->pay.arena_cap[1] = 0;
     H->d_bdesc = H->h_bdesc = H->d_fout = H->h_fdec = nullptr;
     H->d_fres = nullptr;
+    H->d_fst = H->h_fst = nullptr;
     H->bdesc_bytes = H->fout_cap = H->fres_cap = H->h_fdec_cap = 0;
 }
 
@@ -3975,7 +4197,8 @@ int afsk_rx_streams_create_each(int device, int S, const int32_t *h_baud, const 
     H->params.resize((size_t)S);
     for (int s = 0; s < S; s++) H->params[s] = GateParams{h_amp_start[s], h_amp_end[s], h_timeout_frames[s]};
     for (auto *v : {&H->pushed, &H->keep, &H->calls, &H->smp.off, &H->smp.cap, &H->smp.base, &H->np, &H->new_off, &H->new_cap,
-                    &H->pdecided, &H->pw_rec, &H->pw_pushed, &H->pw_keep, &H->pln.off, &H->pln.cap, &H->pln.base})
+                    &H->pdecided, &H->pw_rec, &H->pw_pushed, &H->pw_keep, &H->pln.off, &H->pln.cap, &H->pln.base, &H->py_rec,
+                    &H->py_pushed, &H->py_keep, &H->pay.off, &H->pay.cap, &H->pay.base})
         v->assign((size_t)S, 0);
     H->pending.assign((size_t)S, -1);
     H->pclock.assign((size_t)S, -1);
@@ -4014,13 +4237,15 @@ int afsk_rx_streams_create(int device, int S, int baud, int amp_start, int amp_e
 int afsk_rx_streams_set_retention(AfskRxStreams *H, int mode)
 {
     const char *fn = "afsk_rx_streams_set_retention";
-    if (!H || (mode != AFSK_RETAIN_SAMPLES && mode != AFSK_RETAIN_BITS)) { afsk_set_error("%s: bad argument", fn); return AFSK_E_ARG; }
+    if (!H || (mode != AFSK_RETAIN_SAMPLES && mode != AFSK_RETAIN_BITS && mode != AFSK_RETAIN_PAYLOAD)) {
+        afsk_set_error("%s: bad argument", fn);
+        return AFSK_E_ARG;
+    }
     if (H->used) { afsk_set_error("%s: the retention mode is chosen before the first push or finish", fn); return AFSK_E_ARG; }
     AfskDeviceGuard guard(H->device);
     if (!guard.ok) { afsk_set_error("cannot select device %d", H->device); return AFSK_E_CUDA; }
-    if (mode == AFSK_RETAIN_SAMPLES) {
-        streams_free_bits(H);
-    } else if (!H->d_bdesc) {
+    streams_free_bits(H);
+    if (mode != AFSK_RETAIN_SAMPLES) {
         const size_t S = (size_t)H->S;
         size_t o = 0;
         auto carve = [&](size_t bytes) { const size_t at = o; o += (bytes + 15) & ~(size_t)15; return at; };
@@ -4029,9 +4254,19 @@ int afsk_rx_streams_set_retention(AfskRxStreams *H, int mode)
         H->o_seg_pmov = carve(sizeof(CopySeg) * S); H->o_tf_pmov = carve(8 * (S + 1));
         H->o_win = carve(sizeof(WinJob) * 2 * S); H->o_tf_win = carve(8 * (2 * S + 1));   // a final tail and a new recording per channel
         H->o_fcap = carve(sizeof(CapDesc) * S); H->o_fclk = carve(sizeof(int32_t) * S);
+        if (mode == AFSK_RETAIN_PAYLOAD) {
+            H->o_seg_ymov = carve(sizeof(CopySeg) * S); H->o_tf_ymov = carve(8 * (S + 1));
+            H->o_fjob = carve(sizeof(FrameJob) * 2 * S);                                      // a final and a pending recording per channel
+        }
         H->bdesc_bytes = o;
         cudaError_t e = cudaMalloc((void **)&H->d_bdesc, o);
         if (e == cudaSuccess) e = cudaMallocHost((void **)&H->h_bdesc, o);
+        if (e == cudaSuccess && mode == AFSK_RETAIN_PAYLOAD) {
+            e = cudaMalloc((void **)&H->d_fst, sizeof(FrameState) * S);
+            if (e == cudaSuccess) e = cudaMallocHost((void **)&H->h_fst, sizeof(FrameState) * S);
+            if (e == cudaSuccess) e = cudaMemset(H->d_fst, 0, sizeof(FrameState) * S);
+            if (e == cudaSuccess) memset(H->h_fst, 0, sizeof(FrameState) * S);
+        }
         if (e != cudaSuccess) {
             streams_free_bits(H);
             return streams_fail(e);
@@ -4142,7 +4377,8 @@ int afsk_rx_streams_arena_bytes(const AfskRxStreams *H, int64_t *bytes)
     if (!H || !bytes) return AFSK_E_ARG;
     *bytes = (int64_t)(H->smp.arena_cap[0] + H->smp.arena_cap[1] + H->stage_cap + H->desc_bytes + H->amp_cap + H->ranges_cap + H->out_cap +
                        H->res_cap + (sizeof(GateState) + sizeof(int32_t) + sizeof(GateParams)) * (size_t)H->S +
-                       H->pln.arena_cap[0] + H->pln.arena_cap[1] + H->bdesc_bytes + H->fout_cap + H->fres_cap);
+                       H->pln.arena_cap[0] + H->pln.arena_cap[1] + H->bdesc_bytes + H->fout_cap + H->fres_cap +
+                       H->pay.arena_cap[0] + H->pay.arena_cap[1] + (H->d_fst ? sizeof(FrameState) * (size_t)H->S : 0));
     return AFSK_OK;
 }
 
@@ -4160,6 +4396,41 @@ int afsk_rx_streams_plane_counters(const AfskRxStreams *H, int64_t *moved_words,
     if (!H) { afsk_set_error("afsk_rx_streams_plane_counters: bad argument"); return AFSK_E_ARG; }
     if (moved_words) *moved_words = H->pln.n_moved / 4;
     if (compactions) *compactions = H->pln.n_compactions;
+    return AFSK_OK;
+}
+
+int afsk_rx_streams_pending_payload(const AfskRxStreams *H, int s, int64_t *train_end, int64_t *nbits, int32_t *ended, uint8_t *out,
+                                    int64_t cap, int64_t *nbytes)
+{
+    if (!H || s < 0 || s >= H->S || !train_end || !nbits || !ended || !nbytes || cap < 0 || (cap > 0 && !out)) {
+        afsk_set_error("afsk_rx_streams_pending_payload: bad argument");
+        return AFSK_E_ARG;
+    }
+    *train_end = -1; *nbits = 0; *ended = 0; *nbytes = 0;
+    if (H->retain != AFSK_RETAIN_PAYLOAD || H->pending[s] < 0 || H->pclock[s] < 0) return AFSK_OK;
+    const FrameState &f = H->h_fst[s];
+    if (f.phase >= 1) {
+        *train_end = H->pclock[s] + f.k0 * (int64_t)bits_bf(H->baud[s]);
+        *nbits = (f.phase == 2 ? f.k1 : f.consumed) - f.k0;
+    }
+    *ended = f.phase == 2;
+    *nbytes = f.nbytes;
+    const int64_t n = std::min<int64_t>(cap, f.nbytes);
+    if (n > 0) {
+        AfskDeviceGuard guard(H->device);
+        if (!guard.ok) { afsk_set_error("cannot select device %d", H->device); return AFSK_E_CUDA; }
+        const Slots &Y = H->pay;
+        const uint8_t *src = reinterpret_cast<const uint8_t *>(Y.arena[Y.cur]) + 2 * (Y.off[s] + H->py_rec[s] - Y.base[s]);
+        AFSK_CUDA(cudaMemcpy(out, src, (size_t)n, cudaMemcpyDeviceToHost));
+    }
+    return AFSK_OK;
+}
+
+int afsk_rx_streams_payload_counters(const AfskRxStreams *H, int64_t *moved_bytes, int64_t *compactions)
+{
+    if (!H) { afsk_set_error("afsk_rx_streams_payload_counters: bad argument"); return AFSK_E_ARG; }
+    if (moved_bytes) *moved_bytes = 2 * H->pay.n_moved;
+    if (compactions) *compactions = H->pay.n_compactions;
     return AFSK_OK;
 }
 

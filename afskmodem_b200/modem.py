@@ -944,8 +944,12 @@ def open_receive_streams(receivers, timeout, device: int | None = None, retain: 
     keeps all its samples until it ends: 96 KB per second of audio.  ``"bits"`` demodulates it as it arrives:
     once 4096 frames are in, its clock is recovered, and every push decides its bit windows 32 at a time into
     2 bits per window (1/320 of the samples at 1200 baud); the channel keeps its samples only from its first
-    undecided window (less than max(4096, 33 bit lengths) frames).  Both modes return the same events, results
-    and values.  See ``StreamReceiver``."""
+    undecided window (less than max(4096, 33 bit lengths) frames).  ``"payload"`` does what ``"bits"`` does and
+    also frames the recording as its windows are decided: it finds the training sequence's end, Hamming-decodes
+    whole bytes into a payload slot (``pending_payload`` reads them), and keeps only the bit windows it still
+    needs; once the first quiet window after the message is found the result is fixed, and the channel keeps no
+    windows until the recording ends.  All modes return the same events, results and values.  See
+    ``StreamReceiver``."""
     receivers = list(receivers)
     if not receivers:
         raise ValueError("open_receive_streams needs at least one receiver")
@@ -1004,11 +1008,11 @@ class StreamReceiver:
     of cutting a stream into pushes, the events of all pushes plus ``finish`` are ``listen_gate_multi``
     over the whole stream, and their values ``receive_all(stream, keep_timeouts=True)``."""
 
-    RETAIN = {"samples": 0, "bits": 1}                           # AFSK_RETAIN_SAMPLES / AFSK_RETAIN_BITS
+    RETAIN = {"samples": 0, "bits": 1, "payload": 2}             # AFSK_RETAIN_SAMPLES / _BITS / _PAYLOAD
 
     def __init__(self, receivers, timeout, device: int = 0, retain: str = "samples"):
         if retain not in self.RETAIN:
-            raise ValueError(f"retain must be 'samples' or 'bits', got {retain!r}")
+            raise ValueError(f"retain must be 'samples', 'bits' or 'payload', got {retain!r}")
         _cabi.require_device(device)
         self.receivers, self.S, self.device = tuple(receivers), len(receivers), device
         self.timeout_frames = _timeout_frames(timeout, self.S)
@@ -1195,13 +1199,16 @@ class StreamReceiver:
 
     def counters(self) -> dict:
         """Since this receiver was opened: kernel launches (decodes included), frames moved to keep retained
-        samples (appends aside) and whole-arena compactions; in bits mode also the plane words moved to keep
-        open recordings' planes and the plane arena's compactions (both 0 in samples mode)."""
-        a, b, c, d, e = (C.c_int64(0) for _ in range(5))
-        _cabi.check(_cabi.lib().afsk_rx_streams_counters(self._h, C.byref(a), C.byref(b), C.byref(c)))
-        _cabi.check(_cabi.lib().afsk_rx_streams_plane_counters(self._h, C.byref(d), C.byref(e)))
+        samples (appends aside) and whole-arena compactions; in bits and payload mode also the plane words moved to
+        keep open recordings' planes and the plane arena's compactions (both 0 in samples mode); in payload mode the
+        decoded bytes moved to keep open recordings' payloads and the payload arena's compactions (both 0 otherwise)."""
+        a, b, c, d, e, f, g = (C.c_int64(0) for _ in range(7))
+        L = _cabi.lib()
+        _cabi.check(L.afsk_rx_streams_counters(self._h, C.byref(a), C.byref(b), C.byref(c)))
+        _cabi.check(L.afsk_rx_streams_plane_counters(self._h, C.byref(d), C.byref(e)))
+        _cabi.check(L.afsk_rx_streams_payload_counters(self._h, C.byref(f), C.byref(g)))
         return {"launches": a.value, "moved_frames": b.value, "compactions": c.value, "moved_plane_words": d.value,
-                "plane_compactions": e.value}
+                "plane_compactions": e.value, "moved_payload_bytes": f.value, "payload_compactions": g.value}
 
     def pending_bits(self, s: int) -> tuple[int, int]:
         """(stored clock, windows decided so far) of stream s's pending recording in bits mode: (-1, 0) while its
@@ -1210,8 +1217,25 @@ class StreamReceiver:
         _cabi.check(_cabi.lib().afsk_rx_streams_pending_bits(self._h, int(s), C.byref(a), C.byref(b)))
         return a.value, b.value
 
+    def pending_payload(self, s: int) -> tuple[int, int, bool, bytes]:
+        """(train_end, nbits, ended, bytes) of stream s's pending recording in payload mode, as framed so far:
+        train_end is -1 until the end of the training sequence is seen, nbits the coded bits framed after it, ended
+        True once the first quiet window after it was found (the call's result is then fixed), and bytes the payload
+        decoded so far, a prefix of what the call returns.  (-1, 0, False, b"") in other modes, with no recording
+        pending, or before its clock is recovered."""
+        L = _cabi.lib()
+        te, nb, n = C.c_int64(0), C.c_int64(0), C.c_int64(0)
+        ended = C.c_int32(0)
+        _cabi.check(L.afsk_rx_streams_pending_payload(self._h, int(s), C.byref(te), C.byref(nb), C.byref(ended), None, 0, C.byref(n)))
+        buf = (C.c_uint8 * max(n.value, 1))()
+        if n.value > 0:
+            _cabi.check(L.afsk_rx_streams_pending_payload(self._h, int(s), C.byref(te), C.byref(nb), C.byref(ended), buf, n.value,
+                                                          C.byref(n)))
+        return te.value, nb.value, bool(ended.value), bytes(buf[:n.value])
+
     def arena_bytes(self) -> int:
-        """Device bytes this receiver holds (sample arenas, plane arenas in bits mode, staging, scratch)."""
+        """Device bytes this receiver holds (sample arenas, plane arenas in bits and payload mode, payload arenas
+        in payload mode, staging, scratch)."""
         n = C.c_int64(0)
         _cabi.check(_cabi.lib().afsk_rx_streams_arena_bytes(self._h, C.byref(n)))
         return n.value

@@ -257,19 +257,39 @@ int afsk_rx_streams_destroy(AfskRxStreams *h);
  * 4096 of its frames are in, its clock is recovered and stored, every push decides its complete 32-window plane
  * words (2 bits per window, in a plane arena with the sample arena's policy), and the channel keeps its samples
  * only from its first undecided window (or its partial chunk, if earlier).  Recordings whose status follows from
- * baud and length keep no samples.  Events, results and payloads are those of AFSK_RETAIN_SAMPLES; only state's
- * retained frames, the counters and arena_bytes differ. */
+ * baud and length keep no samples.  AFSK_RETAIN_PAYLOAD does what AFSK_RETAIN_BITS does and also frames each
+ * pending recording with a stored clock as its windows are decided: every push searches the windows that fall in
+ * chunks the gate has walked for the terminator, then for the first quiet window, and Hamming-decodes whole bytes
+ * in between into a payload slot (a third arena with the same policy, two bytes counting as one sample).  The
+ * channel keeps plane words only from the one its search or its next incomplete byte needs; once the first quiet
+ * window is found the result is fixed, and it keeps no planes, decides no more windows and keeps samples only from
+ * its partial chunk.  A recording whose clock is not stored when it ends is decoded as in AFSK_RETAIN_BITS.  In
+ * every mode, events, results and payloads are those of AFSK_RETAIN_SAMPLES; only state's retained frames, the
+ * counters and arena_bytes differ. */
 #define AFSK_RETAIN_SAMPLES 0
 #define AFSK_RETAIN_BITS 1
-/* before the first push or finish only; AFSK_E_ARG (nothing changed) after it or for an unknown mode.  A bits-mode
- * push of more than 2^32 frames on one channel returns AFSK_E_ARG and changes nothing. */
+#define AFSK_RETAIN_PAYLOAD 2
+/* before the first push or finish only; AFSK_E_ARG (nothing changed) after it or for an unknown mode.  A bits- or
+ * payload-mode push of more than 2^32 frames on one channel returns AFSK_E_ARG and changes nothing. */
 int afsk_rx_streams_set_retention(AfskRxStreams *h, int mode);
-/* channel s's pending recording in bits mode: its stored clock (-1: not yet, or no recording pending) and the
- * windows decided so far (0 in samples mode) */
+/* channel s's pending recording in bits or payload mode: its stored clock (-1: not yet, or no recording pending)
+ * and the windows decided so far (0 in samples mode; in payload mode it stops growing once the recording's first
+ * quiet window after the terminator is found) */
 int afsk_rx_streams_pending_bits(const AfskRxStreams *h, int s, int32_t *clock, int64_t *windows);
 /* since creation: plane words moved to keep pending recordings' planes, and whole plane-arena compactions (both
  * 0 in samples mode) */
 int afsk_rx_streams_plane_counters(const AfskRxStreams *h, int64_t *moved_words, int64_t *compactions);
+/* channel s's pending recording in payload mode, as framed so far: *train_end = clock + k0 * bit length once the
+ * terminator was seen (-1 before), *nbits the coded bits framed since k0, *ended 1 once the first quiet window at
+ * or after k0 was found (the result is then fixed), and its first min(cap, *nbytes) decoded bytes copied to out
+ * (out may be NULL when cap is 0).  -1 / 0 / 0 / 0 in other modes, with no recording pending, or before its clock
+ * is stored.  Synchronous (one device-to-host copy); AFSK_E_ARG for a NULL handle or pointer, a negative cap or
+ * an s out of range. */
+int afsk_rx_streams_pending_payload(const AfskRxStreams *h, int s, int64_t *train_end, int64_t *nbits, int32_t *ended,
+                                    uint8_t *out, int64_t cap, int64_t *nbytes);
+/* since creation: payload bytes moved to keep pending recordings' decoded bytes, and whole payload-arena
+ * compactions (both 0 in the other modes) */
+int afsk_rx_streams_payload_counters(const AfskRxStreams *h, int64_t *moved_bytes, int64_t *compactions);
 
 /* ---------------------------------------------------------------- transmitter ---------- */
 /* frames Transmitter.save writes for a payload of n bytes (afskmodem.py:452-469 then :239-244).

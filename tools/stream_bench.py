@@ -20,12 +20,15 @@ a host numpy transpose into the pinned planar buffer followed by push, and .t().
 by push, which is what a user had to do without push_interleaved.  The profiled run then times
 k_stream_deinterleave and k_stream_copy's planar append over the same pieces (4 bytes moved per appended frame).
 
---retain samples,bits runs every configuration once per retention mode, one after the other, on the same traffic
-(open_receive_streams(..., retain=...)), and adds a profiled bits-mode run that times k_stream_windows over the
-frames it demodulates (2 bytes read per frame of every window it decides, counted from pending_bits and the final
+--retain samples,bits,payload runs every configuration once per retention mode, one after the other, on the same
+traffic (open_receive_streams(..., retain=...)), and adds a profiled bits-mode run that times k_stream_windows over
+the frames it demodulates (2 bytes read per frame of every window it decides, counted from pending_bits and the final
 calls).  --windows-bauds profiles it alone at the given bauds on channels whose recordings never close, --stuck
-records arena_bytes() against pushed seconds on such channels for each mode (samples mode stops after 60 s), and
---loopback S times BASELINE config 4 (64 KB at 300 baud) looped back from a transmitter on S channels in bits mode."""
+records arena_bytes() against pushed seconds on such channels for each mode (samples mode stops after 60 s) and each
+--stuck-variants entry: "message" (a short message, then a full-scale carrier), "tone" (the mark tone alone: no
+message, no terminator) and "gap" (a message, one quiet window inside a loud chunk, then the carrier), and
+--loopback S times BASELINE config 4 (64 KB at 300 baud) looped back from a transmitter on S channels in the
+--loopback-retain mode."""
 from __future__ import annotations
 
 import argparse
@@ -40,6 +43,7 @@ import numpy as np
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), ".."))
 import afskmodem_b200 as A  # noqa: E402
 from afskmodem_b200 import _cabi  # noqa: E402
+from oracle import oracle as O  # noqa: E402
 
 SHIFT = 12345
 MIX_BAUDS = [300, 600, 1200, 2400, 4000, 6000]
@@ -205,23 +209,32 @@ def profile_bits(d_base, S: int, piece: int, T: int, timeout: float):
             "kernel_ms": ms, "kernel_us_per_push": ms * 1e3 / n_push, "GBps": nbytes / (ms * 1e-3) / 1e9 if ms else None}
 
 
-def stuck_carrier(S: int, seconds: int, mode: str, samples_cap_s: int = 60):
-    """arena_bytes() against pushed seconds on recordings that never close: a short message, then a full-scale 1200 Hz
-    carrier with no quiet chunk, 1 s device pushes at 1200 baud (samples mode stops after samples_cap_s seconds)"""
+def stuck_carrier(S: int, seconds: int, mode: str, variant: str = "message", samples_cap_s: int = 60):
+    """arena_bytes() against pushed seconds on recordings that never close, 1 s device pushes at 1200 baud (samples
+    mode stops after samples_cap_s seconds).  variant "message": a short message, then a full-scale 1200 Hz carrier
+    with no quiet chunk; "tone": the mark tone alone (every window decides 1: no terminator); "gap": the message, 3
+    bit lengths of silence (a quiet window inside a loud chunk), then the carrier"""
     import torch
     t = torch.arange(48000, device="cuda", dtype=torch.float64)
-    block = torch.round(30000 * torch.sin(2 * np.pi * 1200 * t / 48000)).to(torch.int16)
-    fr = torch.from_numpy(A.Transmitter(1200, 0.1).encode_batch([b"stuck"]).frames(0)[:-4800].copy()).cuda()
+    if variant == "tone":
+        block = torch.from_numpy(np.tile(O.tone("mark", 1200), 1200)).cuda()     # the Receiver's mark template
+    else:
+        block = torch.round(30000 * torch.sin(2 * np.pi * 1200 * t / 48000)).to(torch.int16)
     head = block.clone()
-    head[100:100 + len(fr)] = fr
+    if variant != "tone":
+        fr = torch.from_numpy(A.Transmitter(1200, 0.1).encode_batch([b"stuck"]).frames(0)[:-4800].copy()).cuda()
+        head[100:100 + len(fr)] = fr
+        if variant == "gap":
+            head[100 + len(fr):100 + len(fr) + 120] = 0
     offsets = np.arange(S + 1, dtype=np.int64) * 48000
     out = []
     with A.Receiver(1200).open_streams(S, 5.0, retain=mode) as st:
-        for i in range(seconds if mode == "bits" else min(seconds, samples_cap_s)):
+        for i in range(seconds if mode != "samples" else min(seconds, samples_cap_s)):
             st.push((head if i == 0 else block).repeat(S), offsets)
             out.append([i + 1, st.arena_bytes()])
+        ended = sum(st.pending_payload(s)[2] for s in range(S)) if mode == "payload" else None
         st.finish()
-    return {"S": S, "retain": mode, "seconds_vs_arena_bytes": out}
+    return {"S": S, "retain": mode, "variant": variant, "ended_channels": ended, "seconds_vs_arena_bytes": out}
 
 
 def profile_windows(baud: int, S: int, pushes: int):
@@ -254,7 +267,7 @@ def profile_windows(baud: int, S: int, pushes: int):
             "kernel_us_per_push": ms * 1e3 / pushes, "GBps": 2 * frames / (ms * 1e-3) / 1e9 if ms else None}
 
 
-def loopback_config4(S: int):
+def loopback_config4(S: int, retain: str = "bits"):
     """BASELINE config 4 on S channels: 64 KB random payloads at 300 baud (146.8 M frames each) from a streaming
     transmitter, pulled into a device tensor and pushed in 1 s pieces into a bits-mode receiver; start frames spread
     over chunk phases.  Wall time, decoded messages, peak arena_bytes()"""
@@ -264,7 +277,7 @@ def loopback_config4(S: int):
     ok, peak = 0, 0
     torch.cuda.synchronize()
     t0 = time.perf_counter()
-    with A.open_transmit_streams([A.Transmitter(300, 0.1)] * S) as tx, A.Receiver(300).open_streams(S, 10.0, retain="bits") as st:
+    with A.open_transmit_streams([A.Transmitter(300, 0.1)] * S) as tx, A.Receiver(300).open_streams(S, 10.0, retain=retain) as st:
         buf = torch.empty(S * 48000, dtype=torch.int16, device="cuda")
         ends, pushed = 0, 0
         for g in range(8):
@@ -290,7 +303,7 @@ def loopback_config4(S: int):
                 ok += int(b.status[k] == 0 and b.nbits[k] == 917504 and b.payload(k) == pays[int(ev.stream[i])])
                 k += 1
         torch.cuda.synchronize()
-    return {"S": S, "frames_per_channel": total, "wall_s": time.perf_counter() - t0, "decoded_ok": ok,
+    return {"S": S, "retain": retain, "frames_per_channel": total, "wall_s": time.perf_counter() - t0, "decoded_ok": ok,
             "peak_arena_bytes": peak}
 
 
@@ -373,8 +386,10 @@ def main():
     ap.add_argument("--stuck", type=int, default=0, help="seconds of stuck-carrier traffic per retention mode")
     ap.add_argument("--stuck-S", type=int, default=256, help="channels of the stuck-carrier run")
     ap.add_argument("--windows-bauds", default="", help="bauds at which to profile k_stream_windows alone (bits mode)")
-    ap.add_argument("--loopback", type=int, default=0, help="channels of a config-4 loopback in bits mode (0: none)")
-    ap.add_argument("--retain", default="samples", help="retention modes, run in turn per configuration: samples,bits")
+    ap.add_argument("--stuck-variants", default="message", help="stuck-carrier variants: message,tone,gap")
+    ap.add_argument("--loopback", type=int, default=0, help="channels of a config-4 loopback (0: none)")
+    ap.add_argument("--loopback-retain", default="bits", help="retention mode of the config-4 loopback")
+    ap.add_argument("--retain", default="samples", help="retention modes, run in turn per configuration: samples,bits,payload")
     ap.add_argument("--out", default=None)
     ap.add_argument("--no-profile", action="store_true", help="skip the profiled run of the largest device configuration")
     a = ap.parse_args()
@@ -415,15 +430,16 @@ def main():
             res["profile_interleaved"] = profile_config(d_base, max(Ss), max(pieces), T, a.timeout, out_dir, "interleaved")
             print(json.dumps({k: v for k, v in res["profile_interleaved"].items() if k != "by_kernel_or_copy"}), flush=True)
     if a.stuck:
-        res["stuck_carrier"] = [stuck_carrier(a.stuck_S, a.stuck, m) for m in modes]
+        res["stuck_carrier"] = [stuck_carrier(a.stuck_S, a.stuck, m, v) for v in a.stuck_variants.split(",") for m in modes]
         for r in res["stuck_carrier"]:
-            print(json.dumps({"retain": r["retain"], "last": r["seconds_vs_arena_bytes"][-1]}), flush=True)
+            print(json.dumps({"retain": r["retain"], "variant": r["variant"], "ended_channels": r["ended_channels"],
+                              "last": r["seconds_vs_arena_bytes"][-1]}), flush=True)
     if a.windows_bauds:
         res["windows_by_baud"] = [profile_windows(int(b), max(Ss), 4) for b in a.windows_bauds.split(",")]
         for r in res["windows_by_baud"]:
             print(json.dumps(r), flush=True)
     if a.loopback:
-        res["loopback_config4"] = loopback_config4(a.loopback)
+        res["loopback_config4"] = loopback_config4(a.loopback, a.loopback_retain)
         print(json.dumps(res["loopback_config4"]), flush=True)
     if not a.mix and "bits" in modes:
         res["profile_bits"] = profile_bits(d_base, max(Ss), max(pieces), T, a.timeout)
