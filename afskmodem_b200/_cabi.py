@@ -17,6 +17,8 @@ LIB_PATH = os.environ.get("AFSK_LIB_PATH") or os.path.join(_HERE, "libafsk_b200.
 AFSK_OK, AFSK_E_ARG, AFSK_E_CUDA, AFSK_E_BAUD, AFSK_E_UNSUPPORTED = 0, -1, -2, -3, -4
 ST_OK, ST_NO_CLOCK, ST_NO_DATA = 0, 1, 2
 ST_EXC_WAVELEN, ST_EXC_INDEX, ST_EXC_BAUD = -1, -2, -3
+# AFSK_SAMPLE_*: formats of interleaved frames (afsk_rx_streams_push_frames, afsk_tx_streams_pull_frames)
+SAMPLE_S16, SAMPLE_S32, SAMPLE_F32 = 0, 1, 2
 OPT_FRAME_KERNEL, OPT_L2_HINT, OPT_FUSED, OPT_CLOCK_KERNEL, OPT_GROUP_STREAMS = 1, 2, 3, 4, 5
 
 # every symbol include/afsk_b200.h declares (tests check the library exports them all)
@@ -35,7 +37,8 @@ SYMBOLS = [
     "afsk_tx_streams_destroy", "afsk_rx_streams_create_each", "afsk_rx_streams_finish_some", "afsk_tx_streams_create_each",
     "afsk_tx_streams_configure", "afsk_rx_streams_push_interleaved", "afsk_tx_streams_pull_interleaved",
     "afsk_rx_streams_set_retention", "afsk_rx_streams_pending_bits", "afsk_rx_streams_plane_counters",
-    "afsk_rx_streams_pending_payload", "afsk_rx_streams_payload_counters",
+    "afsk_rx_streams_pending_payload", "afsk_rx_streams_payload_counters", "afsk_rx_streams_push_frames",
+    "afsk_tx_streams_pull_frames",
 ]
 
 
@@ -108,6 +111,7 @@ def lib():
     L.afsk_rx_streams_create.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int64, C.POINTER(vp)]
     L.afsk_rx_streams_push.argtypes = [vp, vp, C.c_int, i64p, vp, i64p]
     L.afsk_rx_streams_push_interleaved.argtypes = [vp, vp, C.c_int, C.c_int64, vp, i64p]
+    L.afsk_rx_streams_push_frames.argtypes = [vp, vp, C.c_int, C.c_int, C.c_int64, C.c_int64, vp, i64p]
     L.afsk_rx_streams_create_each.argtypes = [C.c_int, C.c_int, i32p, i32p, i32p, i64p, C.POINTER(vp)]
     L.afsk_rx_streams_finish.argtypes = [vp, vp, i64p]
     L.afsk_rx_streams_finish_some.argtypes = [vp, C.c_int, i32p, i32p, i32p, i32p, i64p, vp, i64p]
@@ -134,6 +138,7 @@ def lib():
     L.afsk_tx_streams_send.argtypes = [vp, C.c_int, i32p, i64p, u8p, i64p, i64p]
     L.afsk_tx_streams_pull.argtypes = [vp, C.c_int64, vp, C.c_int, vp]
     L.afsk_tx_streams_pull_interleaved.argtypes = [vp, C.c_int64, vp, C.c_int, vp]
+    L.afsk_tx_streams_pull_frames.argtypes = [vp, C.c_int64, vp, C.c_int, C.c_int, C.c_int64, vp]
     L.afsk_tx_streams_state.argtypes = [vp, C.c_int, i64p, i64p, i64p]
     L.afsk_tx_streams_arena_bytes.argtypes = [vp, i64p]
     L.afsk_tx_streams_counters.argtypes = [vp, i64p, i64p, i64p]

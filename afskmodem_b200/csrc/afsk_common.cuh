@@ -181,4 +181,20 @@ __device__ __forceinline__ uint4 ld_nc_v4(const void *p)
                  : "l"(p));
     return r;
 }
+
+// the sample-format rules of include/afsk_b200.h (AFSK_SAMPLE_*), element by element.  x * 32768 is exact in float,
+// and cvt.rni.s32.f32 rounds half to even, saturates and maps NaN to 0, so the clamp finishes the receive rule.
+__device__ __forceinline__ int16_t sample_to_s16(int16_t x) { return x; }
+__device__ __forceinline__ int16_t sample_to_s16(int32_t x) { return (int16_t)(x >> 16); }
+__device__ __forceinline__ int16_t sample_to_s16(float x) { return (int16_t)min(max(__float2int_rn(x * 32768.f), -32768), 32767); }
+template <typename T> __device__ __forceinline__ T sample_from_s16(int16_t s);
+template <> __device__ __forceinline__ int16_t sample_from_s16<int16_t>(int16_t s) { return s; }
+template <> __device__ __forceinline__ int32_t sample_from_s16<int32_t>(int16_t s) { return (int32_t)((uint32_t)(int32_t)s << 16); }
+template <> __device__ __forceinline__ float sample_from_s16<float>(int16_t s) { return (float)s * (1.f / 32768.f); }
 #endif
+
+// bytes per sample of an AFSK_SAMPLE_* format, 0 for an unknown one
+static inline int afsk_sample_size(int format)
+{
+    return format == AFSK_SAMPLE_S16 ? 2 : format == AFSK_SAMPLE_S32 || format == AFSK_SAMPLE_F32 ? 4 : 0;
+}

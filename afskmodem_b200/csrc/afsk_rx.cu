@@ -2240,22 +2240,29 @@ __global__ void __launch_bounds__(kCopyThreads) k_stream_copy(const int16_t *__r
     }
 }
 
-// Appends one interleaved piece (src[f * S + s] = frame f of channel s, n frames, 16-byte aligned) to every
-// channel's slot: frame f of channel s goes to dst[seg[s].dst + f], an arbitrary alignment per channel.
-// A CTA owns kDiC consecutive channels x kDiF destination frames, in destination-vector coordinates: tile fb
-// writes channel s's vectors (seg[s].dst >> 3) + fb * kDiF / 8 + j, j < kDiF / 8, which hold frames
-// fb * kDiF - a + 8j .. + 7 with a = seg[s].dst & 7.  So the tile reads frame rows fb * kDiF - 7 .. fb * kDiF +
-// kDiF - 1 (a halo of 7 frames in front), each row's kDiC channels as 128 contiguous bytes: eight lanes per row,
-// aligned 128-bit loads realigned with funnel shifts when S % 8 != 0.  Each frame lands in shared memory at its
-// channel's destination position, so every thread then writes aligned 16-byte vectors of one channel, sixteen
-// lanes one 256-byte run; only a channel's head and tail vectors are written frame by frame.  64 x 128 keeps a
-// row load at one 128-byte line and the tile at 17 KB (several CTAs per SM); the halo costs 7 / 128 extra reads.
-// Shared rows are channels in the order (s & 7) * 8 + (s >> 3), 136 samples apart (68 words = 4 banks): the
-// eight lanes of a row load write eight consecutive rows, in disjoint bank groups.
+// k_stream_frames<Tin> appends one interleaved piece to every channel's slot: frame f of channel s is element
+// e0 + f * pitch + s of src
+// (src 16-byte aligned, e0 < 16 / sizeof(Tin) the window's offset in its first vector, pitch >= S, n frames), converted
+// to int16 by the rule of its format (sample_to_s16) as it is loaded; it goes to dst[seg[s].dst + f], an arbitrary
+// alignment per channel.  A CTA owns kDiC consecutive channels x kDiF destination frames, in destination-vector
+// coordinates: tile fb writes channel s's vectors (seg[s].dst >> 3) + fb * kDiF / 8 + j, j < kDiF / 8, which hold
+// frames fb * kDiF - a + 8j .. + 7 with a = seg[s].dst & 7.  So the tile reads frame rows fb * kDiF - 7 .. fb * kDiF +
+// kDiF - 1 (a halo of 7 frames in front), each row's kDiC channels as contiguous bytes with aligned 128-bit loads,
+// realigned to the window with funnel shifts (16-bit) or word selects (32-bit): only the vectors holding window
+// samples are read.  A 16-bit row is 128 bytes, eight lanes of 8 samples; a 32-bit row is 256 bytes, sixteen lanes of
+// 4 samples, so that every load instruction still covers whole 128-byte lines and the tile, its shared layout and the
+// store half stay those of the 16-bit case.  Each frame lands in shared memory at its channel's destination position,
+// so every thread then writes aligned 16-byte vectors of one channel, sixteen lanes one 256-byte run; only a channel's
+// head and tail vectors are written frame by frame.  64 x 128 keeps the tile at 17 KB (several CTAs per SM); the halo
+// costs 7 / 128 extra reads.  Shared rows are channels in the order (s & 7) * 8 + (s >> 3), 136 samples apart (68 words
+// = 4 banks): the eight lanes of a 16-bit row load write eight consecutive rows, in disjoint bank groups (a 32-bit row's
+// sixteen lanes fall on eight bank groups, two lanes each).
 constexpr int kDiC = 64, kDiF = 128, kDiHalo = 7, kDiThreads = 256, kDiStride = kDiF + 8;
 
 __device__ __forceinline__ int di_row(int c) { return (c & 7) * 8 + (c >> 3); }
 
+// k_stream_frames<int16_t> for contiguous frames of a 16-byte aligned piece (pitch S, e0 = 0), the layout of
+// afsk_rx_streams_push_interleaved: its row arithmetic is cheaper, and it measured faster (DESIGN.md §5)
 __global__ void __launch_bounds__(kDiThreads) k_stream_deinterleave(const int16_t *__restrict__ src, int16_t *__restrict__ dst,
                                                                      const CopySeg *__restrict__ seg, int S, long long n,
                                                                      int cblocks)
@@ -2285,6 +2292,75 @@ __global__ void __launch_bounds__(kDiThreads) k_stream_deinterleave(const int16_
             if (c >= nc) break;
             const long long p = f - F0 + (sdst[c] & 7);           // destination position in the tile
             if (p >= 0 && p < kDiF) T[di_row(c) * kDiStride + p] = (int16_t)(o[e >> 1] >> (16 * (e & 1)));
+        }
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < nc * (kDiF / 8); i += kDiThreads) {
+        const int j = i % (kDiF / 8), c = i / (kDiF / 8);
+        const long long g = sdst[c];
+        const long long d0 = ((g >> 3) * 8) + F0 + 8 * j, f0 = d0 - g;   // the vector and its first frame
+        if (f0 >= n) continue;
+        const uint4 v = *reinterpret_cast<const uint4 *>(T + di_row(c) * kDiStride + 8 * j);
+        if (f0 >= 0 && f0 + 8 <= n) {
+            *reinterpret_cast<uint4 *>(dst + d0) = v;
+        } else {
+            const uint32_t o[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+            for (int e = 0; e < 8; e++)
+                if (f0 + e >= 0 && f0 + e < n) dst[d0 + e] = (int16_t)(o[e >> 1] >> (16 * (e & 1)));
+        }
+    }
+}
+
+// samples k .. k + 3 of the eight 32-bit samples in two consecutive aligned vectors
+__device__ __forceinline__ void realign4(const uint4 &lo, const uint4 &hi, int k, uint32_t (&o)[4])
+{
+    const uint32_t w[8] = {lo.x, lo.y, lo.z, lo.w, hi.x, hi.y, hi.z, hi.w};
+#pragma unroll
+    for (int t = 0; t < 4; t++) o[t] = k == 0 ? w[t] : k == 1 ? w[t + 1] : k == 2 ? w[t + 2] : w[t + 3];
+}
+
+template <typename Tin>
+__global__ void __launch_bounds__(kDiThreads) k_stream_frames(const Tin *__restrict__ src, int16_t *__restrict__ dst,
+                                                                     const CopySeg *__restrict__ seg, int S, long long n,
+                                                                     long long pitch, int e0, int cblocks)
+{
+    constexpr int V = 16 / sizeof(Tin), L = kDiC / V;             // samples per vector, lanes per row
+    constexpr int lgV = V == 8 ? 3 : 2, lgL = V == 8 ? 3 : 4;
+    __shared__ __align__(16) int16_t T[kDiC * kDiStride];
+    __shared__ long long sdst[kDiC];
+    const int c0 = (int)(blockIdx.x % cblocks) * kDiC, nc = min(kDiC, S - c0);
+    const long long F0 = (long long)(blockIdx.x / cblocks) * kDiF;
+    if (threadIdx.x < nc) sdst[threadIdx.x] = seg[c0 + threadIdx.x].dst;
+    __syncthreads();
+    const long long f_lo = max(F0 - kDiHalo, 0LL), f_hi = min(F0 + kDiF, n);
+    const int nq = (nc + V - 1) / V;
+    for (int i = threadIdx.x; i < (int)(f_hi - f_lo) * L; i += kDiThreads) {
+        const int q = i & (L - 1);
+        if (q >= nq) continue;
+        const long long f = f_lo + (i >> lgL), row = e0 + f * pitch + c0, row_end = row + nc;
+        const long long qs = row + V * q;                         // first sample of channels c0 + Vq ..
+        const long long sv = qs >> lgV;
+        const int k = (int)(qs & (V - 1));
+        const uint4 lo = ld_nc_v4(src + sv * V);                  // holds qs, inside the row
+        const uint4 hi = k && (sv + 1) * V < row_end ? ld_nc_v4(src + (sv + 1) * V) : make_uint4(0, 0, 0, 0);
+        uint32_t o[4];
+        Tin v[V];
+        if constexpr (V == 8) {
+            realign8(lo, hi, k, o);
+#pragma unroll
+            for (int e = 0; e < 8; e++) v[e] = (Tin)(o[e >> 1] >> (16 * (e & 1)));
+        } else {
+            realign4(lo, hi, k, o);
+#pragma unroll
+            for (int e = 0; e < 4; e++) memcpy(&v[e], &o[e], 4);
+        }
+#pragma unroll
+        for (int e = 0; e < V; e++) {
+            const int c = V * q + e;
+            if (c >= nc) break;
+            const long long p = f - F0 + (sdst[c] & 7);           // destination position in the tile
+            if (p >= 0 && p < kDiF) T[di_row(c) * kDiStride + p] = sample_to_s16(v[e]);
         }
     }
     __syncthreads();
@@ -3677,10 +3753,11 @@ static int streams_bits(AfskRxStreams *H, cudaStream_t st, const int64_t *out_fi
 
 // one push (fin == NULL) or the end of the streams s with fin[s] != 0 (no samples); then, when new_baud is
 // given, every channel's settings become new_baud[s] / new_params[s] for its next stream.  A push is planar
-// (inter < 0: channel s's piece is samples[off[s] .. off[s + 1])) or interleaved (inter frames of every
-// channel, samples[f * S + s] = frame f of channel s; off unused)
-static int streams_run(AfskRxStreams *H, const int16_t *samples, int on_device, const int64_t *off, int64_t inter, cudaStream_t st,
-                       const uint8_t *fin, const int32_t *new_baud, const GateParams *new_params, int64_t *n_events)
+// (inter < 0: channel s's piece is samples[off[s] .. off[s + 1]), int16) or interleaved (inter frames of every
+// channel, samples[f * pitch + s] = frame f of channel s in the AFSK_SAMPLE_* format; off unused)
+static int streams_run(AfskRxStreams *H, const void *samples, int on_device, const int64_t *off, int64_t inter, int format,
+                       int64_t pitch, cudaStream_t st, const uint8_t *fin, const int32_t *new_baud, const GateParams *new_params,
+                       int64_t *n_events)
 {
     const int S = H->S;
     const bool finish = fin != nullptr, interleaved = inter >= 0;
@@ -3693,8 +3770,9 @@ static int streams_run(AfskRxStreams *H, const int16_t *samples, int on_device, 
     }
     // buffers first: a failed allocation leaves the channels as they were
     const int64_t in_samples = finish ? 0 : interleaved ? inter * S : off[S] - off[0];
+    const int size = interleaved ? afsk_sample_size(format) : 2;
     cudaError_t e = cudaSuccess;
-    if (!on_device && in_samples > 0) e = grow_device((void **)&H->d_stage, &H->stage_cap, (size_t)in_samples * 2 + 32);
+    if (!on_device && in_samples > 0) e = grow_device((void **)&H->d_stage, &H->stage_cap, (size_t)in_samples * size + 32);
     if (e == cudaSuccess) e = grow_device((void **)&H->d_amp, &H->amp_cap, sizeof(int32_t) * (size_t)nch);
     if (e == cudaSuccess) e = grow_device((void **)&H->d_ranges, &H->ranges_cap, sizeof(int64_t) * 3 * (size_t)(nch + S));
     if (e == cudaSuccess) e = grow_pinned((void **)&H->h_ranges, &H->h_ranges_cap, sizeof(int64_t) * 3 * (size_t)(nch + S));
@@ -3712,9 +3790,14 @@ static int streams_run(AfskRxStreams *H, const int16_t *samples, int on_device, 
     Slots &A = H->smp;
     tf_app[0] = 0;
     first[0] = 0;
+    // interleaved device input is read from the 16-byte vector holding its first sample, e0 samples in; host input
+    // is copied packed (pitch S) into the staging buffer
+    const int e0 = interleaved && on_device ? (int)((reinterpret_cast<uintptr_t>(samples) & 15) / size) : 0;
+    const int64_t kpitch = on_device ? pitch : S;                 // the pitch the kernel reads
     for (int s = 0; s < S; s++) {
-        // (interleaved: src is the channel's column, which only a one-channel push reads as a k_stream_copy segment)
-        const int64_t src = finish ? 0 : interleaved ? s : off[s] - (on_device ? 0 : off[0]);
+        // (interleaved: src is the channel's column, which only a one-channel contiguous int16 push reads as a
+        // k_stream_copy segment)
+        const int64_t src = finish ? 0 : interleaved ? e0 + s : off[s] - (on_device ? 0 : off[0]);
         add_seg(seg_app, tf_app, napp, src, A.off[s] + H->pushed[s] - A.base[s], piece(s));
         const int64_t c_old = H->pushed[s] / C;
         first[s + 1] = first[s] + H->np[s] / C - c_old;
@@ -3727,18 +3810,28 @@ static int streams_run(AfskRxStreams *H, const int16_t *samples, int on_device, 
     slots_move(A, compact, nmov, dd + H->o_seg_mov, dd + H->o_tf_mov, tf_mov[nmov], st, H->n_launches);
     int16_t *x = A.arena[A.cur];
     if (napp > 0) {
-        const int16_t *src = samples;
-        if (!on_device) {
-            AFSK_CUDA(cudaMemcpyAsync(H->d_stage, samples + (interleaved ? 0 : off[0]), (size_t)in_samples * 2, cudaMemcpyHostToDevice, st));
-            src = H->d_stage;
+        const void *src = on_device ? reinterpret_cast<const void *>(reinterpret_cast<uintptr_t>(samples) & ~(uintptr_t)15) : H->d_stage;
+        if (!on_device && interleaved) {
+            AFSK_CUDA(cudaMemcpy2DAsync(H->d_stage, (size_t)S * size, samples, (size_t)pitch * size, (size_t)S * size, (size_t)inter,
+                                        cudaMemcpyHostToDevice, st));
+        } else if (!on_device) {
+            AFSK_CUDA(cudaMemcpyAsync(H->d_stage, static_cast<const int16_t *>(samples) + off[0], (size_t)in_samples * 2,
+                                      cudaMemcpyHostToDevice, st));
         }
-        if (interleaved && S > 1) {
+        const CopySeg *sg = reinterpret_cast<const CopySeg *>(dd + H->o_seg_app);
+        if (interleaved && (S > 1 || format != AFSK_SAMPLE_S16 || kpitch != 1)) {
             const int cblocks = (S + kDiC - 1) / kDiC;
-            const int64_t ftiles = (inter + kDiF + kDiHalo - 1) / kDiF;
-            k_stream_deinterleave<<<(unsigned)(cblocks * ftiles), kDiThreads, 0, st>>>(
-                src, x, reinterpret_cast<const CopySeg *>(dd + H->o_seg_app), S, inter, cblocks);
+            const unsigned grid = (unsigned)(cblocks * ((inter + kDiF + kDiHalo - 1) / kDiF));
+            if (format == AFSK_SAMPLE_S16 && kpitch == S && e0 == 0)
+                k_stream_deinterleave<<<grid, kDiThreads, 0, st>>>(static_cast<const int16_t *>(src), x, sg, S, inter, cblocks);
+            else if (format == AFSK_SAMPLE_S16)
+                k_stream_frames<<<grid, kDiThreads, 0, st>>>(static_cast<const int16_t *>(src), x, sg, S, inter, kpitch, e0, cblocks);
+            else if (format == AFSK_SAMPLE_S32)
+                k_stream_frames<<<grid, kDiThreads, 0, st>>>(static_cast<const int32_t *>(src), x, sg, S, inter, kpitch, e0, cblocks);
+            else
+                k_stream_frames<<<grid, kDiThreads, 0, st>>>(static_cast<const float *>(src), x, sg, S, inter, kpitch, e0, cblocks);
         } else {
-            k_stream_copy<<<(unsigned)tf_app[napp], kCopyThreads, 0, st>>>(src, x, reinterpret_cast<const CopySeg *>(dd + H->o_seg_app),
+            k_stream_copy<<<(unsigned)tf_app[napp], kCopyThreads, 0, st>>>(static_cast<const int16_t *>(src), x, sg,
                                                                           reinterpret_cast<const int64_t *>(dd + H->o_tf_app), napp);
         }
         H->n_launches++;
@@ -4128,7 +4221,8 @@ static int streams_bits(AfskRxStreams *H, cudaStream_t st, const int64_t *out_fi
 
 // a push or finish with valid arguments: any failure may leave the channels between two states, so the
 // handle refuses every later push / finish
-static int streams_call(AfskRxStreams *H, const int16_t *samples, int on_device, const int64_t *off, int64_t inter, void *stream,
+static int streams_call(AfskRxStreams *H, const void *samples, int on_device, const int64_t *off, int64_t inter, int format,
+                        int64_t pitch, void *stream,
                         const uint8_t *fin, const int32_t *new_baud, const GateParams *new_params, int64_t *n_events)
 {
     if (H->failed) { afsk_set_error("afsk_rx_streams: an earlier push failed; destroy the handle"); return AFSK_E_CUDA; }
@@ -4143,7 +4237,7 @@ static int streams_call(AfskRxStreams *H, const int16_t *samples, int on_device,
             }
     }
     H->used = true;
-    const int rc = streams_run(H, samples, on_device, off, inter, (cudaStream_t)stream, fin, new_baud, new_params, n_events);
+    const int rc = streams_run(H, samples, on_device, off, inter, format, pitch, (cudaStream_t)stream, fin, new_baud, new_params, n_events);
     if (rc != AFSK_OK) {
         H->failed = true;
         H->ev.clear(); H->res.clear(); H->payload.clear(); H->payload_off.clear();
@@ -4288,24 +4382,48 @@ int afsk_rx_streams_push(AfskRxStreams *H, const int16_t *samples, int on_device
         afsk_set_error("afsk_rx_streams_push: device samples must be 16-byte aligned");
         return AFSK_E_ARG;
     }
-    return streams_call(H, samples, on_device, h_offsets, -1, stream, nullptr, nullptr, nullptr, n_events);
+    return streams_call(H, samples, on_device, h_offsets, -1, AFSK_SAMPLE_S16, 0, stream, nullptr, nullptr, nullptr, n_events);
+}
+
+// the argument checks of an interleaved push (fn names the entry point in the error)
+static int push_frames_check(const char *fn, AfskRxStreams *H, const void *frames, int format, int64_t n_frames, int64_t row_pitch,
+                             int64_t *n_events)
+{
+    if (!H || !n_events || n_frames < 0 || (n_frames > 0 && !frames)) { afsk_set_error("%s: bad argument", fn); return AFSK_E_ARG; }
+    const int size = afsk_sample_size(format);
+    if (!size) { afsk_set_error("%s: unknown sample format %d", fn, format); return AFSK_E_ARG; }
+    if (row_pitch < H->S) { afsk_set_error("%s: row_pitch %lld < S = %d", fn, (long long)row_pitch, H->S); return AFSK_E_ARG; }
+    if ((reinterpret_cast<uintptr_t>(frames) & (uintptr_t)(size - 1)) != 0) {
+        afsk_set_error("%s: frames must be aligned to the sample size (%d bytes)", fn, size);
+        return AFSK_E_ARG;
+    }
+    if (n_frames > (INT64_MAX / 16) / row_pitch) { afsk_set_error("%s: row_pitch * n_frames overflows", fn); return AFSK_E_ARG; }
+    if ((int64_t)((H->S + kDiC - 1) / kDiC) * ((n_frames + kDiF + kDiHalo - 1) / kDiF) > 0x7FFFFFFFLL) {
+        afsk_set_error("%s: piece too large", fn);
+        return AFSK_E_ARG;
+    }
+    return AFSK_OK;
 }
 
 int afsk_rx_streams_push_interleaved(AfskRxStreams *H, const int16_t *frames, int on_device, int64_t n_frames, void *stream,
                                      int64_t *n_events)
 {
     const char *fn = "afsk_rx_streams_push_interleaved";
-    if (!H || !n_events || n_frames < 0 || (n_frames > 0 && !frames)) { afsk_set_error("%s: bad argument", fn); return AFSK_E_ARG; }
-    if (n_frames > (INT64_MAX / 16) / H->S) { afsk_set_error("%s: S * n_frames overflows", fn); return AFSK_E_ARG; }
-    if ((int64_t)((H->S + kDiC - 1) / kDiC) * ((n_frames + kDiF + kDiHalo - 1) / kDiF) > 0x7FFFFFFFLL) {
-        afsk_set_error("%s: piece too large", fn);
-        return AFSK_E_ARG;
-    }
+    const int rc = push_frames_check(fn, H, frames, AFSK_SAMPLE_S16, n_frames, H ? H->S : 0, n_events);
+    if (rc != AFSK_OK) return rc;
     if (on_device && (reinterpret_cast<uintptr_t>(frames) & 15) != 0) {
         afsk_set_error("%s: device frames must be 16-byte aligned", fn);
         return AFSK_E_ARG;
     }
-    return streams_call(H, frames, on_device, nullptr, n_frames, stream, nullptr, nullptr, nullptr, n_events);
+    return streams_call(H, frames, on_device, nullptr, n_frames, AFSK_SAMPLE_S16, H->S, stream, nullptr, nullptr, nullptr, n_events);
+}
+
+int afsk_rx_streams_push_frames(AfskRxStreams *H, const void *frames, int format, int on_device, int64_t n_frames, int64_t row_pitch,
+                                void *stream, int64_t *n_events)
+{
+    const int rc = push_frames_check("afsk_rx_streams_push_frames", H, frames, format, n_frames, row_pitch, n_events);
+    if (rc != AFSK_OK) return rc;
+    return streams_call(H, frames, on_device, nullptr, n_frames, format, row_pitch, stream, nullptr, nullptr, nullptr, n_events);
 }
 
 int afsk_rx_streams_finish_some(AfskRxStreams *H, int n, const int32_t *h_streams, const int32_t *h_baud, const int32_t *h_amp_start,
@@ -4322,7 +4440,7 @@ int afsk_rx_streams_finish_some(AfskRxStreams *H, int n, const int32_t *h_stream
         if (fin[s]) { afsk_set_error("%s: stream %d listed twice", fn, s); return AFSK_E_ARG; }
         fin[s] = 1;
     }
-    if (!given) return streams_call(H, nullptr, 0, nullptr, -1, stream, fin.data(), nullptr, nullptr, n_events);
+    if (!given) return streams_call(H, nullptr, 0, nullptr, -1, AFSK_SAMPLE_S16, 0, stream, fin.data(), nullptr, nullptr, n_events);
     for (int i = 0; i < n; i++) {
         const int rc = rx_settings_check(fn, h_streams[i], h_baud[i], h_timeout_frames[i]);
         if (rc != AFSK_OK) return rc;
@@ -4333,7 +4451,7 @@ int afsk_rx_streams_finish_some(AfskRxStreams *H, int n, const int32_t *h_stream
         baud[h_streams[i]] = h_baud[i];
         params[h_streams[i]] = GateParams{h_amp_start[i], h_amp_end[i], h_timeout_frames[i]};
     }
-    return streams_call(H, nullptr, 0, nullptr, -1, stream, fin.data(), baud.data(), params.data(), n_events);
+    return streams_call(H, nullptr, 0, nullptr, -1, AFSK_SAMPLE_S16, 0, stream, fin.data(), baud.data(), params.data(), n_events);
 }
 
 int afsk_rx_streams_finish(AfskRxStreams *H, void *stream, int64_t *n_events)

@@ -507,16 +507,21 @@ __global__ void __launch_bounds__(kWinThreads) k_tx_window(const uint8_t *__rest
     }
 }
 
-// The interleaved window, out[c * S + s] = frame P + c of channel s (what a multi-channel sound card takes).  A CTA
-// computes kIlC consecutive channels x kIlV column vectors of 8 frames (aligned on the window column, so no vector
-// straddles two channels) with win_vec, or win_frame for a vector across a message boundary or the window's end: one
-// thread per vector, consecutive threads along a channel as in k_tx_window, into shared memory.  It then writes the
-// tile frame-major: each of its frame rows is the contiguous run out[f * S + c0 .. + kIlC), as aligned 16-byte
-// vectors of the output, the row's partial head and tail vectors (S % 8 != 0) sample by sample.  Shared rows are
-// channels in the order (s & 7) * 8 + (s >> 3), 136 samples apart, so that the lanes of one output row read
-// consecutive shared rows in distinct bank groups.
+// k_tx_window_frames<Tout>: the interleaved window, written into a window of a wider output: frame P + c of channel s,
+// converted by the rule of the output format (sample_from_s16), is element e0 + c * pitch + s of out (out 16-byte
+// aligned, e0 < 16 / sizeof(Tout) the window's offset in its first vector, pitch >= S): what a multi-channel sound card
+// takes, or some columns of it. A CTA computes kIlC consecutive channels x kIlV column vectors of 8 frames (aligned on
+// the window column, so no vector straddles two channels) with win_vec, or win_frame for a vector across a message
+// boundary or the window's end: one thread per vector, consecutive threads along a channel as in k_tx_window, into
+// shared memory. It then writes the tile frame-major: each of its frame rows is the contiguous run of kIlC samples at
+// e0 + f * pitch + c0, written from its absolute alignment as aligned 16-byte vectors of the output, the row's partial
+// head and tail vectors sample by sample, so nothing outside the window is written and handles may fill disjoint
+// windows of one buffer. Shared rows are channels in the order (s & 7) * 8 + (s >> 3), 136 samples apart, so that the
+// lanes of one output row read consecutive shared rows in distinct bank groups.
 constexpr int kIlC = 64, kIlV = 16, kIlStride = 8 * kIlV + 8;
 
+// k_tx_window_frames<int16_t> for a contiguous, 16-byte aligned output (pitch S, e0 = 0), the layout of
+// afsk_tx_streams_pull_interleaved: its row arithmetic is cheaper, and it measured faster (DESIGN.md §5)
 __global__ void __launch_bounds__(kWinThreads) k_tx_window_interleaved(const uint8_t *__restrict__ pay, const int64_t *__restrict__ nib,
                                                                        const TxDesc *__restrict__ descs,
                                                                        const int32_t *__restrict__ row_off, long long P, long long n,
@@ -563,6 +568,63 @@ __global__ void __launch_bounds__(kWinThreads) k_tx_window_interleaved(const uin
 #pragma unroll
             for (int e = 0; e < 8; e++)
                 if (d0 + e >= a && d0 + e < b) out[d0 + e] = (int16_t)(w[e >> 1] >> (16 * (e & 1)));
+        }
+    }
+}
+
+// (__maxnreg__ in place of __launch_bounds__(kWinThreads): with the calls of the synthesis loop, ptxas otherwise settles
+// on 40 registers and spills two values across them)
+template <typename Tout>
+__global__ void __maxnreg__(48) k_tx_window_frames(const uint8_t *__restrict__ pay, const int64_t *__restrict__ nib,
+                                                                       const TxDesc *__restrict__ descs,
+                                                                       const int32_t *__restrict__ row_off, long long P, long long n,
+                                                                       int S, int cblocks, long long pitch, int e0,
+                                                                       Tout *__restrict__ out)
+{
+    constexpr int V = 16 / sizeof(Tout), NV = kIlC / V + 1;      // samples per vector; a row spans at most NV vectors
+    __shared__ __align__(16) int16_t T[kIlC * kIlStride];
+    const int c0 = (int)(blockIdx.x % cblocks) * kIlC, nc = min(kIlC, S - c0);
+    const long long F0 = (long long)(blockIdx.x / cblocks) * (8 * kIlV);
+    const int nf = (int)min(8LL * kIlV, n - F0);
+    const int col = 8 * (threadIdx.x % kIlV);                    // this thread's column vector, on every channel
+    if (col < nf) {
+        const long long t0 = P + F0 + col;
+        const int m = min(8, nf - col);
+#pragma unroll 1
+        for (int c = threadIdx.x / kIlV; c < nc; c += kWinThreads / kIlV) {
+            uint4 o;
+            if (m < 8 || !win_vec(descs, row_off, c0 + c, t0, pay, nib, o)) {   // frame by frame, 0 past the window
+                unsigned long long w = 0, x = 0;
+#pragma unroll 1
+                for (int e = 0; e < m; e++) {
+                    const unsigned long long f = (uint16_t)win_frame(descs, row_off, c0 + c, t0 + e, pay, nib);
+                    if (e < 4) w |= f << (16 * e); else x |= f << (16 * (e - 4));
+                }
+                o = make_uint4((uint32_t)w, (uint32_t)(w >> 32), (uint32_t)x, (uint32_t)(x >> 32));
+            }
+            *reinterpret_cast<uint4 *>(T + ((c & 7) * 8 + (c >> 3)) * kIlStride + col) = o;
+        }
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < nf * NV; i += kWinThreads) {
+        const int q = i % NV, fl = i / NV;
+        const long long a = e0 + (F0 + fl) * pitch + c0, b = a + nc;    // the row's samples in out
+        const long long d0 = ((a >> (V == 8 ? 3 : 2)) + q) * V;
+        if (d0 >= b) continue;
+        Tout w[V];
+#pragma unroll
+        for (int e = 0; e < V; e++) {
+            const int c = (int)(d0 + e - a);
+            w[e] = c >= 0 && c < nc ? sample_from_s16<Tout>(T[((c & 7) * 8 + (c >> 3)) * kIlStride + fl]) : Tout(0);
+        }
+        if (d0 >= a && d0 + V <= b) {
+            uint4 v;
+            memcpy(&v, w, 16);
+            *reinterpret_cast<uint4 *>(out + d0) = v;
+        } else {
+#pragma unroll
+            for (int e = 0; e < V; e++)
+                if (d0 + e >= a && d0 + e < b) out[d0 + e] = w[e];
         }
     }
 }
@@ -912,8 +974,10 @@ static int tx_send_run(AfskTxStreams *H, int n, const int32_t *h_stream, const i
     return AFSK_OK;
 }
 
-// the window as S x n_frames row-major (planar) or n_frames x S (interleaved)
-static int tx_pull_run(AfskTxStreams *H, int64_t n_frames, int16_t *dst, int on_device, bool interleaved, cudaStream_t st)
+// the window as S x n_frames row-major int16 (planar) or interleaved: frame f of channel s at dst[f * pitch + s] in the
+// AFSK_SAMPLE_* format (host output: synthesized packed, then copied row by row)
+static int tx_pull_run(AfskTxStreams *H, int64_t n_frames, void *dst, int on_device, bool interleaved, int format, int64_t pitch,
+                       cudaStream_t st)
 {
     if (n_frames == 0) return AFSK_OK;
     const int S = H->S;
@@ -929,7 +993,8 @@ static int tx_pull_run(AfskTxStreams *H, int64_t n_frames, int16_t *dst, int on_
     const size_t desc_bytes = sizeof(TxDesc) * (size_t)nwin, bytes = desc_bytes + sizeof(int32_t) * ((size_t)S + 1);
     AFSK_CUDA(grow_pinned((void **)&H->h_stage, &H->h_stage_cap, bytes));
     AFSK_CUDA(grow_device((void **)&H->d_scratch, &H->d_scratch_cap, bytes));
-    if (!on_device) AFSK_CUDA(grow_device((void **)&H->d_out, &H->out_cap, (size_t)nvec * 16));
+    const int size = interleaved ? afsk_sample_size(format) : 2;
+    if (!on_device) AFSK_CUDA(grow_device((void **)&H->d_out, &H->out_cap, ((size_t)total * size + 15) / 16 * 16));
     TxDesc *hd = reinterpret_cast<TxDesc *>(H->h_stage);
     int32_t *row_off = reinterpret_cast<int32_t *>(H->h_stage + desc_bytes);
     int32_t k = 0;
@@ -942,22 +1007,40 @@ static int tx_pull_run(AfskTxStreams *H, int64_t n_frames, int16_t *dst, int on_
     }
     row_off[S] = k;
     AFSK_CUDA(cudaMemcpyAsync(H->d_scratch, H->h_stage, bytes, cudaMemcpyHostToDevice, st));
-    int16_t *out = on_device ? dst : H->d_out;
+    // device output is written from the 16-byte vector holding its first sample, e0 samples in
+    void *out = on_device ? reinterpret_cast<void *>(reinterpret_cast<uintptr_t>(dst) & ~(uintptr_t)15) : H->d_out;
+    const int e0 = on_device ? (int)((reinterpret_cast<uintptr_t>(dst) & 15) / size) : 0;
+    const int64_t kpitch = on_device ? pitch : S;
     const uint8_t *a = H->arena[H->cur];
+    const int64_t *nib = reinterpret_cast<const int64_t *>(a);
     const TxDesc *d_descs = reinterpret_cast<const TxDesc *>(H->d_scratch);
     const int32_t *d_row_off = reinterpret_cast<const int32_t *>(H->d_scratch + desc_bytes);
     if (interleaved) {
         const int cblocks = (S + kIlC - 1) / kIlC;
-        const int64_t ftiles = (n + 8 * kIlV - 1) / (8 * kIlV);
-        k_tx_window_interleaved<<<(unsigned)(cblocks * ftiles), kWinThreads, 0, st>>>(a, reinterpret_cast<const int64_t *>(a), d_descs,
-                                                                                     d_row_off, H->P, n, S, cblocks, out);
+        const unsigned grid = (unsigned)(cblocks * ((n + 8 * kIlV - 1) / (8 * kIlV)));
+        if (format == AFSK_SAMPLE_S16 && kpitch == S && e0 == 0)
+            k_tx_window_interleaved<<<grid, kWinThreads, 0, st>>>(a, nib, d_descs, d_row_off, H->P, n, S, cblocks,
+                                                                  static_cast<int16_t *>(out));
+        else if (format == AFSK_SAMPLE_S16)
+            k_tx_window_frames<<<grid, kWinThreads, 0, st>>>(a, nib, d_descs, d_row_off, H->P, n, S, cblocks, kpitch, e0,
+                                                             static_cast<int16_t *>(out));
+        else if (format == AFSK_SAMPLE_S32)
+            k_tx_window_frames<<<grid, kWinThreads, 0, st>>>(a, nib, d_descs, d_row_off, H->P, n, S, cblocks, kpitch, e0,
+                                                             static_cast<int32_t *>(out));
+        else
+            k_tx_window_frames<<<grid, kWinThreads, 0, st>>>(a, nib, d_descs, d_row_off, H->P, n, S, cblocks, kpitch, e0,
+                                                             static_cast<float *>(out));
     } else {
         k_tx_window<<<(unsigned)((nvec + kWinThreads - 1) / kWinThreads), kWinThreads, 0, st>>>(
-            a, reinterpret_cast<const int64_t *>(a), d_descs, d_row_off, H->P, n, total, out);
+            a, nib, d_descs, d_row_off, H->P, n, total, static_cast<int16_t *>(out));
     }
     AFSK_CUDA(cudaGetLastError());
     H->n_launches++;
-    if (!on_device) AFSK_CUDA(cudaMemcpyAsync(dst, H->d_out, (size_t)total * 2, cudaMemcpyDeviceToHost, st));
+    if (!on_device && interleaved)
+        AFSK_CUDA(cudaMemcpy2DAsync(dst, (size_t)pitch * size, H->d_out, (size_t)S * size, (size_t)S * size, (size_t)n,
+                                    cudaMemcpyDeviceToHost, st));
+    else if (!on_device)
+        AFSK_CUDA(cudaMemcpyAsync(dst, H->d_out, (size_t)total * 2, cudaMemcpyDeviceToHost, st));
     AFSK_CUDA(cudaStreamSynchronize(st));
     H->P = wend;
     for (auto &qs : H->q)
@@ -1071,23 +1154,45 @@ int afsk_tx_streams_pull(AfskTxStreams *H, int64_t n_frames, int16_t *dst, int o
         afsk_set_error("afsk_tx_streams_pull: window too large");
         return AFSK_E_ARG;
     }
-    return tx_streams_call(H, [&] { return tx_pull_run(H, n_frames, dst, on_device, false, (cudaStream_t)stream); });
+    return tx_streams_call(H, [&] { return tx_pull_run(H, n_frames, dst, on_device, false, AFSK_SAMPLE_S16, 0, (cudaStream_t)stream); });
+}
+
+// the argument checks of an interleaved pull (fn names the entry point in the error)
+static int pull_frames_check(const char *fn, AfskTxStreams *H, int64_t n_frames, const void *dst, int format, int64_t row_pitch)
+{
+    if (!H || n_frames < 0 || (n_frames > 0 && !dst)) { afsk_set_error("%s: bad argument", fn); return AFSK_E_ARG; }
+    const int size = afsk_sample_size(format);
+    if (!size) { afsk_set_error("%s: unknown sample format %d", fn, format); return AFSK_E_ARG; }
+    if (row_pitch < H->S) { afsk_set_error("%s: row_pitch %lld < S = %d", fn, (long long)row_pitch, H->S); return AFSK_E_ARG; }
+    if ((reinterpret_cast<uintptr_t>(dst) & (uintptr_t)(size - 1)) != 0) {
+        afsk_set_error("%s: dst must be aligned to the sample size (%d bytes)", fn, size);
+        return AFSK_E_ARG;
+    }
+    if (n_frames > (INT64_MAX / 16) / row_pitch) { afsk_set_error("%s: row_pitch * n_frames overflows", fn); return AFSK_E_ARG; }
+    if ((int64_t)((H->S + kIlC - 1) / kIlC) * ((n_frames + 8 * kIlV - 1) / (8 * kIlV)) > 0x7FFFFFFFLL) {
+        afsk_set_error("%s: window too large", fn);
+        return AFSK_E_ARG;
+    }
+    return AFSK_OK;
 }
 
 int afsk_tx_streams_pull_interleaved(AfskTxStreams *H, int64_t n_frames, int16_t *dst, int on_device, void *stream)
 {
     const char *fn = "afsk_tx_streams_pull_interleaved";
-    if (!H || n_frames < 0 || (n_frames > 0 && !dst)) { afsk_set_error("%s: bad argument", fn); return AFSK_E_ARG; }
-    if (n_frames > (INT64_MAX / 16) / H->S) { afsk_set_error("%s: S * n_frames overflows", fn); return AFSK_E_ARG; }
+    const int rc = pull_frames_check(fn, H, n_frames, dst, AFSK_SAMPLE_S16, H ? H->S : 0);
+    if (rc != AFSK_OK) return rc;
     if (on_device && (reinterpret_cast<uintptr_t>(dst) & 15) != 0) {
         afsk_set_error("%s: device output must be 16-byte aligned", fn);
         return AFSK_E_ARG;
     }
-    if ((int64_t)((H->S + kIlC - 1) / kIlC) * ((n_frames + 8 * kIlV - 1) / (8 * kIlV)) > 0x7FFFFFFFLL) {
-        afsk_set_error("%s: window too large", fn);
-        return AFSK_E_ARG;
-    }
-    return tx_streams_call(H, [&] { return tx_pull_run(H, n_frames, dst, on_device, true, (cudaStream_t)stream); });
+    return tx_streams_call(H, [&] { return tx_pull_run(H, n_frames, dst, on_device, true, AFSK_SAMPLE_S16, H->S, (cudaStream_t)stream); });
+}
+
+int afsk_tx_streams_pull_frames(AfskTxStreams *H, int64_t n_frames, void *dst, int format, int on_device, int64_t row_pitch, void *stream)
+{
+    const int rc = pull_frames_check("afsk_tx_streams_pull_frames", H, n_frames, dst, format, row_pitch);
+    if (rc != AFSK_OK) return rc;
+    return tx_streams_call(H, [&] { return tx_pull_run(H, n_frames, dst, on_device, true, format, row_pitch, (cudaStream_t)stream); });
 }
 
 int afsk_tx_streams_state(const AfskTxStreams *H, int s, int64_t *pulled, int64_t *busy_until, int64_t *pending)

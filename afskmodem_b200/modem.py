@@ -965,6 +965,31 @@ def _timeout_frames(timeout, n: int) -> np.ndarray:
     return np.array([max(0, int(float(x) * 48000)) for x in t], dtype=np.int64)
 
 
+# sample formats of interleaved frames (AFSK_SAMPLE_* of afsk_b200.h)
+_FRAME_FORMATS = {np.dtype(np.int16): _cabi.SAMPLE_S16, np.dtype(np.int32): _cabi.SAMPLE_S32,
+                  np.dtype(np.float32): _cabi.SAMPLE_F32}
+
+
+def _frame_format(dtype) -> tuple[np.dtype, int]:
+    """dtype (None: int16; a numpy or torch dtype, or its name) -> (numpy dtype, AFSK_SAMPLE_* code)"""
+    try:
+        dt = np.dtype(np.int16 if dtype is None else str(dtype).removeprefix("torch.") if "torch." in str(dtype) else dtype)
+    except TypeError:
+        dt = None
+    if dt not in _FRAME_FORMATS:
+        raise ValueError(f"dtype must be int16, int32 or float32, got {dtype!r}")
+    return dt, _FRAME_FORMATS[dt]
+
+
+def _row_pitch(n: int, S: int, s0: int, s1: int, what: str) -> int:
+    """the row pitch (in samples) of an (n, S) window with element strides (s0, s1): rows of unit stride, s0 >= S"""
+    if n == 0:                                                  # (an empty array's strides may be anything)
+        return S
+    if (S > 1 and s1 != 1) or (n > 1 and s0 < S):
+        raise ValueError(f"{what} must be rows of unit stride, row_pitch >= {S}: strides ({s0}, {s1}) in samples")
+    return int(s0) if n > 1 else S
+
+
 class StreamEvents:
     """The ``receive`` calls that became final with one push (or ``finish``), ordered by (stream, call):
     numpy arrays ``stream``, ``call``, ``recorded``, ``start``, ``end`` (stream frames of the recording)
@@ -1096,41 +1121,58 @@ class StreamReceiver:
             raise ValueError(f"samples holds {len(arr)} frames, the offsets need {int(offsets[-1])}")
         return self._run(arr.ctypes.data, 0, offsets, stream)
 
-    def push_interleaved(self, frames, stream=None) -> StreamEvents:
+    def push_interleaved(self, frames, stream=None, dtype=None) -> StreamEvents:
         """``push`` of the next n frames of every channel, given interleaved as a multi-channel sound card
-        delivers them: frame f of channel s is ``frames[f, s]``.  ``frames``: a C-contiguous (n, S) int16 numpy
-        array; any buffer (bytes, bytearray, memoryview) of 2 * n * S bytes of little-endian int16, which is what
-        pyaudio's ``Stream.read(n)`` returns for ``channels=S``; or a contiguous CUDA int16 tensor on this
-        receiver's device, of shape (n, S) or (n * S,).  Host input is copied once, as is, into a pinned
-        buffer; the GPU de-interleaves it.  Returns what ``push([frames[:, s] for s in range(S)])`` returns."""
+        delivers them: frame f of channel s is ``frames[f, s]``.  ``dtype`` is the sample format: int16 (the default),
+        int32 or float32, converted to int16 by the rules of ``afsk_b200.h`` (int32: the top 16 bits; float32:
+        ``clip(rint(x * 32768), -32768, 32767)``, NaN -> 0).  ``frames``: an (n, S) numpy array of that dtype whose
+        rows may be a window of wider frames, strides (row_pitch * itemsize, itemsize) with row_pitch >= S (such as
+        ``card[:, c0:c0 + S]``), or a C-contiguous (n * S,) one; any buffer (bytes, bytearray, memoryview) of
+        n * S little-endian samples, which is what pyaudio's ``Stream.read(n)`` returns for ``channels=S``; or a CUDA
+        tensor of that dtype on this receiver's device, (n, S) with strides (row_pitch, 1) or contiguous (n * S,),
+        read in place.  Host input is copied once, packed and still in its format, into a pinned buffer; the GPU
+        converts and de-interleaves it.  Returns what ``push([x[:, s] for s in range(S)])`` returns, x the frames
+        converted to int16."""
         S = self.S
+        dt, fmt = _frame_format(dtype)
         if hasattr(frames, "data_ptr"):                         # a torch tensor: passed by device pointer
             if not frames.is_cuda or frames.device.index != self.device:
                 raise ValueError(f"device frames must live on cuda:{self.device}")
-            if str(frames.dtype) != "torch.int16" or not frames.is_contiguous():
-                raise ValueError("device frames must be a contiguous int16 tensor")
-            if not (frames.dim() == 2 and frames.shape[1] == S) and not (frames.dim() == 1 and frames.numel() % S == 0):
+            if str(frames.dtype) != f"torch.{dt.name}":
+                raise ValueError(f"device frames must be a {dt.name} tensor (dtype=), got {frames.dtype}")
+            if frames.dim() == 1 and frames.is_contiguous() and frames.numel() % S == 0:
+                n, pitch = frames.numel() // S, S
+            elif frames.dim() == 2 and frames.shape[1] == S:
+                n, pitch = frames.shape[0], _row_pitch(frames.shape[0], S, frames.stride(0), frames.stride(1), "device frames")
+            else:
                 raise ValueError(f"device frames must have shape (n, {S}) or (n * {S},), got {tuple(frames.shape)}")
-            return self._run_interleaved(frames.data_ptr(), 1, frames.numel() // S, stream)
+            return self._run_frames(frames.data_ptr(), fmt, 1, n, pitch, stream)
         if isinstance(frames, np.ndarray):
-            if frames.dtype != np.int16 or not frames.flags.c_contiguous:
-                raise ValueError("host frames must be a C-contiguous int16 array")
-            if not (frames.ndim == 2 and frames.shape[1] == S) and not (frames.ndim == 1 and frames.size % S == 0):
-                raise ValueError(f"host frames must have shape (n, {S}) or (n * {S},), got {frames.shape}")
-            src = frames.reshape(-1)
+            if frames.dtype != dt:
+                raise ValueError(f"host frames must be a {dt.name} array (dtype=), got {frames.dtype}")
+            if frames.ndim == 1 and frames.flags.c_contiguous and frames.size % S == 0:
+                src = frames.reshape(-1, S)
+            elif frames.ndim == 2 and frames.shape[1] == S and all(x % dt.itemsize == 0 for x in frames.strides):
+                _row_pitch(frames.shape[0], S, frames.strides[0] // dt.itemsize, frames.strides[1] // dt.itemsize, "host frames")
+                src = frames
+            else:
+                raise ValueError(f"host frames must have shape (n, {S}) with rows of unit stride, or (n * {S},), got "
+                                 f"{frames.shape} with strides {frames.strides}")
         else:
             mv = memoryview(frames).cast("B")
-            if mv.nbytes % (2 * S):
-                raise ValueError(f"{mv.nbytes} bytes are not whole frames of {S} int16 samples")
-            src = np.frombuffer(mv, dtype="<i2")
-        buf = self._staging(src.size)
-        buf[:src.size] = src
-        return self._run_interleaved(buf.ctypes.data, 0, src.size // S, stream)
+            if mv.nbytes % (dt.itemsize * S):
+                raise ValueError(f"{mv.nbytes} bytes are not whole frames of {S} {dt.name} samples")
+            src = np.frombuffer(mv, dtype=dt.newbyteorder("<")).reshape(-1, S)
+        n = src.shape[0]
+        nbytes = n * S * dt.itemsize
+        buf = self._staging((nbytes + 1) // 2).view(np.uint8)[:nbytes].view(dt).reshape(n, S)
+        buf[...] = src
+        return self._run_frames(buf.ctypes.data, fmt, 0, n, S, stream)
 
-    def _run_interleaved(self, ptr: int, on_device: int, n_frames: int, stream) -> StreamEvents:
+    def _run_frames(self, ptr: int, fmt: int, on_device: int, n_frames: int, pitch: int, stream) -> StreamEvents:
         n = C.c_int64(0)
-        _cabi.check(_cabi.lib().afsk_rx_streams_push_interleaved(self._h, C.c_void_p(ptr), on_device, n_frames,
-                                                                  C.c_void_p(stream or 0), C.byref(n)))
+        _cabi.check(_cabi.lib().afsk_rx_streams_push_frames(self._h, C.c_void_p(ptr), fmt, on_device, n_frames, pitch,
+                                                             C.c_void_p(stream or 0), C.byref(n)))
         return self._events(n.value)
 
     def finish(self, streams=None, receivers=None, timeout=None, stream=None) -> StreamEvents:
@@ -1521,18 +1563,59 @@ class StreamTransmitter:
         r = self._pull(_cabi.lib().afsk_tx_streams_pull, n, out, stream)
         return r if out is not None else r.reshape(self.S, int(n))
 
-    def pull_interleaved(self, n: int, out=None, stream=None):
+    def pull_interleaved(self, n: int, out=None, stream=None, dtype=None):
         """``pull`` with the window interleaved, as a multi-channel sound card takes it: frame f of channel s is
-        element [f, s], bitwise ``pull(n).T``.  Default: a host (n, S) int16 array in the grow-only pinned buffer,
+        element [f, s], bitwise ``pull(n).T`` converted to ``dtype``: int16 (the default), int32 (``s << 16``) or
+        float32 (``s / 32768``, exact).  Default: a host (n, S) array of that dtype in the grow-only pinned buffer,
         valid until the next pull; its ``tobytes()`` is what pyaudio's ``Stream.write`` takes for ``channels=S``.
-        ``out``: a contiguous CUDA int16 tensor of at least n * S elements on this transmitter's device, written
-        frame-major and returned; nothing past n * S is written."""
-        r = self._pull(_cabi.lib().afsk_tx_streams_pull_interleaved, n, out, stream)
-        return r if out is not None else r.reshape(int(n), self.S)
+        ``out``: a CUDA tensor of that dtype on this transmitter's device, contiguous with at least n * S elements
+        (written frame-major; nothing past n * S is written), or an (n, S) window of a wider buffer with strides
+        (row_pitch, 1); or a host numpy array with such a window layout (strides in bytes), such as
+        ``playback[:, c0:c0 + S]``.  Only the window is written, and ``out`` is returned."""
+        n = int(n)
+        if n < 0:
+            raise ValueError("pull needs n >= 0")
+        S = self.S
+        dt, fmt = _frame_format(dtype)
+        fn = _cabi.lib().afsk_tx_streams_pull_frames
+        if out is None:
+            nbytes = S * n * dt.itemsize
+            buf = self._pinned_buffer((nbytes + 1) // 2).view(np.uint8)[:nbytes].view(dt)
+            _cabi.check(fn(self._h, n, C.c_void_p(buf.ctypes.data), fmt, 0, S, C.c_void_p(stream or 0)))
+            return buf.reshape(n, S)
+        if isinstance(out, np.ndarray):
+            if out.dtype != dt or out.ndim != 2 or out.shape != (n, S) or any(x % dt.itemsize for x in out.strides) \
+                    or not out.flags.writeable:
+                raise ValueError(f"host out must be a writable ({n}, {S}) {dt.name} array, got {out.dtype} {out.shape}")
+            pitch = _row_pitch(n, S, out.strides[0] // dt.itemsize, out.strides[1] // dt.itemsize, "host out")
+            _cabi.check(fn(self._h, n, C.c_void_p(out.ctypes.data), fmt, 0, pitch, C.c_void_p(stream or 0)))
+            return out
+        if not out.is_cuda or out.device.index != self.device:
+            raise ValueError(f"out must live on cuda:{self.device}")
+        if str(out.dtype) != f"torch.{dt.name}":
+            raise ValueError(f"out must be a {dt.name} tensor (dtype=), got {out.dtype}")
+        if out.dim() == 2 and tuple(out.shape) == (n, S):
+            pitch = _row_pitch(n, S, out.stride(0), out.stride(1), "out")
+        elif out.is_contiguous():
+            if out.numel() < S * n:
+                raise ValueError(f"out holds {out.numel()} frames, the pull needs {S * n}")
+            pitch = S
+        else:
+            raise ValueError(f"out must be contiguous or an ({n}, {S}) window with strides (row_pitch, 1)")
+        _cabi.check(fn(self._h, n, C.c_void_p(out.data_ptr()), fmt, 1, pitch, C.c_void_p(stream or 0)))
+        return out
+
+    def _pinned_buffer(self, total: int) -> np.ndarray:
+        """the grow-only pinned int16 buffer host output is copied into, >= total samples"""
+        if self._pinned is None or self._pinned.array.size < total:
+            if self._pinned is not None:
+                self._pinned.close()
+            self._pinned = _cabi.PinnedArray((max(total + total // 4, 16),), np.int16)
+        return self._pinned.array
 
     def _pull(self, fn, n, out, stream):
-        """the next n frames of every channel through fn (planar or interleaved pull): into ``out``, or into the
-        pinned buffer, returned flat"""
+        """the next n frames of every channel through fn (the planar pull): into ``out``, or into the pinned buffer,
+        returned flat"""
         n = int(n)
         if n < 0:
             raise ValueError("pull needs n >= 0")
@@ -1546,11 +1629,7 @@ class StreamTransmitter:
                 raise ValueError(f"out holds {out.numel()} frames, the pull needs {total}")
             _cabi.check(fn(self._h, n, C.c_void_p(out.data_ptr()), 1, C.c_void_p(stream or 0)))
             return out
-        if self._pinned is None or self._pinned.array.size < total:
-            if self._pinned is not None:
-                self._pinned.close()
-            self._pinned = _cabi.PinnedArray((max(total + total // 4, 16),), np.int16)
-        buf = self._pinned.array[:total]
+        buf = self._pinned_buffer(total)[:total]
         _cabi.check(fn(self._h, n, C.c_void_p(buf.ctypes.data), 0, C.c_void_p(stream or 0)))
         return buf
 

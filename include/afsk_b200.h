@@ -228,6 +228,27 @@ int afsk_rx_streams_push(AfskRxStreams *h, const int16_t *samples, int on_device
  * planar push of the same pieces. */
 int afsk_rx_streams_push_interleaved(AfskRxStreams *h, const int16_t *frames, int on_device, int64_t n_frames,
                                      void *stream, int64_t *n_events);
+/* sample formats of afsk_rx_streams_push_frames / afsk_tx_streams_pull_frames, each defined by its conversion to
+ * and from the int16 samples the modem works on:
+ *   S16  int16     receive x                                        transmit s
+ *   S32  int32     receive x >> 16 (arithmetic: the top 16 bits)   transmit s << 16
+ *   F32  float32   receive clamp(rint(x * 32768), -32768, 32767)    transmit s / 32768 (exact)
+ *                  (round half to even, NaN -> 0, +-inf saturate)
+ * Transmit then receive is the identity in every format.  Float scales by 32768, not 32767, so that the receive
+ * rule is the exact inverse of the transmit rule and -1.0 is -32768. */
+#define AFSK_SAMPLE_S16 0
+#define AFSK_SAMPLE_S32 1
+#define AFSK_SAMPLE_F32 2
+/* afsk_rx_streams_push_interleaved of n_frames frames of every channel, read from a window of wider frames:
+ * frame f of channel s is element frames[f * row_pitch + s] of the given format (row_pitch >= S, in samples;
+ * frames points at row 0's first window sample, aligned to the sample size), converted to int16 by the rule of
+ * its format.  Events, state and counters are those of afsk_rx_streams_push_interleaved of the converted,
+ * contiguous frames.  Device reads may touch the aligned 16-byte vectors holding window samples, never beyond.
+ * A host window is copied packed, in its own format, to the device and converted there.  AFSK_E_ARG (nothing
+ * changes) for an unknown format, row_pitch < S, a misaligned pointer, a NULL frames with n_frames > 0, a negative
+ * n_frames, an n_frames * row_pitch * size that overflows or a piece too large for one launch. */
+int afsk_rx_streams_push_frames(AfskRxStreams *h, const void *frames, int format, int on_device, int64_t n_frames,
+                                int64_t row_pitch, void *stream, int64_t *n_events);
 /* ends the streams of the n distinct channels h_streams[n] (finite-stream conventions of afsk_rx_gate_multi: a
  * pending recording ends at the last full chunk, a call that has neither opened nor timed out is dropped, a
  * partial chunk is ignored) and returns their final calls.  Each listed channel's next push is frame 0 of a new
@@ -343,6 +364,12 @@ int afsk_tx_streams_pull(AfskTxStreams *h, int64_t n_frames, int16_t *dst, int o
  * of channel s (n_frames x S, frame-major), the transpose of afsk_tx_streams_pull's array; nothing past
  * S * n_frames is written.  Arguments and errors as for afsk_tx_streams_pull. */
 int afsk_tx_streams_pull_interleaved(AfskTxStreams *h, int64_t n_frames, int16_t *dst, int on_device, void *stream);
+/* afsk_tx_streams_pull_interleaved into a window: dst[f * row_pitch + s] = frame f of channel s, converted by the
+ * rule of format (AFSK_SAMPLE_*; dst aligned to the sample size, row_pitch >= S).  Nothing outside the window's
+ * n_frames x S elements is written, so handles may write disjoint windows of one buffer.  Host output is
+ * synthesized packed on the device and copied out row by row.  Errors as for afsk_rx_streams_push_frames. */
+int afsk_tx_streams_pull_frames(AfskTxStreams *h, int64_t n_frames, void *dst, int format, int on_device,
+                                int64_t row_pitch, void *stream);
 /* channel s: frames pulled (P), end of its last message sent (<= P: idle), messages not yet fully pulled */
 int afsk_tx_streams_state(const AfskTxStreams *h, int s, int64_t *pulled, int64_t *busy_until, int64_t *pending);
 /* device bytes the handle holds (payload arenas, descriptors, host-output staging) */

@@ -14,6 +14,14 @@ traffic at its own baud, and within a group cycles through the three (amp_start,
 the c5 corpus; the handle is then opened with open_receive_streams.  A push then decodes one group per distinct
 baud among its final recordings.
 
+--format s16,s32,f32 feeds each piece as the columns of a wider card in that sample format (--pitch-extra K: the card
+has S + K columns and the window starts at column 1 when K > 0, an odd column): push_interleaved(card[:, c0:c0 + S],
+dtype=...) beside the route it replaces, the slice made contiguous, the conversion to int16 and push_interleaved, with
+numpy on the host (a pageable card) or torch on the device, run alternately three times on two receivers.  The profiled
+run then times the append kernel in each format over device windows (k_stream_frames; k_stream_deinterleave
+for contiguous int16), its bytes/s counted over the bytes it must
+read and write (n * S * (sample size + 2)).
+
 --layout interleaved feeds each piece as a multi-channel sound card delivers it, n x S frame-major (host input: a
 pageable array, as pyaudio's read returns it), three ways in one run: push_interleaved (the GPU de-interleaves it),
 a host numpy transpose into the pinned planar buffer followed by push, and .t().contiguous() on the device followed
@@ -356,6 +364,99 @@ def profile_config(d_base, S: int, piece: int, T: int, timeout: float, out_dir: 
             "by_kernel_or_copy": dict(sorted(rows.items(), key=lambda kv: -kv[1]["ms"]))}
 
 
+FORMATS = {"s16": np.int16, "s32": np.int32, "f32": np.float32}
+
+
+def run_frames(d_base, S: int, piece: int, T: int, device: bool, fmt: str, extra: int, timeout: float, reps: int = 3):
+    """--format: the pieces as a window of an (n, S + extra) card of fmt; route "window" (push_interleaved of the
+    window) and "replaced" (contiguous copy, conversion, push_interleaved of int16), alternately on two receivers"""
+    import torch
+    dt = FORMATS[fmt]
+    c0 = 1 if extra else 0
+    n_push = max(T // piece, 1)
+    cards = []
+    for i in range(n_push):
+        x = torch.as_strided(d_base, (S, piece), (SHIFT, 1), i * piece).t()
+        y = x if dt == np.int16 else x.to(torch.int32) << 16 if dt == np.int32 else x.to(torch.float32) / 32768
+        c = torch.zeros((piece, S + extra), dtype=y.dtype, device="cuda")
+        c[:, c0:c0 + S] = y
+        cards.append(c if device else c.cpu().numpy())
+    torch.cuda.synchronize()
+
+    def window(st, c):
+        return st.push_interleaved(c[:, c0:c0 + S], dtype=dt)
+
+    def replaced(st, c):
+        w = c[:, c0:c0 + S]
+        if device:
+            w = w.contiguous()
+            w = w if dt == np.int16 else (w >> 16).to(torch.int16) if dt == np.int32 else \
+                torch.clamp(torch.round(torch.nan_to_num(w, nan=0.0) * 32768), -32768, 32767).to(torch.int16)
+        else:
+            w = np.ascontiguousarray(w)
+            w = w if dt == np.int16 else (w >> 16).astype(np.int16) if dt == np.int32 else \
+                np.clip(np.rint(np.nan_to_num(w, nan=0.0).astype(np.float64) * 32768), -32768, 32767).astype(np.int16)
+        return st.push_interleaved(w)
+    routes = {"window": window, "replaced": replaced}
+    times = {r: [] for r in routes}
+    rx = A.Receiver(1200)
+    events = {}
+    with rx.open_streams(S, timeout) as a, rx.open_streams(S, timeout) as b:
+        hs = {"window": a, "replaced": b}
+        for rep in range(reps + 1):                       # rep 0 warms up every shape
+            for r, fn in routes.items():
+                n_ev = 0
+                for c in cards:
+                    torch.cuda.synchronize()
+                    t0 = time.perf_counter()
+                    n_ev += len(fn(hs[r], c))
+                    if rep:
+                        times[r].append(time.perf_counter() - t0)
+                events[r] = n_ev
+    out = []
+    for r in routes:
+        t = np.array(times[r])
+        out.append({"S": S, "piece": piece, "input": "device" if device else "host", "format": fmt, "pitch_extra": extra,
+                    "route": r, "pushes": len(t), "push_ms_median": float(np.median(t) * 1e3),
+                    "push_ms_min": float(t.min() * 1e3), "push_ms_max": float(t.max() * 1e3),
+                    "frames_per_s": S * piece * len(t) / float(t.sum()), "events_last_rep": events[r]})
+    return out
+
+
+def profile_frames(d_base, S: int, piece: int, T: int, fmt: str, extra: int, timeout: float):
+    """the append kernel's device time over device-window pushes in one format (torch.profiler)"""
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+    dt = FORMATS[fmt]
+    c0 = 1 if extra else 0
+    n_push = max(T // piece, 1)
+    cards = []
+    for i in range(n_push):
+        x = torch.as_strided(d_base, (S, piece), (SHIFT, 1), i * piece).t()
+        y = x if dt == np.int16 else x.to(torch.int32) << 16 if dt == np.int32 else x.to(torch.float32) / 32768
+        c = torch.zeros((piece, S + extra), dtype=y.dtype, device="cuda")
+        c[:, c0:c0 + S] = y
+        cards.append(c)
+    with A.Receiver(1200).open_streams(S, timeout) as st:
+        for c in cards:
+            st.push_interleaved(c[:, c0:c0 + S], dtype=dt)
+        st.finish()
+        torch.cuda.synchronize()
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            for c in cards:
+                st.push_interleaved(c[:, c0:c0 + S], dtype=dt)
+    ms = 0.0
+    for e in prof.key_averages():
+        if "k_stream_frames" in e.key or "k_stream_deinterleave" in e.key:
+            us = getattr(e, "device_time_total", None)
+            ms += (us if us is not None else getattr(e, "cuda_time_total", 0.0)) / 1e3
+    nbytes = S * piece * n_push * (np.dtype(dt).itemsize + 2)
+    kernel = "k_stream_deinterleave" if dt == np.int16 and not extra else "k_stream_frames"
+    return {"S": S, "piece": piece, "pushes": n_push, "format": fmt, "pitch_extra": extra, "kernel": kernel,
+            "kernel_ms": ms, "kernel_us_per_push": ms * 1e3 / n_push, "bytes_read_and_written": nbytes,
+            "kernel_TBps": nbytes / (ms * 1e-3) / 1e12 if ms else None}
+
+
 def whole_stream_reference(base: np.ndarray, T: int, n_streams: int, timeout: float):
     rx = A.Receiver(1200)
     streams = [base[s * SHIFT:s * SHIFT + T] for s in range(n_streams)]
@@ -390,6 +491,8 @@ def main():
     ap.add_argument("--loopback", type=int, default=0, help="channels of a config-4 loopback (0: none)")
     ap.add_argument("--loopback-retain", default="bits", help="retention mode of the config-4 loopback")
     ap.add_argument("--retain", default="samples", help="retention modes, run in turn per configuration: samples,bits,payload")
+    ap.add_argument("--format", default="", help="sample formats of a window of a wider card: s16,s32,f32")
+    ap.add_argument("--pitch-extra", type=int, default=0, help="columns of the card beyond the S of the window")
     ap.add_argument("--out", default=None)
     ap.add_argument("--no-profile", action="store_true", help="skip the profiled run of the largest device configuration")
     a = ap.parse_args()
@@ -410,6 +513,26 @@ def main():
     res = {"card": card(), "torch_device": torch.cuda.get_device_name(0), "seconds_per_channel": a.seconds,
            "timeout_s": a.timeout, "mix": a.mix, "layout": a.layout, "retain": a.retain, "configs": []}
     modes = a.retain.split(",")
+    fmts = [f for f in a.format.split(",") if f]
+    if fmts:                                              # the format measurements alone
+        res.update({"pitch_extra": a.pitch_extra, "configs": [], "profile_formats": []})
+        for S in Ss:
+            for piece in pieces:
+                for inp in a.input.split(","):
+                    for f in fmts:
+                        for r in run_frames(d_base, S, piece, T, inp == "device", f, a.pitch_extra, a.timeout):
+                            print(json.dumps(r), flush=True)
+                            res["configs"].append(r)
+        if not a.no_profile:
+            for f in fmts:
+                r = profile_frames(d_base, max(Ss), max(pieces), T, f, a.pitch_extra, a.timeout)
+                print(json.dumps(r), flush=True)
+                res["profile_formats"].append(r)
+        res["card_after"] = card()
+        if a.out:
+            os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
+            json.dump(res, open(a.out, "w"), indent=1)
+        return
     routes = {False: ["planar"], True: ["planar"]}
     if a.layout == "interleaved":
         routes = {False: ["interleaved", "host-transpose"], True: ["interleaved", "device-transpose"]}

@@ -18,7 +18,14 @@ each sending messages of its own length at the same duty.
 run: pull_interleaved (the GPU writes it interleaved), a planar pull followed by a host numpy transpose into a
 preallocated array (host output), and a planar pull into a CUDA tensor followed by .t().contiguous() (device output),
 which is what a user had to do without pull_interleaved.  The profiled run then times k_tx_window_interleaved and
-k_tx_window over the same sequence (2 bytes written per pulled frame)."""
+k_tx_window over the same sequence (2 bytes written per pulled frame).
+
+--format s16,s32,f32 measures, per format, the window written into columns of a wider playback buffer (--pitch-extra K:
+the card has S + K columns and the window starts at column 1 when K > 0, an odd column): pull_interleaved(n,
+out=card[:, c0:c0 + S], dtype=...) beside the route it replaces, pull_interleaved(n) of int16 frames, the conversion
+(s << 16, s / 32768) and the copy into the card's columns, with numpy on the host or torch on the device.  The
+profiled run then times k_tx_window_frames in each format (k_tx_window_interleaved for contiguous int16), its bytes/s
+counted over the bytes it writes (n * S * sample size)."""
 from __future__ import annotations
 
 import argparse
@@ -64,6 +71,41 @@ class Traffic:
     def sent(self, streams, end):
         hi = 2 * (self.mean_len if np.ndim(self.mean_len) == 0 else self.mean_len[streams])
         self.next_at[streams] = end + self.rng.integers(0, hi, len(streams))
+
+
+FORMATS = {"s16": np.int16, "s32": np.int32, "f32": np.float32}
+
+
+def convert_host(x, dt):
+    """the transmit rule of afsk_b200.h, with numpy"""
+    return x if dt == np.int16 else (x.astype(np.int32) << 16) if dt == np.int32 else x.astype(np.float32) / np.float32(32768)
+
+
+def frames_route(st, S, n, route, fmt, extra, device):
+    """--format: the window of an (n, S + extra) card of format fmt, written by pull_interleaved ("window") or by the
+    route it replaces ("replaced": an int16 pull, the conversion, the copy into the card's columns)"""
+    import torch
+    dt = FORMATS[fmt]
+    c0 = 1 if extra else 0
+    if device:
+        cardt = torch.zeros((n, S + extra), dtype=getattr(torch, np.dtype(dt).name), device="cuda")
+        tmp = torch.empty((n, S), dtype=torch.int16, device="cuda")
+        if route == "window":
+            return lambda: st.pull_interleaved(n, out=cardt[:, c0:c0 + S], dtype=dt)
+
+        def dev():
+            x = st.pull_interleaved(n, out=tmp)
+            y = x if dt == np.int16 else x.to(torch.int32) << 16 if dt == np.int32 else x.to(torch.float32) / 32768
+            cardt[:, c0:c0 + S].copy_(y)
+            torch.cuda.synchronize()
+        return dev
+    cardh = np.zeros((n, S + extra), dt)
+    if route == "window":
+        return lambda: st.pull_interleaved(n, out=cardh[:, c0:c0 + S], dtype=dt)
+
+    def host():
+        cardh[:, c0:c0 + S] = convert_host(st.pull_interleaved(n), dt)
+    return host
 
 
 def pull_route(st, S, n, route, out_t):
@@ -112,19 +154,21 @@ def mix_bauds(S: int) -> np.ndarray:
     return np.array([MIX_BAUDS[s * len(MIX_BAUDS) // S] for s in range(S)], np.int64)
 
 
-def run_config(S: int, n: int, T: int, device: bool, baud, route: str = "planar"):
-    """baud: one for every channel, or "mix" (mix_bauds); route: see pull_route"""
+def run_config(S: int, n: int, T: int, device: bool, baud, route: str = "planar", fmt: str | None = None, extra: int = 0):
+    """baud: one for every channel, or "mix" (mix_bauds); route: see pull_route, or with fmt frames_route"""
     import torch
     n_pull = max(T // n, 1)
     out_t = torch.empty(S * n, dtype=torch.int16, device="cuda") if device else None
     res = {"S": S, "pull": n, "baud": baud, "output": "device" if device else "host-pinned", "pulls": n_pull, "route": route}
+    if fmt:
+        res.update({"format": fmt, "pitch_extra": extra, "output": "device" if device else "host"})
     if baud == "mix":
         baud = mix_bauds(S)
         st = A.open_transmit_streams([A.Transmitter(int(b), 0.1) for b in baud])
     else:
         st = A.Transmitter(baud, 0.1).open_streams(S)
     with st:
-        pull = pull_route(st, S, n, route, out_t)
+        pull = frames_route(st, S, n, route, fmt, extra, device) if fmt else pull_route(st, S, n, route, out_t)
         run_sequence(st, S, n, n_pull, baud, 1, out_t, pull)          # warm-up: same shapes
         c0 = st.counters()
         tp, ts, busy = run_sequence(st, S, n, n_pull, baud, 2, out_t, pull)
@@ -143,7 +187,8 @@ def run_config(S: int, n: int, T: int, device: bool, baud, route: str = "planar"
     return res
 
 
-def profile_config(S: int, n: int, T: int, baud: int, out_dir: str | None, route: str = "planar"):
+def profile_config(S: int, n: int, T: int, baud: int, out_dir: str | None, route: str = "planar", fmt: str | None = None,
+                   extra: int = 0):
     """Device time of every kernel and copy over one device-output pull sequence (torch.profiler, CUDA activity),
     beside the host wall time of the same pulls."""
     import torch
@@ -152,7 +197,7 @@ def profile_config(S: int, n: int, T: int, baud: int, out_dir: str | None, route
     out_t = torch.empty(S * n, dtype=torch.int16, device="cuda")
     tx = A.Transmitter(baud, 0.1)
     with tx.open_streams(S) as st:
-        pull = pull_route(st, S, n, route, out_t)
+        pull = frames_route(st, S, n, route, fmt, extra, True) if fmt else pull_route(st, S, n, route, out_t)
         run_sequence(st, S, n, n_pull, baud, 1, out_t, pull)
         torch.cuda.synchronize()
         with profile(activities=[ProfilerActivity.CUDA]) as prof:
@@ -167,13 +212,15 @@ def profile_config(S: int, n: int, T: int, baud: int, out_dir: str | None, route
         if us > 0:
             rows[e.key] = {"count": int(e.count), "ms": us / 1e3}
     busy = sum(r["ms"] for r in rows.values())
-    kernel = "k_tx_window_interleaved" if route == "interleaved" else "k_tx_window"
+    kernel = "k_tx_window_interleaved" if route == "interleaved" or (route == "window" and fmt == "s16" and not extra) else \
+        "k_tx_window_frames" if route == "window" else "k_tx_window"
     win = [v for k, v in rows.items() if re.search(kernel + r"\b(?!_)", k)]
     win_ms = sum(r["ms"] for r in win)
-    win_bytes = 2 * S * n * n_pull
+    win_bytes = (np.dtype(FORMATS[fmt]).itemsize if fmt else 2) * S * n * n_pull
     if out_dir:
         prof.export_chrome_trace(os.path.join(out_dir, f"stream_tx_profile_{route}.pt.trace.json"))
     return {"S": S, "pull": n, "baud": baud, "pulls": n_pull, "output": "device", "route": route, "kernel": kernel,
+            "format": fmt, "pitch_extra": extra,
             "host_wall_ms": wall * 1e3,
             "host_ms_per_pull": wall * 1e3 / n_pull, "pull_ms_per_pull": float(tp.sum()) * 1e3 / n_pull,
             "send_ms_per_pull": float(ts.sum()) * 1e3 / n_pull,
@@ -193,6 +240,8 @@ def main():
     ap.add_argument("--output", default="device,host")
     ap.add_argument("--mix", action="store_true", help="six bauds across the channels")
     ap.add_argument("--layout", default="planar", choices=["planar", "interleaved"])
+    ap.add_argument("--format", default="", help="sample formats of a window of a wider card: s16,s32,f32")
+    ap.add_argument("--pitch-extra", type=int, default=0, help="columns of the card beyond the S of the window")
     ap.add_argument("--out", default=None)
     ap.add_argument("--no-profile", action="store_true", help="skip the profiled run of the largest device configuration")
     a = ap.parse_args()
@@ -212,11 +261,27 @@ def main():
              for r in routes[o == "device"]]
     if not a.mix:
         lines += [(max(Ss), max(pulls), True, 4800, r) for r in routes[True]]
+    fmts = [f for f in a.format.split(",") if f]
+    if fmts:
+        res["pitch_extra"] = a.pitch_extra
+        for S in Ss:
+            for n in pulls:
+                for o in a.output.split(","):
+                    for f in fmts:
+                        for route in ("window", "replaced"):
+                            r = run_config(S, n, T, o == "device", 1200, route, f, a.pitch_extra)
+                            print(json.dumps(r), flush=True)
+                            res["configs"].append(r)
+        if not a.no_profile:
+            res["profile_formats"] = [profile_config(max(Ss), max(pulls), T, 1200, None, "window", f, a.pitch_extra) for f in fmts]
+            for r in res["profile_formats"]:
+                print(json.dumps({k: v for k, v in r.items() if k != "by_kernel_or_copy"}), flush=True)
+        lines = []
     for S, n, dev, baud, route in lines:
         r = run_config(S, n, T, dev, baud, route)
         print(json.dumps(r), flush=True)
         res["configs"].append(r)
-    if not a.mix and not a.no_profile:
+    if not a.mix and not a.no_profile and not fmts:
         out_dir = os.path.dirname(os.path.abspath(a.out)) if a.out else None
         res["profile"] = profile_config(max(Ss), max(pulls), T, 1200, out_dir)
         print(json.dumps({k: v for k, v in res["profile"].items() if k != "by_kernel_or_copy"}), flush=True)
