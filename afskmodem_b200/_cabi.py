@@ -38,7 +38,7 @@ SYMBOLS = [
     "afsk_tx_streams_configure", "afsk_rx_streams_push_interleaved", "afsk_tx_streams_pull_interleaved",
     "afsk_rx_streams_set_retention", "afsk_rx_streams_pending_bits", "afsk_rx_streams_plane_counters",
     "afsk_rx_streams_pending_payload", "afsk_rx_streams_payload_counters", "afsk_rx_streams_push_frames",
-    "afsk_tx_streams_pull_frames",
+    "afsk_tx_streams_pull_frames", "afsk_rx_streams_pending_planes",
 ]
 
 
@@ -122,6 +122,7 @@ def lib():
     L.afsk_rx_streams_destroy.argtypes = [vp]
     L.afsk_rx_streams_set_retention.argtypes = [vp, C.c_int]
     L.afsk_rx_streams_pending_bits.argtypes = [vp, C.c_int, i32p, i64p]
+    L.afsk_rx_streams_pending_planes.argtypes = [vp, C.c_int, C.POINTER(vp), i64p, i64p]
     L.afsk_rx_streams_plane_counters.argtypes = [vp, i64p, i64p]
     L.afsk_rx_streams_pending_payload.argtypes = [vp, C.c_int, i64p, i64p, i32p, vp, C.c_int64, i64p]
     L.afsk_rx_streams_payload_counters.argtypes = [vp, i64p, i64p]

@@ -2773,7 +2773,8 @@ static bool configure_group(Group &g, int bf)
         g.stages = pick_stages(g.stage_bytes);
         if (long_shift) g.stages = (int)std::min<size_t>(3, (size_t)(220 * 1024) / (size_t)g.stage_bytes);
         g.smem = demod_smem_bytes(g);
-        return true;
+        // a ring needs one stage: a tile larger than the budget (AFSK_DEMOD_NSUB=3 at 480 / 240 baud, ~307 KB) is refused
+        return g.stages >= 1;
     }
     if ((bf == 32 || bf == 64 || bf == 128) && !getenv("AFSK_NO_PAD")) {
         // 1500 / 750 / 375 baud: power-of-two windows.  Four / two / one windows per thread over the padded layout
@@ -2795,7 +2796,7 @@ static bool configure_group(Group &g, int bf)
         g.stages = (int)std::min<size_t>(3, (size_t)(220 * 1024) / (size_t)g.stage_bytes);
         if (const char *ev = getenv("AFSK_DEMOD_STAGES")) g.stages = std::max(1, std::min(kMaxStages, atoi(ev)));
         g.smem = demod_smem_bytes(g);
-        return g.smem <= 227 * 1024;
+        return g.stages >= 1 && g.smem <= 227 * 1024;
     }
     // Segments of at most 48 samples per thread.  The thread stride in shared memory is 2 * seg bytes:
     // 40 samples (80 B) is conflict-free for 128-bit loads and 48 is 2-way, both reach the HBM ceiling;
@@ -4487,6 +4488,25 @@ int afsk_rx_streams_pending_bits(const AfskRxStreams *H, int s, int32_t *clock, 
     if (!H || s < 0 || s >= H->S) { afsk_set_error("afsk_rx_streams_pending_bits: bad argument"); return AFSK_E_ARG; }
     if (clock) *clock = H->pending[s] >= 0 ? (int32_t)H->pclock[s] : -1;
     if (windows) *windows = H->pending[s] >= 0 ? H->pdecided[s] : 0;
+    return AFSK_OK;
+}
+
+int afsk_rx_streams_pending_planes(const AfskRxStreams *H, int s, const uint32_t **d_planes, int64_t *first_window, int64_t *n_windows)
+{
+    if (!H || s < 0 || s >= H->S || !d_planes || !first_window || !n_windows) {
+        afsk_set_error("afsk_rx_streams_pending_planes: bad argument");
+        return AFSK_E_ARG;
+    }
+    *d_planes = nullptr; *first_window = 0; *n_windows = 0;
+    if (H->retain == AFSK_RETAIN_SAMPLES || H->pending[s] < 0 || H->pclock[s] < 0) return AFSK_OK;
+    // plane positions count four samples per word: the recording's word 0 is at pw_rec, the channel keeps from pw_keep
+    const int64_t base = (H->pw_keep[s] - H->pw_rec[s]) / 4;
+    const int64_t n = H->pdecided[s] - 32 * base;
+    if (n <= 0) return AFSK_OK;
+    const Slots &Pl = H->pln;
+    *d_planes = reinterpret_cast<const uint32_t *>(reinterpret_cast<const uint2 *>(Pl.arena[Pl.cur]) + (Pl.off[s] + H->pw_keep[s] - Pl.base[s]) / 4);
+    *first_window = 32 * base;
+    *n_windows = n;
     return AFSK_OK;
 }
 

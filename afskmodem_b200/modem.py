@@ -1259,6 +1259,24 @@ class StreamReceiver:
         _cabi.check(_cabi.lib().afsk_rx_streams_pending_bits(self._h, int(s), C.byref(a), C.byref(b)))
         return a.value, b.value
 
+    def pending_planes(self, s: int) -> tuple[int, np.ndarray, np.ndarray]:
+        """(first_window, bits, quiet) of stream s's pending recording in bits or payload mode: the decision and quiet
+        flags of the windows it keeps on the device, windows first_window, first_window + 1, ... of the recording
+        (window k starts at frame ``state(s)[1] + pending_bits(s)[0] + k * bit length``), up to the windows decided.
+        Empty in samples mode, with no recording pending, before its clock is recovered, or in payload mode once its
+        result is fixed.  For diagnostics and stage-level tests (one device-to-host copy)."""
+        L = _cabi.lib()
+        pp, first, n = C.c_void_p(), C.c_int64(0), C.c_int64(0)
+        _cabi.check(L.afsk_rx_streams_pending_planes(self._h, int(s), C.byref(pp), C.byref(first), C.byref(n)))
+        nw = (n.value + 31) // 32
+        words = np.zeros((max(nw, 1), 2), dtype=np.uint32)
+        if nw:
+            _cabi.check(L.afsk_memcpy_d2h(self.device, C.c_void_p(words.ctypes.data), pp, nw * 8, None))
+            _cabi.stream_sync(self.device)
+        unpack = lambda col: np.unpackbits(np.ascontiguousarray(words[:, col]).view(np.uint8),  # noqa: E731
+                                           bitorder="little")[:n.value].astype(bool)
+        return first.value, unpack(0), unpack(1)
+
     def pending_payload(self, s: int) -> tuple[int, int, bool, bytes]:
         """(train_end, nbits, ended, bytes) of stream s's pending recording in payload mode, as framed so far:
         train_end is -1 until the end of the training sequence is seen, nbits the coded bits framed after it, ended

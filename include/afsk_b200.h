@@ -152,7 +152,10 @@ int afsk_rx_plan_set_timing(AfskRxPlan *plan, int enable);
 int afsk_rx_plan_demod_time(AfskRxPlan *plan, float *ms_total, int *launches);
 /* raw decision / quiet flags of capture c after a decode, for diagnostics and stage-level parity
  * tests: d_planes points at interleaved uint32 pairs {bits, quiet}; window k of the capture is
- * bit (k & 31) of pair k >> 5 (LSB first). */
+ * bit (k & 31) of pair k >> 5 (LSB first).  *max_windows counts the windows at clock 0; a decode decides
+ * the K = #{k >= 0 : clock + k * bit length < n - bit length} windows at the capture's clock, in every
+ * schedule and layout, and writes 0 (bit and quiet) for windows K .. of the pair holding window K - 1.  Later
+ * pairs are undefined. */
 int afsk_rx_plan_planes(const AfskRxPlan *plan, int capture, const uint32_t **d_planes, int64_t *max_windows);
 /*
  * Host-buffer convenience (what a drop-in Receiver.load calls): H2D, decode, D2H on `device`.
@@ -297,6 +300,14 @@ int afsk_rx_streams_set_retention(AfskRxStreams *h, int mode);
  * and the windows decided so far (0 in samples mode; in payload mode it stops growing once the recording's first
  * quiet window after the terminator is found) */
 int afsk_rx_streams_pending_bits(const AfskRxStreams *h, int s, int32_t *clock, int64_t *windows);
+/* channel s's pending recording in bits or payload mode, for diagnostics and stage-level tests: the plane words it
+ * keeps on the device, in afsk_rx_plan_planes' {bits, quiet} pair layout.  The first pair holds windows *first_window ..
+ * + 31 (a multiple of 32) of the recording, window k starting at frame pending_start + clock + k * bit length; there
+ * are *n_windows of them, up to the windows decided.  0 windows (d_planes NULL) in samples mode, with no recording
+ * pending, before its clock is stored, or in payload mode once its result is fixed.  The device pointer is valid
+ * until the next push or finish. */
+int afsk_rx_streams_pending_planes(const AfskRxStreams *h, int s, const uint32_t **d_planes, int64_t *first_window,
+                                   int64_t *n_windows);
 /* since creation: plane words moved to keep pending recordings' planes, and whole plane-arena compactions (both
  * 0 in samples mode) */
 int afsk_rx_streams_plane_counters(const AfskRxStreams *h, int64_t *moved_words, int64_t *compactions);

@@ -9,7 +9,8 @@ from afskmodem_b200 import _cabi, modem
 
 def test_bits_symbols_are_exported():
     L = _cabi.lib()
-    for name in ("afsk_rx_streams_set_retention", "afsk_rx_streams_pending_bits", "afsk_rx_streams_plane_counters"):
+    for name in ("afsk_rx_streams_set_retention", "afsk_rx_streams_pending_bits", "afsk_rx_streams_plane_counters",
+                 "afsk_rx_streams_pending_planes"):
         assert name in _cabi.SYMBOLS
         assert hasattr(L, name)
 
@@ -21,6 +22,8 @@ def test_null_handle_or_bad_mode_is_a_bad_argument():
         assert L.afsk_rx_streams_set_retention(None, mode) == _cabi.AFSK_E_ARG
     assert L.afsk_rx_streams_pending_bits(None, 0, C.byref(clk), C.byref(win)) == _cabi.AFSK_E_ARG
     assert L.afsk_rx_streams_plane_counters(None, C.byref(win), C.byref(win)) == _cabi.AFSK_E_ARG
+    ptr, first = C.c_void_p(), C.c_int64(0)
+    assert L.afsk_rx_streams_pending_planes(None, 0, C.byref(ptr), C.byref(first), C.byref(win)) == _cabi.AFSK_E_ARG
 
 
 def test_unknown_retention_is_refused_before_any_device_work():
